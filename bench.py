@@ -25,6 +25,9 @@ whole batch.
               oracle env, 1 env, 1 core (live when /root/reference exists, else the committed measurement).
 * --impl reference  the reference arm: the same oracle port timed on the host cores (the reference's env
               arithmetic lives in un-vendored racecar_gym + pybullet, so no reference build exists: DESIGN.md).
+* --dump-outputs DIR  what the headline's last timed step returned (obs, reward, done, info) as DIR/<name>.npy in
+              float32 / float64, at most 64 MB (beyond that a fixed sample of envs).  The inputs depend only on the
+              arguments, so the files of two builds can be compared array by array.
 """
 import argparse
 import dataclasses
@@ -57,6 +60,8 @@ ALGO_BYTES_PER_ENV_STEP = 4624
 # per kernel: k_lidar writes 1080 f32 ranges and reads one 48-byte origin record per env; k_occupancy writes 64x64 u8 and
 # reads the record + pose; k_step reads and writes the state groups, reads the action, writes scalars + pose/velocity + record
 KERNEL_BYTES_PER_ENV = {"k_lidar": N_BEAMS * 4 + 48, "k_occupancy": 4096 + 48 + 24, "k_step": 224 + 8 + 24 + 48 + 48}
+# --dump-outputs: total size of the .npy files written
+DUMP_LIMIT_BYTES = 64 * 10**6
 
 
 @dataclasses.dataclass
@@ -350,8 +355,39 @@ class Ctx:
         return [float(x) for x in t]
 
 
-def device_leg(cx, wl, n, steps, warmup, sampler=None, back_to_back=True):
-    """K steps of BatchedRaceEnv.step() with inputs resident in HBM; per-step CUDA events, L2 flushed between steps."""
+def step_outputs(obs, reward, done, info, limit=DUMP_LIMIT_BYTES):
+    """What one BatchedRaceEnv.step() handed its caller, as host arrays with one row per env: floats as they are, other
+    types converted exactly (to float32 up to two bytes, else float64).  When the rows exceed `limit` bytes, a fixed
+    sample of envs (seed 0, ascending) is taken from every array alike and its indices are added as `env_index`."""
+    import torch
+    named = {}
+    for k, v in list(obs.items()) + [("reward", reward), ("done", done)] + list(info.items()):
+        named.setdefault(k, v)
+
+    def host_dtype(t):
+        if t.dtype in (torch.float32, torch.float64):
+            return t.dtype
+        return torch.float32 if t.element_size() <= 2 else torch.float64
+
+    n = reward.shape[0]
+    per_env = sum(t[0].numel() * torch.empty((), dtype=host_dtype(t)).element_size() for t in named.values())
+    m = min(n, (limit - 4096) // (per_env + 8))      # 4 KiB for the .npy headers, 8 bytes per env for env_index
+    rows = None
+    if m < n:
+        rows = torch.from_numpy(np.sort(np.random.default_rng(0).choice(n, m, replace=False))).to(reward.device)
+    out = {}
+    for k, t in named.items():
+        if rows is not None:
+            t = t.index_select(0, rows)
+        out[k] = t.to(host_dtype(t)).cpu().numpy()
+    if rows is not None:
+        out["env_index"] = rows.cpu().numpy().astype(np.float64)
+    return out
+
+
+def device_leg(cx, wl, n, steps, warmup, sampler=None, back_to_back=True, keep_outputs=False):
+    """K steps of BatchedRaceEnv.step() with inputs resident in HBM; per-step CUDA events, L2 flushed between steps.
+    keep_outputs: also return what the last timed step returned (`step_outputs`), copied after the timed region."""
     torch = cx.torch
     from racing_dreamer_b200 import BatchedRaceEnv
     env = BatchedRaceEnv(env_config(wl, n, cx.rank), device=cx.dev)
@@ -372,13 +408,14 @@ def device_leg(cx, wl, n, steps, warmup, sampler=None, back_to_back=True):
     for k in range(steps):
         cx.flush.zero_()
         ev[k][0].record()
-        env.step(acts[(warmup + k) % PERIOD])      # the public API (launches only k_* kernels)
+        last = env.step(acts[(warmup + k) % PERIOD])      # the public API (launches only k_* kernels)
         ev[k][1].record()
     cx.barrier()
     wall = time.perf_counter() - wall0
     launches = env.launch_count - launches0
     timing = env.read_timing(reset=True)
     env.enable_timing(False)
+    outputs = step_outputs(*last) if keep_outputs else None
     gpu_ms = float(sum(a.elapsed_time(b) for a, b in ev))
     stats = env.read_stats()
     b2b_ms = 0.0
@@ -399,7 +436,7 @@ def device_leg(cx, wl, n, steps, warmup, sampler=None, back_to_back=True):
     return {"value": value, "ms_per_step": gpu_ms_max / steps,
             "ms_per_step_back_to_back": b2b_ms_max / steps if back_to_back else None,
             "kernel_ms": per, "roofline": roof, "launches": int(launches), "wall_s": wall, "stats": stats, "clocks": clocks,
-            "steps": steps, "warmup": warmup}
+            "steps": steps, "warmup": warmup, "outputs": outputs}
 
 
 def e2e_leg(cx, wl, n, steps, shards, **over):
@@ -618,7 +655,11 @@ def main():
     ap.add_argument("--config-steps", type=int, default=0, help="timed steps of the other configs' legs (0 = min(steps, 20))")
     ap.add_argument("--e2e-steps", type=int, default=0, help="0 = min(steps, 200)")
     ap.add_argument("--e2e-shards", type=int, default=8, help="stream shards of the host-facing env")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step returned (rank 0's envs) as DIR/<name>.npy, float32/float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     wl = workload_of(args.config, args.envs, args.obs)
     if args.impl == "reference":
@@ -632,7 +673,13 @@ def main():
 
     cx = Ctx()
     n = wl.envs
-    main_leg = device_leg(cx, wl, n, args.steps, args.warmup, sampler=ClockSampler(cx.local) if cx.rank == 0 else None)
+    main_leg = device_leg(cx, wl, n, args.steps, args.warmup, sampler=ClockSampler(cx.local) if cx.rank == 0 else None,
+                          keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs and cx.rank == 0:
+        out_dir = Path(args.dump_outputs)
+        out_dir.mkdir(parents=True, exist_ok=True)
+        for name, a in main_leg.pop("outputs").items():
+            np.save(out_dir / f"{name}.npy", a)
 
     e2e_steps = args.e2e_steps or min(args.steps, 200)
     e2e = e2e_leg(cx, wl, n, e2e_steps, args.e2e_shards)

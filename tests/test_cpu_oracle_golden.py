@@ -40,7 +40,6 @@ def test_baselines_stack_replay(golden_dir):
     helpers.assert_matches_baselines_golden(rec, g)
 
 
-@pytest.mark.skipif(not ref_stubs.available(), reason="/root/reference not present (GPU box)")
 def test_library_stages_against_scipy_and_pillow():
     """The two library stages of a5, restated in the oracle, against the libraries themselves."""
     from PIL import Image
