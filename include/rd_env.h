@@ -323,6 +323,72 @@ int rd_policy_dreamer_set_state(rd_env* env, const float* stoch_dev, const float
 /* n_steps x (agent step -> rd_step) enqueued on `stream` with no host synchronisation (see rd_rollout_gap_follower). */
 int rd_rollout_dreamer(rd_env* env, int n_steps, const rd_outputs* out, float* actions_dev, int noise, void* stream);
 
+/* ---- device-resident episode store (SURVEY.md §8-f1): records the Collect rows of every env's episodes on the device
+ *      [REF dreamer/wrappers.py:198-250], exactly the episodes episodes.EpisodeRecorder hands to its callbacks, and
+ *      samples fixed-length chunks the way tools.load_episodes does [REF dreamer/tools.py:235-264].  The env must have
+ *      auto_reset = 0: the store resets the envs whose episode ended, after recording the terminal row.
+ *      Storage: a ring of capacity_rows rows per env (memory n_envs x capacity_rows x row bytes); an env's oldest
+ *      committed episodes are evicted as its ring wraps.  capacity_rows must exceed the longest episode the config
+ *      allows (time_limit_steps, time_limit_ticks / action_repeat, the task's time_limit / (dt * action_repeat)). ---- */
+enum { RD_STORE_LIDAR = 1, RD_STORE_POSE = 2, RD_STORE_VELOCITY = 4, RD_STORE_SPEED = 8,
+       RD_STORE_OCCUPANCY = 16 /* 'lidar_occupancy', u8 [64,64,1]; needs RD_OBS_OCCUPANCY */ };   /* keep_obs bits */
+enum { RD_STORE_POLICY_GAP_FOLLOWER = 0, RD_STORE_POLICY_DREAMER = 1 };                         /* rd_rollout_store */
+typedef struct rd_store_config {
+  int32_t capacity_rows;      /* rows per env */
+  int32_t precision;          /* 32 | 16: float keys as float32 | IEEE half [REF dreamer/wrappers.py:240-250 _convert] */
+  int32_t keep_obs;           /* RD_STORE_* observation keys to store (action, reward, discount, progress, time always) */
+  int32_t reset_mode;         /* RD_RESET_* of the resets of finished envs; -1 = cfg.reset_mode */
+  uint64_t seed;              /* sampler: Philox key (seed_lo, seed_hi ^ stream tag) */
+} rd_store_config;
+/* A sampled batch: caller-owned device buffers [B, L, ...] in the store's precision; NULL = not produced. */
+typedef struct rd_store_batch {
+  void* lidar_dev;            /* [B, L, n_beams] */
+  uint8_t* occupancy_dev;     /* [B, L, 64*64]   */
+  void* pose_dev;             /* [B, L, 6] */
+  void* velocity_dev;         /* [B, L, 6] */
+  void* speed_dev;            /* [B, L] */
+  void* action_dev;           /* [B, L, 2] */
+  void* reward_dev;           /* [B, L] */
+  void* discount_dev;         /* [B, L] */
+  void* progress_dev;         /* [B, L] */
+  void* time_dev;             /* [B, L] */
+  int64_t* episode_id_dev;    /* [B] id of the chunk's episode, -1 = no chunk (zero rows) */
+  int32_t* start_dev;         /* [B] first row of the chunk in its episode, -1 = no chunk */
+} rd_store_batch;
+typedef struct rd_store_summary {
+  int64_t committed;          /* episodes committed since rd_store_init (the next episode id) */
+  int64_t held;               /* episodes held (committed and not evicted) */
+  int64_t held_rows;          /* rows of the held episodes */
+  int64_t evicted;            /* committed - held */
+  int64_t invalid_requests;   /* caller-given sample indices that named no held chunk */
+  int64_t draws;              /* drawing rd_store_sample calls so far (the counter k of the draw law) */
+  int64_t capacity_rows, max_episode_steps;
+} rd_store_summary;
+typedef struct rd_store_episode { int64_t id, env, length; } rd_store_episode;
+
+/* Allocates the store of the handle (replaces an existing one). */
+int rd_store_init(rd_env* env, const rd_store_config* sc);
+/* rd_reset of every env + the first row of each env's new episode (episodes in progress are dropped, held ones kept). */
+int rd_store_reset(rd_env* env, const rd_outputs* out, void* stream);
+/* rd_step -> record every env's row -> commit the episodes of the worlds with a done car (ids in env order) -> reset
+ * exactly those envs (the others are not observed again) -> record their first rows.  Afterwards `out` holds, for reset
+ * envs, the first observation of the next episode, with reward and done of the finished step.  No host synchronisation.
+ * out must provide lidar (if stored), occupancy (if stored), pose, velocity, speed, reward, done, progress, lap, time. */
+int rd_store_step(rd_env* env, const float* actions_dev, const rd_outputs* out, void* stream);
+/* n_steps x (policy -> rd_store_step); policy RD_STORE_POLICY_*, noise as rd_rollout_dreamer (ignored for the gap
+ * follower); the actions of the last step are left in actions_dev (may be NULL). */
+int rd_rollout_store(rd_env* env, int policy, int n_steps, const rd_outputs* out, float* actions_dev, int noise,
+                     void* stream);
+/* batch chunks of `length` rows.  ids_dev == NULL: drawn over the held episodes of at least length + 1 rows in commit
+ * order (draw law in csrc/rd_store.cuh; balance: the reference's balance=True start).  Else ids_dev i64 [B] and
+ * starts_dev i32 [B] name the chunks; they are checked on the device, and must not overlap the episode_id / start
+ * outputs (RD_ERR_INVALID).  Asynchronous. */
+int rd_store_sample(rd_env* env, int batch, int length, int balance, const int64_t* ids_dev, const int32_t* starts_dev,
+                    const rd_store_batch* out, void* stream);
+/* Synchronises `stream`.  episodes_host (may be NULL): the first max_episodes held episodes in commit order. */
+int rd_store_info(rd_env* env, rd_store_summary* out_host, rd_store_episode* episodes_host, int64_t max_episodes,
+                  void* stream);
+
 /* ---- stage entry points (teacher-forced parity tests; each is one kernel of the step) ---- */
 /* a2 LiDAR [REF dreamer/scenarios/max_progress/austria.yml:7 'lidar' sensor]: poses f64 [n,3]=(x,y,yaw),
  * map_ids i32[n] sorted ascending or NULL (= map 0), ranges f32 [n, n_beams].  With agents_per_world = A > 1 consecutive

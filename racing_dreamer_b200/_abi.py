@@ -115,6 +115,36 @@ class RdDreamerWeights(C.Structure):
         ("n_samples", C.c_int32), ("precision", C.c_int32)]
 
 
+class RdStoreConfig(C.Structure):
+    """rd_store_config (include/rd_env.h): the device-resident episode store."""
+    _fields_ = [("capacity_rows", C.c_int32), ("precision", C.c_int32), ("keep_obs", C.c_int32), ("reset_mode", C.c_int32),
+                ("seed", C.c_uint64)]
+
+
+class RdStoreBatch(C.Structure):
+    """rd_store_batch: device pointers of a sampled [B, L, ...] batch (NULL = not produced)."""
+    _fields_ = [(n, C.c_void_p) for n in (
+        "lidar_dev", "occupancy_dev", "pose_dev", "velocity_dev", "speed_dev", "action_dev", "reward_dev", "discount_dev",
+        "progress_dev", "time_dev", "episode_id_dev", "start_dev")]
+
+
+class RdStoreSummary(C.Structure):
+    _fields_ = [(n, C.c_int64) for n in (
+        "committed", "held", "held_rows", "evicted", "invalid_requests", "draws", "capacity_rows", "max_episode_steps")]
+
+    def as_dict(self):
+        return {n: int(getattr(self, n)) for n, _ in self._fields_}
+
+
+class RdStoreEpisode(C.Structure):
+    _fields_ = [("id", C.c_int64), ("env", C.c_int64), ("length", C.c_int64)]
+
+
+STORE_LIDAR, STORE_POSE, STORE_VELOCITY, STORE_SPEED, STORE_OCCUPANCY = 1, 2, 4, 8, 16
+STORE_KEYS = {"lidar": STORE_LIDAR, "pose": STORE_POSE, "velocity": STORE_VELOCITY, "speed": STORE_SPEED,
+              "lidar_occupancy": STORE_OCCUPANCY}
+STORE_POLICY_GAP_FOLLOWER, STORE_POLICY_DREAMER = 0, 1
+
 RD_NOISE_ZERO, RD_NOISE_PHILOX, RD_NOISE_EXPLICIT = 0, 1, 2
 RD_DREAMER_DEBUG_FLOATS = 68
 RD_PRECISION_TF32X3, RD_PRECISION_TF32 = 0, 1
@@ -127,6 +157,7 @@ EXPORTS = (
     "rd_gap_follower_defaults", "rd_policy_gap_follower_init", "rd_policy_gap_follower", "rd_rollout_gap_follower",
     "rd_policy_dreamer_init", "rd_policy_dreamer", "rd_policy_dreamer_get_state", "rd_policy_dreamer_set_state",
     "rd_rollout_dreamer",
+    "rd_store_init", "rd_store_reset", "rd_store_step", "rd_rollout_store", "rd_store_sample", "rd_store_info",
 )
 
 LIB_PATH = Path(__file__).resolve().parent / "librd_env.so"
@@ -219,6 +250,18 @@ def load_library() -> C.CDLL:
     lib.rd_policy_dreamer_set_state.restype = i32
     lib.rd_rollout_dreamer.argtypes = [vp, i32, C.POINTER(RdOutputs), vp, i32, vp]
     lib.rd_rollout_dreamer.restype = i32
+    lib.rd_store_init.argtypes = [vp, C.POINTER(RdStoreConfig)]
+    lib.rd_store_init.restype = i32
+    lib.rd_store_reset.argtypes = [vp, C.POINTER(RdOutputs), vp]
+    lib.rd_store_reset.restype = i32
+    lib.rd_store_step.argtypes = [vp, vp, C.POINTER(RdOutputs), vp]
+    lib.rd_store_step.restype = i32
+    lib.rd_rollout_store.argtypes = [vp, i32, i32, C.POINTER(RdOutputs), vp, i32, vp]
+    lib.rd_rollout_store.restype = i32
+    lib.rd_store_sample.argtypes = [vp, i32, i32, i32, vp, vp, C.POINTER(RdStoreBatch), vp]
+    lib.rd_store_sample.restype = i32
+    lib.rd_store_info.argtypes = [vp, C.POINTER(RdStoreSummary), vp, i64, vp]
+    lib.rd_store_info.restype = i32
     if lib.rd_abi_version() != ABI_VERSION:
         raise NativeLibraryError(f"{path}: ABI version {lib.rd_abi_version()} != {ABI_VERSION}")
     _lib = lib

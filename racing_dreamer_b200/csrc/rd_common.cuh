@@ -75,6 +75,7 @@ __device__ __forceinline__ void philox4x32_10(uint32_t (&c)[4], uint32_t k0, uin
 }
 #define RD_STREAM_RESET 0x52455345u
 #define RD_STREAM_LIDAR 0x4c494441u
+#define RD_STREAM_STORE 0x53544f52u   // episode-store sampler (rd_store.cuh)
 
 // ---- map lookups (global memory, read-only path) ----
 __device__ __forceinline__ bool rd_cell_of(const DevMap& m, double x, double y, int& cx, int& cy) {

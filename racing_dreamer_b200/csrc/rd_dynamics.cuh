@@ -301,7 +301,10 @@ __device__ __forceinline__ void rd_stats_reduce(double* stats, const double (&st
   }
 }
 
-__global__ void __launch_bounds__(128) k_reset(StepParams P, OutPtrs o, const uint8_t* __restrict__ mask, int mode) {
+// keep_others: envs outside the mask are marked frozen (was_reset = 2: the LiDAR / occupancy kernels leave their rows as
+// they are) instead of being observed again (3); their rows are the same either way (pose and noise counters unchanged)
+__global__ void __launch_bounds__(128) k_reset(StepParams P, OutPtrs o, const uint8_t* __restrict__ mask, int mode,
+                                               int keep_others) {
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");   // k_lidar may start its set-up (see launch_lidar_t)
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= P.n) return;
@@ -322,7 +325,8 @@ __global__ void __launch_bounds__(128) k_reset(StepParams P, OutPtrs o, const ui
     q[0] = xy.x; q[1] = xy.y; q[2] = sv.x; q[3] = sv.y; q[4] = yw.x; q[5] = yw.y; q[6] = rd_ldp(P.S, RD_P_ST, e).x;
     agent_step = (uint32_t)P.S.i4[e].w;
   }
-  rd_write_obs(P, o, m, e, jv.y, q, episode, agent_step, sel ? 1 : 3, false, 0.0, 0.0);  // 3: not reset here -> occupancy untouched
+  rd_write_obs(P, o, m, e, jv.y, q, episode, agent_step, sel ? 1 : (keep_others ? 2 : 3), false, 0.0,
+               0.0);  // 3: not reset here -> occupancy untouched
   if (sel) {
     rd_write_scalars(o, e, 0.f, 0, p, 1, 0.0, 0);
     if (o.rank) o.rank[e] = 1 + (P.cfg.agents_per_world > 1 ? e % P.cfg.agents_per_world : 0);  // refined by the first step

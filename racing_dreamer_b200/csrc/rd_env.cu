@@ -23,6 +23,7 @@
 #include "rd_occupancy.cuh"
 #include "rd_policy.cuh"
 #include "rd_dreamer.cuh"
+#include "rd_store.cuh"
 
 #define RD_API extern "C" __attribute__((visibility("default")))
 
@@ -114,6 +115,21 @@ struct rd_env {
     bool attr_set = false;        // kernel opted in to > 48 KB of dynamic shared memory
   } pol;
   DreamerPolicy dr;   // on-device Dreamer agent (rd_policy_dreamer_init)
+  // device-resident episode store (rd_store_init, csrc/rd_store.cuh)
+  struct Store {
+    bool ready = false, started = false;   // started: rd_store_reset has run
+    rd_store_config sc{};
+    int64_t max_steps = 0;
+    StoreDev d{};
+    uint8_t* d_all = nullptr;               // [n] ones: the reset mask of rd_store_reset
+    unsigned long long* d_invalid = nullptr;
+    int64_t* d_elig = nullptr; int* d_n_elig = nullptr;   // eligibility compaction (ids in commit order, count)
+    void* d_cub = nullptr; size_t cub_bytes = 0;
+    int64_t epoch = 0, elig_epoch = -1; int elig_min = -1;   // the compaction is redone when the store or min_len changed
+    int64_t* d_req_id = nullptr; int32_t* d_req_start = nullptr; int req_cap = 0;
+    int64_t* d_export = nullptr;            // [M][3] (id, env, rows) of rd_store_info
+    int64_t draws = 0;
+  } st;
   // device-resident steps over several tracks: the observation kernels of every track but the first run on their own
   // stream (fork behind the step kernel, join at the end), so that a track's kernels fill the SMs the previous track's
   // persistent CTAs leave in their tail.  RD_FORK_MAPS=0 keeps everything on the caller's stream.
@@ -538,6 +554,14 @@ int stage_runs(rd_env* env, const int32_t* ids, int n, int (*runs)[2], cudaStrea
   return RD_OK;
 }
 
+void store_free(rd_env::Store& st) {
+  for (int k = 0; k < SK_N; ++k) cudaFree(st.d.rows[k]);
+  cudaFree(st.d.head); cudaFree(st.d.ep_start); cudaFree(st.d.table); cudaFree(st.d.next_id); cudaFree(st.d.fin);
+  cudaFree(st.d_all); cudaFree(st.d_invalid); cudaFree(st.d_elig); cudaFree(st.d_n_elig); cudaFree(st.d_cub);
+  cudaFree(st.d_req_id); cudaFree(st.d_req_start); cudaFree(st.d_export);
+  st = rd_env::Store{};
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------------------
@@ -671,6 +695,7 @@ RD_API void rd_destroy(rd_env* env) {
   cudaFree(env->d_stage_recs); cudaFree(env->d_stage_ids);
   cudaFree(env->pol.st.f64); cudaFree(env->pol.st.i32); cudaFree(env->pol.d_actions);
   dreamer_free(env->dr);
+  store_free(env->st);
   occ_free(env->occ);
   {
     auto& h = env->hp;
@@ -826,7 +851,7 @@ RD_API int rd_reset(rd_env* env, const uint8_t* mask_dev, int mode, const rd_out
   cudaStream_t s = (cudaStream_t)stream;
   {
     ScopedTiming tm(env, s, T_RESET);
-    k_reset<<<(env->n + 127) / 128, 128, 0, s>>>(step_params(env), out_ptrs(out), mask_dev, mode);
+    k_reset<<<(env->n + 127) / 128, 128, 0, s>>>(step_params(env), out_ptrs(out), mask_dev, mode, 0);
   }
   env->launches++;
   CUDA_TRY(env, cudaGetLastError());
@@ -1384,5 +1409,314 @@ RD_API int rd_read_timing(rd_env* env, rd_timing* out_host, int reset) {
   env->timed.clear();
   *out_host = env->acc;
   if (reset) env->acc = rd_timing{};
+  return RD_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// device-resident episode store (csrc/rd_store.cuh)
+namespace {
+// Longest episode the config allows, in agent steps (-1: unbounded): TimeLimit in agent steps, the gym TimeLimit in
+// ticks, and the tasks' time > time_limit (time advances by dt per tick, so that tick is at most floor(time_limit / dt)
+// + 2 ticks away even with the rounding of the accumulated time).  A world ends with its first car.
+int64_t store_max_steps(const rd_config& c) {
+  const int64_t R = c.action_repeat;
+  int64_t best = -1;
+  auto take = [&](int64_t v) { if (best < 0 || v < best) best = v; };
+  if (c.time_limit_steps > 0) take(c.time_limit_steps);
+  if (c.time_limit_ticks > 0) take((c.time_limit_ticks + R - 1) / R);
+  bool timed = false;   // max_speed has no time limit of its own [REF baselines/racing/environment/tasks.py:6-18]
+  if (c.agents_per_world > 1) {
+    for (int a = 0; a < c.agents_per_world; ++a) timed = timed || c.agent_task[a] != RD_TASK_MAX_SPEED;
+  } else {
+    timed = c.task != RD_TASK_MAX_SPEED;
+  }
+  if (timed && c.time_limit >= 0.0 && c.time_limit / c.dt < 1.0e15) {
+    const double ticks = std::floor(c.time_limit / c.dt) + 2.0;
+    take((int64_t)std::ceil(ticks / (double)R));
+  }
+  return best;
+}
+
+StoreSrc store_src(const rd_outputs* o, const float* actions) {
+  StoreSrc r{};
+  r.lidar = o->lidar_dev; r.occ = o->occupancy_dev; r.pose = o->pose_dev; r.vel = o->velocity_dev; r.speed = o->speed_dev;
+  r.reward = o->reward_dev; r.done = o->done_dev; r.progress = o->progress_dev; r.lap = o->lap_dev; r.time = o->time_dev;
+  r.actions = actions;
+  return r;
+}
+
+int store_check_out(rd_env* env, const rd_outputs* o) {
+  const auto& d = env->st.d;
+  if (!o || !o->pose_dev || !o->velocity_dev || !o->speed_dev || !o->reward_dev || !o->done_dev || !o->progress_dev ||
+      !o->lap_dev || !o->time_dev || (d.rows[SK_LIDAR] && !o->lidar_dev) || (d.rows[SK_OCC] && !o->occupancy_dev))
+    return fail(env, RD_ERR_INVALID, "the episode store records pose, velocity, speed, reward, done, progress, lap, time "
+                                     "and the stored observations: an output pointer is NULL");
+  return RD_OK;
+}
+
+int store_mode(const rd_env* env) {
+  return env->st.sc.reset_mode < 0 ? env->cfg.reset_mode : env->st.sc.reset_mode;
+}
+
+// ids of the held episodes of at least min_len rows, in commit order -> st.d_elig / st.d_n_elig (cached until the
+// store changes)
+int store_compact(rd_env* env, int min_len, cudaStream_t s) {
+  auto& st = env->st;
+  if (st.elig_epoch == st.epoch && st.elig_min == min_len) return RD_OK;
+  StoreIdIter it(thrust::counting_iterator<int64_t>(0), StoreIdOf{st.d.next_id, st.d.M});
+  size_t bytes = st.cub_bytes;
+  CUDA_TRY(env, cub::DeviceSelect::If(st.d_cub, bytes, it, st.d_elig, st.d_n_elig, (int)st.d.M, StoreEligible{st.d, min_len}, s));
+  env->launches++;
+  st.elig_epoch = st.epoch;
+  st.elig_min = min_len;
+  return RD_OK;
+}
+
+int store_record(rd_env* env, const rd_outputs* out, const float* actions, int reset_rows, cudaStream_t s) {
+  k_store_record<<<env->n, 128, 0, s>>>(env->st.d, store_src(out, actions), reset_rows);
+  env->launches++;
+  CUDA_TRY(env, cudaGetLastError());
+  return RD_OK;
+}
+
+int store_step(rd_env* env, const float* actions_dev, const rd_outputs* out, cudaStream_t s) {
+  auto& st = env->st;
+  int rc = rd_step(env, actions_dev, out, s);
+  if (rc) return rc;
+  if ((rc = store_record(env, out, actions_dev, 0, s))) return rc;
+  k_store_commit<<<1, RD_COMMIT_THREADS, 0, s>>>(st.d, out->done_dev);
+  env->launches++;
+  CUDA_TRY(env, cudaGetLastError());
+  // reset of the committed envs; the others are marked frozen so that the observation kernels skip them, and reward /
+  // done keep the finished step's values (what EpisodeRecorder.step returns)
+  rd_outputs keep = *out;
+  keep.reward_dev = nullptr;
+  keep.done_dev = nullptr;
+  {
+    ScopedTiming tm(env, s, T_RESET);
+    k_reset<<<(env->n + 127) / 128, 128, 0, s>>>(step_params(env), out_ptrs(&keep), st.d.fin, store_mode(env), 1);
+  }
+  env->launches++;
+  CUDA_TRY(env, cudaGetLastError());
+  if ((rc = observe(env, &keep, s, 0, -1, nullptr, true))) return rc;
+  if ((rc = store_record(env, out, actions_dev, 1, s))) return rc;
+  st.epoch++;
+  return RD_OK;
+}
+}  // namespace
+
+RD_API int rd_store_init(rd_env* env, const rd_store_config* sc) {
+  if (!env || !sc) return fail(env, RD_ERR_INVALID, "null argument");
+  const rd_config& c = env->cfg;
+  if (c.auto_reset)
+    return fail(env, RD_ERR_INVALID, "the episode store needs auto_reset = 0: it records the terminal observation, then "
+                                     "resets the finished envs itself");
+  if (sc->precision != 32 && sc->precision != 16) return fail(env, RD_ERR_INVALID, "precision %d: expected 32 or 16", sc->precision);
+  if (sc->keep_obs & ~31) return fail(env, RD_ERR_INVALID, "keep_obs 0x%x: unknown bits", sc->keep_obs);
+  if ((sc->keep_obs & RD_STORE_OCCUPANCY) && !(c.obs_flags & RD_OBS_OCCUPANCY))
+    return fail(env, RD_ERR_INVALID, "keep_obs has lidar_occupancy but the env does not produce it (RD_OBS_OCCUPANCY)");
+  if (sc->reset_mode < -1 || sc->reset_mode > RD_RESET_RANDOM_BALL) return fail(env, RD_ERR_INVALID, "bad reset mode %d", sc->reset_mode);
+  const int64_t max_steps = store_max_steps(c);
+  if (max_steps < 0)
+    return fail(env, RD_ERR_INVALID, "the config bounds no episode length (time_limit_steps, time_limit_ticks or a timed task): "
+                                     "a ring could overwrite the episode in progress");
+  if ((int64_t)sc->capacity_rows < max_steps + 1)
+    return fail(env, RD_ERR_INVALID, "capacity_rows %d: episodes of this config reach %lld steps, so at least %lld rows are needed",
+                sc->capacity_rows, (long long)max_steps, (long long)(max_steps + 1));
+  const int64_t n = env->n, cap = sc->capacity_rows;
+  const int64_t M = n * (cap + 2);
+  if (M >= INT32_MAX) return fail(env, RD_ERR_INVALID, "n_envs x (capacity_rows + 2) = %lld exceeds the episode table's 2^31 slots", (long long)M);
+  store_free(env->st);
+  auto& st = env->st;
+  st.sc = *sc;
+  st.max_steps = max_steps;
+  StoreDev& d = st.d;
+  d.cap = (int)cap; d.n = (int)n; d.nb = c.n_beams; d.A = c.agents_per_world > 1 ? c.agents_per_world : 1; d.M = M;
+  d.half = sc->precision == 16 ? 1 : 0;
+  d.lidar_in_half = (c.obs_flags & RD_OBS_LIDAR_F16) ? 1 : 0;
+  const int fe = d.half ? 2 : 4;
+  const int rb[SK_N] = {c.n_beams * fe, 6 * fe, 6 * fe, fe, RD_OCC_OUT * RD_OCC_OUT, 2 * fe, fe, fe, fe, fe};
+  const bool keep[SK_N] = {(sc->keep_obs & RD_STORE_LIDAR) != 0, (sc->keep_obs & RD_STORE_POSE) != 0,
+                           (sc->keep_obs & RD_STORE_VELOCITY) != 0, (sc->keep_obs & RD_STORE_SPEED) != 0,
+                           (sc->keep_obs & RD_STORE_OCCUPANCY) != 0, true, true, true, true, true};
+  cudaError_t e = cudaSuccess;
+  auto alloc = [&](void** p, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc(p, bytes); };
+  for (int k = 0; k < SK_N; ++k) {
+    d.rb[k] = rb[k];
+    if (keep[k]) alloc((void**)&d.rows[k], (size_t)n * (size_t)cap * (size_t)rb[k]);
+  }
+  alloc((void**)&d.head, sizeof(int64_t) * n);
+  alloc((void**)&d.ep_start, sizeof(int64_t) * n);
+  alloc((void**)&d.table, sizeof(StoreEp) * M);
+  alloc((void**)&d.next_id, sizeof(int64_t));
+  alloc((void**)&d.fin, (size_t)n);
+  alloc((void**)&st.d_invalid, sizeof(unsigned long long));
+  alloc((void**)&st.d_elig, sizeof(int64_t) * M);
+  alloc((void**)&st.d_n_elig, sizeof(int));
+  alloc((void**)&st.d_export, sizeof(int64_t) * 3 * M);
+  if (e == cudaSuccess) e = cudaMemset(d.head, 0, sizeof(int64_t) * n);
+  if (e == cudaSuccess) e = cudaMemset(d.ep_start, 0, sizeof(int64_t) * n);
+  if (e == cudaSuccess) e = cudaMemset(d.table, 0xff, sizeof(StoreEp) * M);   // id -1: empty
+  if (e == cudaSuccess) e = cudaMemset(d.next_id, 0, sizeof(int64_t));
+  if (e == cudaSuccess) e = cudaMemset(d.fin, 0, (size_t)n);
+  if (e == cudaSuccess) e = cudaMemset(st.d_invalid, 0, sizeof(unsigned long long));
+  if (e == cudaSuccess) e = cudaMemset(st.d_n_elig, 0, sizeof(int));
+  if (e == cudaSuccess) {
+    StoreIdIter it(thrust::counting_iterator<int64_t>(0), StoreIdOf{d.next_id, M});
+    e = cub::DeviceSelect::If(nullptr, st.cub_bytes, it, st.d_elig, st.d_n_elig, (int)M, StoreEligible{d, 1});
+  }
+  alloc(&st.d_cub, std::max<size_t>(st.cub_bytes, 16));
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    store_free(env->st);
+    return fail(env, e == cudaErrorMemoryAllocation ? RD_ERR_NOMEM : RD_ERR_CUDA, "episode store allocation: %s", cudaGetErrorString(e));
+  }
+  st.ready = true;
+  return RD_OK;
+}
+
+RD_API int rd_store_reset(rd_env* env, const rd_outputs* out, void* stream) {
+  if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
+  auto& st = env->st;
+  if (!st.ready) return fail(env, RD_ERR_STATE, "rd_store_init has not been called");
+  int rc = store_check_out(env, out);
+  if (rc) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  if ((rc = rd_reset(env, nullptr, store_mode(env), out, stream))) return rc;
+  CUDA_TRY(env, cudaMemsetAsync(st.d.fin, 1, (size_t)env->n, s));
+  if ((rc = store_record(env, out, nullptr, 1, s))) return rc;
+  st.started = true;
+  st.epoch++;
+  return RD_OK;
+}
+
+RD_API int rd_store_step(rd_env* env, const float* actions_dev, const rd_outputs* out, void* stream) {
+  if (!env || !actions_dev) return fail(env, RD_ERR_INVALID, "null argument");
+  if (!env->st.ready) return fail(env, RD_ERR_STATE, "rd_store_init has not been called");
+  if (!env->st.started) return fail(env, RD_ERR_STATE, "rd_store_reset has not been called");
+  int rc = store_check_out(env, out);
+  if (rc) return rc;
+  return store_step(env, actions_dev, out, (cudaStream_t)stream);
+}
+
+RD_API int rd_rollout_store(rd_env* env, int policy, int n_steps, const rd_outputs* out, float* actions_dev, int noise,
+                            void* stream) {
+  if (!env || n_steps < 0) return fail(env, RD_ERR_INVALID, "bad argument");
+  if (!env->st.ready) return fail(env, RD_ERR_STATE, "rd_store_init has not been called");
+  if (!env->st.started) return fail(env, RD_ERR_STATE, "rd_store_reset has not been called");
+  int rc = store_check_out(env, out);
+  if (rc) return rc;
+  if (!out->lidar_dev) return fail(env, RD_ERR_INVALID, "the rollout needs out->lidar_dev");
+  if (policy == RD_STORE_POLICY_GAP_FOLLOWER) {
+    if (!env->pol.ready) return fail(env, RD_ERR_STATE, "rd_policy_gap_follower_init has not been called");
+  } else if (policy == RD_STORE_POLICY_DREAMER) {
+    if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
+    if (noise != RD_NOISE_ZERO && noise != RD_NOISE_PHILOX) return fail(env, RD_ERR_INVALID, "a rollout draws its own noise (RD_NOISE_ZERO or RD_NOISE_PHILOX)");
+  } else {
+    return fail(env, RD_ERR_INVALID, "bad policy %d", policy);
+  }
+  cudaStream_t s = (cudaStream_t)stream;
+  float* act = actions_dev ? actions_dev : env->pol.d_actions;
+  for (int k = 0; k < n_steps; ++k) {
+    rc = policy == RD_STORE_POLICY_GAP_FOLLOWER ? launch_gap_follower(env, out->lidar_dev, nullptr, act, nullptr, s)
+                                                : launch_dreamer(env, out->lidar_dev, act, noise, nullptr, nullptr, nullptr, s);
+    if (rc) return rc;
+    if ((rc = store_step(env, act, out, s))) return rc;
+  }
+  return RD_OK;
+}
+
+RD_API int rd_store_sample(rd_env* env, int batch, int length, int balance, const int64_t* ids_dev, const int32_t* starts_dev,
+                           const rd_store_batch* out, void* stream) {
+  if (!env || !out) return fail(env, RD_ERR_INVALID, "null argument");
+  auto& st = env->st;
+  if (!st.ready) return fail(env, RD_ERR_STATE, "rd_store_init has not been called");
+  if (batch < 1 || length < 1 || (int64_t)batch * length >= INT32_MAX)
+    return fail(env, RD_ERR_INVALID, "batch %d x length %d: both must be positive and the product below 2^31", batch, length);
+  if (ids_dev && !starts_dev) return fail(env, RD_ERR_INVALID, "explicit indices need both ids_dev and starts_dev");
+  if (ids_dev) {   // k_store_gather reads the requests of entry b in every CTA of b while one of them writes its outputs
+    auto overlap = [&](const void* a, size_t an, const void* b, size_t bn) {
+      const uintptr_t a0 = (uintptr_t)a, b0 = (uintptr_t)b;
+      return a && b && a0 < b0 + bn && b0 < a0 + an;
+    };
+    const size_t ni = sizeof(int64_t) * (size_t)batch, ns = sizeof(int32_t) * (size_t)batch;
+    if (overlap(ids_dev, ni, out->episode_id_dev, ni) || overlap(ids_dev, ni, out->start_dev, ns) ||
+        overlap(starts_dev, ns, out->episode_id_dev, ni) || overlap(starts_dev, ns, out->start_dev, ns))
+      return fail(env, RD_ERR_INVALID, "the episode_id / start outputs overlap the explicit indices: pass separate buffers");
+  }
+  cudaStream_t s = (cudaStream_t)stream;
+  if (batch > st.req_cap) {   // scratch: requests [batch] and the id / start outputs [batch] when the caller gives none
+    cudaFree(st.d_req_id); cudaFree(st.d_req_start);
+    st.d_req_id = nullptr; st.d_req_start = nullptr; st.req_cap = 0;
+    CUDA_TRY(env, cudaMalloc(&st.d_req_id, sizeof(int64_t) * 2 * (size_t)batch));
+    CUDA_TRY(env, cudaMalloc(&st.d_req_start, sizeof(int32_t) * 2 * (size_t)batch));
+    st.req_cap = batch;
+  }
+  const int64_t* rid = ids_dev;
+  const int32_t* rstart = starts_dev;
+  if (!ids_dev) {
+    int rc = store_compact(env, length + 1, s);   // the reference skips episodes with total - length < 1
+    if (rc) return rc;
+    const uint64_t seed = st.sc.seed;
+    k_store_draw<<<(batch + 127) / 128, 128, 0, s>>>(st.d, st.d_elig, st.d_n_elig, batch, length, balance ? 1 : 0,
+                                                     (uint32_t)seed, (uint32_t)(seed >> 32) ^ RD_STREAM_STORE,
+                                                     (uint32_t)st.draws, st.d_req_id, st.d_req_start);
+    env->launches++;
+    CUDA_TRY(env, cudaGetLastError());
+    st.draws++;
+    rid = st.d_req_id;
+    rstart = st.d_req_start;
+  }
+  StoreOut o{};
+  o.p[SK_LIDAR] = (unsigned char*)out->lidar_dev; o.p[SK_POSE] = (unsigned char*)out->pose_dev;
+  o.p[SK_VELOCITY] = (unsigned char*)out->velocity_dev; o.p[SK_SPEED] = (unsigned char*)out->speed_dev;
+  o.p[SK_OCC] = out->occupancy_dev; o.p[SK_ACTION] = (unsigned char*)out->action_dev;
+  o.p[SK_REWARD] = (unsigned char*)out->reward_dev; o.p[SK_DISCOUNT] = (unsigned char*)out->discount_dev;
+  o.p[SK_PROGRESS] = (unsigned char*)out->progress_dev; o.p[SK_TIME] = (unsigned char*)out->time_dev;
+  o.id = out->episode_id_dev ? out->episode_id_dev : st.d_req_id + st.req_cap;
+  o.start = out->start_dev ? out->start_dev : st.d_req_start + st.req_cap;
+  k_store_gather<<<(unsigned)((int64_t)batch * length), 128, 0, s>>>(st.d, o, rid, rstart, length, ids_dev ? 1 : 0, st.d_invalid);
+  env->launches++;
+  CUDA_TRY(env, cudaGetLastError());
+  return RD_OK;
+}
+
+RD_API int rd_store_info(rd_env* env, rd_store_summary* out_host, rd_store_episode* episodes_host, int64_t max_episodes,
+                         void* stream) {
+  if (!env || !out_host) return fail(env, RD_ERR_INVALID, "null argument");
+  auto& st = env->st;
+  if (!st.ready) return fail(env, RD_ERR_STATE, "rd_store_init has not been called");
+  cudaStream_t s = (cudaStream_t)stream;
+  int rc = store_compact(env, 1, s);
+  if (rc) return rc;
+  int held = 0;
+  int64_t committed = 0;
+  unsigned long long invalid = 0;
+  CUDA_TRY(env, cudaMemcpyAsync(&held, st.d_n_elig, sizeof(int), cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(env, cudaMemcpyAsync(&committed, st.d.next_id, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(env, cudaMemcpyAsync(&invalid, st.d_invalid, sizeof(invalid), cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(env, cudaStreamSynchronize(s));
+  std::vector<int64_t> eps(3 * (size_t)held);
+  if (held > 0) {
+    k_store_export<<<(held + 127) / 128, 128, 0, s>>>(st.d, st.d_elig, held, st.d_export);
+    env->launches++;
+    CUDA_TRY(env, cudaGetLastError());
+    CUDA_TRY(env, cudaMemcpyAsync(eps.data(), st.d_export, sizeof(int64_t) * eps.size(), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(env, cudaStreamSynchronize(s));
+  }
+  int64_t rows = 0;
+  for (int i = 0; i < held; ++i) rows += eps[3 * (size_t)i + 2];
+  out_host->committed = committed;
+  out_host->held = held;
+  out_host->held_rows = rows;
+  out_host->evicted = committed - held;
+  out_host->invalid_requests = (int64_t)invalid;
+  out_host->draws = st.draws;
+  out_host->capacity_rows = st.sc.capacity_rows;
+  out_host->max_episode_steps = st.max_steps;
+  if (episodes_host)
+    for (int64_t i = 0; i < std::min<int64_t>(held, max_episodes); ++i) {
+      episodes_host[i].id = eps[3 * i]; episodes_host[i].env = eps[3 * i + 1]; episodes_host[i].length = eps[3 * i + 2];
+    }
   return RD_OK;
 }

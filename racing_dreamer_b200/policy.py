@@ -18,6 +18,11 @@ from . import _abi
 from .env import BatchedRaceEnv
 
 
+def _check_store(env: BatchedRaceEnv, store) -> None:
+    if getattr(store, "env", None) is not env:
+        raise ValueError("store must be a DeviceEpisodeStore of this policy's env")
+
+
 class GapFollowerPolicy:
     def __init__(self, env: BatchedRaceEnv, **overrides):
         """overrides: fields of ``rd_gap_follower`` (e.g. ``speed_scale=0.6``, ``kp=1.2``)."""
@@ -58,13 +63,20 @@ class GapFollowerPolicy:
                                                       env._stream()))
         return self.actions
 
-    def rollout(self, n_steps: int):
+    def rollout(self, n_steps: int, store=None):
         """n_steps x (controller -> env.step) enqueued on the current stream; returns the env's (obs, reward, done, info)
-        views of the LAST step.  Episode statistics accumulate on the device (env.read_stats())."""
+        views of the LAST step.  Episode statistics accumulate on the device (env.read_stats()).
+        store: a ``DeviceEpisodeStore`` of this env -- every step is recorded and the finished envs are reset
+        (``store.step``), still with no host synchronisation."""
         env = self.env
         with torch.cuda.device(env.device):
-            env._check(env.lib.rd_rollout_gap_follower(env._handle, int(n_steps), C.byref(env._out),
-                                                       self.actions.data_ptr(), env._stream()))
+            if store is not None:
+                _check_store(env, store)
+                env._check(env.lib.rd_rollout_store(env._handle, _abi.STORE_POLICY_GAP_FOLLOWER, int(n_steps),
+                                                    C.byref(env._out), self.actions.data_ptr(), 0, env._stream()))
+            else:
+                env._check(env.lib.rd_rollout_gap_follower(env._handle, int(n_steps), C.byref(env._out),
+                                                           self.actions.data_ptr(), env._stream()))
         return env._obs(), env.buf["reward"], env.buf["done_bool"], env._info()
 
     def drive_command(self) -> Dict[str, torch.Tensor]:
@@ -258,11 +270,17 @@ class DreamerPolicy:
         z = lambda w: torch.zeros((self.env.n, w), dtype=torch.float32, device=self.env.device)   # noqa: E731
         self.set_state(z(_STOCH), z(self.deter), z(2))
 
-    def rollout(self, n_steps: int, noise: Optional[str] = None):
-        """n_steps x (agent step -> env.step) enqueued on the current stream, no host round trip."""
+    def rollout(self, n_steps: int, noise: Optional[str] = None, store=None):
+        """n_steps x (agent step -> env.step) enqueued on the current stream, no host round trip.  store: a
+        ``DeviceEpisodeStore`` of this env that records every step and resets the finished envs (``store.step``)."""
         env = self.env
         mode = self.NOISE[noise or self.noise]
         with torch.cuda.device(env.device):
-            env._check(env.lib.rd_rollout_dreamer(env._handle, int(n_steps), C.byref(env._out), self.actions.data_ptr(),
-                                                  mode, env._stream()))
+            if store is not None:
+                _check_store(env, store)
+                env._check(env.lib.rd_rollout_store(env._handle, _abi.STORE_POLICY_DREAMER, int(n_steps), C.byref(env._out),
+                                                    self.actions.data_ptr(), mode, env._stream()))
+            else:
+                env._check(env.lib.rd_rollout_dreamer(env._handle, int(n_steps), C.byref(env._out),
+                                                      self.actions.data_ptr(), mode, env._stream()))
         return env._obs(), env.buf["reward"], env.buf["done_bool"], env._info()
