@@ -389,6 +389,44 @@ int rd_store_sample(rd_env* env, int batch, int length, int balance, const int64
 int rd_store_info(rd_env* env, rd_store_summary* out_host, rd_store_episode* episodes_host, int64_t max_episodes,
                   void* stream);
 
+/* ---- import arena: episodes from outside the store (saved files, other runs) sampled together with the recorded ones.
+ *      One ring of import_capacity_rows rows per key, same row format and precision as the env rings; imported
+ *      episode k (0, 1, ... in import order since rd_store_import_init) has id RD_STORE_IMPORTED_ID0 + k and env -1.
+ *      It is held while its first row has not been overwritten, so importing past the arena's end evicts the oldest
+ *      imported episodes.  Draws of rd_store_sample pick from one list: the held imported episodes in import order, then
+ *      the held recorded episodes in commit order.  Imports never touch the env rings or the recorded episodes;
+ *      rd_store_reset keeps imported episodes, rd_store_init drops them. ---- */
+#define RD_STORE_IMPORTED_ID0 (INT64_C(1) << 62)
+enum { RD_STORE_U8 = 1, RD_STORE_F16 = 2, RD_STORE_F32 = 4, RD_STORE_F64 = 8 };   /* staged element type (= its bytes) */
+/* Staged rows of the episodes of one rd_store_import call, back to back: caller-owned device buffers [rows, ...] in the
+ * row shapes of rd_store_batch; a kept key needs its pointer and type (float keys F16 | F32 | F64, occupancy U8),
+ * others are ignored.  Floats are rounded once to the store's precision (numpy astype). */
+typedef struct rd_store_import_rows {
+  const void* lidar_dev; const void* occupancy_dev; const void* pose_dev; const void* velocity_dev; const void* speed_dev;
+  const void* action_dev; const void* reward_dev; const void* discount_dev; const void* progress_dev; const void* time_dev;
+  int32_t lidar_type, occupancy_type, pose_type, velocity_type, speed_type, action_type, reward_type, discount_type,
+          progress_type, time_type;
+} rd_store_import_rows;
+typedef struct rd_store_import_summary {
+  int64_t imported;           /* episodes imported since rd_store_import_init (the next imported id - ID0) */
+  int64_t held;               /* imported episodes held */
+  int64_t held_rows;          /* rows of the held imported episodes */
+  int64_t evicted;            /* imported - held */
+  int64_t capacity_rows;      /* arena rows (0: no arena) */
+} rd_store_import_summary;
+
+/* Allocates the import arena of the store (after rd_store_init; replaces an existing arena and its episodes). */
+int rd_store_import_init(rd_env* env, int32_t import_capacity_rows);
+/* Imports n_episodes episodes of lengths_host[i] rows (1 <= length <= import_capacity_rows), staged in `rows`.  rows ==
+ * NULL counts them as imported and at once overwritten (ids and arena rows advance, nothing is held or read): for the
+ * episodes a caller knows later imports overwrite.  Asynchronous; the staged buffers must stay valid until the work
+ * enqueued on `stream` has run. */
+int rd_store_import(rd_env* env, int32_t n_episodes, const int32_t* lengths_host, const rd_store_import_rows* rows,
+                    void* stream);
+/* Synchronises `stream`.  episodes_host (may be NULL): the first max_episodes held imported episodes in import order. */
+int rd_store_import_info(rd_env* env, rd_store_import_summary* out_host, rd_store_episode* episodes_host,
+                         int64_t max_episodes, void* stream);
+
 /* ---- stage entry points (teacher-forced parity tests; each is one kernel of the step) ---- */
 /* a2 LiDAR [REF dreamer/scenarios/max_progress/austria.yml:7 'lidar' sensor]: poses f64 [n,3]=(x,y,yaw),
  * map_ids i32[n] sorted ascending or NULL (= map 0), ranges f32 [n, n_beams].  With agents_per_world = A > 1 consecutive

@@ -140,6 +140,21 @@ class RdStoreEpisode(C.Structure):
     _fields_ = [("id", C.c_int64), ("env", C.c_int64), ("length", C.c_int64)]
 
 
+class RdStoreImportRows(C.Structure):
+    """rd_store_import_rows: device pointers and element types (STORE_U8 / F16 / F32 / F64) of staged import rows."""
+    KEYS = ("lidar", "occupancy", "pose", "velocity", "speed", "action", "reward", "discount", "progress", "time")
+    _fields_ = [(k + "_dev", C.c_void_p) for k in KEYS] + [(k + "_type", C.c_int32) for k in KEYS]
+
+
+class RdStoreImportSummary(C.Structure):
+    _fields_ = [(n, C.c_int64) for n in ("imported", "held", "held_rows", "evicted", "capacity_rows")]
+
+    def as_dict(self):
+        return {n: int(getattr(self, n)) for n, _ in self._fields_}
+
+
+STORE_IMPORTED_ID0 = 1 << 62   # RD_STORE_IMPORTED_ID0
+STORE_U8, STORE_F16, STORE_F32, STORE_F64 = 1, 2, 4, 8
 STORE_LIDAR, STORE_POSE, STORE_VELOCITY, STORE_SPEED, STORE_OCCUPANCY = 1, 2, 4, 8, 16
 STORE_KEYS = {"lidar": STORE_LIDAR, "pose": STORE_POSE, "velocity": STORE_VELOCITY, "speed": STORE_SPEED,
               "lidar_occupancy": STORE_OCCUPANCY}
@@ -158,6 +173,7 @@ EXPORTS = (
     "rd_policy_dreamer_init", "rd_policy_dreamer", "rd_policy_dreamer_get_state", "rd_policy_dreamer_set_state",
     "rd_rollout_dreamer",
     "rd_store_init", "rd_store_reset", "rd_store_step", "rd_rollout_store", "rd_store_sample", "rd_store_info",
+    "rd_store_import_init", "rd_store_import", "rd_store_import_info",
 )
 
 LIB_PATH = Path(__file__).resolve().parent / "librd_env.so"
@@ -262,6 +278,12 @@ def load_library() -> C.CDLL:
     lib.rd_store_sample.restype = i32
     lib.rd_store_info.argtypes = [vp, C.POINTER(RdStoreSummary), vp, i64, vp]
     lib.rd_store_info.restype = i32
+    lib.rd_store_import_init.argtypes = [vp, i32]
+    lib.rd_store_import_init.restype = i32
+    lib.rd_store_import.argtypes = [vp, i32, vp, C.POINTER(RdStoreImportRows), vp]
+    lib.rd_store_import.restype = i32
+    lib.rd_store_import_info.argtypes = [vp, C.POINTER(RdStoreImportSummary), vp, i64, vp]
+    lib.rd_store_import_info.restype = i32
     if lib.rd_abi_version() != ABI_VERSION:
         raise NativeLibraryError(f"{path}: ABI version {lib.rd_abi_version()} != {ABI_VERSION}")
     _lib = lib

@@ -127,8 +127,9 @@ struct rd_env {
     void* d_cub = nullptr; size_t cub_bytes = 0;
     int64_t epoch = 0, elig_epoch = -1; int elig_min = -1;   // the compaction is redone when the store or min_len changed
     int64_t* d_req_id = nullptr; int32_t* d_req_start = nullptr; int req_cap = 0;
-    int64_t* d_export = nullptr;            // [M][3] (id, env, rows) of rd_store_info
+    int64_t* d_export = nullptr;            // [M + Mi][3] (id, env, rows) of rd_store_info
     int64_t draws = 0;
+    int32_t* d_imp_len = nullptr; int64_t* d_imp_first = nullptr; int imp_meta_cap = 0;   // rd_store_import: per episode
   } st;
   // device-resident steps over several tracks: the observation kernels of every track but the first run on their own
   // stream (fork behind the step kernel, join at the end), so that a track's kernels fill the SMs the previous track's
@@ -559,6 +560,8 @@ void store_free(rd_env::Store& st) {
   cudaFree(st.d.head); cudaFree(st.d.ep_start); cudaFree(st.d.table); cudaFree(st.d.next_id); cudaFree(st.d.fin);
   cudaFree(st.d_all); cudaFree(st.d_invalid); cudaFree(st.d_elig); cudaFree(st.d_n_elig); cudaFree(st.d_cub);
   cudaFree(st.d_req_id); cudaFree(st.d_req_start); cudaFree(st.d_export);
+  for (int k = 0; k < SK_N; ++k) cudaFree(st.d.imp[k]);
+  cudaFree(st.d.itable); cudaFree(st.d_imp_len); cudaFree(st.d_imp_first);
   st = rd_env::Store{};
 }
 
@@ -1463,12 +1466,34 @@ int store_mode(const rd_env* env) {
 int store_compact(rd_env* env, int min_len, cudaStream_t s) {
   auto& st = env->st;
   if (st.elig_epoch == st.epoch && st.elig_min == min_len) return RD_OK;
-  StoreIdIter it(thrust::counting_iterator<int64_t>(0), StoreIdOf{st.d.next_id, st.d.M});
+  StoreIdIter it(thrust::counting_iterator<int64_t>(0), StoreIdOf{st.d.next_id, st.d.M, st.d.Mi, st.d.imp_next});
   size_t bytes = st.cub_bytes;
-  CUDA_TRY(env, cub::DeviceSelect::If(st.d_cub, bytes, it, st.d_elig, st.d_n_elig, (int)st.d.M, StoreEligible{st.d, min_len}, s));
+  CUDA_TRY(env, cub::DeviceSelect::If(st.d_cub, bytes, it, st.d_elig, st.d_n_elig, (int)(st.d.M + st.d.Mi),
+                                      StoreEligible{st.d, min_len}, s));
   env->launches++;
   st.elig_epoch = st.epoch;
   st.elig_min = min_len;
+  return RD_OK;
+}
+
+// (id, env, rows) of every held episode, imported ones (n_imp of them) first; synchronises s
+int store_held(rd_env* env, cudaStream_t s, std::vector<int64_t>& eps, int& n_imp) {
+  auto& st = env->st;
+  int rc = store_compact(env, 1, s);
+  if (rc) return rc;
+  int held = 0;
+  CUDA_TRY(env, cudaMemcpyAsync(&held, st.d_n_elig, sizeof(int), cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(env, cudaStreamSynchronize(s));
+  eps.assign(3 * (size_t)held, 0);
+  if (held > 0) {
+    k_store_export<<<(held + 127) / 128, 128, 0, s>>>(st.d, st.d_elig, held, st.d_export);
+    env->launches++;
+    CUDA_TRY(env, cudaGetLastError());
+    CUDA_TRY(env, cudaMemcpyAsync(eps.data(), st.d_export, sizeof(int64_t) * eps.size(), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(env, cudaStreamSynchronize(s));
+  }
+  n_imp = 0;
+  while (n_imp < held && eps[3 * (size_t)n_imp] >= RD_STORE_IMPORTED_ID0) n_imp++;
   return RD_OK;
 }
 
@@ -1562,7 +1587,7 @@ RD_API int rd_store_init(rd_env* env, const rd_store_config* sc) {
   if (e == cudaSuccess) e = cudaMemset(st.d_invalid, 0, sizeof(unsigned long long));
   if (e == cudaSuccess) e = cudaMemset(st.d_n_elig, 0, sizeof(int));
   if (e == cudaSuccess) {
-    StoreIdIter it(thrust::counting_iterator<int64_t>(0), StoreIdOf{d.next_id, M});
+    StoreIdIter it(thrust::counting_iterator<int64_t>(0), StoreIdOf{d.next_id, M, 0, 0});
     e = cub::DeviceSelect::If(nullptr, st.cub_bytes, it, st.d_elig, st.d_n_elig, (int)M, StoreEligible{d, 1});
   }
   alloc(&st.d_cub, std::max<size_t>(st.cub_bytes, 16));
@@ -1687,23 +1712,16 @@ RD_API int rd_store_info(rd_env* env, rd_store_summary* out_host, rd_store_episo
   auto& st = env->st;
   if (!st.ready) return fail(env, RD_ERR_STATE, "rd_store_init has not been called");
   cudaStream_t s = (cudaStream_t)stream;
-  int rc = store_compact(env, 1, s);
-  if (rc) return rc;
-  int held = 0;
   int64_t committed = 0;
   unsigned long long invalid = 0;
-  CUDA_TRY(env, cudaMemcpyAsync(&held, st.d_n_elig, sizeof(int), cudaMemcpyDeviceToHost, s));
   CUDA_TRY(env, cudaMemcpyAsync(&committed, st.d.next_id, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
   CUDA_TRY(env, cudaMemcpyAsync(&invalid, st.d_invalid, sizeof(invalid), cudaMemcpyDeviceToHost, s));
-  CUDA_TRY(env, cudaStreamSynchronize(s));
-  std::vector<int64_t> eps(3 * (size_t)held);
-  if (held > 0) {
-    k_store_export<<<(held + 127) / 128, 128, 0, s>>>(st.d, st.d_elig, held, st.d_export);
-    env->launches++;
-    CUDA_TRY(env, cudaGetLastError());
-    CUDA_TRY(env, cudaMemcpyAsync(eps.data(), st.d_export, sizeof(int64_t) * eps.size(), cudaMemcpyDeviceToHost, s));
-    CUDA_TRY(env, cudaStreamSynchronize(s));
-  }
+  std::vector<int64_t> all;
+  int n_imp = 0;
+  int rc = store_held(env, s, all, n_imp);
+  if (rc) return rc;
+  const int held = (int)(all.size() / 3) - n_imp;   // the recorded episodes follow the imported ones
+  const int64_t* eps = all.data() + 3 * (size_t)n_imp;
   int64_t rows = 0;
   for (int i = 0; i < held; ++i) rows += eps[3 * (size_t)i + 2];
   out_host->committed = committed;
@@ -1716,6 +1734,125 @@ RD_API int rd_store_info(rd_env* env, rd_store_summary* out_host, rd_store_episo
   out_host->max_episode_steps = st.max_steps;
   if (episodes_host)
     for (int64_t i = 0; i < std::min<int64_t>(held, max_episodes); ++i) {
+      episodes_host[i].id = eps[3 * i]; episodes_host[i].env = eps[3 * i + 1]; episodes_host[i].length = eps[3 * i + 2];
+    }
+  return RD_OK;
+}
+
+RD_API int rd_store_import_init(rd_env* env, int32_t import_capacity_rows) {
+  if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
+  auto& st = env->st;
+  if (!st.ready) return fail(env, RD_ERR_STATE, "rd_store_init has not been called");
+  if (import_capacity_rows < 1) return fail(env, RD_ERR_INVALID, "import_capacity_rows %d: expected at least 1", import_capacity_rows);
+  const int64_t icap = import_capacity_rows, Mi = icap + 1;
+  if (st.d.M + Mi >= INT32_MAX)
+    return fail(env, RD_ERR_INVALID, "the recorded and imported episode tables (%lld + %lld slots) exceed 2^31",
+                (long long)st.d.M, (long long)Mi);
+  StoreDev& d = st.d;
+  // the new buffers are allocated first, so that a failed allocation leaves the store as it was
+  unsigned char* imp[SK_N] = {};
+  StoreEp* itable = nullptr; int64_t* elig = nullptr; int64_t* xport = nullptr; void* cub = nullptr;
+  size_t cub_bytes = 0;
+  cudaError_t e = cudaSuccess;
+  auto alloc = [&](void** p, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc(p, bytes); };
+  for (int k = 0; k < SK_N; ++k)
+    if (d.rows[k]) alloc((void**)&imp[k], (size_t)icap * (size_t)d.rb[k]);
+  alloc((void**)&itable, sizeof(StoreEp) * Mi);
+  alloc((void**)&elig, sizeof(int64_t) * (d.M + Mi));
+  alloc((void**)&xport, sizeof(int64_t) * 3 * (d.M + Mi));
+  if (e == cudaSuccess) e = cudaMemset(itable, 0xff, sizeof(StoreEp) * Mi);   // id -1: empty
+  if (e == cudaSuccess) {
+    StoreIdIter it(thrust::counting_iterator<int64_t>(0), StoreIdOf{d.next_id, d.M, Mi, 0});
+    e = cub::DeviceSelect::If(nullptr, cub_bytes, it, elig, st.d_n_elig, (int)(d.M + Mi), StoreEligible{d, 1});
+  }
+  alloc(&cub, std::max<size_t>(cub_bytes, 16));
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    for (int k = 0; k < SK_N; ++k) cudaFree(imp[k]);
+    cudaFree(itable); cudaFree(elig); cudaFree(xport); cudaFree(cub);
+    return fail(env, e == cudaErrorMemoryAllocation ? RD_ERR_NOMEM : RD_ERR_CUDA, "import arena allocation: %s", cudaGetErrorString(e));
+  }
+  for (int k = 0; k < SK_N; ++k) { cudaFree(d.imp[k]); d.imp[k] = imp[k]; }
+  cudaFree(d.itable); cudaFree(st.d_elig); cudaFree(st.d_export); cudaFree(st.d_cub);
+  d.itable = itable; st.d_elig = elig; st.d_export = xport; st.d_cub = cub; st.cub_bytes = cub_bytes;
+  d.icap = (int)icap; d.Mi = Mi; d.imp_head = 0; d.imp_next = 0;
+  st.epoch++;
+  return RD_OK;
+}
+
+RD_API int rd_store_import(rd_env* env, int32_t n_episodes, const int32_t* lengths_host, const rd_store_import_rows* rows,
+                           void* stream) {
+  if (!env || (n_episodes > 0 && !lengths_host) || n_episodes < 0) return fail(env, RD_ERR_INVALID, "bad argument");
+  auto& st = env->st;
+  StoreDev& d = st.d;
+  if (!st.ready) return fail(env, RD_ERR_STATE, "rd_store_init has not been called");
+  if (d.icap == 0) return fail(env, RD_ERR_STATE, "the store has no import arena (rd_store_import_init)");
+  if (n_episodes == 0) return RD_OK;
+  std::vector<int64_t> first((size_t)n_episodes);
+  int64_t total = 0;
+  for (int j = 0; j < n_episodes; ++j) {
+    if (lengths_host[j] < 1 || lengths_host[j] > d.icap)
+      return fail(env, RD_ERR_INVALID, "episode %d of the import has %d rows: expected 1 to import_capacity_rows = %d", j,
+                  lengths_host[j], d.icap);
+    first[(size_t)j] = total;
+    total += lengths_host[j];
+  }
+  cudaStream_t s = (cudaStream_t)stream;
+  if (rows) {
+    StoreStaged in{};
+    const void* p[SK_N] = {rows->lidar_dev, rows->pose_dev, rows->velocity_dev, rows->speed_dev, rows->occupancy_dev,
+                           rows->action_dev, rows->reward_dev, rows->discount_dev, rows->progress_dev, rows->time_dev};
+    const int32_t ty[SK_N] = {rows->lidar_type, rows->pose_type, rows->velocity_type, rows->speed_type, rows->occupancy_type,
+                              rows->action_type, rows->reward_type, rows->discount_type, rows->progress_type, rows->time_type};
+    const int32_t ne[SK_N] = {d.nb, 6, 6, 1, RD_OCC_OUT * RD_OCC_OUT, 2, 1, 1, 1, 1};
+    static const char* names[SK_N] = {"lidar", "pose", "velocity", "speed", "lidar_occupancy", "action", "reward",
+                                      "discount", "progress", "time"};
+    for (int k = 0; k < SK_N; ++k) {
+      if (!d.imp[k]) continue;
+      const bool ok_ty = k == SK_OCC ? ty[k] == RD_STORE_U8 : (ty[k] == RD_STORE_F16 || ty[k] == RD_STORE_F32 || ty[k] == RD_STORE_F64);
+      if (!p[k] || !ok_ty) return fail(env, RD_ERR_INVALID, "import rows of '%s': missing or of element type %d", names[k], ty[k]);
+      in.p[k] = (const unsigned char*)p[k];
+      in.type[k] = ty[k];
+      in.ne[k] = ne[k];
+    }
+    if (n_episodes > st.imp_meta_cap) {
+      cudaFree(st.d_imp_len); cudaFree(st.d_imp_first);
+      st.d_imp_len = nullptr; st.d_imp_first = nullptr; st.imp_meta_cap = 0;
+      CUDA_TRY(env, cudaMalloc(&st.d_imp_len, sizeof(int32_t) * (size_t)n_episodes));
+      CUDA_TRY(env, cudaMalloc(&st.d_imp_first, sizeof(int64_t) * (size_t)n_episodes));
+      st.imp_meta_cap = n_episodes;
+    }
+    CUDA_TRY(env, cudaMemcpyAsync(st.d_imp_len, lengths_host, sizeof(int32_t) * (size_t)n_episodes, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(env, cudaMemcpyAsync(st.d_imp_first, first.data(), sizeof(int64_t) * (size_t)n_episodes, cudaMemcpyHostToDevice, s));
+    const int64_t grid = std::min<int64_t>(total, d.icap);
+    k_store_import<<<(unsigned)grid, 128, 0, s>>>(d, in, total, st.d_imp_len, st.d_imp_first, n_episodes);
+    env->launches++;
+    CUDA_TRY(env, cudaGetLastError());
+  }
+  d.imp_head += total;
+  d.imp_next += n_episodes;
+  st.epoch++;
+  return RD_OK;
+}
+
+RD_API int rd_store_import_info(rd_env* env, rd_store_import_summary* out_host, rd_store_episode* episodes_host,
+                                int64_t max_episodes, void* stream) {
+  if (!env || !out_host) return fail(env, RD_ERR_INVALID, "null argument");
+  auto& st = env->st;
+  if (!st.ready) return fail(env, RD_ERR_STATE, "rd_store_init has not been called");
+  std::vector<int64_t> eps;
+  int n_imp = 0;
+  int rc = store_held(env, (cudaStream_t)stream, eps, n_imp);
+  if (rc) return rc;
+  int64_t rows = 0;
+  for (int i = 0; i < n_imp; ++i) rows += eps[3 * (size_t)i + 2];
+  out_host->imported = st.d.imp_next;
+  out_host->held = n_imp;
+  out_host->held_rows = rows;
+  out_host->evicted = st.d.imp_next - n_imp;
+  out_host->capacity_rows = st.d.icap;
+  if (episodes_host)
+    for (int64_t i = 0; i < std::min<int64_t>(n_imp, max_episodes); ++i) {
       episodes_host[i].id = eps[3 * i]; episodes_host[i].env = eps[3 * i + 1]; episodes_host[i].length = eps[3 * i + 2];
     }
   return RD_OK;

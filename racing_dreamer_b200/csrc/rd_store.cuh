@@ -10,6 +10,14 @@
 // (start >= head[env] - cap), so an env's oldest episodes are evicted as its ring wraps.  M = n_envs * (cap + 2) table
 // slots: a held episode's env writes at most cap rows before the episode is evicted, and no env commits more than
 // cap + 1 episodes in that time, so a held episode's slot is never reused.
+//
+// Import arena (rd_store_import): one more ring of icap rows per key, written from staged host episodes.  Imported
+// episode k has id RD_STORE_IMPORTED_ID0 + k, env -1 and its entry in a table of Mi = icap + 1 slots at k mod Mi; it is
+// held while its first row has not been overwritten (start >= imp_head - icap).  Every episode has at least one row, so
+// a held episode's slot is reused only after icap + 1 later imports, and those overwrite its rows first.  Imports are
+// host-driven, so the arena's counters (imp_head, imp_next) are host values passed in StoreDev: every launch sees the
+// arena as the imports enqueued before it left it.  The recorded table's bound M relies on the envs stepping in lockstep,
+// which imports do not, so imported episodes never go there.
 #pragma once
 #include <thrust/iterator/counting_iterator.h>
 #include <thrust/iterator/transform_iterator.h>
@@ -40,6 +48,11 @@ struct StoreDev {
   int cap, n, nb, A;
   int half;                    // precision 16: float keys stored as IEEE half
   int lidar_in_half;           // the env emits half scans (RD_OBS_LIDAR_F16)
+  // import arena (icap = 0: none)
+  unsigned char* imp[SK_N];    // [icap][rb[k]] or null
+  StoreEp* itable;             // [Mi]
+  int64_t Mi, imp_head, imp_next;   // table slots; arena rows written, episodes imported so far
+  int icap;
 };
 
 struct StoreSrc {                 // the env's outputs of the step / reset being recorded
@@ -90,8 +103,15 @@ __device__ __forceinline__ void st_zero(unsigned char* dst, int bytes) {
   }
 }
 
+// table entry of a recorded or imported id (the caller has checked id >= 0)
+__device__ __forceinline__ StoreEp st_entry(const StoreDev& S, int64_t id) {
+  if (id < RD_STORE_IMPORTED_ID0) return S.table[id % S.M];
+  if (S.Mi == 0) { StoreEp r; r.id = -1; r.start = 0; r.env = -1; r.len = 0; return r; }
+  return S.itable[(id - RD_STORE_IMPORTED_ID0) % S.Mi];
+}
 __device__ __forceinline__ bool st_held(const StoreDev& S, const StoreEp& r, int64_t id) {
-  return r.id == id && r.start >= S.head[r.env] - (int64_t)S.cap;
+  if (r.id != id) return false;
+  return r.env < 0 ? r.start >= S.imp_head - (int64_t)S.icap : r.start >= S.head[r.env] - (int64_t)S.cap;
 }
 
 // One row per env (one CTA per env): the step's row of every env (reset_rows = 0), or the reset row of every env that
@@ -183,16 +203,23 @@ __global__ void __launch_bounds__(RD_COMMIT_THREADS) k_store_commit(StoreDev S, 
   if (threadIdx.x == 0) *S.next_id = base_s;
 }
 
-// eligibility compaction in commit order: the window of the last M ids, kept when held and at least min_len rows long
+// eligibility compaction: the window of the last Mi imported ids in import order, then the window of the last M recorded
+// ids in commit order, kept when held and at least min_len rows long (without an arena Mi = 0: the recorded window alone)
 struct StoreIdOf {
-  const int64_t* next_id; int64_t M;
-  __device__ int64_t operator()(int64_t i) const { return *next_id - M + i; }
+  const int64_t* next_id; int64_t M, Mi, imp_next;
+  __device__ int64_t operator()(int64_t i) const {
+    if (i < Mi) {
+      const int64_t k = imp_next - Mi + i;
+      return k < 0 ? -1 : RD_STORE_IMPORTED_ID0 + k;
+    }
+    return *next_id - M + (i - Mi);
+  }
 };
 struct StoreEligible {
   StoreDev S; int min_len;
   __device__ bool operator()(int64_t id) const {
     if (id < 0) return false;
-    const StoreEp r = S.table[id % S.M];
+    const StoreEp r = st_entry(S, id);
     return st_held(S, r, id) && r.len >= min_len;
   }
 };
@@ -212,7 +239,7 @@ __global__ void __launch_bounds__(128) k_store_draw(StoreDev S, const int64_t* _
   uint32_t c[4] = {(uint32_t)b, call, 0u, 0u};
   philox4x32_10(c, k0, k1);
   const int64_t id = elig[(uint32_t)(((uint64_t)c[0] * (uint64_t)(uint32_t)ne) >> 32)];
-  const uint32_t total = (uint32_t)S.table[id % S.M].len;
+  const uint32_t total = (uint32_t)st_entry(S, id).len;
   uint32_t st;
   if (balance) {
     st = (uint32_t)(((uint64_t)c[1] * (uint64_t)total) >> 32);
@@ -242,22 +269,25 @@ __global__ void __launch_bounds__(128) k_store_gather(StoreDev S, StoreOut O, co
   bool ok = false;
   StoreEp r{};
   if (id >= 0) {
-    r = S.table[id % S.M];
+    r = st_entry(S, id);
     ok = st_held(S, r, id) && st >= 0 && (int64_t)st + L <= (int64_t)r.len;
   }
+  const bool imported = r.env < 0;
   if (t == 0 && threadIdx.x == 0) {
     O.id[b] = ok ? id : -1;
     O.start[b] = ok ? st : -1;
     if (!ok && count_invalid) atomicAdd(invalid, 1ull);
   }
-  const size_t src_slot = ok ? (size_t)r.env * (size_t)S.cap + (size_t)((r.start + st + t) % S.cap) : 0;
+  size_t src_slot = 0;
+  if (ok) src_slot = imported ? (size_t)((r.start + st + t) % S.icap)
+                              : (size_t)r.env * (size_t)S.cap + (size_t)((r.start + st + t) % S.cap);
 #pragma unroll
   for (int k = 0; k < SK_N; ++k) {   // unrolled: the key descriptors stay in the parameter space
     unsigned char* dst = O.p[k];
     if (!dst || !S.rows[k]) continue;
     const int rb = S.rb[k];
     dst += (size_t)row * rb;
-    if (ok) st_copy(dst, S.rows[k] + src_slot * rb, rb);
+    if (ok) st_copy(dst, (imported ? S.imp[k] : S.rows[k]) + src_slot * rb, rb);
     else st_zero(dst, rb);
   }
 }
@@ -266,6 +296,84 @@ __global__ void __launch_bounds__(128) k_store_gather(StoreDev S, StoreOut O, co
 __global__ void k_store_export(StoreDev S, const int64_t* __restrict__ ids, int n, int64_t* out) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  const StoreEp r = S.table[ids[i] % S.M];
+  const StoreEp r = st_entry(S, ids[i]);
   out[3 * i] = r.id; out[3 * i + 1] = r.env; out[3 * i + 2] = r.len;
+}
+
+// Import of staged rows, one CTA per staged row: row r of the call goes to arena row imp_head + r, converted from the
+// staged type to the store's (numpy astype: one rounding); the first CTAs also write the table entries of the call's
+// episodes.  A call of more than icap rows writes only its last icap rows and the entries of its last icap episodes:
+// the others are overwritten within the call (an episode held afterwards has fewer than icap rows after its first, so
+// fewer than icap episodes after it).
+struct StoreStaged {
+  const unsigned char* p[SK_N];   // [rows][elements of the key] or null (key not kept)
+  int32_t type[SK_N];             // RD_STORE_U8 | F16 | F32 | F64 (element bytes)
+  int32_t ne[SK_N];               // elements per row
+};
+
+template <typename T> __device__ __forceinline__ double st_ld(const T* p, int i);
+template <> __device__ __forceinline__ double st_ld<__half>(const __half* p, int i) { return (double)__half2float(p[i]); }
+template <> __device__ __forceinline__ double st_ld<float>(const float* p, int i) { return (double)p[i]; }
+template <> __device__ __forceinline__ double st_ld<double>(const double* p, int i) { return p[i]; }
+
+// one row of n elements of type T into the store's float type; groups of 8 elements as 16-byte loads and stores where
+// n and both addresses allow it (a LiDAR row of 1080 beams), element by element otherwise.  Every value takes the path of
+// st_put_f64: widening to double is exact, so this is one rounding from the staged value.
+template <typename T>
+__device__ __forceinline__ void st_convert_row(unsigned char* dst, const unsigned char* src, int n, int half) {
+  const T* s = reinterpret_cast<const T*>(src);
+  const unsigned al = (unsigned)(uintptr_t)dst | (unsigned)(uintptr_t)src;
+  if ((n & 7) == 0 && (al & 15u) == 0) {
+    for (int g = threadIdx.x; g < n / 8; g += blockDim.x) {
+      alignas(16) T v[8];
+#pragma unroll
+      for (int q = 0; q < (int)(8 * sizeof(T)) / 16; ++q)
+        reinterpret_cast<uint4*>(v)[q] = __ldg(reinterpret_cast<const uint4*>(s + 8 * g) + q);
+      if (half) {
+        alignas(16) uint16_t h[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) h[j] = st_f64_to_f16(st_ld(v, j));
+        reinterpret_cast<uint4*>(dst)[g] = *reinterpret_cast<const uint4*>(h);
+      } else {
+        alignas(16) float f[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) f[j] = __double2float_rn(st_ld(v, j));
+        reinterpret_cast<uint4*>(dst)[2 * g] = *reinterpret_cast<const uint4*>(f);
+        reinterpret_cast<uint4*>(dst)[2 * g + 1] = *reinterpret_cast<const uint4*>(f + 4);
+      }
+    }
+  } else {
+    for (int i = threadIdx.x; i < n; i += blockDim.x) st_put_f64(dst, i, st_ld(s, i), half);
+  }
+}
+
+__global__ void __launch_bounds__(128) k_store_import(StoreDev S, StoreStaged in, int64_t rows, const int32_t* __restrict__ lens,
+                                                      const int64_t* __restrict__ first, int n_ep) {
+  const int64_t r = (int64_t)blockIdx.x + (rows > S.icap ? rows - S.icap : 0);
+  const int n_w = min(n_ep, S.icap);   // <= gridDim.x = min(rows, icap)
+  if ((int)blockIdx.x < n_w && threadIdx.x == 0) {
+    const int j = (int)blockIdx.x + (n_ep - n_w);
+    StoreEp e;
+    e.id = RD_STORE_IMPORTED_ID0 + S.imp_next + j;
+    e.start = S.imp_head + first[j];
+    e.env = -1;
+    e.len = lens[j];
+    S.itable[(S.imp_next + j) % S.Mi] = e;
+  }
+  if (r >= rows) return;
+  const size_t slot = (size_t)((S.imp_head + r) % S.icap);
+#pragma unroll
+  for (int k = 0; k < SK_N; ++k) {
+    unsigned char* dst = S.imp[k];
+    if (!dst) continue;
+    const int rb = S.rb[k];
+    dst += slot * rb;
+    const int ne = in.ne[k], ty = in.type[k];
+    const unsigned char* src = in.p[k] + (size_t)r * (size_t)ne * (size_t)ty;
+    const int store_ty = k == SK_OCC ? RD_STORE_U8 : (S.half ? RD_STORE_F16 : RD_STORE_F32);
+    if (ty == store_ty) st_copy(dst, src, rb);
+    else if (ty == RD_STORE_F16) st_convert_row<__half>(dst, src, ne, S.half);
+    else if (ty == RD_STORE_F32) st_convert_row<float>(dst, src, ne, S.half);
+    else st_convert_row<double>(dst, src, ne, S.half);
+  }
 }

@@ -20,9 +20,12 @@ from __future__ import annotations
 
 import datetime
 import io
+import os
 import pathlib
 import uuid
-from typing import Callable, Dict, Iterator, List, Optional, Sequence
+import zipfile
+from concurrent.futures import ThreadPoolExecutor
+from typing import Callable, Dict, Iterator, List, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -236,6 +239,82 @@ def max_episode_steps(cfg) -> Optional[int]:
     return min(bounds) if bounds else None
 
 
+def episode_files(directory, shard: Optional[Tuple[int, int]] = None) -> List[pathlib.Path]:
+    """The ``*.npz`` files of `directory` in sorted order (``load_episodes``' order); ``shard=(rank, world)`` keeps those
+    whose index in that order is ``rank`` modulo ``world``, so that the ranks of one run split a directory."""
+    files = sorted(pathlib.Path(directory).expanduser().glob("*.npz"))
+    if shard is None:
+        return files
+    rank, world = (int(v) for v in shard)
+    if world < 1 or not 0 <= rank < world:
+        raise ValueError(f"shard {shard}: expected (rank, world) with 0 <= rank < world")
+    return files[rank::world]
+
+
+def npz_meta(path, keys: Sequence[str]) -> Dict[str, Tuple[tuple, np.dtype]]:
+    """(shape, dtype) of the arrays `keys` of an ``.npz`` file, read from the ``.npy`` headers without decompressing
+    the data; keys the file lacks are left out.  Raises on a file that is not a readable archive."""
+    from numpy.lib import format as npf
+    readers = {(1, 0): npf.read_array_header_1_0, (2, 0): npf.read_array_header_2_0}
+    out = {}
+    with zipfile.ZipFile(path) as z:
+        names = set(z.namelist())
+        for k in keys:
+            if k + ".npy" not in names:
+                continue
+            with z.open(k + ".npy") as f:
+                version = npf.read_magic(f)
+                if version in readers:
+                    shape, _, dtype = readers[version](f)
+                else:       # a newer header format: decode the array
+                    a = npf.read_array(f)
+                    shape, dtype = a.shape, a.dtype
+            out[k] = (tuple(shape), np.dtype(dtype))
+    return out
+
+
+_FLOAT_DTYPES = (np.dtype(np.float16), np.dtype(np.float32), np.dtype(np.float64))
+
+
+def check_import(metas: Sequence[Dict[str, Tuple[tuple, np.dtype]]], row_shapes: Dict[str, tuple],
+                 capacity_rows: int, names: Optional[Sequence[str]] = None) -> List[int]:
+    """Lengths of the episodes described by `metas` (key -> (shape, dtype)), or ValueError naming the first episode a
+    ``DeviceEpisodeStore`` with these row shapes and import arena cannot take: a missing key, keys of different
+    lengths or of no rows, a row shape other than the store's, a float key that is not float16/32/64, a
+    ``lidar_occupancy`` that is not uint8, or more rows than the arena holds.  Extra keys are ignored."""
+    lengths = []
+    for i, meta in enumerate(metas):
+        what = names[i] if names is not None else f"episode {i}"
+        missing = [k for k in row_shapes if k not in meta]
+        if missing:
+            raise ValueError(f"{what}: missing keys {missing}")
+        n = {meta[k][0][0] if len(meta[k][0]) else None for k in row_shapes}
+        if len(n) != 1 or None in n or min(n) < 1:
+            raise ValueError(f"{what}: the keys need one common length of at least one row, got "
+                             f"{ {k: meta[k][0] for k in row_shapes} }")
+        length = n.pop()
+        for k, row in row_shapes.items():
+            shape, dtype = meta[k]
+            if tuple(shape[1:]) != tuple(row):
+                raise ValueError(f"{what}: '{k}' rows have shape {tuple(shape[1:])}, the store's are {tuple(row)}")
+            if k == "lidar_occupancy" and dtype != np.uint8:
+                raise ValueError(f"{what}: 'lidar_occupancy' is {dtype}, expected uint8")
+            if k != "lidar_occupancy" and dtype not in _FLOAT_DTYPES:
+                raise ValueError(f"{what}: '{k}' is {dtype}, expected float16, float32 or float64")
+        if length > capacity_rows:
+            raise ValueError(f"{what}: {length} rows exceed import_capacity_rows = {capacity_rows}")
+        lengths.append(int(length))
+    return lengths
+
+
+def imported_held(lengths: Sequence[int], capacity_rows: int) -> np.ndarray:
+    """Which of the episodes imported in this order, with these lengths, an import arena of `capacity_rows` rows holds:
+    those whose first row has not been overwritten by the rows imported after it."""
+    lengths = np.asarray(lengths, np.int64)
+    first = np.cumsum(lengths) - lengths
+    return first >= lengths.sum() - int(capacity_rows)
+
+
 # keys of the dict DeviceEpisodeStore.step / reset return: those of HostSteppedEnv (what EpisodeRecorder.step returns)
 _ENV_OUT_KEYS = ("lidar", "occupancy", "pose", "velocity", "speed", "reward", "done", "progress", "lap", "time", "flags",
                  "rank", "opponents", "wrong_way", "wall_collision")
@@ -249,10 +328,21 @@ class DeviceEpisodeStore:
     The committed episodes are, bit for bit, those ``EpisodeRecorder`` over ``HostSteppedEnv`` hands to its callbacks for
     the same config, seed and actions, in the same order (``episodes()``).  Each env keeps a ring of ``capacity_rows``
     rows (memory: n_envs x capacity_rows x row bytes); an env's oldest episodes are evicted as its ring wraps.
-    ``capacity_rows`` must exceed ``max_episode_steps(env.cfg)``.  ``seed`` keys the sampler's Philox stream."""
+    ``capacity_rows`` must exceed ``max_episode_steps(env.cfg)``.  ``seed`` keys the sampler's Philox stream.
+
+    ``import_capacity_rows > 0`` adds an import arena of that many rows (same row format and precision), which
+    ``insert`` / ``load`` fill with episodes from outside the store -- saved files of this or another run, the
+    reference's own episodes -- so that a resumed learner samples what it saved.  Imported episode k gets id
+    ``IMPORTED_ID0 + k`` and is held while its first row has not been overwritten; importing past the arena's end evicts
+    the oldest imported episodes.  Draws pick from the held imported episodes in import order, then the held recorded
+    ones in commit order.  Imports never touch the recording: ``reset()`` keeps imported episodes, and ``episodes()``,
+    ``held()`` and ``save()`` leave them out unless asked with ``imported=True``."""
+
+    IMPORTED_ID0 = 1 << 62
+    _IMPORT_CHUNK_BYTES = 64 << 20    # staged bytes per device import (two such buffers, pinned and on the device)
 
     def __init__(self, env, capacity_rows: int, precision: int = 32, keep_obs: Sequence[str] = OBS_KEYS,
-                 reset_mode: Optional[str] = None, seed: int = 0):
+                 reset_mode: Optional[str] = None, seed: int = 0, import_capacity_rows: int = 0):
         import ctypes as C
         from . import _abi
         self._C, self._abi = C, _abi
@@ -279,8 +369,14 @@ class DeviceEpisodeStore:
         self._spec = {"lidar": ((env.n_beams,), fdt), "pose": ((6,), fdt), "velocity": ((6,), fdt), "speed": ((), fdt),
                       "lidar_occupancy": ((64, 64, 1), torch.uint8), "action": ((2,), fdt), "reward": ((), fdt),
                       "discount": ((), fdt), "progress": ((), fdt), "time": ((), fdt)}
+        self.import_capacity_rows = int(import_capacity_rows)
+        if self.import_capacity_rows < 0:
+            raise ValueError("import_capacity_rows must be >= 0")
+        self._stage = None
         with torch.cuda.device(env.device):
             env._check(env.lib.rd_store_init(env._handle, C.byref(sc)))
+            if self.import_capacity_rows:
+                env._check(env.lib.rd_store_import_init(env._handle, self.import_capacity_rows))
 
     # -- recording --
     def _outputs(self):
@@ -313,8 +409,9 @@ class DeviceEpisodeStore:
     def sample(self, batch: Optional[int] = None, length: Optional[int] = None, balance: bool = False,
                indices=None, check: bool = False) -> Dict[str, "torch.Tensor"]:
         """``batch`` chunks of ``length`` rows as CUDA tensors ``[B, L, ...]`` per key, plus ``episode_id`` i64 [B] and
-        ``start`` i32 [B].  Drawn uniformly over the held episodes of at least ``length + 1`` rows, in commit order, with
-        the start law of ``load_episodes`` (``balance``); or ``indices=(episode_id, start)`` names the chunks.  Entries
+        ``start`` i32 [B].  Drawn uniformly over the held episodes of at least ``length + 1`` rows -- imported ones in
+        import order, then recorded ones in commit order -- with the start law of ``load_episodes`` (``balance``); or
+        ``indices=(episode_id, start)`` names the chunks (recorded or imported ids).  Entries
         with no chunk (nothing eligible, or an index that names no held chunk) are zero rows with id and start -1;
         invalid indices are counted (``info()['invalid_requests']``) and ``check=True`` raises on them.  Asynchronous
         unless ``check``."""
@@ -360,27 +457,39 @@ class DeviceEpisodeStore:
     # -- bookkeeping / export --
     def info(self) -> Dict[str, int]:
         """Synchronising: committed, held, held_rows, evicted, invalid_requests, draws, capacity_rows,
-        max_episode_steps."""
+        max_episode_steps (recorded episodes), and imported, imported_held, imported_rows, imported_evicted,
+        import_capacity_rows (the import arena)."""
         env = self.env
         s = self._abi.RdStoreSummary()
+        si = self._abi.RdStoreImportSummary()
         with self._torch.cuda.device(env.device):
             env._check(env.lib.rd_store_info(env._handle, self._C.byref(s), None, 0, env._stream()))
-        return s.as_dict()
+            env._check(env.lib.rd_store_import_info(env._handle, self._C.byref(si), None, 0, env._stream()))
+        out = s.as_dict()
+        i = si.as_dict()
+        out.update(imported=i["imported"], imported_held=i["held"], imported_rows=i["held_rows"],
+                   imported_evicted=i["evicted"], import_capacity_rows=i["capacity_rows"])
+        return out
 
-    def held(self) -> np.ndarray:
-        """(id, env, length) of the held episodes in commit order, int64 [held, 3]."""
-        env, C = self.env, self._C
-        n = self.info()["held"]
-        arr = (self._abi.RdStoreEpisode * max(n, 1))()
-        s = self._abi.RdStoreSummary()
+    def held(self, imported: bool = False) -> np.ndarray:
+        """(id, env, length) of the held episodes in commit order, int64 [held, 3]; ``imported=True``: of the held
+        imported episodes in import order (env -1)."""
+        env, C, abi = self.env, self._C, self._abi
+        fn, summary = ((env.lib.rd_store_import_info, abi.RdStoreImportSummary) if imported else
+                       (env.lib.rd_store_info, abi.RdStoreSummary))
+        n = self.info()["imported_held" if imported else "held"]
+        arr = (abi.RdStoreEpisode * max(n, 1))()
+        s = summary()
         with self._torch.cuda.device(env.device):
-            env._check(env.lib.rd_store_info(env._handle, C.byref(s), arr, n, env._stream()))
+            env._check(fn(env._handle, C.byref(s), arr, n, env._stream()))
         return np.array([(e.id, e.env, e.length) for e in arr[:min(n, int(s.held))]], np.int64).reshape(-1, 3)
 
-    def episodes(self, since_id: Optional[int] = None, max_rows_per_gather: int = 1 << 18) -> List[Dict[str, np.ndarray]]:
+    def episodes(self, since_id: Optional[int] = None, max_rows_per_gather: int = 1 << 18,
+                 imported: bool = False) -> List[Dict[str, np.ndarray]]:
         """Host dicts of the held episodes (id >= since_id) in commit order, the format ``EpisodeRecorder`` hands to its
-        callbacks.  Gathered on the device, episodes of one length at a time."""
-        h = self.held()
+        callbacks; ``imported=True``: of the held imported episodes in import order.  Gathered on the device, episodes
+        of one length at a time."""
+        h = self.held(imported)
         if since_id is not None:
             h = h[h[:, 0] >= int(since_id)]
         out: List[Optional[Dict[str, np.ndarray]]] = [None] * len(h)
@@ -396,5 +505,143 @@ class DeviceEpisodeStore:
         return out
 
     def save(self, directory, since_id: Optional[int] = None) -> List[pathlib.Path]:
-        """``save_episodes`` of ``episodes(since_id)``: files ``load_episodes`` / ``count_episodes`` read."""
+        """``save_episodes`` of ``episodes(since_id)``: files ``load_episodes`` / ``count_episodes`` read.  Imported
+        episodes are not written again (after a resume they are on disk already)."""
         return save_episodes(directory, self.episodes(since_id))
+
+    # -- import --
+    def _row_shapes(self) -> Dict[str, tuple]:
+        return {k: self._spec[k][0] for k in self.keys}
+
+    def insert(self, episodes: Sequence[Dict[str, np.ndarray]]) -> np.ndarray:
+        """Imports episode dicts -- those ``EpisodeRecorder`` hands to its callbacks, ``episodes()`` returns or
+        ``dict(np.load(file))`` reads -- into the import arena; returns their ids (int64, in order).
+
+        Every kept key must be present (others are ignored), all with one length of 1 to ``import_capacity_rows`` rows,
+        the store's row shapes, float16/32/64 floats and uint8 ``lidar_occupancy``.  All episodes are checked before any
+        device work, so a call that raises ``ValueError`` imports nothing.  Rows are converted on the device to the
+        store's precision exactly as ``_convert`` does (numpy ``astype``).  Whether the observations were normalised as
+        the env's are (``normalize_lidar``, the baselines' normalisation) cannot be told from the data and is not
+        checked.  Asynchronous: the arrays are copied before it returns."""
+        episodes = list(episodes)
+        metas = [{k: (np.shape(v), np.asarray(v).dtype) for k, v in ep.items() if k in self.keys} for ep in episodes]
+        lengths = self._check_import(metas)
+        return self._import(lengths, [lambda ep=ep: ep for ep in episodes])
+
+    def load(self, directory, shard: Optional[Tuple[int, int]] = None, workers: Optional[int] = None) -> np.ndarray:
+        """Imports the ``*.npz`` episodes of `directory` in sorted file order (``load_episodes``' order), as ``insert``
+        does; ``shard=(rank, world)`` takes the files whose index in that order is ``rank`` modulo ``world``.  A file
+        that cannot be read is skipped with a message, as ``load_episodes`` does.  The files' headers are checked
+        before any device work; their data is decompressed on `workers` threads, overlapped with the copies to the
+        device, and files the arena would not hold at the end of the call are not decompressed.  Returns the ids."""
+        paths, metas = [], []
+        for path in episode_files(directory, shard):
+            try:
+                metas.append(npz_meta(path, self.keys))
+            except Exception as e:  # noqa: BLE001 - a half-written file must not stop training (reference behaviour)
+                print(f"Could not load episode: {e}")
+                continue
+            paths.append(path)
+        lengths = self._check_import(metas, [str(p) for p in paths])
+        keys = self.keys
+
+        def read(path):
+            try:
+                with np.load(path) as z:
+                    return {k: z[k] for k in keys}
+            except Exception as e:  # noqa: BLE001
+                print(f"Could not load episode: {e}")
+                return None
+        workers = int(workers or min(8, os.cpu_count() or 1))
+        with ThreadPoolExecutor(max_workers=workers) as pool:
+            return self._import(lengths, [lambda p=p: read(p) for p in paths], pool, 2 * workers)
+
+    def _check_import(self, metas, names=None) -> List[int]:
+        if self.import_capacity_rows == 0:
+            raise ValueError("this store has no import arena: create it with import_capacity_rows > 0")
+        return check_import(metas, self._row_shapes(), self.import_capacity_rows, names)
+
+    def _import(self, lengths: List[int], readers, pool=None, ahead: int = 1) -> np.ndarray:
+        """Registers the episodes the arena will not hold after the call without their data, then stages the others in
+        chunks of up to _IMPORT_CHUNK_BYTES (one element type per key and chunk) through two pinned buffers, each
+        chunk's copy and k_store_import enqueued on the current stream.  readers[i]() -> the dict of episode i, or None
+        (skipped).  With a pool, up to `ahead` readers run ahead of the staging."""
+        torch, env, C = self._torch, self.env, self._C
+        n_before = self.info()["imported"]
+        keep = imported_held(lengths, self.import_capacity_rows) if lengths else np.zeros(0, bool)
+        n_drop = int(np.argmax(keep)) if keep.any() else len(lengths)
+        registered = []                              # indices of the episodes imported, in order
+        with torch.cuda.device(env.device):
+            if n_drop:
+                lens = (C.c_int32 * n_drop)(*lengths[:n_drop])
+                env._check(env.lib.rd_store_import(env._handle, n_drop, lens, None, env._stream()))
+                registered.extend(range(n_drop))
+            todo = list(range(n_drop, len(lengths)))
+            if pool is None:
+                results = ((i, readers[i]()) for i in todo)
+            else:
+                def results():
+                    futs = {}
+                    for j, i in enumerate(todo):
+                        for i2 in todo[j:j + ahead]:
+                            if i2 not in futs:
+                                futs[i2] = pool.submit(readers[i2])
+                        yield i, futs.pop(i).result()
+                results = results()
+            chunk, chunk_bytes, chunk_types = [], 0, None
+            for i, ep in results:
+                if ep is None:
+                    continue
+                arrs = {k: np.ascontiguousarray(ep[k]) for k in self.keys}
+                types = tuple(arrs[k].dtype for k in self.keys)
+                nbytes = sum(a.nbytes + 16 for a in arrs.values())
+                if chunk and (types != chunk_types or chunk_bytes + nbytes > self._IMPORT_CHUNK_BYTES):
+                    self._stage_chunk(chunk)
+                    chunk, chunk_bytes = [], 0
+                chunk.append(arrs)
+                chunk_bytes += nbytes
+                chunk_types = types
+                registered.append(i)
+            if chunk:
+                self._stage_chunk(chunk)
+        return self.IMPORTED_ID0 + n_before + np.arange(len(registered), dtype=np.int64)
+
+    def _stage_chunk(self, chunk: List[Dict[str, np.ndarray]]) -> None:
+        torch, env, C, abi = self._torch, self.env, self._C, self._abi
+        offs, total = {}, 0
+        for k in self.keys:
+            offs[k] = total
+            total += -(-sum(ep[k].nbytes for ep in chunk) // 16) * 16
+        if self._stage is None or self._stage["host"][0].numel() < total:
+            for ev in (self._stage or {}).get("done", ()):
+                if ev is not None:
+                    ev.synchronize()
+            size = max(total, self._IMPORT_CHUNK_BYTES)
+            self._stage = {"host": [torch.empty(size, dtype=torch.uint8, pin_memory=True) for _ in range(2)],
+                           "dev": [torch.empty(size, dtype=torch.uint8, device=env.device) for _ in range(2)],
+                           "done": [None, None], "next": 0}
+        st = self._stage
+        b = st["next"]
+        st["next"] ^= 1
+        if st["done"][b] is not None:
+            st["done"][b].synchronize()              # the previous copy out of this pinned buffer has run
+        host, dev = st["host"][b], st["dev"][b]
+        hnp = host.numpy()
+        for k in self.keys:
+            o = offs[k]
+            for ep in chunk:
+                a = ep[k]
+                hnp[o:o + a.nbytes] = a.reshape(-1).view(np.uint8)
+                o += a.nbytes
+        dev[:total].copy_(host[:total], non_blocking=True)
+        ev = torch.cuda.Event()
+        ev.record()
+        st["done"][b] = ev
+        rows = abi.RdStoreImportRows()
+        field = {"lidar_occupancy": "occupancy"}
+        for k in self.keys:
+            f = field.get(k, k)
+            setattr(rows, f + "_dev", dev.data_ptr() + offs[k])
+            setattr(rows, f + "_type", chunk[0][k].dtype.itemsize)
+        lens = (C.c_int32 * len(chunk))(*[len(ep["reward"]) for ep in chunk])
+        env._check(env.lib.rd_store_import(env._handle, len(chunk), lens, C.byref(rows), env._stream()))
