@@ -323,6 +323,38 @@ int rd_policy_dreamer_set_state(rd_env* env, const float* stoch_dev, const float
 /* n_steps x (agent step -> rd_step) enqueued on `stream` with no host synchronisation (see rd_rollout_gap_follower). */
 int rd_rollout_dreamer(rd_env* env, int n_steps, const rd_outputs* out, float* actions_dev, int noise, void* stream);
 
+/* Training mode: Dreamer.policy(obs, state, training=True) [REF dreamer/dreamer.py, Dreamer.policy, _exploration].
+ * The head takes ONE sample of the actor distribution, a = tanh(mean + sd e1), and explores:
+ * a' = clip(a + amount_k e2, -1, 1) in float32, one rounding per operation.  a' is written to actions_dev and kept in
+ * the latent state as the previous action.  amount_k = expl amount * 0.5^(env_steps / decay) (decay > 0), at least
+ * min_amount (min_amount > 0), computed in float64 and rounded once to float32; env_steps then advances by
+ * n_envs * action_repeat (evaluation steps leave it).  noise: RD_NOISE_PHILOX draws (e1, e2) from one Philox block,
+ * counter (env id, agent step, 0, tag), key (seed_lo, seed_hi ^ tag), apart from the evaluation-mode and posterior
+ * streams; RD_NOISE_ZERO: e1 = e2 = 0; RD_NOISE_EXPLICIT reads eps_stoch_dev f32 [N,30], eps_sample_dev f32 [N,2] (e1)
+ * and eps_expl_dev f32 [N,2] (e2).  debug_dev as rd_policy_dreamer's; its action is a (before exploration), its
+ * log_prob that of a, its index 0. */
+typedef struct rd_dreamer_exploration {
+  double amount;              /* expl_amount: 0.3 */
+  double decay;               /* expl_decay: 0 = constant amount */
+  double min_amount;          /* expl_min: 0 = no floor */
+  int64_t env_steps;          /* the schedule's env-step counter */
+} rd_dreamer_exploration;
+/* rd_policy_dreamer_init sets env_steps to 0 and leaves the rest (0.3, 0, 0 until set). */
+int rd_policy_dreamer_set_exploration(rd_env* env, const rd_dreamer_exploration* x);
+int rd_policy_dreamer_get_exploration(rd_env* env, rd_dreamer_exploration* x);
+int rd_policy_dreamer_train(rd_env* env, const float* lidar_dev, float* actions_dev, int noise, const float* eps_stoch_dev,
+                            const float* eps_sample_dev, const float* eps_expl_dev, float* debug_dev, void* stream);
+/* n_steps x (training agent step -> rd_step) enqueued on `stream`, no host synchronisation. */
+int rd_rollout_dreamer_train(rd_env* env, int n_steps, const rd_outputs* out, float* actions_dev, int noise, void* stream);
+/* New weights for an initialised agent, packed on the device on `stream` into the buffers rd_policy_dreamer_init
+ * allocated, bit for bit as init packs them.  w: the layout rd_policy_dreamer_init takes, its array pointers DEVICE
+ * memory of the env's device (on_device = 1, e.g. a learner's tensors) or host memory (on_device = 0: copied with
+ * cudaMemcpyAsync on `stream` through a staging buffer the handle owns).  No allocation; the latent state, the Philox
+ * step counter and the exploration state are kept.  Steps enqueued on `stream` before the call use the old weights,
+ * the ones after it the new ones.  The architecture, BN presence, precision and head scalars must equal the init's
+ * (else RD_ERR_INVALID and nothing changes). */
+int rd_policy_dreamer_set_weights(rd_env* env, const rd_dreamer_weights* w, int on_device, void* stream);
+
 /* ---- device-resident episode store (SURVEY.md §8-f1): records the Collect rows of every env's episodes on the device
  *      [REF dreamer/wrappers.py:198-250], exactly the episodes episodes.EpisodeRecorder hands to its callbacks, and
  *      samples fixed-length chunks the way tools.load_episodes does [REF dreamer/tools.py:235-264].  The env must have
@@ -332,7 +364,8 @@ int rd_rollout_dreamer(rd_env* env, int n_steps, const rd_outputs* out, float* a
  *      allows (time_limit_steps, time_limit_ticks / action_repeat, the task's time_limit / (dt * action_repeat)). ---- */
 enum { RD_STORE_LIDAR = 1, RD_STORE_POSE = 2, RD_STORE_VELOCITY = 4, RD_STORE_SPEED = 8,
        RD_STORE_OCCUPANCY = 16 /* 'lidar_occupancy', u8 [64,64,1]; needs RD_OBS_OCCUPANCY */ };   /* keep_obs bits */
-enum { RD_STORE_POLICY_GAP_FOLLOWER = 0, RD_STORE_POLICY_DREAMER = 1 };                         /* rd_rollout_store */
+enum { RD_STORE_POLICY_GAP_FOLLOWER = 0, RD_STORE_POLICY_DREAMER = 1,
+       RD_STORE_POLICY_DREAMER_TRAIN = 2 /* rd_rollout_dreamer_train's agent step */ };          /* rd_rollout_store */
 typedef struct rd_store_config {
   int32_t capacity_rows;      /* rows per env */
   int32_t precision;          /* 32 | 16: float keys as float32 | IEEE half [REF dreamer/wrappers.py:240-250 _convert] */

@@ -115,6 +115,11 @@ class RdDreamerWeights(C.Structure):
         ("n_samples", C.c_int32), ("precision", C.c_int32)]
 
 
+class RdDreamerExploration(C.Structure):
+    """rd_dreamer_exploration: the training-mode exploration schedule and its env-step counter."""
+    _fields_ = [("amount", C.c_double), ("decay", C.c_double), ("min_amount", C.c_double), ("env_steps", C.c_int64)]
+
+
 class RdStoreConfig(C.Structure):
     """rd_store_config (include/rd_env.h): the device-resident episode store."""
     _fields_ = [("capacity_rows", C.c_int32), ("precision", C.c_int32), ("keep_obs", C.c_int32), ("reset_mode", C.c_int32),
@@ -158,7 +163,7 @@ STORE_U8, STORE_F16, STORE_F32, STORE_F64 = 1, 2, 4, 8
 STORE_LIDAR, STORE_POSE, STORE_VELOCITY, STORE_SPEED, STORE_OCCUPANCY = 1, 2, 4, 8, 16
 STORE_KEYS = {"lidar": STORE_LIDAR, "pose": STORE_POSE, "velocity": STORE_VELOCITY, "speed": STORE_SPEED,
               "lidar_occupancy": STORE_OCCUPANCY}
-STORE_POLICY_GAP_FOLLOWER, STORE_POLICY_DREAMER = 0, 1
+STORE_POLICY_GAP_FOLLOWER, STORE_POLICY_DREAMER, STORE_POLICY_DREAMER_TRAIN = 0, 1, 2
 
 RD_NOISE_ZERO, RD_NOISE_PHILOX, RD_NOISE_EXPLICIT = 0, 1, 2
 RD_DREAMER_DEBUG_FLOATS = 68
@@ -171,7 +176,8 @@ EXPORTS = (
     "rd_host_init", "rd_reset_host", "rd_step_host", "rd_step_host_begin", "rd_step_host_end",
     "rd_gap_follower_defaults", "rd_policy_gap_follower_init", "rd_policy_gap_follower", "rd_rollout_gap_follower",
     "rd_policy_dreamer_init", "rd_policy_dreamer", "rd_policy_dreamer_get_state", "rd_policy_dreamer_set_state",
-    "rd_rollout_dreamer",
+    "rd_rollout_dreamer", "rd_policy_dreamer_set_exploration", "rd_policy_dreamer_get_exploration",
+    "rd_policy_dreamer_train", "rd_rollout_dreamer_train", "rd_policy_dreamer_set_weights",
     "rd_store_init", "rd_store_reset", "rd_store_step", "rd_rollout_store", "rd_store_sample", "rd_store_info",
     "rd_store_import_init", "rd_store_import", "rd_store_import_info",
 )
@@ -266,6 +272,16 @@ def load_library() -> C.CDLL:
     lib.rd_policy_dreamer_set_state.restype = i32
     lib.rd_rollout_dreamer.argtypes = [vp, i32, C.POINTER(RdOutputs), vp, i32, vp]
     lib.rd_rollout_dreamer.restype = i32
+    lib.rd_policy_dreamer_set_exploration.argtypes = [vp, C.POINTER(RdDreamerExploration)]
+    lib.rd_policy_dreamer_set_exploration.restype = i32
+    lib.rd_policy_dreamer_get_exploration.argtypes = [vp, C.POINTER(RdDreamerExploration)]
+    lib.rd_policy_dreamer_get_exploration.restype = i32
+    lib.rd_policy_dreamer_train.argtypes = [vp, vp, vp, i32, vp, vp, vp, vp, vp]
+    lib.rd_policy_dreamer_train.restype = i32
+    lib.rd_rollout_dreamer_train.argtypes = [vp, i32, C.POINTER(RdOutputs), vp, i32, vp]
+    lib.rd_rollout_dreamer_train.restype = i32
+    lib.rd_policy_dreamer_set_weights.argtypes = [vp, C.POINTER(RdDreamerWeights), i32, vp]
+    lib.rd_policy_dreamer_set_weights.restype = i32
     lib.rd_store_init.argtypes = [vp, C.POINTER(RdStoreConfig)]
     lib.rd_store_init.restype = i32
     lib.rd_store_reset.argtypes = [vp, C.POINTER(RdOutputs), vp]

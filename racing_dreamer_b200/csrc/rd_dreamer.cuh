@@ -64,6 +64,11 @@ struct DreamerPolicy {
   int sm_count = 148;
   int cur = 0;           // feat[cur] holds the latest latent
   uint32_t step = 0;     // agent steps taken (Philox counter)
+  // training-mode exploration [REF dreamer/dreamer.py, Dreamer._exploration]: amount * 0.5^(env_steps / decay) (decay > 0),
+  // at least min_amount (min_amount > 0); env_steps = Dreamer's step counter, + n_envs * action_repeat per training step
+  double expl_amount = 0.3, expl_decay = 0.0, expl_min = 0.0;
+  int64_t env_steps = 0;
+  float* stage = nullptr;      // device copy of host-pointer weights for dreamer_set_weights (sized at init)
   std::string err;
 };
 
@@ -79,8 +84,43 @@ static inline void dreamer_free(DreamerPolicy& d) {
   for (float* p : d.owned) cudaFree(p);
   d.owned.clear();
   d.bn = nullptr;
+  d.stage = nullptr;
   d.ready = false;
 }
+
+// The policy's weight layout: each checkpoint array, where it goes and how.  Matrices ([in][out] Keras kernels) become
+// K-major TF32 operands (dr_upload_t: pitch ld, the K slots from k_from on shifted by k_shift); vectors (op == null)
+// are copied as they are to *vec.  Both dreamer_init and dreamer_set_weights walk this one list.
+struct DrPart { const float* src; DreamerPolicy::Operand* op; float** vec; int in, out, ld, k_from, k_shift; };
+static inline int dr_parts(DreamerPolicy& d, const rd_dreamer_weights* w, DrPart* p) {
+  const int H = d.hidden, D = d.deter, E = d.embed, U = d.units, L = d.layers, NO = 1 << 30;
+  int k = 0;
+  auto mat = [&](const float* src, DreamerPolicy::Operand& op, int in, int out, int ld, int k_from, int k_shift) {
+    p[k++] = DrPart{src, &op, nullptr, in, out, ld, k_from, k_shift};
+  };
+  auto vec = [&](const float* src, float*& dst, int count) { p[k++] = DrPart{src, nullptr, &dst, 1, count, 0, NO, 0}; };
+  mat(w->img1_w, d.w_img1, GM_STOCH + 2, H, 32, NO, 0);
+  vec(w->img1_b, d.b_img1, H);
+  mat(w->gru_kernel, d.w_gruk, H, 3 * D, H, NO, 0);
+  mat(w->gru_recurrent, d.w_grur, D, 3 * D, D, NO, 0);
+  vec(w->gru_bias, d.b_gru, 6 * D);
+  mat(w->obs1_w, d.w_obs1, D + E, H, D + E, NO, 0);
+  vec(w->obs1_b, d.b_obs1, H);
+  mat(w->obs2_w, d.w_obs2, H, 2 * GM_STOCH, H, NO, 0);
+  vec(w->obs2_b, d.b_obs2, 2 * GM_STOCH);
+  // actor h0: rows [stoch | deter] -> K slots [0, 30) and [32, 32 + deter); the two action slots get zero weights
+  mat(w->actor_w[0], d.w_act[0], GM_STOCH + D, U, d.ldf, GM_STOCH, 2);
+  vec(w->actor_b[0], d.b_act[0], U);
+  for (int i = 1; i < L; ++i) {
+    mat(w->actor_w[i], d.w_act[i], U, U, U, NO, 0);
+    vec(w->actor_b[i], d.b_act[i], U);
+  }
+  mat(w->actor_w[L], d.w_act[L], U, 4, U, NO, 0);
+  vec(w->actor_b[L], d.b_act[L], 4);
+  if (w->bn) vec(w->bn, d.bn, 16);
+  return k;
+}
+#define DR_MAX_PARTS (9 + 2 * 8 + 1)
 
 // [in][out] host matrix -> device [out][ld] (K-major), element (o, kmap(i)) = scale_i * W[i][o], split into its TF32
 // rounding (op.p[0]) and, in x3 mode, the TF32 rounding of the remainder (op.p[1])
@@ -166,26 +206,17 @@ static inline int dreamer_init(DreamerPolicy& d, int n, int n_beams, bool lidar_
   d.raw_init_std = (float)std::log(std::exp((double)w->init_std) - 1.0);   // [REF models.py:321]
   d.min_std = w->min_std; d.mean_scale = w->mean_scale; d.bn_eps = w->bn_eps; d.n_samples = w->n_samples;
   const int H = d.hidden, D = d.deter, E = d.embed, U = d.units;
-  const int NO = 1 << 30;
-  DR_TRY(dr_upload_t(d, d.w_img1, w->img1_w, GM_STOCH + 2, H, 32, NO, 0));
-  DR_TRY(dr_upload(d, &d.b_img1, w->img1_b, H));
-  DR_TRY(dr_upload_t(d, d.w_gruk, w->gru_kernel, H, 3 * D, H, NO, 0));
-  DR_TRY(dr_upload_t(d, d.w_grur, w->gru_recurrent, D, 3 * D, D, NO, 0));
-  DR_TRY(dr_upload(d, &d.b_gru, w->gru_bias, (size_t)6 * D));
-  DR_TRY(dr_upload_t(d, d.w_obs1, w->obs1_w, D + E, H, D + E, NO, 0));
-  DR_TRY(dr_upload(d, &d.b_obs1, w->obs1_b, H));
-  DR_TRY(dr_upload_t(d, d.w_obs2, w->obs2_w, H, 2 * GM_STOCH, H, NO, 0));
-  DR_TRY(dr_upload(d, &d.b_obs2, w->obs2_b, 2 * GM_STOCH));
-  // actor h0: rows [stoch | deter] -> K slots [0, 30) and [32, 32 + deter); the two action slots get zero weights
-  DR_TRY(dr_upload_t(d, d.w_act[0], w->actor_w[0], GM_STOCH + D, U, d.ldf, GM_STOCH, 2));
-  DR_TRY(dr_upload(d, &d.b_act[0], w->actor_b[0], U));
-  for (int i = 1; i < d.layers; ++i) {
-    DR_TRY(dr_upload_t(d, d.w_act[i], w->actor_w[i], U, U, U, NO, 0));
-    DR_TRY(dr_upload(d, &d.b_act[i], w->actor_b[i], U));
+  DrPart parts[DR_MAX_PARTS];
+  const int n_parts = dr_parts(d, w, parts);
+  size_t stage_floats = 0;
+  for (int k = 0; k < n_parts; ++k) {
+    const DrPart& p = parts[k];
+    if (p.op) DR_TRY(dr_upload_t(d, *p.op, p.src, p.in, p.out, p.ld, p.k_from, p.k_shift));
+    else DR_TRY(dr_upload(d, p.vec, p.src, (size_t)p.out));
+    stage_floats += (size_t)p.in * p.out;
   }
-  DR_TRY(dr_upload_t(d, d.w_act[d.layers], w->actor_w[d.layers], U, 4, U, NO, 0));
-  DR_TRY(dr_upload(d, &d.b_act[d.layers], w->actor_b[d.layers], 4));
-  if (w->bn) DR_TRY(dr_upload(d, &d.bn, w->bn, 16));
+  DR_TRY(cudaMalloc(&d.stage, stage_floats * sizeof(float)));
+  d.owned.push_back(d.stage);
   const size_t N = (size_t)n;
   for (int p = 0; p < 2; ++p) {
     DR_TRY(dr_alloc(d, d.feat[p], N, d.ldf));
@@ -233,7 +264,69 @@ static inline int dreamer_init(DreamerPolicy& d, int n, int n_beams, bool lidar_
   DR_MAP(dr_view(d, d.w_act[d.layers], d.w_act[d.layers], 0, U, 4, U, GM_BN));
   d.cur = 0;
   d.step = 0;
+  d.env_steps = 0;
   d.ready = true;
+  return RD_OK;
+}
+
+// the exploration amount of the next training step, rounded once to float32
+static inline float dreamer_expl_amount(const DreamerPolicy& d) {
+  double a = d.expl_amount;
+  if (d.expl_decay > 0.0) a *= std::pow(0.5, (double)d.env_steps / d.expl_decay);
+  if (d.expl_min > 0.0) a = std::max(d.expl_min, a);
+  return (float)a;
+}
+
+// New values for every weight of an initialised policy, packed on the device on `s` into the buffers it already owns
+// (no allocation; the tensor maps stay valid) bit for bit as dreamer_init packs them.  Latent state, Philox step and
+// env_steps are kept.  w holds device pointers (on_device) or host pointers, which are first copied to d.stage.  The
+// architecture, precision and head scalars must be the init's; otherwise RD_ERR_INVALID and nothing changes.
+static inline int dreamer_set_weights(DreamerPolicy& d, const rd_dreamer_weights* w, bool on_device, cudaStream_t s) {
+  if (!w) { d.err = "null weights"; return RD_ERR_INVALID; }
+  const float raw_init_std = (float)std::log(std::exp((double)w->init_std) - 1.0);
+  if (w->stoch != GM_STOCH || w->deter != d.deter || w->hidden != d.hidden || w->embed != d.embed ||
+      w->actor_units != d.units || w->actor_layers != d.layers || (w->bn != nullptr) != (d.bn != nullptr) ||
+      (w->precision != RD_PRECISION_TF32X3 && w->precision != RD_PRECISION_TF32) ||
+      (w->precision == RD_PRECISION_TF32X3) != d.x3 || w->n_samples != d.n_samples || raw_init_std != d.raw_init_std ||
+      w->min_std != d.min_std || w->mean_scale != d.mean_scale || w->bn_eps != d.bn_eps) {
+    d.err = "the weights' architecture, precision or head scalars differ from the ones the policy was initialised with";
+    return RD_ERR_INVALID;
+  }
+  DrPart parts[DR_MAX_PARTS];
+  const int n_parts = dr_parts(d, w, parts);
+  int dev = 0;
+  DR_TRY(cudaGetDevice(&dev));
+  for (int k = 0; k < n_parts; ++k) {
+    if (!parts[k].src) { d.err = "null weight pointer"; return RD_ERR_INVALID; }
+    cudaPointerAttributes at{};
+    DR_TRY(cudaPointerGetAttributes(&at, parts[k].src));
+    const bool device_ptr = at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged;
+    if (on_device && (!device_ptr || at.device != dev)) { d.err = "on_device: a weight pointer is not memory of the policy's device"; return RD_ERR_INVALID; }
+    if (!on_device && at.type == cudaMemoryTypeDevice) { d.err = "a device pointer was passed with on_device = 0"; return RD_ERR_INVALID; }
+  }
+  PackArgs a{};
+  a.n_jobs = n_parts;
+  size_t off = 0;
+  for (int k = 0; k < n_parts; ++k) {
+    const DrPart& p = parts[k];
+    const size_t count = (size_t)p.in * p.out;
+    const float* src = p.src;
+    if (!on_device) {
+      DR_TRY(cudaMemcpyAsync(d.stage + off, p.src, count * sizeof(float), cudaMemcpyHostToDevice, s));
+      src = d.stage + off;
+    }
+    PackJob& J = a.job[k];
+    J.src = src;
+    J.hi = p.op ? p.op->p[0] : *p.vec;
+    J.lo = p.op ? p.op->p[1] : nullptr;
+    J.in = p.in; J.out = p.out; J.ld = p.ld; J.k_from = p.k_from; J.k_shift = p.k_shift; J.raw = p.op ? 0 : 1;
+    J.begin = (long long)off;
+    off += count;
+  }
+  a.total = (long long)off;
+  const unsigned grid = (unsigned)std::min<size_t>((off + 255) / 256, (size_t)d.sm_count * 8);
+  k_pack_weights<<<grid, 256, 0, s>>>(a);
+  DR_TRY(cudaGetLastError());
   return RD_OK;
 }
 
@@ -292,8 +385,12 @@ static inline void dr_build(const DreamerPolicy& d, GemmMaps& maps, GemmArgs& g,
 }
 
 // Enqueues one agent step for all envs on `s`; returns the number of kernels launched in *launched.
+// train: null = evaluation mode (SampleDist.mode(), eps_actor [N][n_samples][2]); else the training head k_actor_train
+// with exploration amount train->amount (eps_actor = the sample's draws [N][2], train->eps_expl the exploration's).
+struct DrTrain { const float* eps_expl; float amount; };
 static inline int dreamer_step(DreamerPolicy& d, const float* lidar, float* actions, int noise, const float* eps_stoch,
-                               const float* eps_actor, float* debug, uint64_t seed, uint32_t gid0, cudaStream_t s, int* launched) {
+                               const float* eps_actor, float* debug, uint64_t seed, uint32_t gid0, cudaStream_t s, int* launched,
+                               const DrTrain* train = nullptr) {
   *launched = 0;
   const int cur = d.cur, nxt = cur ^ 1;
   const int H = d.hidden, D = d.deter, U = d.units;
@@ -427,11 +524,18 @@ static inline int dreamer_step(DreamerPolicy& d, const float* lidar, float* acti
       cfg.blockDim = dim3(256);
       cfg.stream = s;
       cudaLaunchAttribute attrs[1];
-      attrs[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;   // griddepcontrol.wait in k_actor_mode
+      attrs[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;   // griddepcontrol.wait in k_actor_mode / k_actor_train
       attrs[0].val.programmaticStreamSerializationAllowed = 1;
       cfg.attrs = attrs;
       cfg.numAttrs = 1;
-      DR_TRY(cudaLaunchKernelEx(&cfg, k_actor_mode, g));
+      if (train) {
+        cfg.gridDim = dim3((unsigned)((d.n + 255) / 256));   // one thread per env
+        g.ld_eps = 2;
+        g.key1 = (uint32_t)(seed >> 32) ^ RD_STREAM_TRAIN;
+        DR_TRY(cudaLaunchKernelEx(&cfg, k_actor_train, g, train->eps_expl, train->amount));
+      } else {
+        DR_TRY(cudaLaunchKernelEx(&cfg, k_actor_mode, g));
+      }
     }
     ++*launched;
   }

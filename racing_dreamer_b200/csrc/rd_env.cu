@@ -1210,16 +1210,21 @@ RD_API int rd_policy_dreamer_init(rd_env* env, const rd_dreamer_weights* w) {
 }
 
 namespace {
+// training: Dreamer.policy(training=True) -- one sample + exploration (k_actor_train), and the env-step counter of the
+// exploration schedule advances by n_envs * action_repeat [REF dreamer/dreamer.py, Dreamer.__call__ self._step]
 int launch_dreamer(rd_env* env, const float* lidar_dev, float* actions_dev, int noise, const float* eps_stoch_dev,
-                   const float* eps_actor_dev, float* debug_dev, cudaStream_t s) {
+                   const float* eps_actor_dev, float* debug_dev, cudaStream_t s, bool training = false,
+                   const float* eps_expl_dev = nullptr) {
   int launched = 0, rc;
+  const DrTrain tr{eps_expl_dev, dreamer_expl_amount(env->dr)};
   {
     ScopedTiming tm(env, s, T_POLICY);
     rc = dreamer_step(env->dr, lidar_dev, actions_dev, noise, eps_stoch_dev, eps_actor_dev, debug_dev, env->cfg.seed,
-                      (uint32_t)env->cfg.env_id_offset, s, &launched);
+                      (uint32_t)env->cfg.env_id_offset, s, &launched, training ? &tr : nullptr);
   }
   env->launches += launched;
   if (rc) return fail(env, rc, "rd_policy_dreamer: %s", env->dr.err.c_str());
+  if (training) env->dr.env_steps += (int64_t)env->n * env->cfg.action_repeat;
   return RD_OK;
 }
 }  // namespace
@@ -1263,6 +1268,62 @@ RD_API int rd_rollout_dreamer(rd_env* env, int n_steps, const rd_outputs* out, f
     if (rc) return rc;
     if ((rc = rd_step(env, act, out, stream))) return rc;
   }
+  return RD_OK;
+}
+
+RD_API int rd_policy_dreamer_train(rd_env* env, const float* lidar_dev, float* actions_dev, int noise, const float* eps_stoch_dev,
+                                   const float* eps_sample_dev, const float* eps_expl_dev, float* debug_dev, void* stream) {
+  if (!env || !lidar_dev || !actions_dev) return fail(env, RD_ERR_INVALID, "null argument");
+  if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
+  if (noise < RD_NOISE_ZERO || noise > RD_NOISE_EXPLICIT) return fail(env, RD_ERR_INVALID, "bad noise mode %d", noise);
+  if (noise == RD_NOISE_EXPLICIT && (!eps_stoch_dev || !eps_sample_dev || !eps_expl_dev))
+    return fail(env, RD_ERR_INVALID, "RD_NOISE_EXPLICIT needs eps_stoch_dev, eps_sample_dev and eps_expl_dev");
+  return launch_dreamer(env, lidar_dev, actions_dev, noise, eps_stoch_dev, eps_sample_dev, debug_dev, (cudaStream_t)stream,
+                        true, eps_expl_dev);
+}
+
+RD_API int rd_rollout_dreamer_train(rd_env* env, int n_steps, const rd_outputs* out, float* actions_dev, int noise, void* stream) {
+  if (!env || !out || !out->lidar_dev || n_steps < 0) return fail(env, RD_ERR_INVALID, "bad argument (the rollout needs out->lidar_dev)");
+  if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
+  if (noise != RD_NOISE_ZERO && noise != RD_NOISE_PHILOX) return fail(env, RD_ERR_INVALID, "a rollout draws its own noise (RD_NOISE_ZERO or RD_NOISE_PHILOX)");
+  if (!env->was_reset) return fail(env, RD_ERR_STATE, "Must reset environment.");
+  float* act = actions_dev ? actions_dev : env->pol.d_actions;
+  for (int k = 0; k < n_steps; ++k) {
+    int rc = launch_dreamer(env, out->lidar_dev, act, noise, nullptr, nullptr, nullptr, (cudaStream_t)stream, true);
+    if (rc) return rc;
+    if ((rc = rd_step(env, act, out, stream))) return rc;
+  }
+  return RD_OK;
+}
+
+RD_API int rd_policy_dreamer_set_exploration(rd_env* env, const rd_dreamer_exploration* x) {
+  if (!env || !x) return fail(env, RD_ERR_INVALID, "null argument");
+  if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
+  if (!(x->amount >= 0.0) || !(x->decay >= 0.0) || !(x->min_amount >= 0.0) || x->env_steps < 0)
+    return fail(env, RD_ERR_INVALID, "exploration: amount, decay, min_amount and env_steps must be >= 0");
+  env->dr.expl_amount = x->amount;
+  env->dr.expl_decay = x->decay;
+  env->dr.expl_min = x->min_amount;
+  env->dr.env_steps = x->env_steps;
+  return RD_OK;
+}
+
+RD_API int rd_policy_dreamer_get_exploration(rd_env* env, rd_dreamer_exploration* x) {
+  if (!env || !x) return fail(env, RD_ERR_INVALID, "null argument");
+  if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
+  x->amount = env->dr.expl_amount;
+  x->decay = env->dr.expl_decay;
+  x->min_amount = env->dr.expl_min;
+  x->env_steps = env->dr.env_steps;
+  return RD_OK;
+}
+
+RD_API int rd_policy_dreamer_set_weights(rd_env* env, const rd_dreamer_weights* w, int on_device, void* stream) {
+  if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
+  if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
+  const int rc = dreamer_set_weights(env->dr, w, on_device != 0, (cudaStream_t)stream);
+  if (rc) return fail(env, rc, "rd_policy_dreamer_set_weights: %s", env->dr.err.c_str());
+  env->launches++;
   return RD_OK;
 }
 
@@ -1634,7 +1695,7 @@ RD_API int rd_rollout_store(rd_env* env, int policy, int n_steps, const rd_outpu
   if (!out->lidar_dev) return fail(env, RD_ERR_INVALID, "the rollout needs out->lidar_dev");
   if (policy == RD_STORE_POLICY_GAP_FOLLOWER) {
     if (!env->pol.ready) return fail(env, RD_ERR_STATE, "rd_policy_gap_follower_init has not been called");
-  } else if (policy == RD_STORE_POLICY_DREAMER) {
+  } else if (policy == RD_STORE_POLICY_DREAMER || policy == RD_STORE_POLICY_DREAMER_TRAIN) {
     if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
     if (noise != RD_NOISE_ZERO && noise != RD_NOISE_PHILOX) return fail(env, RD_ERR_INVALID, "a rollout draws its own noise (RD_NOISE_ZERO or RD_NOISE_PHILOX)");
   } else {
@@ -1644,7 +1705,8 @@ RD_API int rd_rollout_store(rd_env* env, int policy, int n_steps, const rd_outpu
   float* act = actions_dev ? actions_dev : env->pol.d_actions;
   for (int k = 0; k < n_steps; ++k) {
     rc = policy == RD_STORE_POLICY_GAP_FOLLOWER ? launch_gap_follower(env, out->lidar_dev, nullptr, act, nullptr, s)
-                                                : launch_dreamer(env, out->lidar_dev, act, noise, nullptr, nullptr, nullptr, s);
+                                                : launch_dreamer(env, out->lidar_dev, act, noise, nullptr, nullptr, nullptr, s,
+                                                                 policy == RD_STORE_POLICY_DREAMER_TRAIN);
     if (rc) return rc;
     if ((rc = store_step(env, act, out, s))) return rc;
   }

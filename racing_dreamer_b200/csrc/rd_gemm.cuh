@@ -69,6 +69,7 @@ enum { EPI_DENSE = 0, EPI_GRU = 1, EPI_STOCH = 2, EPI_ACTOR = 3 };
 enum { GM_NOISE_ZERO = 0, GM_NOISE_PHILOX = 1, GM_NOISE_EXPLICIT = 2 };
 #define RD_STREAM_STOCH 0x53544f43u
 #define RD_STREAM_ACTOR 0x41435452u
+#define RD_STREAM_TRAIN 0x5452414eu   // training head: the action sample and its exploration noise (k_actor_train)
 
 struct GemmArgs {
   int M, N;                 // rows (envs), valid output columns
@@ -667,7 +668,37 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
 #undef GM_TRD
 }
 
-// ActionDecoder distribution head [REF models.py:323-346] + SampleDist.mode() [REF ros_agent/helpers/tools.py:70-73]:
+// ActionDecoder distribution head [REF models.py:323-346]: mean and sd of the pre-tanh Normal from hout's
+// pre-activations g.out[row][0..3]
+__device__ __forceinline__ void gm_actor_dist(const GemmArgs& g, int row, float (&mean)[2], float (&sd)[2]) {
+  const float4 x4 = *reinterpret_cast<const float4*>(g.out + (size_t)row * 4);
+  float x[4] = {x4.x, x4.y, x4.z, x4.w};
+  if (g.bn) {   // 'normalized_tanhtransformed_normal': BatchNormalization in inference mode, linear mean
+#pragma unroll
+    for (int t = 0; t < 4; ++t)
+      x[t] = (x[t] - __ldg(g.bn + 8 + t)) * (__ldg(g.bn + t) * rsqrtf(__ldg(g.bn + 12 + t) + g.bn_eps)) + __ldg(g.bn + 4 + t);
+    mean[0] = x[0]; mean[1] = x[1];
+    sd[0] = gm_softplus(x[2]) + g.min_std; sd[1] = gm_softplus(x[3]) + g.min_std;
+  } else {      // 'tanh_normal'
+    mean[0] = g.mean_scale * tanhf(x[0] / g.mean_scale); mean[1] = g.mean_scale * tanhf(x[1] / g.mean_scale);
+    sd[0] = gm_softplus(x[2] + g.raw_init_std) + g.min_std; sd[1] = gm_softplus(x[3] + g.raw_init_std) + g.min_std;
+  }
+}
+// the chosen action -> g.actions[row] and the latent's action slots (TF32 hi [+ lo]), which the next img1 reads
+__device__ __forceinline__ void gm_actor_store(const GemmArgs& g, int row, float a0, float a1) {
+  g.actions[2 * (size_t)row] = a0;
+  g.actions[2 * (size_t)row + 1] = a1;
+  float* frow = g.feat + (size_t)row * g.ldf;
+  const float h0 = gm_round_tf32(a0), h1 = gm_round_tf32(a1);
+  frow[GM_STOCH] = h0;
+  frow[GM_STOCH + 1] = h1;
+  if (g.feat_lo) {
+    g.feat_lo[(size_t)row * g.ldf + GM_STOCH] = gm_round_tf32(a0 - h0);
+    g.feat_lo[(size_t)row * g.ldf + GM_STOCH + 1] = gm_round_tf32(a1 - h1);
+  }
+}
+
+// ActionDecoder distribution head + SampleDist.mode() [REF ros_agent/helpers/tools.py:70-73]:
 // one warp per env, lanes over pairs of draws (one Philox block = the four normals of two draws), warp arg-max.
 // `g.out` holds hout's pre-activations [M][4] (k_dense<EPI_ACTOR>); the other fields are the ACTOR ones of GemmArgs.
 __global__ void __launch_bounds__(256) k_actor_mode(const GemmArgs g) {
@@ -684,19 +715,8 @@ __global__ void __launch_bounds__(256) k_actor_mode(const GemmArgs g) {
         gm_normal4(g.gid0 + (uint32_t)row, g.step, (uint32_t)(2 * lane + 64 * it), RD_STREAM_ACTOR, g.key0, g.key1, zp[it]);
   }
   asm volatile("griddepcontrol.wait;" ::: "memory");
-  const float4 x4 = *reinterpret_cast<const float4*>(g.out + (size_t)row * 4);
-  float x[4] = {x4.x, x4.y, x4.z, x4.w};
   float mean[2], sd[2];
-  if (g.bn) {   // 'normalized_tanhtransformed_normal': BatchNormalization in inference mode, linear mean
-#pragma unroll
-    for (int t = 0; t < 4; ++t)
-      x[t] = (x[t] - __ldg(g.bn + 8 + t)) * (__ldg(g.bn + t) * rsqrtf(__ldg(g.bn + 12 + t) + g.bn_eps)) + __ldg(g.bn + 4 + t);
-    mean[0] = x[0]; mean[1] = x[1];
-    sd[0] = gm_softplus(x[2]) + g.min_std; sd[1] = gm_softplus(x[3]) + g.min_std;
-  } else {      // 'tanh_normal'
-    mean[0] = g.mean_scale * tanhf(x[0] / g.mean_scale); mean[1] = g.mean_scale * tanhf(x[1] / g.mean_scale);
-    sd[0] = gm_softplus(x[2] + g.raw_init_std) + g.min_std; sd[1] = gm_softplus(x[3] + g.raw_init_std) + g.min_std;
-  }
+  gm_actor_dist(g, row, mean, sd);
   // mode(): argmax over n_samples draws of log_prob(tanh(u)), u ~ N(mean, sd): the Normal's log density minus the tanh
   // bijector's forward log-det-Jacobian 2 (log 2 - u - softplus(-2u)), summed over the two actions
   const float log2f_ = 0.69314718f, half_log_2pi = 0.91893853f;
@@ -749,20 +769,76 @@ __global__ void __launch_bounds__(256) k_actor_mode(const GemmArgs g) {
   }
   if (lane == 0) {
     const float a0 = tanhf(bu0), a1 = tanhf(bu1);
-    g.actions[2 * (size_t)row] = a0;
-    g.actions[2 * (size_t)row + 1] = a1;
-    float* frow = g.feat + (size_t)row * g.ldf;
-    const float h0 = gm_round_tf32(a0), h1 = gm_round_tf32(a1);
-    frow[GM_STOCH] = h0;
-    frow[GM_STOCH + 1] = h1;
-    if (g.feat_lo) {
-      g.feat_lo[(size_t)row * g.ldf + GM_STOCH] = gm_round_tf32(a0 - h0);
-      g.feat_lo[(size_t)row * g.ldf + GM_STOCH + 1] = gm_round_tf32(a1 - h1);
-    }
+    gm_actor_store(g, row, a0, a1);
     if (g.dbg) {
       float* d = g.dbg + (size_t)row * 8;
       d[0] = mean[0]; d[1] = mean[1]; d[2] = sd[0]; d[3] = sd[1]; d[4] = a0; d[5] = a1; d[6] = best; d[7] = (float)bi;
     }
+  }
+}
+
+// Dreamer.policy(training=True)'s head [REF dreamer/dreamer.py, Dreamer.policy and _exploration]: ONE draw of the
+// ActionDecoder distribution, a = tanh(mean + sd e1) (`actor(feat).sample()`), then the additive Gaussian exploration
+// a' = clip(a + amount e2, -1, 1), rounded once per operation so that a' is reproducible bit for bit from a.  a' is the
+// executed action and the one the latent keeps for the next obs_step.  One thread per env; noise: Philox block
+// (env id, step, 0, RD_STREAM_TRAIN) -> e1 = z0..1, e2 = z2..3, zero (a = tanh(mean), a' = a) or explicit
+// (g.eps [M][2] = e1, eps_expl [M][2] = e2).  Debug row: mean, sd, a (before exploration), log_prob(a), index 0.
+__global__ void __launch_bounds__(256) k_actor_train(const GemmArgs g, const float* __restrict__ eps_expl, float amount) {
+  const int row = blockIdx.x * blockDim.x + threadIdx.x;
+  if (row >= g.M) return;
+  float z[4] = {0.f, 0.f, 0.f, 0.f};
+  // made before the wait, as in k_actor_mode: the draws do not depend on the head's k_dense
+  if (g.noise == GM_NOISE_PHILOX) gm_normal4(g.gid0 + (uint32_t)row, g.step, 0u, RD_STREAM_TRAIN, g.key0, g.key1, z);
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  if (g.noise == GM_NOISE_EXPLICIT) {
+    z[0] = g.eps[2 * (size_t)row]; z[1] = g.eps[2 * (size_t)row + 1];
+    z[2] = eps_expl[2 * (size_t)row]; z[3] = eps_expl[2 * (size_t)row + 1];
+  }
+  float mean[2], sd[2];
+  gm_actor_dist(g, row, mean, sd);
+  const float log2f_ = 0.69314718f, half_log_2pi = 0.91893853f;
+  float a[2], x[2], lp = 0.f;
+#pragma unroll
+  for (int d = 0; d < 2; ++d) {
+    const float e = z[d], u = mean[d] + sd[d] * e;
+    lp += ((-0.5f * e * e - logf(sd[d])) - half_log_2pi) - 2.f * ((log2f_ - u) - gm_softplus(-2.f * u));
+    a[d] = tanhf(u);
+    x[d] = fminf(fmaxf(__fadd_rn(a[d], __fmul_rn(amount, z[2 + d])), -1.f), 1.f);
+  }
+  gm_actor_store(g, row, x[0], x[1]);
+  if (g.dbg) {
+    float* d = g.dbg + (size_t)row * 8;
+    d[0] = mean[0]; d[1] = mean[1]; d[2] = sd[0]; d[3] = sd[1]; d[4] = a[0]; d[5] = a[1]; d[6] = lp; d[7] = 0.f;
+  }
+}
+
+// Weight refresh (rd_policy_dreamer_set_weights): checkpoint arrays -> the policy's packed operands, on the device.
+// Job j: src [in][out] -> dst (o, kmap(i)) = tf32(x) and, if lo, tf32(x - tf32(x)), kmap(i) = i >= k_from ? i + k_shift
+// : i (dr_upload_t's layout; the K slots it skips keep their zeros); raw jobs copy [out] values as they are (biases,
+// BN).  The rounding is dr_tf32's integer one, so the packed bits equal the host packing of rd_policy_dreamer_init.
+#define GM_PACK_MAX 32
+struct PackJob {
+  const float* src; float* hi; float* lo;
+  int in, out, ld, k_from, k_shift, raw;
+  long long begin;         // first element of the job in the launch's flat index
+};
+struct PackArgs { int n_jobs; long long total; PackJob job[GM_PACK_MAX]; };
+__device__ __forceinline__ float gm_tf32_bits(float x) {   // == dr_tf32 (rd_dreamer.cuh)
+  return __uint_as_float((__float_as_uint(x) + 0x1000u) & ~0x1fffu);
+}
+__global__ void __launch_bounds__(256) k_pack_weights(const __grid_constant__ PackArgs a) {
+  for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < a.total; t += (long long)gridDim.x * blockDim.x) {
+    int j = 0;
+    while (j + 1 < a.n_jobs && t >= a.job[j + 1].begin) ++j;
+    const PackJob& J = a.job[j];
+    const long long e = t - J.begin;
+    const float x = J.src[e];
+    if (J.raw) { J.hi[e] = x; continue; }
+    const int i = (int)(e / J.out), o = (int)(e % J.out);
+    const size_t f = (size_t)o * J.ld + (i >= J.k_from ? i + J.k_shift : i);
+    const float h = gm_tf32_bits(x);
+    J.hi[f] = h;
+    if (J.lo) J.lo[f] = gm_tf32_bits(__fsub_rn(x, h));
   }
 }
 
