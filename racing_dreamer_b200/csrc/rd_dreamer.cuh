@@ -2,10 +2,9 @@
 //
 // One agent step = RacingDreamer.action [REF ros_agent/models/dreamer/racing_dreamer.py:62-82] for every env:
 //   img1 -> GRU cell -> obs1 (concat([deter, embed])) -> obs2 + posterior sample -> actor h0..h3 -> hout + mode()
-// = k_embed_lidar, five launches of k_dense, one of k_dense_chain (the actor trunk; with RD_DREAMER_HEAD=1 and up to
-// 33 x 128 envs also hout, which is the fifth k_dense launch otherwise) and k_actor_mode (rd_gemm.cuh);
-// activations live in a handful of [envs][width] float32 arrays that stay in
-// L2 between launches, the recurrent state in two ping-pong "latent" arrays whose rows are
+// = k_embed_lidar, five launches of k_dense (the fifth is hout), one of k_dense_chain per four layers of the actor trunk
+// and k_actor_mode (rd_gemm.cuh); activations live in a handful of [envs][width] float32 arrays that stay in L2 between
+// launches, the recurrent state in two ping-pong "latent" arrays whose rows are
 //   [ stoch (30) | previous action (2) | deter (200) ]          (232 floats, 928 bytes)
 // so that img1's input concat([stoch, action]), the GRU's state, obs1's concat([deter, ...]) and the actor's
 // concat([stoch, deter]) are all plain TMA views of one row (the actor's weight rows for the two action slots are
@@ -24,16 +23,12 @@
 // 128-wide tiles make 4 N tiles instead of 7: 128 CTAs, one per SM (two 64-wide CTAs on half the SMs share the SM's L2
 // ingress), which also leaves room for three 64 KB stages and four epilogue groups.  Measured: 64/2/2 0.190 ms,
 // 128/2/2 0.191, 128/2/4 0.188, 128/3/4 0.181 ms per agent step.
-#ifndef DR_ACT_BN
 #define DR_ACT_BN 128
 #define DR_ACT_STAGES 3
 #define DR_ACT_EW 4
-#endif
 
 // epilogue warp groups of the launches that have an SM to themselves (GRU cell, obs1, obs2 + posterior)
-#ifndef DR_EW_WIDE
 #define DR_EW_WIDE 4
-#endif
 
 struct DreamerPolicy {
   bool ready = false;
@@ -54,11 +49,6 @@ struct DreamerPolicy {
   float* head_raw = nullptr;   // [n][4] hout pre-activations
   // k_dense_chain (the actor trunk in one launch): per-row-block layer counters and the values they have reached
   bool chain = true;           // RD_DREAMER_CHAIN=0: one k_dense launch per actor layer instead
-  bool head_fused = false;     // RD_DREAMER_HEAD=1: hout inside the last k_dense_chain launch (cluster launches of <= 33 row
-                               // blocks).  Opt-in: 4 % faster, tests / memcheck / synccheck green, but racecheck flags the
-                               // remote stores ("block might not have entered yet"), see profiles/r5b_dreamer_chain.txt
-  bool chain_cluster = true;   // the N tiles of a row block are launched as a thread-block cluster (RD_DREAMER_CLUSTER=0: plain grid)
-  bool tma_out = true;         // RD_DREAMER_TMA_OUT=0: Dense / GRU epilogues store from registers (see gm_stage_f4)
   unsigned* chain_flags = nullptr;
   unsigned chain_count[GM_CHAIN_MAX] = {};
   int sm_count = 148;
@@ -235,12 +225,6 @@ static inline int dreamer_init(DreamerPolicy& d, int n, int n_beams, bool lidar_
     DR_TRY(cudaDeviceGetAttribute(&d.sm_count, cudaDevAttrMultiProcessorCount, dev));
     d.chain = true;
     if (const char* ev = std::getenv("RD_DREAMER_CHAIN")) d.chain = std::atoi(ev) != 0;
-    d.head_fused = false;
-    if (const char* ev = std::getenv("RD_DREAMER_HEAD")) d.head_fused = std::atoi(ev) != 0;
-    d.chain_cluster = true;
-    if (const char* ev = std::getenv("RD_DREAMER_CLUSTER")) d.chain_cluster = std::atoi(ev) != 0;
-    d.tma_out = true;
-    if (const char* ev = std::getenv("RD_DREAMER_TMA_OUT")) d.tma_out = std::atoi(ev) != 0;
   }
   DR_TRY(dr_alloc(d, d.x1, N, H));
   DR_TRY(dr_alloc(d, d.hobs, N, H));
@@ -410,7 +394,7 @@ static inline int dreamer_step(DreamerPolicy& d, const float* lidar, float* acti
     const DrTerm t[1] = {{&d.v_sa[cur], &d.w_img1, 32, 0}};
     dr_build(d, maps, g, t, 1, 1, nullptr, nullptr, 1, 4);
     g.step = d.step; g.bias = d.b_img1; g.out = d.x1.p[0]; g.out_lo = d.x1.p[1]; g.ldo = H; g.act = 1;
-    g.tma_out = d.tma_out; maps.o[0] = d.x1.m[0]; maps.o[1] = d.x1.m[1];
+    maps.o[0] = d.x1.m[0]; maps.o[1] = d.x1.m[1];
     if (d.x3) DR_TRY((gm_launch<EPI_DENSE, 1, 4, 2, true, DR_EW_WIDE>(maps, g, s)));
     else DR_TRY((gm_launch<EPI_DENSE, 1, 4, 4>(maps, g, s)));
     ++*launched;
@@ -425,7 +409,7 @@ static inline int dreamer_step(DreamerPolicy& d, const float* lidar, float* acti
     dr_build(d, maps, g, t, 2, 3, rows, gate, 4, d.x3 ? 8 : 4);   // one main group (every gate slot must be fed), one small
     g.step = d.step; g.bias = d.b_gru; g.out = d.v_det[nxt].p[0]; g.out_lo = d.v_det[nxt].p[1]; g.ldo = d.ldf;
     g.hold = d.v_det[cur].p[0]; g.hold_lo = d.v_det[cur].p[1]; g.ldh = d.ldf;
-    g.tma_out = d.tma_out; maps.o[0] = d.v_det[nxt].m[0]; maps.o[1] = d.v_det[nxt].m[1];
+    maps.o[0] = d.v_det[nxt].m[0]; maps.o[1] = d.v_det[nxt].m[1];
     if (d.x3) DR_TRY((gm_launch<EPI_GRU, 3, 8, 2, true, DR_EW_WIDE>(maps, g, s)));
     else DR_TRY((gm_launch<EPI_GRU, 3, 8, 4>(maps, g, s)));
     ++*launched;
@@ -437,7 +421,7 @@ static inline int dreamer_step(DreamerPolicy& d, const float* lidar, float* acti
     const DrTerm t[2] = {{&d.v_det[nxt], &d.w_obs1, D, 0}, {&d.lidar, &d.w_obs1, d.embed, D}};
     dr_build(d, maps, g, t, 2, 1, nullptr, nullptr, 1, 8);
     g.step = d.step; g.bias = d.b_obs1; g.out = d.hobs.p[0]; g.out_lo = d.hobs.p[1]; g.ldo = H; g.act = 1;
-    g.tma_out = d.tma_out; maps.o[0] = d.hobs.m[0]; maps.o[1] = d.hobs.m[1];
+    maps.o[0] = d.hobs.m[0]; maps.o[1] = d.hobs.m[1];
     if (d.x3) DR_TRY((gm_launch<EPI_DENSE, 1, 8, 4, true, DR_EW_WIDE>(maps, g, s)));
     else DR_TRY((gm_launch<EPI_DENSE, 1, 8, 8>(maps, g, s)));
     ++*launched;
@@ -458,7 +442,6 @@ static inline int dreamer_step(DreamerPolicy& d, const float* lidar, float* acti
   }
   // 5. actor trunk [REF models.py:321-322]: float32-grade mode runs up to GM_CHAIN_MAX layers per launch (k_dense_chain)
   const bool chain = d.x3 && d.chain;
-  bool head_fused = false;   // hout computed by the last chain launch (k_dense_chain's fused head)
   for (int i0 = 0; chain && i0 < d.layers; i0 += GM_CHAIN_MAX) {
     ChainMaps cm;
     ChainArgs c{};
@@ -482,11 +465,7 @@ static inline int dreamer_step(DreamerPolicy& d, const float* lidar, float* acti
       cm.w[j][0] = d.w_act[i].m[0]; cm.w[j][1] = d.w_act[i].m[1];
       if (j + 1 == c.n_layers) { cm.o_last[0] = d.hid[i & 1].m[0]; cm.o_last[1] = d.hid[i & 1].m[1]; }
     }
-    if (d.head_fused && i0 + c.n_layers == d.layers) {
-      c.head = 1; c.head_bias = d.b_act[d.layers]; c.head_out = d.head_raw;
-      cm.wh[0] = d.w_act[d.layers].m[0]; cm.wh[1] = d.w_act[d.layers].m[1];
-    }
-    DR_TRY((gm_launch_chain<DR_ACT_STAGES, DR_ACT_EW, DR_ACT_BN>(cm, c, d.sm_count, d.chain_cluster, s, &head_fused)));
+    DR_TRY((gm_launch_chain<DR_ACT_STAGES, DR_ACT_EW, DR_ACT_BN>(cm, c, d.sm_count, s)));
     ++*launched;
   }
   for (int i = 0; !chain && i < d.layers; ++i) {
@@ -495,7 +474,7 @@ static inline int dreamer_step(DreamerPolicy& d, const float* lidar, float* acti
     const DrTerm t[1] = {{i == 0 ? &d.feat[nxt] : &d.hid[(i - 1) & 1], &d.w_act[i], i == 0 ? d.ldf : U, 0}};
     dr_build(d, maps, g, t, 1, 1, nullptr, nullptr, 1, 4);
     g.bias = d.b_act[i]; g.out = d.hid[i & 1].p[0]; g.out_lo = d.hid[i & 1].p[1]; g.ldo = U; g.act = 1;
-    g.tma_out = d.tma_out; maps.o[0] = d.hid[i & 1].m[0]; maps.o[1] = d.hid[i & 1].m[1];
+    maps.o[0] = d.hid[i & 1].m[0]; maps.o[1] = d.hid[i & 1].m[1];
     if (d.x3) DR_TRY((gm_launch<EPI_DENSE, 1, 4, DR_ACT_STAGES, true, DR_ACT_EW, DR_ACT_BN>(maps, g, s)));
     else DR_TRY((gm_launch<EPI_DENSE, 1, 4, 4>(maps, g, s)));
     ++*launched;
@@ -513,11 +492,9 @@ static inline int dreamer_step(DreamerPolicy& d, const float* lidar, float* acti
     g.n_samples = d.n_samples;
     g.dbg = debug ? debug + (size_t)d.n * 2 * GM_STOCH : nullptr;
     g.out = d.head_raw;
-    if (!head_fused) {
-      if (d.x3) DR_TRY((gm_launch<EPI_ACTOR, 1, 4, 4, true>(maps, g, s)));
-      else DR_TRY((gm_launch<EPI_ACTOR, 1, 4, 4>(maps, g, s)));
-      ++*launched;
-    }
+    if (d.x3) DR_TRY((gm_launch<EPI_ACTOR, 1, 4, 4, true>(maps, g, s)));
+    else DR_TRY((gm_launch<EPI_ACTOR, 1, 4, 4>(maps, g, s)));
+    ++*launched;
     {
       cudaLaunchConfig_t cfg = {};
       cfg.gridDim = dim3((unsigned)((d.n + 7) / 8));

@@ -54,9 +54,6 @@ struct rd_env {
   int smem_per_sm = 0;            // shared memory per SM, bytes
   size_t l2_window_max = 0;       // > 0: L2 persistence is set up; the largest access-policy window the device takes
   bool lidar_centre_first = true; // k_lidar work order (RD_LIDAR_ORDER=0: env-major)
-  int lidar_gpi_min = 45;         // beam groups per resident warp from which a work item holds two groups (RD_LIDAR_GPI_MIN)
-  int lidar_gpi_force = 0;        // RD_LIDAR_GPI=1|2
-  bool lidar_pdl = true;          // k_lidar is launched as a programmatic dependent of the kernel in front of it (RD_LIDAR_PDL=0: off)
   bool lidar_attr_set[12] = {};   // k_lidar<16|24|32, groups per item, cars> opted in to smem_optin
   int n = 0;
   int step_block = 128;           // k_step threads per CTA (small batches: fewer, so that every SM gets a warp)
@@ -102,7 +99,6 @@ struct rd_env {
     float* lidar_dev = nullptr; float* lidar_host = nullptr;   // float32 rows, or IEEE half rows (lidar_elem == 2)
     size_t lidar_elem = 4;
     uint8_t* occ_dev = nullptr; uint8_t* occ_host = nullptr;
-    bool zero_copy = false;                  // k_lidar stores straight into the pinned host mirror (no staging copy)
     bool pending = false;                    // rd_step_host_begin enqueued a step whose results rd_step_host_end has not awaited
     rd_outputs dev_out{}, host_out{};
   } hp;
@@ -363,7 +359,7 @@ int launch_lidar_t(rd_env* env, int map_id, const OriginRec* recs, const int32_t
     cudaLaunchConfig_t lc{};
     lc.gridDim = dim3((unsigned)grid); lc.blockDim = dim3(WARPS * 32); lc.dynamicSmemBytes = smem; lc.stream = s;
     cudaLaunchAttribute at[2];
-    lc.attrs = at; lc.numAttrs = launch_attrs(env, map_id, env->lidar_pdl, at);
+    lc.attrs = at; lc.numAttrs = launch_attrs(env, map_id, true, at);
     const DevMap* a_maps = env->d_maps; const double* a_tab = env->d_beam_tab;
     cudaError_t le = cudaLaunchKernelEx(&lc, kern, a_maps, map_id, recs, order, n_env, lp, a_tab, out, ctr);
     if (le != cudaSuccess) { cudaGetLastError(); return fail(env, RD_ERR_CUDA, "k_lidar launch: %s", cudaGetErrorString(le)); }
@@ -379,16 +375,14 @@ int launch_lidar(rd_env* env, int map_id, const OriginRec* recs, const int32_t* 
   if (!ctr) ctr = env->d_lidar_ctr + 2 * (env->lidar_ctr_next++ % RD_CTR_RING);
   // 48 resident warps per SM wherever the shared-memory copies of the map allow it (the kernel is capped at 40
   // registers for that): three 16-warp CTAs for small maps, two 24-warp CTAs for maps of which two copies fit, one
-  // 32-warp CTA otherwise.  RD_LIDAR_WARPS=16|24|32 overrides (tuning).
+  // 32-warp CTA otherwise.
   const size_t smem1 = 16 + (((size_t)2 * env->cfg.n_beams * 8 + 15) & ~(size_t)15) + (size_t)m.bits_bytes + 1024;   // + the per-CTA reserve
   const size_t sm_total = (size_t)env->smem_per_sm;
-  int warps = 3 * smem1 <= sm_total ? 16 : (2 * smem1 <= sm_total ? 24 : 32);
-  if (const char* ev = std::getenv("RD_LIDAR_WARPS")) { const int w = std::atoi(ev); if (w == 16 || w == 24 || w == 32) warps = w; }
+  const int warps = 3 * smem1 <= sm_total ? 16 : (2 * smem1 <= sm_total ? 24 : 32);
   // Two beam groups per work item once a resident warp gets enough of them (see k_lidar): 45 groups per warp is where
-  // the curves cross (profiles/r3o_lidar_groups_per_item.txt).  RD_LIDAR_GPI=1|2 overrides.
+  // the curves cross (profiles/r3o_lidar_groups_per_item.txt).
   const long long resident_warps = (long long)env->sm_count * (warps == 32 ? 32 : 48);
-  int gpi = (long long)n_env * ((env->cfg.n_beams + 31) / 32) >= (long long)env->lidar_gpi_min * resident_warps ? 2 : 1;
-  if (env->lidar_gpi_force) gpi = env->lidar_gpi_force;
+  const int gpi = (long long)n_env * ((env->cfg.n_beams + 31) / 32) >= 45LL * resident_warps ? 2 : 1;
   const bool cars = env->cfg.agents_per_world > 1;   // worlds: the scans also see the other cars (own instantiation, so
                                                       // that the single-car kernel keeps its register budget)
 #define RD_LIDAR_GO(W, G, C) launch_lidar_t<W, G, C>(env, map_id, recs, order, n_env, out, s, ctr)
@@ -620,33 +614,25 @@ RD_API int rd_create(const rd_config* cfg, rd_env** out) {
   env->n = cfg->n_envs;
   env->order_offset.assign(RD_MAX_MAPS + 1, 0);
   // L2 residency of the tracks (launch_attrs): set aside a slice of L2 for persisting lines, once per device; the
-  // slice only ever grows (another handle or the application may have asked for more).  RD_L2_PERSIST=0 turns it off.
-  {
-    bool on = prop.persistingL2CacheMaxSize > 0 && prop.accessPolicyMaxWindowSize > 0;
-    if (const char* ev = std::getenv("RD_L2_PERSIST")) on = on && std::atoi(ev) != 0;
-    if (on) {
-      size_t cur = 0;
-      const size_t want = std::min<size_t>((size_t)prop.persistingL2CacheMaxSize, (size_t)8 << 20);
-      if (cudaDeviceGetLimit(&cur, cudaLimitPersistingL2CacheSize) == cudaSuccess &&
-          (cur >= want || cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want) == cudaSuccess))
-        env->l2_window_max = std::min<size_t>((size_t)prop.accessPolicyMaxWindowSize, std::max(cur, want));
-      cudaGetLastError();
-    }
+  // slice only ever grows (another handle or the application may have asked for more).
+  if (prop.persistingL2CacheMaxSize > 0 && prop.accessPolicyMaxWindowSize > 0) {
+    size_t cur = 0;
+    const size_t want = std::min<size_t>((size_t)prop.persistingL2CacheMaxSize, (size_t)8 << 20);
+    if (cudaDeviceGetLimit(&cur, cudaLimitPersistingL2CacheSize) == cudaSuccess &&
+        (cur >= want || cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want) == cudaSuccess))
+      env->l2_window_max = std::min<size_t>((size_t)prop.accessPolicyMaxWindowSize, std::max(cur, want));
+    cudaGetLastError();
   }
   // k_step is one long float64 instruction stream per warp: spread the warps over as many SM sub-partitions as the
-  // batch allows (RD_STEP_BLOCK overrides, tuning)
+  // batch allows
   env->step_block = (env->n >= 128 * 4 * env->sm_count) ? 128 : ((env->n >= 64 * 4 * env->sm_count) ? 64 : 32);
-  if (const char* ev = std::getenv("RD_LIDAR_PDL")) env->lidar_pdl = std::atoi(ev) != 0;
   if (const char* ev = std::getenv("RD_LIDAR_ORDER")) env->lidar_centre_first = std::atoi(ev) != 0;
-  if (const char* ev = std::getenv("RD_LIDAR_GPI")) { const int v = std::atoi(ev); if (v == 1 || v == 2) env->lidar_gpi_force = v; }
-  if (const char* ev = std::getenv("RD_LIDAR_GPI_MIN")) { const int v = std::atoi(ev); if (v > 0) env->lidar_gpi_min = v; }
   env->step_split = env->n <= 64 * env->sm_count;   // up to two CTAs per SM -- what the kernel's registers allow, a third CTA
                                                      // would wait for a second wave (measured: 22.9 vs 31.9 us at 8192 envs, 39.1 vs
                                                      // 33.0 us at 12 288; rotating the warp roles of co-resident CTAs over the
                                                      // schedulers changes nothing, profiles/r6b_two_tracks_strong_scaling.txt)
   if (const char* ev = std::getenv("RD_STEP_SPLIT")) env->step_split = std::atoi(ev) != 0;
   if (const char* ev = std::getenv("RD_FORK_MAPS")) env->fork_maps = std::atoi(ev) != 0;
-  if (const char* ev = std::getenv("RD_STEP_BLOCK")) { int v = std::atoi(ev); if (v == 32 || v == 64 || v == 128) env->step_block = v; }
   const size_t n = (size_t)env->n;
   cudaError_t e = cudaSuccess;
   auto alloc = [&](void** p, size_t bytes) { if (e == cudaSuccess) { e = cudaMalloc(p, bytes); if (e == cudaSuccess) e = cudaMemset(*p, 0, bytes); } };
@@ -706,8 +692,7 @@ RD_API void rd_destroy(rd_env* env) {
     for (auto ev : h.ev_done) cudaEventDestroy(ev);
     if (h.ev_act) cudaEventDestroy(h.ev_act);
     cudaFreeHost(h.act_host); cudaFree(h.act_dev); cudaFree(h.mask_dev); cudaFree(h.small_dev); cudaFreeHost(h.small_host);
-    if (!h.zero_copy) cudaFree(h.lidar_dev);
-    cudaFreeHost(h.lidar_host); cudaFree(h.occ_dev); cudaFreeHost(h.occ_host);
+    cudaFree(h.lidar_dev); cudaFreeHost(h.lidar_host); cudaFree(h.occ_dev); cudaFreeHost(h.occ_host);
   }
   for (auto& t : env->timed) { cudaEventDestroy(t.a); cudaEventDestroy(t.b); }
   for (auto& e : env->event_pool) cudaEventDestroy(e);
@@ -750,11 +735,10 @@ RD_API int rd_upload_map(rd_env* env, int map_id, const uint32_t* bits_host, int
   int ch = 0, cw = 0;
   // Block size of the clearance field: the finest that still fits in shared memory next to the bits and the beam
   // table.  Measured on B200: 2x2 blocks beat 4x4 by 10-13 % even where they halve the resident warps (fewer exact-DDA
-  // steps at the end of each ray matter more than occupancy); RD_LIDAR_CSHIFT overrides (tuning).
+  // steps at the end of each ray matter more than occupancy).
   int cshift = 1;
   const size_t fixed = 16 + (((size_t)2 * env->cfg.n_beams * 8 + 15) & ~(size_t)15) + bits_padded;
   while (cshift < 5 && fixed + (size_t)(((h >> cshift) + 1) * ((w >> cshift) + 1)) + 16 > (size_t)env->smem_optin) ++cshift;
-  if (const char* ev = std::getenv("RD_LIDAR_CSHIFT")) { int v = std::atoi(ev); if (v >= 0 && v <= 5) cshift = v; }
   rd_build_clearance(bits_host, h, w, row_words, cshift, coarse, ch, cw);
   const size_t coarse_padded = (coarse.size() + 15) & ~(size_t)15;
   std::vector<unsigned char> packed(bits_padded + coarse_padded, 0);
@@ -882,29 +866,14 @@ RD_API int rd_host_init(rd_env* env, int n_chunks, rd_outputs* host_out) {
   const int n = env->n;
   n_chunks = std::max(1, std::min(n_chunks, n));
   h.n_chunks = n_chunks;
-  h.bounds.resize(n_chunks + 1);
   // progressive chunk sizes (1 : 2 : 4 : ... capped at 16x, measured with the round-2 kernels): the first chunk is small so that the copy engine starts
   // early; from then on it is the bottleneck and each chunk's ray casting hides behind the previous chunk's copy.
-  // RD_HOST_CHUNKS="1,3,12" overrides the weights (and the chunk count) for tuning.
   {
-    std::vector<double> w;
-    if (const char* ev = std::getenv("RD_HOST_CHUNKS")) {
-      for (const char* p = ev; *p;) {
-        char* end = nullptr;
-        const double v = std::strtod(p, &end);
-        if (end == p) break;
-        if (v > 0.0) w.push_back(v);
-        p = (*end == ',') ? end + 1 : end;
-      }
-      if ((int)w.size() > n) w.resize(n);
-    }
-    if (w.empty()) { w.resize(n_chunks); for (int c = 0; c < n_chunks; ++c) w[c] = (double)(1 << std::min(c, 4)); }
-    n_chunks = (int)w.size();
-    h.n_chunks = n_chunks;
+    auto weight = [](int c) { return (double)(1 << std::min(c, 4)); };
     h.bounds.assign(n_chunks + 1, 0);
     double tot = 0.0, acc = 0.0;
-    for (double v : w) tot += v;
-    for (int c = 0; c < n_chunks; ++c) { acc += w[c]; h.bounds[c + 1] = (int)std::llround((double)n * acc / tot); }
+    for (int c = 0; c < n_chunks; ++c) tot += weight(c);
+    for (int c = 0; c < n_chunks; ++c) { acc += weight(c); h.bounds[c + 1] = (int)std::llround((double)n * acc / tot); }
     h.bounds[n_chunks] = n;
   }
   // small arrays share one slab (one device->host copy per step); offsets 256-byte aligned
@@ -924,17 +893,10 @@ RD_API int rd_host_init(rd_env* env, int n_chunks, rd_outputs* host_out) {
   CUDA_TRY(env, cudaMemset(h.small_dev, 0, h.small_bytes));
   CUDA_TRY(env, cudaHostAlloc(&h.small_host, h.small_bytes, cudaHostAllocDefault));
   std::memset(h.small_host, 0, h.small_bytes);
-  // RD_HOST_ZEROCOPY=1: the ray-cast kernel writes its (fully coalesced, 128 B per warp) range rows directly into the
-  // pinned host mirror over PCIe -- the transfer then overlaps the ray casting store by store, with no copy phase.
-  if (const char* ev = std::getenv("RD_HOST_ZEROCOPY")) h.zero_copy = std::atoi(ev) != 0;
-  CUDA_TRY(env, cudaHostAlloc(&h.lidar_host, lidar_bytes, cudaHostAllocMapped));
+  CUDA_TRY(env, cudaHostAlloc(&h.lidar_host, lidar_bytes, cudaHostAllocDefault));
   std::memset(h.lidar_host, 0, lidar_bytes);
-  if (h.zero_copy) {
-    CUDA_TRY(env, cudaHostGetDevicePointer((void**)&h.lidar_dev, h.lidar_host, 0));
-  } else {
-    CUDA_TRY(env, cudaMalloc(&h.lidar_dev, lidar_bytes));
-    CUDA_TRY(env, cudaMemset(h.lidar_dev, 0, lidar_bytes));
-  }
+  CUDA_TRY(env, cudaMalloc(&h.lidar_dev, lidar_bytes));
+  CUDA_TRY(env, cudaMemset(h.lidar_dev, 0, lidar_bytes));
   if (occ) {
     CUDA_TRY(env, cudaMalloc(&h.occ_dev, (size_t)n * 4096));
     CUDA_TRY(env, cudaMemset(h.occ_dev, 0, (size_t)n * 4096));
@@ -978,11 +940,9 @@ int host_copy_back(rd_env* env, int c) {
   auto& h = env->hp;
   const size_t e0 = (size_t)h.bounds[c], cnt = (size_t)(h.bounds[c + 1] - h.bounds[c]);
   const size_t nb = (size_t)env->cfg.n_beams;
-  if (!h.zero_copy) {
-    const size_t off = e0 * nb * h.lidar_elem;
-    CUDA_TRY(env, cudaMemcpyAsync(reinterpret_cast<unsigned char*>(h.lidar_host) + off, reinterpret_cast<unsigned char*>(h.lidar_dev) + off,
-                                  h.lidar_elem * cnt * nb, cudaMemcpyDeviceToHost, h.streams[c]));
-  }
+  const size_t off = e0 * nb * h.lidar_elem;
+  CUDA_TRY(env, cudaMemcpyAsync(reinterpret_cast<unsigned char*>(h.lidar_host) + off, reinterpret_cast<unsigned char*>(h.lidar_dev) + off,
+                                h.lidar_elem * cnt * nb, cudaMemcpyDeviceToHost, h.streams[c]));
   if (h.occ_dev) CUDA_TRY(env, cudaMemcpyAsync(h.occ_host + e0 * 4096, h.occ_dev + e0 * 4096, cnt * 4096, cudaMemcpyDeviceToHost, h.streams[c]));
   return RD_OK;
 }
@@ -1011,7 +971,7 @@ RD_API int rd_reset_host(rd_env* env, const uint8_t* mask_host, int mode) {
   if (rc) return rc;
   const int saved = h.n_chunks;   // everything ran on stream 0: copy it back as one chunk
   const size_t nb = (size_t)env->cfg.n_beams, n = (size_t)env->n;
-  if (!h.zero_copy) CUDA_TRY(env, cudaMemcpyAsync(h.lidar_host, h.lidar_dev, h.lidar_elem * n * nb, cudaMemcpyDeviceToHost, s0));
+  CUDA_TRY(env, cudaMemcpyAsync(h.lidar_host, h.lidar_dev, h.lidar_elem * n * nb, cudaMemcpyDeviceToHost, s0));
   if (h.occ_dev) CUDA_TRY(env, cudaMemcpyAsync(h.occ_host, h.occ_dev, n * 4096, cudaMemcpyDeviceToHost, s0));
   CUDA_TRY(env, cudaMemcpyAsync(h.small_host, h.small_dev, h.small_bytes, cudaMemcpyDeviceToHost, s0));
   CUDA_TRY(env, cudaStreamSynchronize(s0));

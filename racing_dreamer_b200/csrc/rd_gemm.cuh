@@ -29,8 +29,6 @@
 #include <cuda.h>
 
 #include <algorithm>
-#include <cstdio>
-#include <cstdlib>
 
 #include "rd_common.cuh"
 
@@ -38,10 +36,7 @@
 #define GM_BN 64
 #define GM_BK 32                      // float32 elements per K block = one 128-byte swizzle row
 #define GM_A_BYTES (GM_BM * 128)      // 16 KB
-#define GM_W_BYTES (GM_BN * 128)      // 8 KB
-#ifndef GM_EPI_GROUPS
 #define GM_EPI_GROUPS 2               // epilogue warp groups: group p of 4 warps handles columns [p, p + 1) * 64 / GROUPS of the tile
-#endif
 #define GM_THREADS (64 + 128 * GM_EPI_GROUPS)   // warp 0: TMA producer, warp 1: TMEM allocator + MMA issuer, then the epilogue warps
 #define GM_STOCH 30                   // RSSM stochastic state size of the shipped agents [REF racing_dreamer.py:20]
 
@@ -49,7 +44,7 @@
 struct GemmMaps {   // tensor maps of one launch: A sources and weight matrices, hi parts and (x3 mode) lo parts
   CUtensorMap a[4];
   CUtensorMap w[4];
-  CUtensorMap o[2];  // GemmArgs::tma_out: the output rows (hi, lo), box 32 columns x 128 rows -- the view the next layer loads
+  CUtensorMap o[2];  // DENSE / GRU: the output rows (hi, lo), box 32 columns x 128 rows -- the view the next layer loads
 };
 struct GemmPhase {
   int a_map, w_map; // indices into GemmMaps
@@ -80,7 +75,6 @@ struct GemmArgs {
   float* out; int ldo;      // DENSE / GRU: output rows, TF32-rounded (they are only ever read as MMA operands)
   float* out_lo;            // x3 mode: TF32-rounded remainder of the same rows (same pitch), or null
   int act;                  // DENSE: 1 = ELU, 0 = linear
-  int tma_out;              // DENSE / GRU: 1 = the tile leaves through shared memory and the copy engine (maps.o), see gm_stage_f4
   const float* hold; const float* hold_lo; int ldh;   // GRU: previous deterministic state (hi [+ lo])
   // STOCH / ACTOR
   int noise;                // GM_NOISE_*
@@ -271,12 +265,6 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
   extern __shared__ uint8_t gm_smem_raw[];
   __shared__ uint64_t full_bar[GM_STAGES], empty_bar[GM_STAGES], acc_bar;
   __shared__ uint32_t tmem_slot;
-#ifdef GM_CHAIN_TRACE   // per-role clock stamps (tools/gpu_chain_trace.sh)
-  __shared__ long long trd[8];
-#define GM_TRD(k) trd[k] = clock64()
-#else
-#define GM_TRD(k) do { } while (0)
-#endif
   // X3: a ring stage holds the hi AND the lo tiles of a K block ([A_hi | W_hi slabs | A_lo | W_lo slabs]) and feeds all
   // three products of the float32-grade scheme from one load: two thirds of the operand bytes of three separate passes
   // and a third of the producer / issuer hand-offs.
@@ -310,7 +298,6 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
   // Programmatic dependent launch: the next k_dense of the stream may start its own set-up (barriers, TMEM, tensor-map
   // fetch) now; everything that touches global memory first waits for the previous kernel to have completed.
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  if (threadIdx.x == 0) GM_TRD(0);
 
   if (warp == 0) {
     if (gm_elect_one()) {   // ===== TMA producer =====
@@ -320,7 +307,7 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
       // are requested BEFORE griddepcontrol.wait (pass 0), the activation tiles of those K blocks and everything else
       // after it (pass 1) -- the ring is full of weights by the time the previous layer's outputs exist.
       for (int pass = 0; pass < 2; ++pass) {
-        if (pass == 1) { asm volatile("griddepcontrol.wait;" ::: "memory"); GM_TRD(1); }
+        if (pass == 1) asm volatile("griddepcontrol.wait;" ::: "memory");
         uint32_t it = 0;
         for (int p = 0; p < g.n_phases; ++p) {
           const GemmPhase& ph = g.ph[p];
@@ -387,7 +374,6 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
           const uint32_t s = it % GM_STAGES, par = (it / GM_STAGES) & 1u;
           gm_mbar_wait(&full_bar[s], par);
           gm_tc_fence_after();
-          if (it == 0) GM_TRD(2);
           const uint32_t a_lo = lo_base + s * (STAGE_BYTES >> 4);
 #pragma unroll
           for (int i = 0; i < 3; ++i) {
@@ -413,7 +399,6 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
         }
       }
       gm_commit(&acc_bar);            // accumulators complete
-      GM_TRD(3);
     }
     __syncwarp();
   } else {
@@ -457,8 +442,7 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
     }
     gm_mbar_wait(&acc_bar, 0, true);
     gm_tc_fence_after();
-    if (threadIdx.x == 64) GM_TRD(4);
-    // tma_out: this part's 32-column staging tile (hi, lo) in the idle ring, and who shares it
+    // DENSE / GRU: this part's 32-column staging tile (hi, lo) in the idle ring, and who shares it
     constexpr int TILE_PARTS = PART_COLS >= 32 ? 1 : 32 / PART_COLS;       // column parts per staging tile
     static_assert(PART_COLS == 16 || PART_COLS % 32 == 0, "staging tiles are 32 columns wide");
     const uint32_t rt = (uint32_t)(q * 32 + lane);                          // tile row
@@ -472,7 +456,7 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
 #pragma unroll
         for (int j = 0; j < 16; j += 4) {
           const int col = n0 + c0 + j;
-          if ((live || g.tma_out) && col < g.N) {   // N % 4 == 0
+          if (col < g.N) {   // N % 4 == 0
             float4 o, ol;
             float* po = &o.x;
             float* pl = &ol.x;
@@ -483,23 +467,16 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
               po[t] = gm_round_tf32(x);
               pl[t] = gm_round_tf32(x - po[t]);
             }
-            if (g.tma_out) {
-              gm_stage_f4(s_hi, rt, (c0 + j) & 31, o);
-              if (g.out_lo) gm_stage_f4(s_lo, rt, (c0 + j) & 31, ol);
-            } else {
-              *reinterpret_cast<float4*>(g.out + (size_t)row * g.ldo + col) = o;
-              if (g.out_lo) *reinterpret_cast<float4*>(g.out_lo + (size_t)row * g.ldo + col) = ol;
-            }
+            gm_stage_f4(s_hi, rt, (c0 + j) & 31, o);
+            if (g.out_lo) gm_stage_f4(s_lo, rt, (c0 + j) & 31, ol);
           }
         }
       }
-      if (g.tma_out) {
 #pragma unroll 1
-        for (int t0 = cbeg & ~31; t0 < cend; t0 += 32) {   // the 32-column tiles this part contributes to (one, unless PART_COLS > 32)
-          const uint32_t s_hi = smem_base + (uint32_t)(t0 >> 5) * (2u * GM_A_BYTES);
-          gm_tiles_out(1 + (t0 >> 5), 128 * TILE_PARTS, (part % TILE_PARTS) == 0 && q == 0 && lane == 0, n0 + t0 < g.N, &maps.o[0],
-                       g.out_lo ? &maps.o[1] : nullptr, n0 + t0, m0, s_hi, s_hi + GM_A_BYTES);
-        }
+      for (int t0 = cbeg & ~31; t0 < cend; t0 += 32) {   // the 32-column tiles this part contributes to (one, unless PART_COLS > 32)
+        const uint32_t s_hi = smem_base + (uint32_t)(t0 >> 5) * (2u * GM_A_BYTES);
+        gm_tiles_out(1 + (t0 >> 5), 128 * TILE_PARTS, (part % TILE_PARTS) == 0 && q == 0 && lane == 0, n0 + t0 < g.N, &maps.o[0],
+                     g.out_lo ? &maps.o[1] : nullptr, n0 + t0, m0, s_hi, s_hi + GM_A_BYTES);
       }
     } else if constexpr (EPI == EPI_GRU) {
       // tf.keras GRUCell (reset_after=True): z, r, h gates; bias[0] input side, bias[1] recurrent side
@@ -543,24 +520,17 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
               po[t] = gm_round_tf32(hn);
               pl[t] = gm_round_tf32(hn - po[t]);
             }
-            if (g.tma_out) {
-              const uint32_t s_hi = smem_base + (uint32_t)(c0 >> 5) * (2u * GM_A_BYTES);
-              gm_stage_f4(s_hi, rt, (c0 + j) & 31, o);
-              if (g.out_lo) gm_stage_f4(s_hi + GM_A_BYTES, rt, (c0 + j) & 31, ol);
-            } else {
-              *reinterpret_cast<float4*>(g.out + (size_t)row * g.ldo + col) = o;
-              if (g.out_lo) *reinterpret_cast<float4*>(g.out_lo + (size_t)row * g.ldo + col) = ol;
-            }
+            const uint32_t s_hi = smem_base + (uint32_t)(c0 >> 5) * (2u * GM_A_BYTES);
+            gm_stage_f4(s_hi, rt, (c0 + j) & 31, o);
+            if (g.out_lo) gm_stage_f4(s_hi + GM_A_BYTES, rt, (c0 + j) & 31, ol);
           }
         }
       }
-      if (g.tma_out) {
 #pragma unroll 1
-        for (int t0 = cbeg & ~31; t0 < cend; t0 += 32) {
-          const uint32_t s_hi = smem_base + (uint32_t)(t0 >> 5) * (2u * GM_A_BYTES);
-          gm_tiles_out(1 + (t0 >> 5), 128 * TILE_PARTS, (part % TILE_PARTS) == 0 && q == 0 && lane == 0, n0 + t0 < H, &maps.o[0],
-                       g.out_lo ? &maps.o[1] : nullptr, n0 + t0, m0, s_hi, s_hi + GM_A_BYTES);
-        }
+      for (int t0 = cbeg & ~31; t0 < cend; t0 += 32) {
+        const uint32_t s_hi = smem_base + (uint32_t)(t0 >> 5) * (2u * GM_A_BYTES);
+        gm_tiles_out(1 + (t0 >> 5), 128 * TILE_PARTS, (part % TILE_PARTS) == 0 && q == 0 && lane == 0, n0 + t0 < H, &maps.o[0],
+                     g.out_lo ? &maps.o[1] : nullptr, n0 + t0, m0, s_hi, s_hi + GM_A_BYTES);
       }
     } else if constexpr (EPI == EPI_STOCH) {
       // RSSM posterior [REF models.py:69-73]: mean, std = split(x); std = softplus(std) + 0.1; stoch = mean + std * eps
@@ -653,19 +623,12 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
       }
     }
     gm_tc_fence_before();
-    if (threadIdx.x == 64) GM_TRD(5);
   }
   __syncthreads();
   if (warp == 1) {
     gm_tc_fence_after();
     gm_tmem_free(tmem, TM_COLS);
   }
-#ifdef GM_CHAIN_TRACE
-  if (threadIdx.x == 0 && g.step == 40u && blockIdx.x % 16 == 0)
-    printf("DENSE epi %d cta (%d,%d): inputs ready %lld | first full %lld | MMAs issued %lld | acc ready %lld | epilogue done %lld | end %lld\n",
-           EPI, blockIdx.x, blockIdx.y, trd[1] - trd[0], trd[2] - trd[0], trd[3] - trd[0], trd[4] - trd[0], trd[5] - trd[0], clock64() - trd[0]);
-#endif
-#undef GM_TRD
 }
 
 // ActionDecoder distribution head [REF models.py:323-346]: mean and sd of the pre-tanh Normal from hout's
@@ -908,7 +871,6 @@ struct ChainMaps {   // [layer][hi, lo]; layer l stores its output through a[l +
   CUtensorMap a[GM_CHAIN_MAX][2];
   CUtensorMap w[GM_CHAIN_MAX][2];
   CUtensorMap o_last[2];
-  CUtensorMap wh[2];          // ChainArgs::head: the head's weights [4][K] (hi, lo), box 32 x 64 rows
 };
 struct ChainLayer {
   int kb_total;            // K blocks of the layer
@@ -923,13 +885,6 @@ struct ChainArgs {
   int M, N, ldo, n_layers, row_blocks;
   unsigned* flags;         // [GM_CHAIN_MAX][row_blocks]
   ChainLayer L[GM_CHAIN_MAX];
-  // Fused output head (ActionDecoder hout, 4 columns): cluster launches with one row block per cluster only.  The last
-  // layer's output tiles never leave shared memory: every CTA multiplies its own 128 columns -- staged as MMA-ready
-  // 128-byte-swizzled tiles anyway -- with its K slice of the head's weights, and the cluster's first CTA adds the
-  // four partial [128][4] products (distributed shared memory) and the bias.
-  int head;
-  const float* head_bias;  // [4]
-  float* head_out;         // [M][4] pre-activations (k_actor_mode reads them)
 };
 
 __device__ __forceinline__ void gm_flag_wait(const unsigned* flag, unsigned target) {
@@ -947,16 +902,7 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
     k_dense_chain(const __grid_constant__ ChainMaps maps, const ChainArgs g) {
   extern __shared__ uint8_t gm_smem_raw[];
   __shared__ uint64_t full_bar[GM_STAGES], empty_bar[GM_STAGES], acc_bar, tmem_free_bar, epi_done_bar;
-  __shared__ uint64_t head_full_bar, stage_ready_bar, head_acc_bar;   // fused head (g.head)
-  __shared__ float4 head_red[4][GM_BM];                              // CTA 0 of the cluster: the four partial products
   __shared__ uint32_t tmem_slot;
-#ifdef GM_CHAIN_TRACE   // per-role clock stamps of the first row block (tools/gpu_chain_trace.sh)
-  __shared__ long long tr[GM_CHAIN_MAX][16];
-  __shared__ long long tr0;
-#define GM_TR(l, k) do { if (mb == (int)blockIdx.y) tr[l][k] = clock64(); } while (0)
-#else
-#define GM_TR(l, k) do { } while (0)
-#endif
   static_assert(BN % 16 == 0 && BN <= 256 && 4 * BN <= 512, "MMA N and the accumulators' TMEM columns");
   constexpr uint32_t W_BYTES = BN * 128, IDESC = GM_IDESC_N(BN);
   constexpr uint32_t SUB_BYTES = GM_A_BYTES + W_BYTES, STAGE_BYTES = 2u * SUB_BYTES;
@@ -964,23 +910,8 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
   const uint32_t smem_base = (rd_smem_u32(gm_smem_raw) + 1023u) & ~1023u;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int n0 = blockIdx.x * BN;
-  // fused head: this CTA's live 32-column parts, and where the ring stands after the last K block (g.head implies one
-  // row block per CTA, so the K blocks of the launch are those of its layers)
-  const int head_parts = g.head ? min(EW, (g.N - n0 + 31) / 32) : 0;
-  uint32_t head_it = 0;
-  for (int l = 0; l < g.n_layers; ++l) head_it += (uint32_t)g.L[l].kb_total;
-  // staging tile of part p (see the epilogue) and the idle weight slot that receives the head's K slice for it
-  auto head_a_hi = [&](int p) -> uint32_t {
-    const uint32_t st = p < 2 ? (head_it + (uint32_t)p) % 3u : (head_it + 2u) % 3u;
-    return smem_base + st * STAGE_BYTES + (p == 3 ? GM_A_BYTES : 0u);
-  };
-  auto head_w_hi = [&](int p) -> uint32_t {   // parts 0, 1 -> W slots of stage head_it % 3; parts 2, 3 -> of the next stage
-    const uint32_t st = (head_it + (uint32_t)(p >> 1)) % 3u;
-    return smem_base + st * STAGE_BYTES + GM_A_BYTES + (uint32_t)(p & 1) * SUB_BYTES;
-  };
 
   if (threadIdx.x == 0) {
-    if (g.head) { gm_prefetch_map(&maps.wh[0]); gm_prefetch_map(&maps.wh[1]); }
     for (int l = 0; l < g.n_layers; ++l) {
       gm_prefetch_map(&maps.a[l][0]); gm_prefetch_map(&maps.a[l][1]);
       gm_prefetch_map(&maps.w[l][0]); gm_prefetch_map(&maps.w[l][1]);
@@ -993,9 +924,6 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
     asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(rd_smem_u32(&acc_bar)));
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(rd_smem_u32(&tmem_free_bar)), "r"(4 * EW));
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(rd_smem_u32(&epi_done_bar)), "r"(EW));
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(rd_smem_u32(&head_full_bar)));
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(rd_smem_u32(&stage_ready_bar)), "r"(EW));
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(rd_smem_u32(&head_acc_bar)));
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == 1) gm_tmem_alloc(&tmem_slot, TM_COLS);
@@ -1004,9 +932,6 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
   gm_tc_fence_after();
   const uint32_t tmem = tmem_slot;
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#ifdef GM_CHAIN_TRACE
-  if (threadIdx.x == 0) tr0 = clock64();
-#endif
 
   if (warp == 0) {
     if (gm_elect_one()) {   // ===== TMA producer =====
@@ -1031,13 +956,10 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
             gm_tma_2d(sa + GM_A_BYTES, mw, j * GM_BK, n0, &full_bar[s]);
             gm_tma_2d(sb + GM_A_BYTES, mw2, j * GM_BK, n0, &full_bar[s]);
           }
-          GM_TR(l, 0);
           // the layer's input rows: the kernel in front of this one (first layer) or every N tile of the layer before
           if (first) { asm volatile("griddepcontrol.wait;" ::: "memory"); first = false; }
           if (tile > 0) gm_mbar_wait(&epi_done_bar, (tile - 1) & 1u);   // the copy engine has read the staged tiles
-          GM_TR(l, 14);
           if (l > 0) gm_flag_wait(g.flags + (size_t)(l - 1) * g.row_blocks + mb, g.L[l - 1].target);
-          GM_TR(l, 1);
           for (int j = 0; j < pre; ++j) {
             const uint32_t s = (it + (uint32_t)j) % GM_STAGES;
             const uint32_t sa = smem_base + s * STAGE_BYTES, sb = sa + SUB_BYTES;
@@ -1056,16 +978,6 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
           }
           it += (uint32_t)kbs;
           ++tile;
-        }
-      }
-      if (g.head) {
-        // the head's weights go into ring slots no staging tile uses; the ring is idle once the last MMAs are complete
-        gm_mbar_wait(&acc_bar, (tile - 1) & 1u);
-        rd_mbar_expect_tx(&head_full_bar, (uint32_t)head_parts * 2u * GM_W_BYTES);
-        for (int p = 0; p < head_parts; ++p) {
-          const uint32_t w = head_w_hi(p);
-          gm_tma_2d(w, &maps.wh[0], n0 + 32 * p, 0, &head_full_bar);
-          gm_tma_2d(w + GM_W_BYTES, &maps.wh[1], n0 + 32 * p, 0, &head_full_bar);
         }
       }
     }
@@ -1090,7 +1002,6 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
               const uint32_t s = it % GM_STAGES, par = (it / GM_STAGES) & 1u;
               gm_mbar_wait(&full_bar[s], par);
               gm_tc_fence_after();
-              if (grp == 0 && kb == 0) GM_TR(l, 2);
               const uint32_t a_lo = lo_base + s * (STAGE_BYTES >> 4);
               const uint32_t w_lo = a_lo + (GM_A_BYTES >> 4);
               const uint32_t a2 = a_lo + (SUB_BYTES >> 4), w2 = w_lo + (SUB_BYTES >> 4);
@@ -1109,31 +1020,7 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
             }
           }
           gm_commit(&acc_bar);
-          GM_TR(l, 3);
         }
-      }
-      if (g.head) {
-        // hout's partial product over this CTA's K slice, straight from the staged output tiles: hi*hi into TMEM
-        // columns 0..15, the two cross products into columns 16..31 (N = 16: the head's 4 rows + zero-filled ones)
-        gm_mbar_wait(&tmem_free_bar, (tile - 1) & 1u);   // the last layer's accumulators have been read
-        gm_mbar_wait(&stage_ready_bar, 0);                // its output tiles are staged (and fenced for the async proxy)
-        gm_mbar_wait(&head_full_bar, 0);                  // the weights' K slice has landed
-        gm_tc_fence_after();
-        constexpr uint32_t IDESC16 = GM_IDESC_N(16);
-        for (int p = 0; p < head_parts; ++p) {
-          const uint32_t a_hi = gm_desc_lo(head_a_hi(p)), a_lo = a_hi + (SUB_BYTES >> 4);
-          const uint32_t w_hi = gm_desc_lo(head_w_hi(p)), w_lo = w_hi + (GM_W_BYTES >> 4);
-#pragma unroll
-          for (int k = 0; k < GM_BK / 8; ++k)
-            gm_mma_tf32(tmem + 16u, gm_desc(a_lo + 2 * k), gm_desc(w_hi + 2 * k), IDESC16, (p > 0 || k > 0) ? 1u : 0u);
-#pragma unroll
-          for (int k = 0; k < GM_BK / 8; ++k)
-            gm_mma_tf32(tmem + 16u, gm_desc(a_hi + 2 * k), gm_desc(w_lo + 2 * k), IDESC16, 1u);
-#pragma unroll
-          for (int k = 0; k < GM_BK / 8; ++k)
-            gm_mma_tf32(tmem, gm_desc(a_hi + 2 * k), gm_desc(w_hi + 2 * k), IDESC16, (p > 0 || k > 0) ? 1u : 0u);
-        }
-        gm_commit(&head_acc_bar);
       }
     }
     __syncwarp();
@@ -1166,7 +1053,6 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
         const bool any = n0 + cbeg < g.N;   // warp-uniform (and uniform over the part's four warps)
         gm_mbar_wait(&acc_bar, tile & 1u, true);
         gm_tc_fence_after();
-        if (threadIdx.x == 64) GM_TR(l, 4);
 #pragma unroll 1
         for (int c0 = cbeg; c0 < cend; c0 += 16) {
           if (n0 + c0 >= g.N) break;   // warp-uniform
@@ -1197,10 +1083,7 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
         __syncwarp();
         if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(rd_smem_u32(&tmem_free_bar)) : "memory");
         asm volatile("bar.sync %0, 128;" ::"r"(1 + part) : "memory");    // the part's four warps
-        const bool to_head = g.head && l + 1 == g.n_layers;   // the tiles feed the fused head instead of leaving the SM
-        if (q == 0 && lane == 0 && to_head) {
-          asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(rd_smem_u32(&stage_ready_bar)) : "memory");
-        } else if (q == 0 && lane == 0) {
+        if (q == 0 && lane == 0) {
           if (any) {
             const CUtensorMap* mo = l + 1 < g.n_layers ? &maps.a[l + 1][0] : &maps.o_last[0];
             const CUtensorMap* mo2 = l + 1 < g.n_layers ? &maps.a[l + 1][1] : &maps.o_last[1];
@@ -1209,7 +1092,6 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
             asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%1, %2}], [%3];" ::"l"(
                              reinterpret_cast<uint64_t>(mo2)), "r"(n0 + cbeg), "r"(mb * GM_BM), "r"(s_lo) : "memory");
             asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            GM_TR(l, 6 + part);
             asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
           }
           asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(rd_smem_u32(&epi_done_bar)) : "memory");
@@ -1218,31 +1100,13 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
               asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
               asm volatile("fence.proxy.async;" ::: "memory");
             }
-            GM_TR(l, 10 + part);
             __threadfence();
             atomicAdd(g.flags + (size_t)l * g.row_blocks + mb, 1u);
           }
         }
-        if (threadIdx.x == 64) GM_TR(l, 5);
       }
     }
     if (q == 0 && lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // the last tile's stores
-    if (g.head && part == 0) {
-      // this CTA's partial [128][4] of hout -> slot blockIdx.x of the cluster's first CTA (distributed shared memory).
-      // NOTE (why the fused head is opt-in): nothing but the co-scheduling of a cluster and the row-block counters this
-      // CTA has consumed tells it that the first CTA is running; the programming model wants a cluster barrier before the
-      // first remote access (a plain arrive + wait right after the set-up would do), and racecheck says so.  That
-      // variant is not shipped because it could not be re-validated on a GPU (profiles/r5b_dreamer_chain.txt).
-      gm_mbar_wait(&head_acc_bar, 0, true);
-      gm_tc_fence_after();
-      float m8[8], s8[8];
-      gm_tmem_ld8(tl, m8);
-      gm_tmem_ld8(tl + 16u, s8);
-      const float4 v = make_float4(m8[0] + s8[0], m8[1] + s8[1], m8[2] + s8[2], m8[3] + s8[3]);
-      uint32_t remote;
-      asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(rd_smem_u32(&head_red[blockIdx.x][r])), "r"(0));
-      asm volatile("st.shared::cluster.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(remote), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-    }
     gm_tc_fence_before();
   }
   __syncthreads();
@@ -1250,34 +1114,6 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
     gm_tc_fence_after();
     gm_tmem_free(tmem, TM_COLS);
   }
-  if (g.head) {
-    // every thread of the cluster arrives; the first CTA waits for the other three's partials, adds them in CTA order
-    // and stores hout's pre-activations (the others may exit: nobody writes into their shared memory)
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    if (blockIdx.x == 0) {
-      asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-      if (warp >= 2 && ((warp - 2) >> 2) == 0) {
-        const int rr = (warp & 3) * 32 + lane;
-        const int row = (int)blockIdx.y * GM_BM + rr;
-        if (row < g.M) {
-          float4 o = head_red[0][rr];
-          for (int x = 1; x < (int)gridDim.x; ++x) { const float4 t = head_red[x][rr]; o.x += t.x; o.y += t.y; o.z += t.z; o.w += t.w; }
-          o.x += __ldg(g.head_bias + 0); o.y += __ldg(g.head_bias + 1); o.z += __ldg(g.head_bias + 2); o.w += __ldg(g.head_bias + 3);
-          *reinterpret_cast<float4*>(g.head_out + (size_t)row * 4) = o;
-        }
-      }
-    }
-  }
-#ifdef GM_CHAIN_TRACE
-  if (threadIdx.x == 0 && g.L[0].target == 40u * gridDim.x * EW && (blockIdx.y % 8) == 0)
-    for (int l = 0; l < g.n_layers; ++l)
-      printf("CHAIN cta (%d,%d) layer %d: W issued %lld | staged tiles read %lld | A issued %lld | first full %lld | MMAs issued %lld | acc ready %lld | "
-             "stores issued %lld %lld %lld %lld | stores complete %lld %lld %lld %lld | part 0 counted %lld\n",
-             blockIdx.x, blockIdx.y, l, tr[l][0] - tr0, tr[l][14] - tr0, tr[l][1] - tr0, tr[l][2] - tr0, tr[l][3] - tr0, tr[l][4] - tr0,
-             tr[l][6] - tr0, tr[l][7] - tr0, tr[l][8] - tr0, tr[l][9] - tr0, tr[l][10] - tr0, tr[l][11] - tr0, tr[l][12] - tr0,
-             tr[l][13] - tr0, tr[l][5] - tr0);
-#endif
-#undef GM_TR
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1337,11 +1173,7 @@ static inline cudaError_t gm_launch(const GemmMaps& maps, const GemmArgs& g, cud
 }
 
 template <int GM_STAGES, int EW, int BN>
-// g.head != 0 asks for the fused output head; *head_fused tells whether this launch could take it (cluster launch, one
-// row block per cluster) -- if not, the caller runs the head as a k_dense launch of its own.
-static inline cudaError_t gm_launch_chain(const ChainMaps& maps, const ChainArgs& g_in, int sm_count, bool cluster, cudaStream_t s,
-                                          bool* head_fused) {
-  ChainArgs g = g_in;
+static inline cudaError_t gm_launch_chain(const ChainMaps& maps, const ChainArgs& g, int sm_count, cudaStream_t s) {
   constexpr size_t smem = (size_t)GM_STAGES * 2 * (GM_A_BYTES + BN * 128) + 1024;
   static bool attr = false;
   static int max_clusters = -1;   // co-resident clusters of this shape on this device (cluster launches)
@@ -1365,7 +1197,7 @@ static inline cudaError_t gm_launch_chain(const ChainMaps& maps, const ChainArgs
   // the grid is then sized to the clusters that fit at once only to keep the work in one wave.  Without clusters the
   // guarantee is the grid size (one CTA per SM, whole row-block groups, CTAs dispatched in index order).
   int groups = std::max(1, std::min(g.row_blocks, sm_count / nt));
-  if (cluster && nt <= 8) {
+  if (nt <= 8) {
     attrs[1].id = cudaLaunchAttributeClusterDimension;
     attrs[1].val.clusterDim.x = (unsigned)nt; attrs[1].val.clusterDim.y = 1; attrs[1].val.clusterDim.z = 1;
     cfg.numAttrs = 2;
@@ -1375,12 +1207,9 @@ static inline cudaError_t gm_launch_chain(const ChainMaps& maps, const ChainArgs
       cudaError_t e = cudaOccupancyMaxActiveClusters(&q, k_dense_chain<GM_STAGES, EW, BN>, &cfg);
       if (e != cudaSuccess) return e;
       max_clusters = std::max(1, q);
-      if (std::getenv("RD_DREAMER_DEBUG")) std::fprintf(stderr, "k_dense_chain: %d clusters of %d CTAs fit at once\n", max_clusters, nt);
     }
     groups = std::min(groups, max_clusters);
   }
-  g.head = (g.head && cfg.numAttrs == 2 && groups == g.row_blocks && nt <= 4) ? 1 : 0;
-  if (head_fused) *head_fused = g.head != 0;
   cfg.gridDim = dim3((unsigned)nt, (unsigned)groups);
   return cudaLaunchKernelEx(&cfg, k_dense_chain<GM_STAGES, EW, BN>, maps, g);
 }

@@ -4,7 +4,7 @@ OUT=gpurun_out/${1:-var}; mkdir -p $OUT
 for v in variants/*.so; do
   for rep in 1 2; do
     echo "== $v" | tee -a $OUT/variants.log
-    RD_ENV_LIB=$PWD/$v RD_SWEEP=austria:4096:2 python tools/lidar_sweep.py 2>&1 | tail -1 | tee -a $OUT/variants.log
+    RD_ENV_LIB=$PWD/$v RD_SWEEP=austria:4096 python tools/lidar_sweep.py 2>&1 | tail -1 | tee -a $OUT/variants.log
   done
 done
 timeout 600 python -m pytest tests -x -q -m gpu 2>&1 | tail -3

@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""GPU tuning sweep of k_lidar: clearance block size (RD_LIDAR_CSHIFT) x track, timed with rd_enable_timing."""
+"""Per-launch times of k_lidar and k_step over tracks and batch sizes, timed with rd_enable_timing."""
 import json
 import os
 import sys
@@ -12,8 +12,7 @@ sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
 from racing_dreamer_b200 import BatchedRaceEnv, EnvConfig  # noqa: E402
 
 
-def run(track, n, cshift, steps=200):
-    os.environ["RD_LIDAR_CSHIFT"] = str(cshift)
+def run(track, n, steps=200):
     env = BatchedRaceEnv(EnvConfig(tracks=(track,), n_envs=n, action_repeat=8, auto_reset=True, reset_mode="random", seed=1,
                                    time_limit_steps=250), device="cuda:0")
     rng = np.random.RandomState(0)
@@ -32,18 +31,16 @@ def run(track, n, cshift, steps=200):
 
 if __name__ == "__main__":
     out = []
-    spec = os.environ.get("RD_SWEEP")   # e.g. "austria:4096:2" = one point
+    spec = os.environ.get("RD_SWEEP")   # e.g. "austria:4096" = one point
     if spec:
-        tr, nn, cc = spec.split(":")
-        grid = [(tr, int(nn), int(cc))]
+        tr, nn = spec.split(":")
+        grid = [(tr, int(nn))]
     else:
-        grid = [(t, n, c) for t in ("austria", "columbia", "barcelona") for n in (4096, 16384) for c in (1, 2, 3)]
-    if True:
-        if True:
-            for track, n, cs in grid:
-                try:
-                    l, s = run(track, n, cs)
-                    out.append(dict(track=track, n=n, cshift=cs, lidar_ms=l, step_ms=s, rays_per_s=n * 1080 / l * 1e3))
-                except Exception as e:  # e.g. map + field too large for shared memory
-                    out.append(dict(track=track, n=n, cshift=cs, error=str(e)[:100]))
-                print(json.dumps(out[-1]), flush=True)
+        grid = [(t, n) for t in ("austria", "columbia", "barcelona") for n in (4096, 16384)]
+    for track, n in grid:
+        try:
+            l, s = run(track, n)
+            out.append(dict(track=track, n=n, lidar_ms=l, step_ms=s, rays_per_s=n * 1080 / l * 1e3))
+        except Exception as e:  # e.g. map too large for shared memory
+            out.append(dict(track=track, n=n, error=str(e)[:100]))
+        print(json.dumps(out[-1]), flush=True)

@@ -35,14 +35,16 @@ int main() {
     CK(cudaMemcpy(dW, W.data(), W.size() * 4, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(db, b.data(), N * 4, cudaMemcpyHostToDevice));
     CK(cudaMemset(dO, 0, (size_t)M * N * 4));
-    CUtensorMap ma, mw;
-    if (!gm_make_map(&ma, dA, K, M, K, GM_BM) || !gm_make_map(&mw, dW, K, N, K, GM_BN)) { printf("T1 map encode failed\n"); return 3; }
+    CUtensorMap ma, mw, mo;
+    if (!gm_make_map(&ma, dA, K, M, K, GM_BM) || !gm_make_map(&mw, dW, K, N, K, GM_BN) || !gm_make_map(&mo, dO, N, M, N, GM_BM)) {
+      printf("T1 map encode failed\n"); return 3;
+    }
     GemmArgs g{};
     g.M = M; g.N = N; g.n_phases = 1; g.n_acc = 1;
     g.ph[0].k_blocks = (K + 31) / 32; g.ph[0].nb = 1; g.ph[0].w_row0[0] = 0; g.ph[0].acc[0] = 0;
     g.bias = db; g.out = dO; g.ldo = N; g.act = 1;
     GemmMaps maps{};
-    maps.a[0] = ma; maps.w[0] = mw;
+    maps.a[0] = ma; maps.w[0] = mw; maps.o[0] = mo;
     CK((gm_launch<EPI_DENSE, 1, 4, 4>(maps, g, 0)));
     CK(cudaDeviceSynchronize());
     std::vector<float> O((size_t)M * N);
@@ -73,16 +75,16 @@ int main() {
     CK(cudaMemcpy(dL, L.data(), L.size() * 4, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(dW, W.data(), W.size() * 4, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(db, b.data(), N * 4, cudaMemcpyHostToDevice));
-    CUtensorMap ma0, ma1, mw;
+    CUtensorMap ma0, ma1, mw, mo;
     if (!gm_make_map(&ma0, dF + 32, K0, M, LD0, GM_BM) || !gm_make_map(&ma1, dL, K1, M, K1, GM_BM) ||
-        !gm_make_map(&mw, dW, K0 + K1, N, K0 + K1, GM_BN)) { printf("T2 map encode failed\n"); return 3; }
+        !gm_make_map(&mw, dW, K0 + K1, N, K0 + K1, GM_BN) || !gm_make_map(&mo, dO, N, M, N, GM_BM)) { printf("T2 map encode failed\n"); return 3; }
     GemmArgs g{};
     g.M = M; g.N = N; g.n_phases = 2; g.n_acc = 1;
     g.ph[0].k_blocks = (K0 + 31) / 32; g.ph[0].nb = 1; g.ph[0].w_k0 = 0;
     g.ph[1].k_blocks = (K1 + 31) / 32; g.ph[1].nb = 1; g.ph[1].w_k0 = K0; g.ph[1].a_map = 1;
     g.bias = db; g.out = dO; g.ldo = N; g.act = 0;
     GemmMaps maps{};
-    maps.a[0] = ma0; maps.a[1] = ma1; maps.w[0] = mw;
+    maps.a[0] = ma0; maps.a[1] = ma1; maps.w[0] = mw; maps.o[0] = mo;
     CK((gm_launch<EPI_DENSE, 1, 4, 4>(maps, g, 0)));
     CK(cudaDeviceSynchronize());
     std::vector<float> O((size_t)M * N);
@@ -117,9 +119,10 @@ int main() {
     CK(cudaMemcpy(dWr, Wr.data(), Wr.size() * 4, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(db, b.data(), b.size() * 4, cudaMemcpyHostToDevice));
     CK(cudaMemset(dO, 0, (size_t)M * LD * 4));
-    CUtensorMap mx, mh, mwk, mwr;
+    CUtensorMap mx, mh, mwk, mwr, mo;
     if (!gm_make_map(&mx, dX, H, M, H, GM_BM) || !gm_make_map(&mh, dF + 32, H, M, LD, GM_BM) ||
-        !gm_make_map(&mwk, dWk, H, 3 * H, H, GM_BN) || !gm_make_map(&mwr, dWr, H, 3 * H, H, GM_BN)) { printf("T3 map encode failed\n"); return 3; }
+        !gm_make_map(&mwk, dWk, H, 3 * H, H, GM_BN) || !gm_make_map(&mwr, dWr, H, 3 * H, H, GM_BN) ||
+        !gm_make_map(&mo, dO + 32, H, M, LD, GM_BM)) { printf("T3 map encode failed\n"); return 3; }
     GemmArgs g{};
     g.M = M; g.N = H; g.n_phases = 2; g.n_acc = 1;
     for (int p = 0; p < 2; ++p) {
@@ -129,7 +132,7 @@ int main() {
     }
     g.bias = db; g.out = dO + 32; g.ldo = LD; g.hold = dF + 32; g.ldh = LD;
     GemmMaps maps{};
-    maps.a[0] = mx; maps.a[1] = mh; maps.w[0] = mwk; maps.w[1] = mwr;
+    maps.a[0] = mx; maps.a[1] = mh; maps.w[0] = mwk; maps.w[1] = mwr; maps.o[0] = mo;
     CK((gm_launch<EPI_GRU, 3, 8, 4>(maps, g, 0)));
     CK(cudaDeviceSynchronize());
     std::vector<float> O((size_t)M * LD);
