@@ -71,28 +71,30 @@ def n_actor_layers(w) -> int:
     return sum(1 for k in w if k.startswith("h") and k.endswith("_w") and k[1:-2].isdigit())
 
 
-def random_weights(seed: int, n_beams: int = 1080, normalized: bool = False, actor_layers: int = ACTOR_LAYERS) -> Dict[str, np.ndarray]:
-    """Glorot-ish random weights of the shipped architecture (for tests on machines without the checkpoints);
-    actor_layers other than the shipped four exercise the product's general trunk path."""
+def random_weights(seed: int, n_beams: int = 1080, normalized: bool = False, actor_layers: int = ACTOR_LAYERS,
+                   deter: int = DETER, hidden: int = HIDDEN, units: int = ACTOR_UNITS) -> Dict[str, np.ndarray]:
+    """Glorot-ish random weights (for tests on machines without the checkpoints), by default of the shipped
+    architecture; other trunk depths and widths (deter, hidden, units, n_beams = embed) exercise the product's general
+    paths.  The draws are made in one fixed order, so the default arguments give the same arrays whatever the others."""
     rng = np.random.RandomState(seed)
 
     def dense(i, o):
         return (rng.uniform(-1, 1, (i, o)) * np.sqrt(3.0 / i)).astype(np.float32), (rng.uniform(-0.1, 0.1, o)).astype(np.float32)
 
     w = {}
-    w["gru_kernel"], _ = dense(HIDDEN, 3 * DETER)
-    w["gru_recurrent"], _ = dense(DETER, 3 * DETER)
-    w["gru_bias"] = rng.uniform(-0.1, 0.1, (2, 3 * DETER)).astype(np.float32)
-    w["img1_w"], w["img1_b"] = dense(STOCH + 2, HIDDEN)
-    w["img2_w"], w["img2_b"] = dense(DETER, HIDDEN)
-    w["img3_w"], w["img3_b"] = dense(HIDDEN, 2 * STOCH)
-    w["obs1_w"], w["obs1_b"] = dense(DETER + n_beams, HIDDEN)
-    w["obs2_w"], w["obs2_b"] = dense(HIDDEN, 2 * STOCH)
-    i = STOCH + DETER
+    w["gru_kernel"], _ = dense(hidden, 3 * deter)
+    w["gru_recurrent"], _ = dense(deter, 3 * deter)
+    w["gru_bias"] = rng.uniform(-0.1, 0.1, (2, 3 * deter)).astype(np.float32)
+    w["img1_w"], w["img1_b"] = dense(STOCH + 2, hidden)
+    w["img2_w"], w["img2_b"] = dense(deter, hidden)
+    w["img3_w"], w["img3_b"] = dense(hidden, 2 * STOCH)
+    w["obs1_w"], w["obs1_b"] = dense(deter + n_beams, hidden)
+    w["obs2_w"], w["obs2_b"] = dense(hidden, 2 * STOCH)
+    i = STOCH + deter
     for k in range(actor_layers):
-        w[f"h{k}_w"], w[f"h{k}_b"] = dense(i, ACTOR_UNITS)
-        i = ACTOR_UNITS
-    w["hout_w"], w["hout_b"] = dense(ACTOR_UNITS, 4)
+        w[f"h{k}_w"], w[f"h{k}_b"] = dense(i, units)
+        i = units
+    w["hout_w"], w["hout_b"] = dense(units, 4)
     if normalized:
         w["bn_gamma"] = rng.uniform(0.5, 2.0, 4).astype(np.float32)
         w["bn_beta"] = rng.uniform(-0.5, 0.5, 4).astype(np.float32)
@@ -185,12 +187,13 @@ def mode(mean, std, eps_actor):
 
 
 def policy_step(w, scan, state: Optional[Tuple[np.ndarray, np.ndarray, np.ndarray]], eps_stoch, eps_actor, dtype=np.float64):
-    """RacingDreamer.action for a batch [REF racing_dreamer.py:62-82].  state = (stoch, deter, action) or None.
-    Returns (agent-facing action in [-1, 1], new state, diagnostics)."""
+    """RacingDreamer.action for a batch [REF racing_dreamer.py:62-82].  state = (stoch, deter, action) or None (zeros,
+    deter as wide as the weights' GRU).  Returns (agent-facing action in [-1, 1], new state, diagnostics)."""
     n = scan.shape[0]
     embed = preprocess_lidar(scan)
     if state is None:
-        stoch, deter, action = np.zeros((n, STOCH), dtype), np.zeros((n, DETER), dtype), np.zeros((n, 2), dtype)
+        d = w["gru_recurrent"].shape[0]
+        stoch, deter, action = np.zeros((n, STOCH), dtype), np.zeros((n, d), dtype), np.zeros((n, 2), dtype)
     else:
         stoch, deter, action = state
     mean, std, stoch, deter = obs_step(w, stoch, deter, action, embed, eps_stoch, dtype)

@@ -1176,7 +1176,7 @@ template <int GM_STAGES, int EW, int BN>
 static inline cudaError_t gm_launch_chain(const ChainMaps& maps, const ChainArgs& g, int sm_count, cudaStream_t s) {
   constexpr size_t smem = (size_t)GM_STAGES * 2 * (GM_A_BYTES + BN * 128) + 1024;
   static bool attr = false;
-  static int max_clusters = -1;   // co-resident clusters of this shape on this device (cluster launches)
+  static int max_clusters[9] = {};   // co-resident clusters of this shape on this device, per cluster width (0: not asked yet)
   if (!attr) {
     cudaError_t e = cudaFuncSetAttribute(k_dense_chain<GM_STAGES, EW, BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
@@ -1201,14 +1201,14 @@ static inline cudaError_t gm_launch_chain(const ChainMaps& maps, const ChainArgs
     attrs[1].id = cudaLaunchAttributeClusterDimension;
     attrs[1].val.clusterDim.x = (unsigned)nt; attrs[1].val.clusterDim.y = 1; attrs[1].val.clusterDim.z = 1;
     cfg.numAttrs = 2;
-    if (max_clusters < 0) {
+    if (max_clusters[nt] == 0) {
       cfg.gridDim = dim3((unsigned)nt, (unsigned)groups);
       int q = 0;
       cudaError_t e = cudaOccupancyMaxActiveClusters(&q, k_dense_chain<GM_STAGES, EW, BN>, &cfg);
       if (e != cudaSuccess) return e;
-      max_clusters = std::max(1, q);
+      max_clusters[nt] = std::max(1, q);
     }
-    groups = std::min(groups, max_clusters);
+    groups = std::min(groups, max_clusters[nt]);
   }
   cfg.gridDim = dim3((unsigned)nt, (unsigned)groups);
   return cudaLaunchKernelEx(&cfg, k_dense_chain<GM_STAGES, EW, BN>, maps, g);

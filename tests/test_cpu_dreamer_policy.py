@@ -106,3 +106,93 @@ def test_mode_is_first_argmax_of_log_prob():
     assert np.allclose(act, np.tanh(u[np.arange(5), idx]))
     a0, _, i0, _ = dp.mode(mean, std, None)                 # zero-noise variant
     assert np.allclose(a0, np.tanh(mean)) and (i0 == 0).all()
+
+
+def _torch_step(w, scan, state, eps_stoch, eps_actor):
+    """The agent step restated with torch.nn modules in float64: Linear layers for img1, obs1, obs2, the actor trunk
+    and hout, torch.nn.GRUCell (gate blocks permuted as in test_gru_cell_matches_torch), BatchNorm1d in eval mode for
+    the 'normalized' head, torch.distributions.Normal for the base log-density and log|d tanh(u)/du| = -2 log cosh(u)
+    (torch's TanhTransform clips its softplus at 20, 2e-9 away from the exact value for |u| > 10)."""
+    import torch
+    import torch.nn.functional as F
+    t = lambda a: torch.from_numpy(np.asarray(a, np.float64))   # noqa: E731
+
+    def linear(name_w, name_b):
+        k = w[name_w]
+        lin = torch.nn.Linear(k.shape[0], k.shape[1]).double()
+        with torch.no_grad():
+            lin.weight.copy_(t(k.T))
+            lin.bias.copy_(t(w[name_b]))
+        return lin
+
+    deter_n = w["gru_recurrent"].shape[0]
+    cell = torch.nn.GRUCell(w["gru_kernel"].shape[0], deter_n).double()
+    perm = np.r_[deter_n:2 * deter_n, 0:deter_n, 2 * deter_n:3 * deter_n]
+    with torch.no_grad():
+        cell.weight_ih.copy_(t(w["gru_kernel"].T[perm]))
+        cell.weight_hh.copy_(t(w["gru_recurrent"].T[perm]))
+        cell.bias_ih.copy_(t(w["gru_bias"][0][perm]))
+        cell.bias_hh.copy_(t(w["gru_bias"][1][perm]))
+    softplus = lambda x: F.softplus(x, threshold=50.0)   # noqa: E731  (log1p(exp(x)) over the whole range used here)
+    stoch, deter, action = (t(s) for s in state)
+    with torch.no_grad():
+        embed = (torch.clamp(t(scan), 0.0, 15.0) / 15.0 - 0.5).float().double()   # the scans are preprocessed in float32
+        x = F.elu(linear("img1_w", "img1_b")(torch.cat([stoch, action], -1)))
+        deter = cell(x, deter)
+        x = F.elu(linear("obs1_w", "obs1_b")(torch.cat([deter, embed], -1)))
+        mean, raw = linear("obs2_w", "obs2_b")(x).split(dp.STOCH, -1)
+        std = softplus(raw) + 0.1
+        stoch = mean + std * t(eps_stoch)
+        x = torch.cat([stoch, deter], -1)
+        for i in range(dp.n_actor_layers(w)):
+            x = F.elu(linear(f"h{i}_w", f"h{i}_b")(x))
+        x = linear("hout_w", "hout_b")(x)
+        if "bn_gamma" in w:
+            bn = torch.nn.BatchNorm1d(4, eps=dp.BN_EPS).double().eval()
+            bn.weight.copy_(t(w["bn_gamma"]))
+            bn.bias.copy_(t(w["bn_beta"]))
+            bn.running_mean.copy_(t(w["bn_mean"]))
+            bn.running_var.copy_(t(w["bn_var"]))
+            x = bn(x)
+            amean, astd = x[:, :2], softplus(x[:, 2:]) + dp.MIN_STD
+        else:
+            amean = dp.MEAN_SCALE * torch.tanh(x[:, :2] / dp.MEAN_SCALE)
+            astd = softplus(x[:, 2:] + float(np.log(np.exp(dp.INIT_STD) - 1))) + dp.MIN_STD
+        u = amean[:, None] + astd[:, None] * t(eps_actor)
+        lp = (torch.distributions.Normal(amean[:, None], astd[:, None]).log_prob(u) + 2.0 * torch.log(torch.cosh(u))).sum(-1)
+    return {k: v.numpy() for k, v in dict(mean=mean, std=std, stoch=stoch, deter=deter, actor_mean=amean,
+                                          actor_std=astd, logp_all=lp).items()}
+
+
+@pytest.mark.parametrize("deter,hidden,units,embed,layers,normalized", [
+    (36, 100, 132, 100, 3, False), (4, 4, 4, 4, 1, False), (212, 28, 32, 360, 5, True), (516, 1028, 1028, 2048, 2, False)])
+def test_oracle_matches_torch_at_other_architectures(deter, hidden, units, embed, layers, normalized):
+    """The oracle generalised to any width (random_weights, policy_step) == an independent torch.nn restatement to
+    1e-12: what makes it the yardstick of the kernels at architectures other than the shipped one."""
+    w = dp.random_weights(7, n_beams=embed, normalized=normalized, actor_layers=layers, deter=deter, hidden=hidden, units=units)
+    assert w["gru_recurrent"].shape == (deter, 3 * deter) and w["obs1_w"].shape == (deter + embed, hidden)
+    assert dp.n_actor_layers(w) == layers and w["hout_w"].shape == (units, 4) and w[f"h{layers - 1}_w"].shape[1] == units
+    rng = np.random.RandomState(1)
+    n, S = 24, 37
+    scan = rng.uniform(-1, 18, (n, embed))
+    state = (rng.standard_normal((n, 30)), rng.uniform(-1, 1, (n, deter)), rng.uniform(-1, 1, (n, 2)))
+    es, ea = rng.standard_normal((n, 30)), rng.standard_normal((n, S, 2))
+    act, new_state, d = dp.policy_step(w, scan, state, es, ea, np.float64)
+    ref = _torch_step(w, scan, state, es, ea)
+    got = dict(mean=d["mean"], std=d["std"], stoch=new_state[0], deter=new_state[1], actor_mean=d["actor_mean"],
+               actor_std=d["actor_std"], logp_all=d["logp_all"])
+    for k, v in got.items():
+        assert v.shape == ref[k].shape and np.abs(v - ref[k]).max() <= 1e-12 * max(1.0, np.abs(ref[k]).max()), k
+    assert np.array_equal(d["index"], ref["logp_all"].argmax(-1))
+    # the zero state is as wide as the weights' GRU
+    _, s0, _ = dp.policy_step(w, scan, None, es, ea, np.float64)
+    assert s0[1].shape == (n, deter)
+
+
+def test_random_weights_defaults_unchanged():
+    """the generalised random_weights draws the shipped architecture's arrays exactly as before (the goldens and the
+    GPU tests' weights depend on them): the default widths given explicitly change nothing"""
+    a = dp.random_weights(11, normalized=True)
+    b = dp.random_weights(11, n_beams=1080, normalized=True, actor_layers=4, deter=200, hidden=200, units=400)
+    assert set(a) == set(b) and all(np.array_equal(a[k], b[k]) for k in a)
+    assert a["gru_kernel"].shape == (200, 600) and a["h3_w"].shape == (400, 400) and a["obs1_w"].shape == (1280, 200)

@@ -92,6 +92,14 @@ def posterior_normals(seed, n, step, gid0=0):
     return np.concatenate([normal4(seed, np.arange(n) + gid0, step, j0, STREAM_STOCH) for j0 in range(0, 32, 4)], -1)[:, :30]
 
 
+def actor_normals(seed, n, step, n_samples, gid0=0):
+    """eps_actor [n, n_samples, 2] of evaluation step `step` (k_actor_mode's Philox draws): draw s takes normals
+    2 (s % 2) + d of block (gid, step, s - s % 2, RD_STREAM_ACTOR)."""
+    gid = np.arange(n) + gid0
+    z = [normal4(seed, gid, step, s0, STREAM_ACTOR).reshape(n, 2, 2) for s0 in range(0, n_samples, 2)]
+    return np.concatenate(z, 1)[:, :n_samples]
+
+
 @pytest.mark.parametrize("amount,decay,floor", [(0.3, 0.0, 0.0), (0.3, 5e5, 0.0), (0.3, 5e5, 0.05), (0.3, 0.0, 0.5),
                                                 (1.0, 1234.5, 0.0), (0.0, 0.0, 0.1)])
 def test_schedule_equals_the_restated_formula(amount, decay, floor):
@@ -153,6 +161,21 @@ def test_training_draws_on_the_numpy_philox():
     assert np.array_equal(train_normals(seed, 8, 5, 100)[1], e2)
     z = np.concatenate([np.concatenate(train_normals(7, 4096, s), -1) for s in range(8)]).ravel()
     assert abs(z.mean()) < 0.01 and abs(z.std() - 1.0) < 0.01
+
+
+@pytest.mark.parametrize("n_samples", [1, 3, 100, 257])
+def test_actor_draws_on_the_numpy_philox(n_samples):
+    seed, n, step, gid0 = 0x0123456789ABCDEF, 5, 7, 4096
+    ea = actor_normals(seed, n, step, n_samples, gid0)
+    assert ea.shape == (n, n_samples, 2)
+    for row, s in [(0, 0), (4, n_samples - 1), (2, n_samples // 2)]:
+        z = normal4(seed, np.array([gid0 + row]), step, s - s % 2, STREAM_ACTOR)[0]
+        assert np.array_equal(ea[row, s], z[2 * (s % 2): 2 * (s % 2) + 2])
+    # another step, another rank: other draws; the posterior's stream at the same (env, step) is another one too
+    if n_samples > 1:
+        assert not np.allclose(actor_normals(seed, n, step + 1, n_samples, gid0), ea)
+        assert not np.allclose(actor_normals(seed, n, step, n_samples, 0), ea)
+        assert not np.allclose(posterior_normals(seed, n, step, gid0)[:, :2], ea[:, 0])
 
 
 def test_training_step_restatement_against_an_independent_evaluation():

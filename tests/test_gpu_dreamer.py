@@ -58,14 +58,15 @@ def close(name, got, ref, rtol=RTOL, atol=ATOL, floor=0.0):
     return float(np.abs(got - ref).max())
 
 
-def check_mode(diag, ref, t=None, precision="tf32x3"):
-    """the kernel's argmax is the oracle's, or a near tie under the oracle's log-probabilities"""
+def check_mode(diag, ref, t=None, precision="tf32x3", tie=1.0):
+    """the kernel's argmax is the oracle's, or a near tie under the oracle's log-probabilities (within `tie` x LP_TIE:
+    a wider actor-head bar widens the margin with it)"""
     idx = diag["index"].cpu().numpy().astype(np.int64)
     lp_all = ref["logp_all"] if t is None else ref["logp_all"][t]
     ridx = ref["index"] if t is None else ref["index"][t]
     rows = np.arange(idx.shape[0])
     gap = lp_all[rows, ridx] - lp_all[rows, idx]
-    assert (gap <= LP_TIE[precision]).all(), f"mode(): picked a draw {gap.max():.3e} below the maximum log-probability"
+    assert (gap <= tie * LP_TIE[precision]).all(), f"mode(): picked a draw {gap.max():.3e} below the maximum log-probability"
     return float((idx == ridx).mean())
 
 
@@ -287,10 +288,11 @@ def test_actor_chain_is_bitwise_the_per_layer_launches(torch_cuda, weights, monk
         assert torch.equal(a, b)
 
 
-@pytest.mark.parametrize("layers", [1, 6])
+@pytest.mark.parametrize("layers", [1, 2, 3, 5, 6, 7])
 def test_actor_trunk_depths_other_than_the_shipped_four(torch_cuda, layers):
-    """The C ABI takes 1..7 trunk layers; k_dense_chain runs them four per launch (6 = a launch of four and one of two,
-    1 = a launch without any counter).  Random weights, explicit noise, against the float64 restatement."""
+    """The C ABI takes 1..7 trunk layers; k_dense_chain runs them four per launch (1 = a launch without any counter,
+    2 / 3 = one launch of that many, 5 / 6 / 7 = a launch of four and one of one / two / three).  Random weights,
+    explicit noise, against the float64 restatement."""
     torch = torch_cuda
     from racing_dreamer_b200 import DreamerPolicy
     n = 700
