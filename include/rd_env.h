@@ -355,6 +355,36 @@ int rd_rollout_dreamer_train(rd_env* env, int n_steps, const rd_outputs* out, fl
  * (else RD_ERR_INVALID and nothing changes). */
 int rd_policy_dreamer_set_weights(rd_env* env, const rd_dreamer_weights* w, int on_device, void* stream);
 
+/* Dreamer agent on 'lidar_occupancy' observations [REF dreamer/dream.py:64-66]: the image encoder ConvEncoder
+ * [UPSTREAM-RECALL: danijar Dreamer models.py ConvEncoder] replaces _preprocess_lidar in front of the same RSSM and actor.
+ * The u8 image [N,64,64] is cast to float (no scaling), then four Conv2D(kernel 4, stride 2, 'valid', relu) layers with
+ * depth, 2 depth, 4 depth, 8 depth filters (31x31, 14x14, 6x6, 2x2 outputs); the 2x2x(8 depth) output flattened in
+ * (y, x, c) order is the embed (32 depth floats) obs1 reads.  conv1 runs on CUDA cores, conv2..conv4 as implicit GEMMs
+ * on the k_dense tensor-core kernel (csrc/rd_gemm.cuh).  Only depth 32 (the reference's cnn_depth) is accepted. */
+typedef struct rd_dreamer_conv_encoder {
+  int32_t depth;              /* cnn_depth: 32 */
+  const float* w[4];          /* Keras Conv2D kernels [4][4][Cin][Cout], Cin = 1, d, 2d, 4d; Cout = d, 2d, 4d, 8d */
+  const float* b[4];          /* [Cout] */
+} rd_dreamer_conv_encoder;
+/* As rd_policy_dreamer_init, for an encoder agent: w->embed = 32 * enc->depth (obs1_w [deter + embed][hidden]); the env
+ * must produce occupancy (RD_OBS_OCCUPANCY).  Allocates the encoder's activations (~0.4 MB per env in tf32x3).  Re-init
+ * with either init replaces the agent; a rejected call leaves the current one working. */
+int rd_policy_dreamer_init_occupancy(rd_env* env, const rd_dreamer_weights* w, const rd_dreamer_conv_encoder* enc);
+/* rd_policy_dreamer / rd_policy_dreamer_train for an encoder agent: occupancy_dev u8 [N,64,64] (an rd_step output). */
+int rd_policy_dreamer_occupancy(rd_env* env, const uint8_t* occupancy_dev, float* actions_dev, int noise,
+                                const float* eps_stoch_dev, const float* eps_actor_dev, float* debug_dev, void* stream);
+int rd_policy_dreamer_occupancy_train(rd_env* env, const uint8_t* occupancy_dev, float* actions_dev, int noise,
+                                      const float* eps_stoch_dev, const float* eps_sample_dev, const float* eps_expl_dev,
+                                      float* debug_dev, void* stream);
+/* rd_policy_dreamer_set_weights for an encoder agent: the encoder's arrays follow the same on_device rule. */
+int rd_policy_dreamer_set_weights_occupancy(rd_env* env, const rd_dreamer_weights* w, const rd_dreamer_conv_encoder* enc,
+                                            int on_device, void* stream);
+/* The encoder stage alone: embed_dev f32 [N][32 depth] = hi + lo of what obs1 reads.  The latent state is untouched. */
+int rd_dreamer_encode_occupancy(rd_env* env, const uint8_t* occupancy_dev, float* embed_dev, void* stream);
+/* rd_rollout_dreamer, rd_rollout_dreamer_train, rd_rollout_store (RD_STORE_POLICY_DREAMER*), get/set_state and the
+ * per-env state zeroing serve both agent kinds; an encoder agent's rollout reads out->occupancy_dev.  The lidar entry
+ * points fail for an encoder agent and the occupancy ones for a lidar agent (RD_ERR_INVALID). */
+
 /* ---- device-resident episode store (SURVEY.md §8-f1): records the Collect rows of every env's episodes on the device
  *      [REF dreamer/wrappers.py:198-250], exactly the episodes episodes.EpisodeRecorder hands to its callbacks, and
  *      samples fixed-length chunks the way tools.load_episodes does [REF dreamer/tools.py:235-264].  The env must have

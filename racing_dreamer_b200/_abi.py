@@ -115,6 +115,11 @@ class RdDreamerWeights(C.Structure):
         ("n_samples", C.c_int32), ("precision", C.c_int32)]
 
 
+class RdDreamerConvEncoder(C.Structure):
+    """rd_dreamer_conv_encoder: the ConvEncoder's depth and pointers to its Keras Conv2D kernels and biases."""
+    _fields_ = [("depth", C.c_int32), ("w", C.c_void_p * 4), ("b", C.c_void_p * 4)]
+
+
 class RdDreamerExploration(C.Structure):
     """rd_dreamer_exploration: the training-mode exploration schedule and its env-step counter."""
     _fields_ = [("amount", C.c_double), ("decay", C.c_double), ("min_amount", C.c_double), ("env_steps", C.c_int64)]
@@ -178,6 +183,8 @@ EXPORTS = (
     "rd_policy_dreamer_init", "rd_policy_dreamer", "rd_policy_dreamer_get_state", "rd_policy_dreamer_set_state",
     "rd_rollout_dreamer", "rd_policy_dreamer_set_exploration", "rd_policy_dreamer_get_exploration",
     "rd_policy_dreamer_train", "rd_rollout_dreamer_train", "rd_policy_dreamer_set_weights",
+    "rd_policy_dreamer_init_occupancy", "rd_policy_dreamer_occupancy", "rd_policy_dreamer_occupancy_train",
+    "rd_policy_dreamer_set_weights_occupancy", "rd_dreamer_encode_occupancy",
     "rd_store_init", "rd_store_reset", "rd_store_step", "rd_rollout_store", "rd_store_sample", "rd_store_info",
     "rd_store_import_init", "rd_store_import", "rd_store_import_info",
 )
@@ -282,6 +289,17 @@ def load_library() -> C.CDLL:
     lib.rd_rollout_dreamer_train.restype = i32
     lib.rd_policy_dreamer_set_weights.argtypes = [vp, C.POINTER(RdDreamerWeights), i32, vp]
     lib.rd_policy_dreamer_set_weights.restype = i32
+    lib.rd_policy_dreamer_init_occupancy.argtypes = [vp, C.POINTER(RdDreamerWeights), C.POINTER(RdDreamerConvEncoder)]
+    lib.rd_policy_dreamer_init_occupancy.restype = i32
+    lib.rd_policy_dreamer_occupancy.argtypes = [vp, vp, vp, i32, vp, vp, vp, vp]
+    lib.rd_policy_dreamer_occupancy.restype = i32
+    lib.rd_policy_dreamer_occupancy_train.argtypes = [vp, vp, vp, i32, vp, vp, vp, vp, vp]
+    lib.rd_policy_dreamer_occupancy_train.restype = i32
+    lib.rd_policy_dreamer_set_weights_occupancy.argtypes = [vp, C.POINTER(RdDreamerWeights), C.POINTER(RdDreamerConvEncoder),
+                                                            i32, vp]
+    lib.rd_policy_dreamer_set_weights_occupancy.restype = i32
+    lib.rd_dreamer_encode_occupancy.argtypes = [vp, vp, vp, vp]
+    lib.rd_dreamer_encode_occupancy.restype = i32
     lib.rd_store_init.argtypes = [vp, C.POINTER(RdStoreConfig)]
     lib.rd_store_init.restype = i32
     lib.rd_store_reset.argtypes = [vp, C.POINTER(RdOutputs), vp]

@@ -46,6 +46,13 @@ struct DreamerPolicy {
   float* b_act[8] = {};
   // activations.  feat[p]: latent rows; sa/det/all are views of the same rows (img1 input, deter, actor input)
   Operand feat[2], v_sa[2], v_det[2], x1, hobs, hid[2], lidar;
+  // ConvEncoder agent (depth > 0; 0 = lidar agent): conv1's raw kernel [16][depth] and the biases, conv2..conv4's packed
+  // kernels (k_pack_conv), the activations ping-ponging through enc_a (conv1, conv3) and enc_b (conv2) -- conv4 writes
+  // `lidar`, the embed obs1 reads -- and per layer l = conv2..conv4 the 5-D input view and the 2-D output view
+  int depth = 0;
+  float* w_conv1 = nullptr;
+  float* b_conv[4] = {};
+  Operand w_conv[3], enc_a, enc_b, conv_in[3], conv_out[3];
   float* head_raw = nullptr;   // [n][4] hout pre-activations
   // k_dense_chain (the actor trunk in one launch): per-row-block layer counters and the values they have reached
   bool chain = true;           // RD_DREAMER_CHAIN=0: one k_dense launch per actor layer instead
@@ -82,7 +89,7 @@ static inline void dreamer_free(DreamerPolicy& d) {
 // K-major TF32 operands (dr_upload_t: pitch ld, the K slots from k_from on shifted by k_shift); vectors (op == null)
 // are copied as they are to *vec.  Both dreamer_init and dreamer_set_weights walk this one list.
 struct DrPart { const float* src; DreamerPolicy::Operand* op; float** vec; int in, out, ld, k_from, k_shift; };
-static inline int dr_parts(DreamerPolicy& d, const rd_dreamer_weights* w, DrPart* p) {
+static inline int dr_parts(DreamerPolicy& d, const rd_dreamer_weights* w, const rd_dreamer_conv_encoder* enc, DrPart* p) {
   const int H = d.hidden, D = d.deter, E = d.embed, U = d.units, L = d.layers, NO = 1 << 30;
   int k = 0;
   auto mat = [&](const float* src, DreamerPolicy::Operand& op, int in, int out, int ld, int k_from, int k_shift) {
@@ -108,9 +115,27 @@ static inline int dr_parts(DreamerPolicy& d, const rd_dreamer_weights* w, DrPart
   mat(w->actor_w[L], d.w_act[L], U, 4, U, NO, 0);
   vec(w->actor_b[L], d.b_act[L], 4);
   if (w->bn) vec(w->bn, d.bn, 16);
+  if (enc) {   // conv1 runs on CUDA cores from its Keras kernel as it is; conv2..conv4's kernels: dr_pack_conv
+    vec(enc->w[0], d.w_conv1, 16 * enc->depth);
+    for (int l = 0; l < 4; ++l) vec(enc->b[l], d.b_conv[l], enc->depth << l);
+  }
   return k;
 }
-#define DR_MAX_PARTS (9 + 2 * 8 + 1)
+#define DR_MAX_PARTS (9 + 2 * 8 + 1 + 5)
+
+// Cin of conv layer l = 1..3 (conv2..conv4) of a depth-d encoder; Cout = 2 Cin
+static inline int dr_conv_cin(int depth, int l) { return depth << (l - 1); }
+// packs conv2..conv4's kernels (device pointers src[l - 1]) into the policy's operands on `s` (k_pack_conv)
+static inline cudaError_t dr_pack_conv(DreamerPolicy& d, const float* const* src, cudaStream_t s) {
+  for (int l = 1; l < 4; ++l) {
+    const int cin = dr_conv_cin(d.depth, l), total = 16 * cin * 2 * cin;
+    k_pack_conv<<<(unsigned)std::min((total + 255) / 256, d.sm_count * 8), 256, 0, s>>>(src[l - 1], d.w_conv[l - 1].p[0],
+                                                                                         d.w_conv[l - 1].p[1], cin, 2 * cin);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+  }
+  return cudaSuccess;
+}
 
 // [in][out] host matrix -> device [out][ld] (K-major), element (o, kmap(i)) = scale_i * W[i][o], split into its TF32
 // rounding (op.p[0]) and, in x3 mode, the TF32 rounding of the remainder (op.p[1])
@@ -173,12 +198,20 @@ static inline bool dr_view(const DreamerPolicy& d, DreamerPolicy::Operand& view,
   } while (0)
 
 // lidar_normalised: the env already emits r/15 - 0.5 (RD_OBS_LIDAR_NORM), so k_embed_lidar only splits the values
-static inline int dreamer_init(DreamerPolicy& d, int n, int n_beams, bool lidar_normalised, const rd_dreamer_weights* w) {
+// enc: a ConvEncoder agent (embed = 32 depth) instead of the lidar one (embed = n_beams)
+static inline int dreamer_init(DreamerPolicy& d, int n, int n_beams, bool lidar_normalised, const rd_dreamer_weights* w,
+                               const rd_dreamer_conv_encoder* enc = nullptr) {
   if (!w) { d.err = "null weights"; return RD_ERR_INVALID; }
-  if (w->stoch != GM_STOCH || w->deter <= 0 || w->deter % 4 || w->hidden <= 0 || w->hidden % 4 || w->embed != n_beams ||
-      n_beams % 4 || w->actor_units <= 0 || w->actor_units % 4 || w->actor_layers < 1 || w->actor_layers > 7 ||
+  if (enc) {
+    if (enc->depth != 32) { d.err = "unsupported ConvEncoder depth " + std::to_string(enc->depth) + " (need 32)"; return RD_ERR_INVALID; }
+    if (w->embed != 32 * enc->depth) { d.err = "a ConvEncoder agent's embed must be 32 * depth"; return RD_ERR_INVALID; }
+    for (int l = 0; l < 4; ++l)
+      if (!enc->w[l] || !enc->b[l]) { d.err = "null encoder weight pointer"; return RD_ERR_INVALID; }
+  }
+  if (w->stoch != GM_STOCH || w->deter <= 0 || w->deter % 4 || w->hidden <= 0 || w->hidden % 4 ||
+      (!enc && w->embed != n_beams) || w->embed % 4 || w->actor_units <= 0 || w->actor_units % 4 || w->actor_layers < 1 || w->actor_layers > 7 ||
       w->n_samples < 1 || !(w->mean_scale > 0.f)) {
-    d.err = "unsupported Dreamer architecture (need stoch 30, deter/hidden/units/embed multiples of 4, embed == n_beams, 1..7 actor layers)";
+    d.err = "unsupported Dreamer architecture (need stoch 30, deter/hidden/units/embed multiples of 4, embed == n_beams (lidar agent), 1..7 actor layers)";
     return RD_ERR_INVALID;
   }
   const float* need[] = {w->gru_kernel, w->gru_recurrent, w->gru_bias, w->img1_w, w->img1_b, w->obs1_w, w->obs1_b, w->obs2_w, w->obs2_b};
@@ -192,12 +225,13 @@ static inline int dreamer_init(DreamerPolicy& d, int n, int n_beams, bool lidar_
   d.x3 = w->precision == RD_PRECISION_TF32X3;
   d.lidar_normalised = lidar_normalised;
   d.n = n; d.deter = w->deter; d.hidden = w->hidden; d.embed = w->embed; d.units = w->actor_units; d.layers = w->actor_layers;
+  d.depth = enc ? enc->depth : 0;
   d.ldf = 32 + d.deter;
   d.raw_init_std = (float)std::log(std::exp((double)w->init_std) - 1.0);   // [REF models.py:321]
   d.min_std = w->min_std; d.mean_scale = w->mean_scale; d.bn_eps = w->bn_eps; d.n_samples = w->n_samples;
   const int H = d.hidden, D = d.deter, E = d.embed, U = d.units;
   DrPart parts[DR_MAX_PARTS];
-  const int n_parts = dr_parts(d, w, parts);
+  const int n_parts = dr_parts(d, w, enc, parts);
   size_t stage_floats = 0;
   for (int k = 0; k < n_parts; ++k) {
     const DrPart& p = parts[k];
@@ -205,8 +239,26 @@ static inline int dreamer_init(DreamerPolicy& d, int n, int n_beams, bool lidar_
     else DR_TRY(dr_upload(d, p.vec, p.src, (size_t)p.out));
     stage_floats += (size_t)p.in * p.out;
   }
-  DR_TRY(cudaMalloc(&d.stage, stage_floats * sizeof(float)));
+  size_t conv_floats = 0;   // conv2..conv4 kernels: packed on the device from the stage, as dreamer_set_weights packs them
+  for (int l = 1; d.depth && l < 4; ++l) {
+    const int cin = dr_conv_cin(d.depth, l);
+    DR_TRY(dr_alloc(d, d.w_conv[l - 1], (size_t)2 * cin, (size_t)16 * cin));
+    conv_floats += (size_t)32 * cin * cin;
+  }
+  DR_TRY(cudaMalloc(&d.stage, (stage_floats + conv_floats) * sizeof(float)));
   d.owned.push_back(d.stage);
+  if (d.depth) {
+    const float* src[3];
+    size_t off = 0;
+    for (int l = 1; l < 4; ++l) {
+      const size_t count = (size_t)32 * dr_conv_cin(d.depth, l) * dr_conv_cin(d.depth, l);
+      DR_TRY(cudaMemcpy(d.stage + off, enc->w[l], count * sizeof(float), cudaMemcpyHostToDevice));
+      src[l - 1] = d.stage + off;
+      off += count;
+    }
+    DR_TRY(dr_pack_conv(d, src, 0));
+    DR_TRY(cudaDeviceSynchronize());
+  }
   const size_t N = (size_t)n;
   for (int p = 0; p < 2; ++p) {
     DR_TRY(dr_alloc(d, d.feat[p], N, d.ldf));
@@ -238,6 +290,23 @@ static inline int dreamer_init(DreamerPolicy& d, int n, int n_beams, bool lidar_
   DR_MAP(dr_view(d, d.x1, d.x1, 0, H, N, H, GM_BM));
   DR_MAP(dr_view(d, d.hobs, d.hobs, 0, H, N, H, GM_BM));
   DR_MAP(dr_view(d, d.lidar, d.lidar, 0, E, N, E, GM_BM));
+  if (d.depth) {   // encoder activations: conv1 / conv3 outputs in enc_a, conv2's in enc_b (see dreamer_encode)
+    const int c = d.depth;
+    DR_TRY(dr_alloc(d, d.enc_a, N * 32 * 32, c));
+    DR_TRY(dr_alloc(d, d.enc_b, N * 16 * 16, 2 * c));
+    const DreamerPolicy::Operand* in[3] = {&d.enc_a, &d.enc_b, &d.enc_a};
+    const DreamerPolicy::Operand* out[3] = {&d.enc_b, &d.enc_a, &d.lidar};
+    const int g_in[3] = {32, 16, 8}, g_out[3] = {16, 8, 2};
+    for (int l = 0; l < 3; ++l) {
+      const int cin = dr_conv_cin(c, l + 1);
+      for (int part = 0; part < (d.x3 ? 2 : 1); ++part) {
+        d.conv_in[l].p[part] = in[l]->p[part];
+        DR_MAP(gm_make_map_conv(&d.conv_in[l].m[part], in[l]->p[part], cin, g_in[l], N, g_out[l]));
+      }
+      DR_MAP(dr_view(d, d.conv_out[l], *out[l], 0, 2 * cin, N * g_out[l] * g_out[l], 2 * cin, GM_BM));
+      DR_MAP(dr_view(d, d.w_conv[l], d.w_conv[l], 0, 16 * cin, 2 * cin, 16 * cin, GM_BN));
+    }
+  }
   DR_MAP(dr_view(d, d.w_img1, d.w_img1, 0, 32, H, 32, GM_BN));
   DR_MAP(dr_view(d, d.w_gruk, d.w_gruk, 0, H, 3 * D, H, GM_BN));
   DR_MAP(dr_view(d, d.w_grur, d.w_grur, 0, D, 3 * D, D, GM_BN));
@@ -265,8 +334,13 @@ static inline float dreamer_expl_amount(const DreamerPolicy& d) {
 // (no allocation; the tensor maps stay valid) bit for bit as dreamer_init packs them.  Latent state, Philox step and
 // env_steps are kept.  w holds device pointers (on_device) or host pointers, which are first copied to d.stage.  The
 // architecture, precision and head scalars must be the init's; otherwise RD_ERR_INVALID and nothing changes.
-static inline int dreamer_set_weights(DreamerPolicy& d, const rd_dreamer_weights* w, bool on_device, cudaStream_t s) {
+static inline int dreamer_set_weights(DreamerPolicy& d, const rd_dreamer_weights* w, const rd_dreamer_conv_encoder* enc,
+                                      bool on_device, cudaStream_t s) {
   if (!w) { d.err = "null weights"; return RD_ERR_INVALID; }
+  if ((enc != nullptr) != (d.depth > 0) || (enc && enc->depth != d.depth)) {
+    d.err = "the encoder (present, depth) differs from the one the policy was initialised with";
+    return RD_ERR_INVALID;
+  }
   const float raw_init_std = (float)std::log(std::exp((double)w->init_std) - 1.0);
   if (w->stoch != GM_STOCH || w->deter != d.deter || w->hidden != d.hidden || w->embed != d.embed ||
       w->actor_units != d.units || w->actor_layers != d.layers || (w->bn != nullptr) != (d.bn != nullptr) ||
@@ -277,13 +351,17 @@ static inline int dreamer_set_weights(DreamerPolicy& d, const rd_dreamer_weights
     return RD_ERR_INVALID;
   }
   DrPart parts[DR_MAX_PARTS];
-  const int n_parts = dr_parts(d, w, parts);
+  const int n_parts = dr_parts(d, w, enc, parts);
   int dev = 0;
   DR_TRY(cudaGetDevice(&dev));
-  for (int k = 0; k < n_parts; ++k) {
-    if (!parts[k].src) { d.err = "null weight pointer"; return RD_ERR_INVALID; }
+  const float* srcs[DR_MAX_PARTS + 3];   // every source array: the table's, then conv2..conv4's kernels
+  int n_src = 0;
+  for (int k = 0; k < n_parts; ++k) srcs[n_src++] = parts[k].src;
+  for (int l = 1; enc && l < 4; ++l) srcs[n_src++] = enc->w[l];
+  for (int k = 0; k < n_src; ++k) {
+    if (!srcs[k]) { d.err = "null weight pointer"; return RD_ERR_INVALID; }
     cudaPointerAttributes at{};
-    DR_TRY(cudaPointerGetAttributes(&at, parts[k].src));
+    DR_TRY(cudaPointerGetAttributes(&at, srcs[k]));
     const bool device_ptr = at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged;
     if (on_device && (!device_ptr || at.device != dev)) { d.err = "on_device: a weight pointer is not memory of the policy's device"; return RD_ERR_INVALID; }
     if (!on_device && at.type == cudaMemoryTypeDevice) { d.err = "a device pointer was passed with on_device = 0"; return RD_ERR_INVALID; }
@@ -311,6 +389,19 @@ static inline int dreamer_set_weights(DreamerPolicy& d, const rd_dreamer_weights
   const unsigned grid = (unsigned)std::min<size_t>((off + 255) / 256, (size_t)d.sm_count * 8);
   k_pack_weights<<<grid, 256, 0, s>>>(a);
   DR_TRY(cudaGetLastError());
+  if (enc) {
+    const float* src[3];
+    for (int l = 1; l < 4; ++l) {
+      const size_t count = (size_t)32 * dr_conv_cin(d.depth, l) * dr_conv_cin(d.depth, l);
+      src[l - 1] = enc->w[l];
+      if (!on_device) {
+        DR_TRY(cudaMemcpyAsync(d.stage + off, enc->w[l], count * sizeof(float), cudaMemcpyHostToDevice, s));
+        src[l - 1] = d.stage + off;
+      }
+      off += count;
+    }
+    DR_TRY(dr_pack_conv(d, src, s));
+  }
   return RD_OK;
 }
 
@@ -372,13 +463,51 @@ static inline void dr_build(const DreamerPolicy& d, GemmMaps& maps, GemmArgs& g,
 // train: null = evaluation mode (SampleDist.mode(), eps_actor [N][n_samples][2]); else the training head k_actor_train
 // with exploration amount train->amount (eps_actor = the sample's draws [N][2], train->eps_expl the exploration's).
 struct DrTrain { const float* eps_expl; float amount; };
-static inline int dreamer_step(DreamerPolicy& d, const float* lidar, float* actions, int noise, const float* eps_stoch,
+// ConvEncoder [UPSTREAM-RECALL: danijar Dreamer models.py ConvEncoder] of u8 images [n][64][64] -> d.lidar, the embed
+// operand obs1 reads ([n][32 depth], (y, x, c) order, TF32 hi + lo).  conv1 on CUDA cores (k_conv1) into enc_a's 32 x 32
+// grid; conv2 (16 x 16 grid, 14 x 14 valid) -> enc_b, conv3 (8 x 8 grid, 6 x 6 valid) -> enc_a, conv4 (2 x 2, all valid)
+// -> d.lidar as k_dense implicit GEMMs (gm_conv_a).  The padded grids' extra outputs are finite (they read zeros or other
+// finite outputs) and no valid output reads them.
+template <int G>
+static inline cudaError_t dr_conv_launch(const DreamerPolicy& d, const GemmMaps& maps, const GemmArgs& g, cudaStream_t s) {
+  if (d.x3) return gm_launch<EPI_DENSE, 1, 8, 4, true, DR_EW_WIDE, GM_BN, G>(maps, g, s);
+  return gm_launch<EPI_DENSE, 1, 8, 8, false, GM_EPI_GROUPS, GM_BN, G>(maps, g, s);
+}
+static inline int dreamer_encode(DreamerPolicy& d, const uint8_t* occ, cudaStream_t s, int* launched) {
+  k_conv1<<<(unsigned)d.n * 32, 256, 0, s>>>(occ, d.w_conv1, d.b_conv[0], reinterpret_cast<float4*>(d.enc_a.p[0]),
+                                             reinterpret_cast<float4*>(d.enc_a.p[1]));
+  DR_TRY(cudaGetLastError());
+  ++*launched;
+  GemmMaps maps;
+  const int g_out[3] = {16, 8, 2};
+  for (int l = 0; l < 3; ++l) {
+    const int cin = dr_conv_cin(d.depth, l + 1);
+    GemmArgs g{};
+    g.M = d.n * g_out[l] * g_out[l]; g.N = 2 * cin;
+    const DrTerm t[1] = {{&d.conv_in[l], &d.w_conv[l], 16 * cin, 0}};
+    dr_build(d, maps, g, t, 1, 1, nullptr, nullptr, 1, 8);
+    g.step = d.step; g.bias = d.b_conv[l + 1]; g.out = d.conv_out[l].p[0]; g.out_lo = d.conv_out[l].p[1]; g.ldo = 2 * cin;
+    maps.o[0] = d.conv_out[l].m[0]; maps.o[1] = d.conv_out[l].m[1];
+    if (l == 0) DR_TRY(dr_conv_launch<16>(d, maps, g, s));
+    else if (l == 1) DR_TRY(dr_conv_launch<8>(d, maps, g, s));
+    else DR_TRY(dr_conv_launch<2>(d, maps, g, s));
+    ++*launched;
+  }
+  return RD_OK;
+}
+
+// obs: the lidar scans (f32 [n][n_beams]) or, for a ConvEncoder agent, the occupancy images (u8 [n][64][64])
+static inline int dreamer_step(DreamerPolicy& d, const void* obs, float* actions, int noise, const float* eps_stoch,
                                const float* eps_actor, float* debug, uint64_t seed, uint32_t gid0, cudaStream_t s, int* launched,
                                const DrTrain* train = nullptr) {
   *launched = 0;
   const int cur = d.cur, nxt = cur ^ 1;
   const int H = d.hidden, D = d.deter, U = d.units;
-  {   // 0. embed = _preprocess_lidar(scan), split for the tensor-core passes
+  if (d.depth) {   // 0. embed = ConvEncoder(image)
+    const int rc = dreamer_encode(d, static_cast<const uint8_t*>(obs), s, launched);
+    if (rc) return rc;
+  } else {   // 0. embed = _preprocess_lidar(scan), split for the tensor-core passes
+    const float* lidar = static_cast<const float*>(obs);
     const size_t count4 = (size_t)d.n * d.embed / 4;
     const unsigned grid = (unsigned)std::min<size_t>((count4 + 255) / 256, 148 * 8);
     k_embed_lidar<<<grid, 256, 0, s>>>(reinterpret_cast<const float4*>(lidar), reinterpret_cast<float4*>(d.lidar.p[0]),

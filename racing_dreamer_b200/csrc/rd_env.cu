@@ -1172,14 +1172,14 @@ RD_API int rd_policy_dreamer_init(rd_env* env, const rd_dreamer_weights* w) {
 namespace {
 // training: Dreamer.policy(training=True) -- one sample + exploration (k_actor_train), and the env-step counter of the
 // exploration schedule advances by n_envs * action_repeat [REF dreamer/dreamer.py, Dreamer.__call__ self._step]
-int launch_dreamer(rd_env* env, const float* lidar_dev, float* actions_dev, int noise, const float* eps_stoch_dev,
+int launch_dreamer(rd_env* env, const void* obs_dev, float* actions_dev, int noise, const float* eps_stoch_dev,
                    const float* eps_actor_dev, float* debug_dev, cudaStream_t s, bool training = false,
                    const float* eps_expl_dev = nullptr) {
   int launched = 0, rc;
   const DrTrain tr{eps_expl_dev, dreamer_expl_amount(env->dr)};
   {
     ScopedTiming tm(env, s, T_POLICY);
-    rc = dreamer_step(env->dr, lidar_dev, actions_dev, noise, eps_stoch_dev, eps_actor_dev, debug_dev, env->cfg.seed,
+    rc = dreamer_step(env->dr, obs_dev, actions_dev, noise, eps_stoch_dev, eps_actor_dev, debug_dev, env->cfg.seed,
                       (uint32_t)env->cfg.env_id_offset, s, &launched, training ? &tr : nullptr);
   }
   env->launches += launched;
@@ -1187,12 +1187,27 @@ int launch_dreamer(rd_env* env, const float* lidar_dev, float* actions_dev, int 
   if (training) env->dr.env_steps += (int64_t)env->n * env->cfg.action_repeat;
   return RD_OK;
 }
+// the entry point's agent kind (encoder: the occupancy entry points) must be the initialised agent's
+int dreamer_kind(rd_env* env, bool encoder, const char* fn) {
+  if (!env->dr.ready) return fail(env, RD_ERR_STATE, "%s: rd_policy_dreamer_init has not been called", fn);
+  if (encoder && !env->dr.depth)
+    return fail(env, RD_ERR_INVALID, "%s: the agent reads lidar (rd_policy_dreamer_init); use the lidar entry points", fn);
+  if (!encoder && env->dr.depth)
+    return fail(env, RD_ERR_INVALID, "%s: the agent reads lidar_occupancy (rd_policy_dreamer_init_occupancy); use the "
+                "occupancy entry points", fn);
+  return RD_OK;
+}
+// what a rollout feeds the agent: the scans, or the images for an encoder agent (null if the env does not produce them)
+const void* dreamer_obs(rd_env* env, const rd_outputs* out) {
+  if (!env->dr.depth) return out->lidar_dev;
+  return (env->cfg.obs_flags & RD_OBS_OCCUPANCY) ? out->occupancy_dev : nullptr;
+}
 }  // namespace
 
 RD_API int rd_policy_dreamer(rd_env* env, const float* lidar_dev, float* actions_dev, int noise, const float* eps_stoch_dev,
                              const float* eps_actor_dev, float* debug_dev, void* stream) {
   if (!env || !lidar_dev || !actions_dev) return fail(env, RD_ERR_INVALID, "null argument");
-  if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
+  if (int rc = dreamer_kind(env, false, "rd_policy_dreamer")) return rc;
   if (noise < RD_NOISE_ZERO || noise > RD_NOISE_EXPLICIT) return fail(env, RD_ERR_INVALID, "bad noise mode %d", noise);
   if (noise == RD_NOISE_EXPLICIT && (!eps_stoch_dev || !eps_actor_dev))
     return fail(env, RD_ERR_INVALID, "RD_NOISE_EXPLICIT needs eps_stoch_dev and eps_actor_dev");
@@ -1218,13 +1233,17 @@ RD_API int rd_policy_dreamer_set_state(rd_env* env, const float* stoch_dev, cons
 }
 
 RD_API int rd_rollout_dreamer(rd_env* env, int n_steps, const rd_outputs* out, float* actions_dev, int noise, void* stream) {
-  if (!env || !out || !out->lidar_dev || n_steps < 0) return fail(env, RD_ERR_INVALID, "bad argument (the rollout needs out->lidar_dev)");
+  if (!env || !out || n_steps < 0) return fail(env, RD_ERR_INVALID, "bad argument");
   if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
+  const void* obs = dreamer_obs(env, out);
+  if (!obs)
+    return fail(env, RD_ERR_INVALID, env->dr.depth ? "the rollout needs out->occupancy_dev and an env that produces it (RD_OBS_OCCUPANCY)"
+                                                   : "bad argument (the rollout needs out->lidar_dev)");
   if (noise != RD_NOISE_ZERO && noise != RD_NOISE_PHILOX) return fail(env, RD_ERR_INVALID, "a rollout draws its own noise (RD_NOISE_ZERO or RD_NOISE_PHILOX)");
   if (!env->was_reset) return fail(env, RD_ERR_STATE, "Must reset environment.");
   float* act = actions_dev ? actions_dev : env->pol.d_actions;
   for (int k = 0; k < n_steps; ++k) {
-    int rc = launch_dreamer(env, out->lidar_dev, act, noise, nullptr, nullptr, nullptr, (cudaStream_t)stream);
+    int rc = launch_dreamer(env, obs, act, noise, nullptr, nullptr, nullptr, (cudaStream_t)stream);
     if (rc) return rc;
     if ((rc = rd_step(env, act, out, stream))) return rc;
   }
@@ -1234,7 +1253,7 @@ RD_API int rd_rollout_dreamer(rd_env* env, int n_steps, const rd_outputs* out, f
 RD_API int rd_policy_dreamer_train(rd_env* env, const float* lidar_dev, float* actions_dev, int noise, const float* eps_stoch_dev,
                                    const float* eps_sample_dev, const float* eps_expl_dev, float* debug_dev, void* stream) {
   if (!env || !lidar_dev || !actions_dev) return fail(env, RD_ERR_INVALID, "null argument");
-  if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
+  if (int rc = dreamer_kind(env, false, "rd_policy_dreamer_train")) return rc;
   if (noise < RD_NOISE_ZERO || noise > RD_NOISE_EXPLICIT) return fail(env, RD_ERR_INVALID, "bad noise mode %d", noise);
   if (noise == RD_NOISE_EXPLICIT && (!eps_stoch_dev || !eps_sample_dev || !eps_expl_dev))
     return fail(env, RD_ERR_INVALID, "RD_NOISE_EXPLICIT needs eps_stoch_dev, eps_sample_dev and eps_expl_dev");
@@ -1243,13 +1262,17 @@ RD_API int rd_policy_dreamer_train(rd_env* env, const float* lidar_dev, float* a
 }
 
 RD_API int rd_rollout_dreamer_train(rd_env* env, int n_steps, const rd_outputs* out, float* actions_dev, int noise, void* stream) {
-  if (!env || !out || !out->lidar_dev || n_steps < 0) return fail(env, RD_ERR_INVALID, "bad argument (the rollout needs out->lidar_dev)");
+  if (!env || !out || n_steps < 0) return fail(env, RD_ERR_INVALID, "bad argument");
   if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
+  const void* obs = dreamer_obs(env, out);
+  if (!obs)
+    return fail(env, RD_ERR_INVALID, env->dr.depth ? "the rollout needs out->occupancy_dev and an env that produces it (RD_OBS_OCCUPANCY)"
+                                                   : "bad argument (the rollout needs out->lidar_dev)");
   if (noise != RD_NOISE_ZERO && noise != RD_NOISE_PHILOX) return fail(env, RD_ERR_INVALID, "a rollout draws its own noise (RD_NOISE_ZERO or RD_NOISE_PHILOX)");
   if (!env->was_reset) return fail(env, RD_ERR_STATE, "Must reset environment.");
   float* act = actions_dev ? actions_dev : env->pol.d_actions;
   for (int k = 0; k < n_steps; ++k) {
-    int rc = launch_dreamer(env, out->lidar_dev, act, noise, nullptr, nullptr, nullptr, (cudaStream_t)stream, true);
+    int rc = launch_dreamer(env, obs, act, noise, nullptr, nullptr, nullptr, (cudaStream_t)stream, true);
     if (rc) return rc;
     if ((rc = rd_step(env, act, out, stream))) return rc;
   }
@@ -1280,10 +1303,76 @@ RD_API int rd_policy_dreamer_get_exploration(rd_env* env, rd_dreamer_exploration
 
 RD_API int rd_policy_dreamer_set_weights(rd_env* env, const rd_dreamer_weights* w, int on_device, void* stream) {
   if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
-  if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
-  const int rc = dreamer_set_weights(env->dr, w, on_device != 0, (cudaStream_t)stream);
+  if (int rc = dreamer_kind(env, false, "rd_policy_dreamer_set_weights")) return rc;
+  const int rc = dreamer_set_weights(env->dr, w, nullptr, on_device != 0, (cudaStream_t)stream);
   if (rc) return fail(env, rc, "rd_policy_dreamer_set_weights: %s", env->dr.err.c_str());
   env->launches++;
+  return RD_OK;
+}
+
+RD_API int rd_policy_dreamer_init_occupancy(rd_env* env, const rd_dreamer_weights* w, const rd_dreamer_conv_encoder* enc) {
+  if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
+  if (!enc) return fail(env, RD_ERR_INVALID, "rd_policy_dreamer_init_occupancy: null encoder");
+  if (!(env->cfg.obs_flags & RD_OBS_OCCUPANCY))
+    return fail(env, RD_ERR_INVALID, "rd_policy_dreamer_init_occupancy: the env does not produce lidar_occupancy (RD_OBS_OCCUPANCY)");
+  const int rc = dreamer_init(env->dr, env->n, env->cfg.n_beams, false, w, enc);
+  if (rc) return fail(env, rc, "rd_policy_dreamer_init_occupancy: %s", env->dr.err.c_str());
+  if (!env->pol.d_actions) {
+    CUDA_TRY(env, cudaMalloc(&env->pol.d_actions, sizeof(float) * 2 * (size_t)env->n));
+    CUDA_TRY(env, cudaMemset(env->pol.d_actions, 0, sizeof(float) * 2 * (size_t)env->n));
+  }
+  return RD_OK;
+}
+
+RD_API int rd_policy_dreamer_occupancy(rd_env* env, const uint8_t* occupancy_dev, float* actions_dev, int noise,
+                                       const float* eps_stoch_dev, const float* eps_actor_dev, float* debug_dev, void* stream) {
+  if (!env || !occupancy_dev || !actions_dev) return fail(env, RD_ERR_INVALID, "null argument");
+  if (int rc = dreamer_kind(env, true, "rd_policy_dreamer_occupancy")) return rc;
+  if (noise < RD_NOISE_ZERO || noise > RD_NOISE_EXPLICIT) return fail(env, RD_ERR_INVALID, "bad noise mode %d", noise);
+  if (noise == RD_NOISE_EXPLICIT && (!eps_stoch_dev || !eps_actor_dev))
+    return fail(env, RD_ERR_INVALID, "RD_NOISE_EXPLICIT needs eps_stoch_dev and eps_actor_dev");
+  return launch_dreamer(env, occupancy_dev, actions_dev, noise, eps_stoch_dev, eps_actor_dev, debug_dev, (cudaStream_t)stream);
+}
+
+RD_API int rd_policy_dreamer_occupancy_train(rd_env* env, const uint8_t* occupancy_dev, float* actions_dev, int noise,
+                                             const float* eps_stoch_dev, const float* eps_sample_dev, const float* eps_expl_dev,
+                                             float* debug_dev, void* stream) {
+  if (!env || !occupancy_dev || !actions_dev) return fail(env, RD_ERR_INVALID, "null argument");
+  if (int rc = dreamer_kind(env, true, "rd_policy_dreamer_occupancy_train")) return rc;
+  if (noise < RD_NOISE_ZERO || noise > RD_NOISE_EXPLICIT) return fail(env, RD_ERR_INVALID, "bad noise mode %d", noise);
+  if (noise == RD_NOISE_EXPLICIT && (!eps_stoch_dev || !eps_sample_dev || !eps_expl_dev))
+    return fail(env, RD_ERR_INVALID, "RD_NOISE_EXPLICIT needs eps_stoch_dev, eps_sample_dev and eps_expl_dev");
+  return launch_dreamer(env, occupancy_dev, actions_dev, noise, eps_stoch_dev, eps_sample_dev, debug_dev, (cudaStream_t)stream,
+                        true, eps_expl_dev);
+}
+
+RD_API int rd_policy_dreamer_set_weights_occupancy(rd_env* env, const rd_dreamer_weights* w, const rd_dreamer_conv_encoder* enc,
+                                                   int on_device, void* stream) {
+  if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
+  if (!enc) return fail(env, RD_ERR_INVALID, "rd_policy_dreamer_set_weights_occupancy: null encoder");
+  if (int rc = dreamer_kind(env, true, "rd_policy_dreamer_set_weights_occupancy")) return rc;
+  const int rc = dreamer_set_weights(env->dr, w, enc, on_device != 0, (cudaStream_t)stream);
+  if (rc) return fail(env, rc, "rd_policy_dreamer_set_weights_occupancy: %s", env->dr.err.c_str());
+  env->launches += 4;
+  return RD_OK;
+}
+
+RD_API int rd_dreamer_encode_occupancy(rd_env* env, const uint8_t* occupancy_dev, float* embed_dev, void* stream) {
+  if (!env || !occupancy_dev || !embed_dev) return fail(env, RD_ERR_INVALID, "null argument");
+  if (int rc = dreamer_kind(env, true, "rd_dreamer_encode_occupancy")) return rc;
+  DreamerPolicy& d = env->dr;
+  cudaStream_t s = (cudaStream_t)stream;
+  int launched = 0;
+  int rc = dreamer_encode(d, occupancy_dev, s, &launched);
+  if (!rc) {   // embed = hi + lo: the latent copy kernel over [n][embed] rows
+    const size_t total = (size_t)d.n * d.embed;
+    k_latent_copy<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(d.lidar.p[0], d.lidar.p[1], d.embed, 0, d.embed, embed_dev, d.n, 0);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) { rc = RD_ERR_CUDA; d.err = std::string("k_latent_copy: ") + cudaGetErrorString(e); }
+    ++launched;
+  }
+  env->launches += launched;
+  if (rc) return fail(env, rc, "rd_dreamer_encode_occupancy: %s", d.err.c_str());
   return RD_OK;
 }
 
@@ -1652,11 +1741,15 @@ RD_API int rd_rollout_store(rd_env* env, int policy, int n_steps, const rd_outpu
   if (!env->st.started) return fail(env, RD_ERR_STATE, "rd_store_reset has not been called");
   int rc = store_check_out(env, out);
   if (rc) return rc;
-  if (!out->lidar_dev) return fail(env, RD_ERR_INVALID, "the rollout needs out->lidar_dev");
+  const void* dr_obs = nullptr;
   if (policy == RD_STORE_POLICY_GAP_FOLLOWER) {
+    if (!out->lidar_dev) return fail(env, RD_ERR_INVALID, "the rollout needs out->lidar_dev");
     if (!env->pol.ready) return fail(env, RD_ERR_STATE, "rd_policy_gap_follower_init has not been called");
   } else if (policy == RD_STORE_POLICY_DREAMER || policy == RD_STORE_POLICY_DREAMER_TRAIN) {
     if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
+    if (!(dr_obs = dreamer_obs(env, out)))
+      return fail(env, RD_ERR_INVALID, env->dr.depth ? "the rollout needs out->occupancy_dev and an env that produces it (RD_OBS_OCCUPANCY)"
+                                                     : "the rollout needs out->lidar_dev");
     if (noise != RD_NOISE_ZERO && noise != RD_NOISE_PHILOX) return fail(env, RD_ERR_INVALID, "a rollout draws its own noise (RD_NOISE_ZERO or RD_NOISE_PHILOX)");
   } else {
     return fail(env, RD_ERR_INVALID, "bad policy %d", policy);
@@ -1665,7 +1758,7 @@ RD_API int rd_rollout_store(rd_env* env, int policy, int n_steps, const rd_outpu
   float* act = actions_dev ? actions_dev : env->pol.d_actions;
   for (int k = 0; k < n_steps; ++k) {
     rc = policy == RD_STORE_POLICY_GAP_FOLLOWER ? launch_gap_follower(env, out->lidar_dev, nullptr, act, nullptr, s)
-                                                : launch_dreamer(env, out->lidar_dev, act, noise, nullptr, nullptr, nullptr, s,
+                                                : launch_dreamer(env, dr_obs, act, noise, nullptr, nullptr, nullptr, s,
                                                                  policy == RD_STORE_POLICY_DREAMER_TRAIN);
     if (rc) return rc;
     if ((rc = store_step(env, act, out, s))) return rc;

@@ -98,6 +98,15 @@ __device__ __forceinline__ void gm_tma_2d(uint32_t dst_smem, const CUtensorMap* 
       "l"(reinterpret_cast<uint64_t>(map)), "r"(x), "r"(y), "r"(rd_smem_u32(bar))
       : "memory");
 }
+// implicit-GEMM A operand of a convolution layer (k_dense<..., CONV>): coordinates (K element, bx, dy, by, env)
+__device__ __forceinline__ void gm_tma_5d(uint32_t dst_smem, const CUtensorMap* map, int c0, int c1, int c2, int c3, int c4,
+                                          uint64_t* bar) {
+  asm volatile(
+      "cp.async.bulk.tensor.5d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5, %6}], [%7];" ::"r"(
+          dst_smem),
+      "l"(reinterpret_cast<uint64_t>(map)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4), "r"(rd_smem_u32(bar))
+      : "memory");
+}
 __device__ __forceinline__ void gm_prefetch_map(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(map)) : "memory");
 }
@@ -257,9 +266,27 @@ __device__ __forceinline__ void gm_tiles_out(int bar_id, int n_threads, bool lea
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+// Convolution layers as k_dense launches (CONV = the output grid's width G > 0; EPI_DENSE with ReLU).
+// Conv2D(kernel 4, stride 2, 'valid') over an NHWC input [env][2G'][2G'][Cin] is an implicit GEMM: M rows = output
+// positions (env, oy, ox) on a G x G grid, K = (ky, kx, c).  With ky = 2 py + dy and kx = 2 px + dx the input element of
+// (oy, ox, ky, kx, c) is (by, dy, bx, dx, c) with by = oy + py, bx = ox + px, so for fixed (py, px, dy) the K slice
+// (dx, c) is 2 Cin contiguous floats.  The A map is a 5-D view (2 Cin, bx, dy, by, env) of the previous layer's output
+// (host: gm_make_map_conv) whose 128-row box is a power-of-two rectangle of output positions (bx fastest, then by, then
+// env); out-of-range bx / by / env coordinates are zero-filled by the copy engine.  K is ordered in 32-wide blocks
+// kb = 8 cb + (4 py + 2 px + dy), cb = the 32-float chunk of the (dx, c) slice -- the order k_pack_conv packs the
+// weights in -- so the producer derives a block's coordinates from its K index alone.
+// ---------------------------------------------------------------------------------------------------------------
+template <int CONV>
+__device__ __forceinline__ void gm_conv_a(uint32_t dst, const CUtensorMap* map, int ak, int m0, uint64_t* bar) {
+  const int kb = ak / GM_BK, f = kb & 7;
+  const int rows_env = CONV * CONV;
+  gm_tma_5d(dst, map, (kb >> 3) * GM_BK, (f >> 1) & 1, f & 1, (m0 % rows_env) / CONV + (f >> 2), m0 / rows_env, bar);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
 // the kernel
 // ---------------------------------------------------------------------------------------------------------------
-template <int EPI, int NSLAB, int NACC, int GM_STAGES, bool X3 = false, int EW = GM_EPI_GROUPS, int BN = GM_BN>
+template <int EPI, int NSLAB, int NACC, int GM_STAGES, bool X3 = false, int EW = GM_EPI_GROUPS, int BN = GM_BN, int CONV = 0>
 __global__ void __launch_bounds__(64 + 128 * EW, 1)
     k_dense(const __grid_constant__ GemmMaps maps, const GemmArgs g) {
   extern __shared__ uint8_t gm_smem_raw[];
@@ -338,8 +365,13 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
               }
             }
             if (do_a) {
-              gm_tma_2d(sa, ma, ak, m0, &full_bar[s]);
-              if (X3) gm_tma_2d(sb, ma2, ak, m0, &full_bar[s]);
+              if constexpr (CONV > 0) {
+                gm_conv_a<CONV>(sa, ma, ak, m0, &full_bar[s]);
+                if (X3) gm_conv_a<CONV>(sb, ma2, ak, m0, &full_bar[s]);
+              } else {
+                gm_tma_2d(sa, ma, ak, m0, &full_bar[s]);
+                if (X3) gm_tma_2d(sb, ma2, ak, m0, &full_bar[s]);
+              }
             }
           }
           if (pass == 0 && it >= (uint32_t)GM_STAGES) break;
@@ -463,7 +495,8 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
               float x = v[j + t] + __ldg(g.bias + col + t);
-              if (g.act) x = gm_elu(x);
+              if constexpr (CONV > 0) x = fmaxf(x, 0.f);   // tf.nn.relu
+              else if (g.act) x = gm_elu(x);
               po[t] = gm_round_tf32(x);
               pl[t] = gm_round_tf32(x - po[t]);
             }
@@ -830,6 +863,60 @@ __global__ void __launch_bounds__(256) k_embed_lidar(const float4* __restrict__ 
     if (lo) lo[i] = l4;
   }
 }
+// ConvEncoder's first layer [UPSTREAM-RECALL: Dreamer models.py ConvEncoder]: relu(Conv2D(32, 4, stride 2)) of the
+// occupancy image cast to float, on CUDA cores (K = 16 is too short for a tensor-core K block).  The inputs are 0 / 1 (any
+// u8 is cast exactly), so every product is exact and the float32 sums are float32-grade in both precisions.  Output: NHWC
+// [env][32][32][32] TF32 hi (+ lo) on a 32 x 32 grid whose last row and column (outside the 31 x 31 valid outputs) are
+// zero -- the grid conv2's 5-D view reads.  One CTA per (env, output row), thread = (ox, 4 channels).
+#define GM_CONV1_C 32
+__global__ void __launch_bounds__(256) k_conv1(const uint8_t* __restrict__ occ, const float* __restrict__ w,
+                                               const float* __restrict__ b, float4* __restrict__ hi, float4* __restrict__ lo) {
+  __shared__ float ws[16 * GM_CONV1_C];
+  __shared__ float img[4][64];
+  const int oy = blockIdx.x & 31, t = threadIdx.x;
+  const size_t env = blockIdx.x >> 5;
+  for (int i = t; i < 16 * GM_CONV1_C; i += 256) ws[i] = w[i];
+  img[t >> 6][t & 63] = oy < 31 ? (float)occ[env * 4096 + (size_t)(2 * oy + (t >> 6)) * 64 + (t & 63)] : 0.f;
+  __syncthreads();
+  const int ox = t >> 3, c0 = (t & 7) * 4;
+  float v[4] = {0.f, 0.f, 0.f, 0.f};
+  if (oy < 31 && ox < 31) {
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      float acc = b[c0 + j];
+#pragma unroll
+      for (int k = 0; k < 16; ++k) acc = fmaf(img[k >> 2][2 * ox + (k & 3)], ws[k * GM_CONV1_C + c0 + j], acc);
+      v[j] = fmaxf(acc, 0.f);
+    }
+  }
+  float4 h4, l4;
+  float* h = &h4.x;
+  float* l = &l4.x;
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    h[j] = gm_round_tf32(v[j]);
+    l[j] = gm_round_tf32(v[j] - h[j]);
+  }
+  const size_t o = ((env * 32 + oy) * 32 + ox) * (GM_CONV1_C / 4) + (c0 >> 2);
+  hi[o] = h4;
+  if (lo) lo[o] = l4;
+}
+// Conv2D kernel [4][4][cin][cout] (Keras) -> the K-major operand [cout][16 cin] of k_dense<..., CONV> in its K-block
+// order (see gm_conv_a): (ky, kx, c) -> block 8 cb + (4 py + 2 px + dy), element cc % 32, with ky = 2 py + dy,
+// kx = 2 px + dx, cc = dx cin + c, cb = cc / 32.  Rounding as k_pack_weights'; init and weight refresh both pack with it.
+__global__ void __launch_bounds__(256) k_pack_conv(const float* __restrict__ src, float* __restrict__ hi, float* __restrict__ lo,
+                                                   int cin, int cout) {
+  const int total = 16 * cin * cout;
+  for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < total; t += gridDim.x * blockDim.x) {
+    const int i = t / cout, o = t % cout;
+    const int ky = i / (4 * cin), kx = (i / cin) & 3, c = i % cin;
+    const int f = 4 * (ky >> 1) + 2 * (kx >> 1) + (ky & 1), cc = (kx & 1) * cin + c;
+    const size_t k = (size_t)o * 16 * cin + (size_t)(((cc >> 5) * 8 + f) * GM_BK + (cc & 31));
+    const float x = src[t], h = gm_tf32_bits(x);
+    hi[k] = h;
+    if (lo) lo[k] = gm_tf32_bits(__fsub_rn(x, h));
+  }
+}
 // latent rows <-> the reference's state tuple.  dir 0: out = hi + lo; dir 1: (hi, lo) = split(in)
 __global__ void __launch_bounds__(256) k_latent_copy(float* __restrict__ feat, float* __restrict__ feat_lo, int ldf, int col0,
                                                       int width, float* __restrict__ ext, int n, int dir) {
@@ -1150,12 +1237,27 @@ static inline bool gm_make_map(CUtensorMap* m, const float* base, uint64_t inner
              CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-template <int EPI, int NSLAB, int NACC, int GM_STAGES, bool X3 = false, int EW = GM_EPI_GROUPS, int BN = GM_BN>
+// Conv2D input [env][G_in][G_in][cin] (NHWC, G_in even) as the 5-D view (2 cin, G_in / 2, 2, G_in / 2, env) the K blocks
+// of k_dense<..., CONV = g_out> load; the box covers 128 output positions: g_out x min(g_out, 128 / g_out) x the rest envs
+static inline bool gm_make_map_conv(CUtensorMap* m, const float* base, int cin, int g_in, uint64_t envs, int g_out) {
+  gm_encode_fn enc = gm_get_encoder();
+  if (!enc) return false;
+  const uint32_t bx = (uint32_t)g_out, by = (uint32_t)std::min(g_out, GM_BM / g_out), be = (uint32_t)(GM_BM / (g_out * (int)by));
+  const uint64_t row = (uint64_t)g_in * cin * 4;   // bytes of one input row
+  cuuint64_t gdim[5] = {(cuuint64_t)(2 * cin), (cuuint64_t)(g_in / 2), 2, (cuuint64_t)(g_in / 2), envs};
+  cuuint64_t gstr[4] = {(cuuint64_t)(2 * cin * 4), row, 2 * row, row * g_in};
+  cuuint32_t box[5] = {GM_BK, bx, 1, by, be};
+  cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+  return enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5, (void*)base, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
+template <int EPI, int NSLAB, int NACC, int GM_STAGES, bool X3 = false, int EW = GM_EPI_GROUPS, int BN = GM_BN, int CONV = 0>
 static inline cudaError_t gm_launch(const GemmMaps& maps, const GemmArgs& g, cudaStream_t s) {
   constexpr size_t smem = (size_t)GM_STAGES * (X3 ? 2 : 1) * (GM_A_BYTES + NSLAB * BN * 128) + 1024;
   static bool attr = false;
   if (!attr) {
-    cudaError_t e = cudaFuncSetAttribute(k_dense<EPI, NSLAB, NACC, GM_STAGES, X3, EW, BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(k_dense<EPI, NSLAB, NACC, GM_STAGES, X3, EW, BN, CONV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     attr = true;
   }
@@ -1169,7 +1271,7 @@ static inline cudaError_t gm_launch(const GemmMaps& maps, const GemmArgs& g, cud
   attrs[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attrs;
   cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, k_dense<EPI, NSLAB, NACC, GM_STAGES, X3, EW, BN>, maps, g);
+  return cudaLaunchKernelEx(&cfg, k_dense<EPI, NSLAB, NACC, GM_STAGES, X3, EW, BN, CONV>, maps, g);
 }
 
 template <int GM_STAGES, int EW, int BN>

@@ -170,6 +170,35 @@ def _dreamer_arch(w) -> tuple:
     return deter, hidden, units, embed, layers, has_bn
 
 
+_ENC_KEYS = tuple(f"enc{l}_{p}" for l in range(1, 5) for p in "wb")
+
+
+def _encoder_depth(w, deter: int, embed: int) -> int:
+    """The ConvEncoder depth of a weight dict holding enc1_w, enc1_b .. enc4_w, enc4_b (Keras Conv2D kernels
+    [4][4][Cin][Cout] with Cout = depth, 2 depth, 4 depth, 8 depth; biases [Cout]), 0 if it holds none of them;
+    ValueError if they are incomplete, misshapen, or obs1_w's rows are not deter + 32 depth."""
+    present = [k for k in _ENC_KEYS if k in w]
+    if not present:
+        return 0
+    missing = [k for k in _ENC_KEYS if k not in w]
+    if missing:
+        raise ValueError(f"ConvEncoder arrays {', '.join(missing)} are missing")
+    shape = tuple(w["enc1_w"].shape)
+    if len(shape) != 4 or shape[3] < 1:
+        raise ValueError(f"checkpoint array enc1_w has shape {shape}, expected (4, 4, 1, depth)")
+    depth, cin = shape[3], 1
+    for l in range(4):
+        cout = depth << l
+        for k, shp in ((f"enc{l + 1}_w", (4, 4, cin, cout)), (f"enc{l + 1}_b", (cout,))):
+            if tuple(w[k].shape) != shp:
+                raise ValueError(f"checkpoint array {k} has shape {tuple(w[k].shape)}, expected {shp}")
+        cin = cout
+    if embed != 32 * depth:
+        raise ValueError(f"obs1_w has {deter + embed} rows; a depth-{depth} ConvEncoder needs deter + 32 * depth = "
+                         f"{deter + 32 * depth}")
+    return depth
+
+
 def exploration_amount(amount: float, decay: float, min_amount: float, env_steps: int) -> np.float32:
     """The exploration noise scale of a training step [REF dreamer/dreamer.py, Dreamer._exploration]: amount, times
     0.5 ** (env_steps / decay) if decay > 0, at least min_amount if min_amount > 0 -- in float64, rounded once to
@@ -206,7 +235,13 @@ class DreamerPolicy:
     exploration ``clip(a + amount * N(0, 1), -1, 1)``.  The amount is ``expl_amount``, halved every ``expl_decay`` env
     steps if ``expl_decay`` > 0 and floored at ``expl_min`` if ``expl_min`` > 0; ``env_steps`` counts
     ``n_envs * action_repeat`` per training step.  The defaults 0.3 / 0 / 0 are Dreamer's ``define_config`` values
-    [UPSTREAM-RECALL].  ``load_weights`` hands the agent a learner's new weights without touching its state."""
+    [UPSTREAM-RECALL].  ``load_weights`` hands the agent a learner's new weights without touching its state.
+
+    A weight dict with ``enc1_w, enc1_b .. enc4_w, enc4_b`` builds the ``lidar_occupancy`` agent (the reference's second
+    Dreamer setup [REF dreamer/dream.py:64-66]): the ConvEncoder [UPSTREAM-RECALL: Dreamer models.py ConvEncoder] of the
+    64x64 u8 image replaces ``_preprocess_lidar`` (conv1 on CUDA cores, conv2..conv4 on ``k_dense``), the rest is the
+    same agent.  It needs an env with ``obs_type='lidar_occupancy'``; ``act(occupancy=...)`` and ``encode()`` read the
+    images, ``rollout`` reads the env's own."""
 
     NOISE = {"zero": _abi.RD_NOISE_ZERO, "philox": _abi.RD_NOISE_PHILOX, "explicit": _abi.RD_NOISE_EXPLICIT}
 
@@ -232,7 +267,10 @@ class DreamerPolicy:
         self.weights = w
         self._arch = _dreamer_arch(w)
         deter, hidden, units, embed, layers, _ = self._arch
-        if embed != env.n_beams:
+        self.depth = _encoder_depth(w, deter, embed)
+        if self.depth and not env.cfg.obs_flags & _abi.OBS_OCCUPANCY:
+            raise ValueError("a ConvEncoder agent reads lidar_occupancy: the env needs obs_type='lidar_occupancy'")
+        if not self.depth and embed != env.n_beams:
             raise ValueError(f"the checkpoint embeds {embed} beams, the env casts {env.n_beams}")
         if precision not in self.PRECISION:
             raise ValueError(f"precision {precision!r}: expected one of {sorted(self.PRECISION)}")
@@ -243,7 +281,11 @@ class DreamerPolicy:
             self._bn = np.ascontiguousarray(np.stack([w["bn_gamma"], w["bn_beta"], w["bn_mean"], w["bn_var"]]), np.float32)
         s = self._weights_struct(w, self._bn, lambda a: a.ctypes.data_as(C.c_void_p))
         with torch.cuda.device(env.device):
-            env._check(env.lib.rd_policy_dreamer_init(env._handle, C.byref(s)))
+            if self.depth:
+                e = self._encoder_struct(w, lambda a: a.ctypes.data_as(C.c_void_p))
+                env._check(env.lib.rd_policy_dreamer_init_occupancy(env._handle, C.byref(s), C.byref(e)))
+            else:
+                env._check(env.lib.rd_policy_dreamer_init(env._handle, C.byref(s)))
         self.actions = torch.zeros((env.n, 2), dtype=torch.float32, device=env.device)
         self.debug = torch.zeros(env.n * _abi.RD_DREAMER_DEBUG_FLOATS, dtype=torch.float32, device=env.device)
         self.expl_amount, self.expl_decay, self.expl_min = float(expl_amount), float(expl_decay), float(expl_min)
@@ -265,6 +307,13 @@ class DreamerPolicy:
         s.n_samples = self.n_samples                                            # [REF ros_agent/helpers/tools.py:55]
         s.precision = self.PRECISION[self.precision]
         return s
+
+    def _encoder_struct(self, w, ptr) -> "_abi.RdDreamerConvEncoder":
+        e = _abi.RdDreamerConvEncoder()
+        e.depth = self.depth
+        for l in range(4):
+            e.w[l], e.b[l] = ptr(w[f"enc{l + 1}_w"]), ptr(w[f"enc{l + 1}_b"])
+        return e
 
     def _set_exploration(self, env_steps: int) -> None:
         x = _abi.RdDreamerExploration(self.expl_amount, self.expl_decay, self.expl_min, int(env_steps))
@@ -303,8 +352,12 @@ class DreamerPolicy:
             names = ("deter", "hidden", "units", "embed", "actor layers", "BN head")
             diff = [f"{n} {a} != {b}" for n, a, b in zip(names, arch, self._arch) if a != b]
             raise ValueError("the weights do not match the policy's architecture: " + ", ".join(diff))
-        layers = arch[4]
-        keys = ["gru_kernel", "gru_recurrent", "gru_bias", "img1_w", "img1_b", "obs1_w", "obs1_b", "obs2_w", "obs2_b",
+        deter, _, _, embed, layers, _ = arch
+        depth = _encoder_depth(weights, deter, embed)
+        if depth != self.depth:
+            raise ValueError(f"the weights' ConvEncoder depth {depth} != the policy's {self.depth} (0 = none)")
+        keys = list(_ENC_KEYS) if depth else []
+        keys += ["gru_kernel", "gru_recurrent", "gru_bias", "img1_w", "img1_b", "obs1_w", "obs1_b", "obs2_w", "obs2_b",
                 "hout_w", "hout_b"] + [f"h{i}_{p}" for i in range(layers) for p in "wb"]
         if arch[5]:
             keys += ["bn_gamma", "bn_beta", "bn_mean", "bn_var"]
@@ -334,20 +387,33 @@ class DreamerPolicy:
             ptr = lambda a: a.ctypes.data_as(C.c_void_p)   # noqa: E731
         s = self._weights_struct(staged, bn, ptr)
         with torch.cuda.device(env.device):
-            env._check(env.lib.rd_policy_dreamer_set_weights(env._handle, C.byref(s), int(on_device), env._stream()))
+            if depth:
+                e = self._encoder_struct(staged, ptr)
+                env._check(env.lib.rd_policy_dreamer_set_weights_occupancy(env._handle, C.byref(s), C.byref(e), int(on_device),
+                                                                           env._stream()))
+            else:
+                env._check(env.lib.rd_policy_dreamer_set_weights(env._handle, C.byref(s), int(on_device), env._stream()))
         self._staged = (staged, bn)
 
     def act(self, lidar: Optional[torch.Tensor] = None, eps_stoch: Optional[torch.Tensor] = None,
             eps_actor: Optional[torch.Tensor] = None, debug: bool = False, noise: Optional[str] = None,
             training: bool = False, eps_sample: Optional[torch.Tensor] = None,
-            eps_expl: Optional[torch.Tensor] = None) -> torch.Tensor:
+            eps_expl: Optional[torch.Tensor] = None, occupancy: Optional[torch.Tensor] = None) -> torch.Tensor:
         """lidar f32 [N, n_beams] (default: the env's current observation) -> agent-facing actions f32 [N, 2].
+        A ConvEncoder agent reads ``occupancy`` u8 [N,64,64,1] instead (default: the env's current image).
         training=True: one actor sample plus exploration (the class docstring); noise='explicit' then takes
         ``eps_stoch`` [N,30], ``eps_sample`` [N,2] and ``eps_expl`` [N,2]."""
         env = self.env
-        li = env.buf["lidar"] if lidar is None else lidar
-        if li.shape != (env.n, env.n_beams) or li.dtype != torch.float32 or li.device != env.device or not li.is_contiguous():
-            raise ValueError(f"lidar must be a contiguous float32 CUDA tensor of shape ({env.n}, {env.n_beams})")
+        if self.depth:
+            if lidar is not None:
+                raise ValueError("this agent reads lidar_occupancy: pass occupancy=, not lidar")
+            li = self._occupancy(occupancy)
+        else:
+            if occupancy is not None:
+                raise ValueError("this agent reads lidar: pass lidar=, not occupancy")
+            li = env.buf["lidar"] if lidar is None else lidar
+            if li.shape != (env.n, env.n_beams) or li.dtype != torch.float32 or li.device != env.device or not li.is_contiguous():
+                raise ValueError(f"lidar must be a contiguous float32 CUDA tensor of shape ({env.n}, {env.n_beams})")
         mode = self.NOISE[noise or self.noise]
         cast = lambda t: t.to(device=env.device, dtype=torch.float32).contiguous()   # noqa: E731
         es = ea = ex = None
@@ -365,14 +431,36 @@ class DreamerPolicy:
                 raise ValueError("eps_stoch must be [N,30] and eps_actor [N,n_samples,2]")
         p = lambda t: t.data_ptr() if t is not None else None   # noqa: E731
         dbg = self.debug.data_ptr() if debug else None
+        lib = env.lib
         with torch.cuda.device(env.device):
             if training:
-                env._check(env.lib.rd_policy_dreamer_train(env._handle, li.data_ptr(), self.actions.data_ptr(), mode,
-                                                           p(es), p(ea), p(ex), dbg, env._stream()))
+                run = lib.rd_policy_dreamer_occupancy_train if self.depth else lib.rd_policy_dreamer_train
+                env._check(run(env._handle, li.data_ptr(), self.actions.data_ptr(), mode, p(es), p(ea), p(ex), dbg,
+                               env._stream()))
             else:
-                env._check(env.lib.rd_policy_dreamer(env._handle, li.data_ptr(), self.actions.data_ptr(), mode,
-                                                     p(es), p(ea), dbg, env._stream()))
+                run = lib.rd_policy_dreamer_occupancy if self.depth else lib.rd_policy_dreamer
+                env._check(run(env._handle, li.data_ptr(), self.actions.data_ptr(), mode, p(es), p(ea), dbg, env._stream()))
         return self.actions
+
+    def _occupancy(self, occupancy: Optional[torch.Tensor]) -> torch.Tensor:
+        env = self.env
+        occ = env.buf["occupancy"] if occupancy is None else occupancy
+        if (occ is None or occ.shape != (env.n, 64, 64, 1) or occ.dtype != torch.uint8 or occ.device != env.device
+                or not occ.is_contiguous()):
+            raise ValueError(f"occupancy must be a contiguous uint8 CUDA tensor of shape ({env.n}, 64, 64, 1)")
+        return occ
+
+    def encode(self, occupancy: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The ConvEncoder alone: occupancy u8 [N,64,64,1] (default: the env's current image) -> the embed f32
+        [N, 32 depth] obs1 reads (its hi + lo parts).  The recurrent state is untouched."""
+        if not self.depth:
+            raise ValueError("encode() needs a ConvEncoder agent (weights with enc1_w .. enc4_b)")
+        env = self.env
+        occ = self._occupancy(occupancy)
+        out = torch.empty((env.n, 32 * self.depth), dtype=torch.float32, device=env.device)
+        with torch.cuda.device(env.device):
+            env._check(env.lib.rd_dreamer_encode_occupancy(env._handle, occ.data_ptr(), out.data_ptr(), env._stream()))
+        return out
 
     def diagnostics(self) -> Dict[str, torch.Tensor]:
         """Valid after ``act(debug=True)``: posterior mean/std, actor mean/std, action, log-prob and index of the mode.
