@@ -307,8 +307,10 @@ enum { RD_NOISE_ZERO = 0,      /* none: stoch = mean, action = tanh(actor mean) 
        RD_NOISE_PHILOX = 1,    /* Philox(cfg.seed; env id, policy step)          [NEW-SPEC, the reference uses TF's RNG] */
        RD_NOISE_EXPLICIT = 2   /* caller-provided draws (teacher-forced parity tests) */ };
 #define RD_DREAMER_DEBUG_FLOATS 68   /* per env: posterior mean[30] std[30] | actor mean[2] std[2] action[2] log_prob index */
-/* Uploads the weights (transposed to K-major, lidar normalisation x/15 - 0.5 folded into obs1 unless the env emits
- * normalised scans) and allocates the per-env latent state; idempotent (a second call replaces weights, clears state). */
+/* Allocates the weights and the per-env latent state and packs the weights on the device (K-major TF32 operands, the
+ * packing rd_policy_dreamer_set_weights uses); returns after the packing finished.  The scans are normalised on the
+ * device (x/15 - 0.5) unless the env emits normalised ones.  Idempotent: a second call replaces the agent and clears the
+ * state; a rejected call (RD_ERR_INVALID, e.g. a device pointer in w) leaves the current agent working. */
 int rd_policy_dreamer_init(rd_env* env, const rd_dreamer_weights* w);
 /* One agent step per env.  lidar_dev f32 [N, n_beams] (an rd_step / rd_reset output), actions_dev f32 [N,2]
  * agent-facing (what rd_step takes; its rescale is postprocess_action [REF racing_dreamer.py:54-60]).

@@ -13,7 +13,6 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
-#include <cstring>
 #include <string>
 #include <vector>
 
@@ -65,17 +64,9 @@ struct DreamerPolicy {
   // at least min_amount (min_amount > 0); env_steps = Dreamer's step counter, + n_envs * action_repeat per training step
   double expl_amount = 0.3, expl_decay = 0.0, expl_min = 0.0;
   int64_t env_steps = 0;
-  float* stage = nullptr;      // device copy of host-pointer weights for dreamer_set_weights (sized at init)
+  float* stage = nullptr;      // device copy of host-pointer weights for dr_pack (sized at init)
   std::string err;
 };
-
-static inline float dr_tf32(float x) {   // cvt.rna.tf32.f32 on the host (finite values)
-  uint32_t u;
-  std::memcpy(&u, &x, 4);
-  u = (u + 0x1000u) & ~0x1fffu;
-  std::memcpy(&x, &u, 4);
-  return x;
-}
 
 static inline void dreamer_free(DreamerPolicy& d) {
   for (float* p : d.owned) cudaFree(p);
@@ -86,11 +77,12 @@ static inline void dreamer_free(DreamerPolicy& d) {
 }
 
 // The policy's weight layout: each checkpoint array, where it goes and how.  Matrices ([in][out] Keras kernels) become
-// K-major TF32 operands (dr_upload_t: pitch ld, the K slots from k_from on shifted by k_shift); vectors (op == null)
-// are copied as they are to *vec.  Both dreamer_init and dreamer_set_weights walk this one list.
+// K-major TF32 operands [out][ld] (k_pack_weights: the K slots from k_from on shifted by k_shift, the slots skipped stay
+// as init's zero fill left them); vectors (op == null) are copied as they are to *vec.  Sizes are w's, which the callers
+// have checked (init) or held to the policy's (set_weights).  Init allocates and dr_pack fills what this list names.
 struct DrPart { const float* src; DreamerPolicy::Operand* op; float** vec; int in, out, ld, k_from, k_shift; };
 static inline int dr_parts(DreamerPolicy& d, const rd_dreamer_weights* w, const rd_dreamer_conv_encoder* enc, DrPart* p) {
-  const int H = d.hidden, D = d.deter, E = d.embed, U = d.units, L = d.layers, NO = 1 << 30;
+  const int H = w->hidden, D = w->deter, E = w->embed, U = w->actor_units, L = w->actor_layers, NO = 1 << 30;
   int k = 0;
   auto mat = [&](const float* src, DreamerPolicy::Operand& op, int in, int out, int ld, int k_from, int k_shift) {
     p[k++] = DrPart{src, &op, nullptr, in, out, ld, k_from, k_shift};
@@ -106,7 +98,7 @@ static inline int dr_parts(DreamerPolicy& d, const rd_dreamer_weights* w, const 
   mat(w->obs2_w, d.w_obs2, H, 2 * GM_STOCH, H, NO, 0);
   vec(w->obs2_b, d.b_obs2, 2 * GM_STOCH);
   // actor h0: rows [stoch | deter] -> K slots [0, 30) and [32, 32 + deter); the two action slots get zero weights
-  mat(w->actor_w[0], d.w_act[0], GM_STOCH + D, U, d.ldf, GM_STOCH, 2);
+  mat(w->actor_w[0], d.w_act[0], GM_STOCH + D, U, 32 + D, GM_STOCH, 2);
   vec(w->actor_b[0], d.b_act[0], U);
   for (int i = 1; i < L; ++i) {
     mat(w->actor_w[i], d.w_act[i], U, U, U, NO, 0);
@@ -122,6 +114,7 @@ static inline int dr_parts(DreamerPolicy& d, const rd_dreamer_weights* w, const 
   return k;
 }
 #define DR_MAX_PARTS (9 + 2 * 8 + 1 + 5)
+static_assert(DR_MAX_PARTS <= GM_PACK_MAX, "dr_pack packs the whole table in one k_pack_weights launch");
 
 // Cin of conv layer l = 1..3 (conv2..conv4) of a depth-d encoder; Cout = 2 Cin
 static inline int dr_conv_cin(int depth, int l) { return depth << (l - 1); }
@@ -137,37 +130,10 @@ static inline cudaError_t dr_pack_conv(DreamerPolicy& d, const float* const* src
   return cudaSuccess;
 }
 
-// [in][out] host matrix -> device [out][ld] (K-major), element (o, kmap(i)) = scale_i * W[i][o], split into its TF32
-// rounding (op.p[0]) and, in x3 mode, the TF32 rounding of the remainder (op.p[1])
-static inline cudaError_t dr_upload_t(DreamerPolicy& d, DreamerPolicy::Operand& op, const float* w, int in, int out, int ld,
-                                      int k_shift_from, int k_shift, const std::vector<float>* col_scale = nullptr) {
-  std::vector<float> hi((size_t)out * ld, 0.f), lo((size_t)out * ld, 0.f);
-  for (int i = 0; i < in; ++i) {
-    const int k = i >= k_shift_from ? i + k_shift : i;
-    const float sc = col_scale ? (*col_scale)[i] : 1.f;
-    for (int o = 0; o < out; ++o) {
-      const float x = w[(size_t)i * out + o] * sc, h = dr_tf32(x);
-      hi[(size_t)o * ld + k] = h;
-      lo[(size_t)o * ld + k] = dr_tf32(x - h);
-    }
-  }
-  for (int part = 0; part < (d.x3 ? 2 : 1); ++part) {
-    cudaError_t e = cudaMalloc(&op.p[part], hi.size() * sizeof(float));
-    if (e != cudaSuccess) return e;
-    d.owned.push_back(op.p[part]);
-    e = cudaMemcpy(op.p[part], (part ? lo : hi).data(), hi.size() * sizeof(float), cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) return e;
-  }
-  return cudaSuccess;
-}
-static inline cudaError_t dr_upload(DreamerPolicy& d, float** dst, const float* v, size_t count) {
-  cudaError_t e = cudaMalloc(dst, count * sizeof(float));
-  if (e != cudaSuccess) return e;
-  d.owned.push_back(*dst);
-  return cudaMemcpy(*dst, v, count * sizeof(float), cudaMemcpyHostToDevice);
-}
-// zero-initialised activation array(s) [rows][ld]
+// zero-initialised operand array(s) [rows][ld].  In single-pass mode p[1] is null -- the packer and the epilogues test it
+// -- also where the operand held a freed remainder array of an earlier tf32x3 agent (dr_view likewise).
 static inline cudaError_t dr_alloc(DreamerPolicy& d, DreamerPolicy::Operand& op, size_t rows, size_t ld) {
+  op.p[1] = nullptr;
   for (int part = 0; part < (d.x3 ? 2 : 1); ++part) {
     cudaError_t e = cudaMalloc(&op.p[part], rows * ld * sizeof(float));
     if (e != cudaSuccess) return e;
@@ -184,6 +150,7 @@ static inline bool dr_view(const DreamerPolicy& d, DreamerPolicy::Operand& view,
     view.p[part] = base.p[part] + col0;
     if (!gm_make_map(&view.m[part], view.p[part], inner, rows, ld, box_rows)) return false;
   }
+  if (!d.x3) view.p[1] = nullptr;
   return true;
 }
 
@@ -197,6 +164,74 @@ static inline bool dr_view(const DreamerPolicy& d, DreamerPolicy::Operand& view,
     if (!(expr)) { d.err = "cuTensorMapEncodeTiled failed: " #expr; return RD_ERR_CUDA; }       \
   } while (0)
 
+// Every source array of w and enc (dr_parts' and conv2..conv4's kernels) is non-null and, with on_device, memory of the
+// current device, else not device memory.  Reads w's architecture: run it after that is checked.
+static inline int dr_check_sources(DreamerPolicy& d, const rd_dreamer_weights* w, const rd_dreamer_conv_encoder* enc,
+                                   bool on_device) {
+  DrPart parts[DR_MAX_PARTS];
+  const int n_parts = dr_parts(d, w, enc, parts);
+  const float* srcs[DR_MAX_PARTS + 3];
+  int n_src = 0;
+  for (int k = 0; k < n_parts; ++k) srcs[n_src++] = parts[k].src;
+  for (int l = 1; enc && l < 4; ++l) srcs[n_src++] = enc->w[l];
+  int dev = 0;
+  DR_TRY(cudaGetDevice(&dev));
+  for (int k = 0; k < n_src; ++k) {
+    if (!srcs[k]) { d.err = "null weight pointer"; return RD_ERR_INVALID; }
+    cudaPointerAttributes at{};
+    DR_TRY(cudaPointerGetAttributes(&at, srcs[k]));
+    const bool device_ptr = at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged;
+    if (on_device && (!device_ptr || at.device != dev)) { d.err = "on_device: a weight pointer is not memory of the policy's device"; return RD_ERR_INVALID; }
+    if (!on_device && at.type == cudaMemoryTypeDevice) { d.err = "a weight pointer is device memory where host memory is expected (init, or on_device = 0)"; return RD_ERR_INVALID; }
+  }
+  return RD_OK;
+}
+
+// Packs w and enc (checked by dr_check_sources) into the buffers init allocated, on `s`: host sources (!on_device) are
+// first copied to d.stage, then one k_pack_weights launch packs the dr_parts table and dr_pack_conv conv2..conv4.
+static inline int dr_pack(DreamerPolicy& d, const rd_dreamer_weights* w, const rd_dreamer_conv_encoder* enc, bool on_device,
+                          cudaStream_t s) {
+  DrPart parts[DR_MAX_PARTS];
+  const int n_parts = dr_parts(d, w, enc, parts);
+  PackArgs a{};
+  a.n_jobs = n_parts;
+  size_t off = 0;
+  for (int k = 0; k < n_parts; ++k) {
+    const DrPart& p = parts[k];
+    const size_t count = (size_t)p.in * p.out;
+    const float* src = p.src;
+    if (!on_device) {
+      DR_TRY(cudaMemcpyAsync(d.stage + off, p.src, count * sizeof(float), cudaMemcpyHostToDevice, s));
+      src = d.stage + off;
+    }
+    PackJob& J = a.job[k];
+    J.src = src;
+    J.hi = p.op ? p.op->p[0] : *p.vec;
+    J.lo = p.op ? p.op->p[1] : nullptr;
+    J.in = p.in; J.out = p.out; J.ld = p.ld; J.k_from = p.k_from; J.k_shift = p.k_shift; J.raw = p.op ? 0 : 1;
+    J.begin = (long long)off;
+    off += count;
+  }
+  a.total = (long long)off;
+  const unsigned grid = (unsigned)std::min<size_t>((off + 255) / 256, (size_t)d.sm_count * 8);
+  k_pack_weights<<<grid, 256, 0, s>>>(a);
+  DR_TRY(cudaGetLastError());
+  if (enc) {
+    const float* src[3];
+    for (int l = 1; l < 4; ++l) {
+      const size_t count = (size_t)32 * dr_conv_cin(d.depth, l) * dr_conv_cin(d.depth, l);
+      src[l - 1] = enc->w[l];
+      if (!on_device) {
+        DR_TRY(cudaMemcpyAsync(d.stage + off, enc->w[l], count * sizeof(float), cudaMemcpyHostToDevice, s));
+        src[l - 1] = d.stage + off;
+      }
+      off += count;
+    }
+    DR_TRY(dr_pack_conv(d, src, s));
+  }
+  return RD_OK;
+}
+
 // lidar_normalised: the env already emits r/15 - 0.5 (RD_OBS_LIDAR_NORM), so k_embed_lidar only splits the values
 // enc: a ConvEncoder agent (embed = 32 depth) instead of the lidar one (embed = n_beams)
 static inline int dreamer_init(DreamerPolicy& d, int n, int n_beams, bool lidar_normalised, const rd_dreamer_weights* w,
@@ -205,8 +240,6 @@ static inline int dreamer_init(DreamerPolicy& d, int n, int n_beams, bool lidar_
   if (enc) {
     if (enc->depth != 32) { d.err = "unsupported ConvEncoder depth " + std::to_string(enc->depth) + " (need 32)"; return RD_ERR_INVALID; }
     if (w->embed != 32 * enc->depth) { d.err = "a ConvEncoder agent's embed must be 32 * depth"; return RD_ERR_INVALID; }
-    for (int l = 0; l < 4; ++l)
-      if (!enc->w[l] || !enc->b[l]) { d.err = "null encoder weight pointer"; return RD_ERR_INVALID; }
   }
   if (w->stoch != GM_STOCH || w->deter <= 0 || w->deter % 4 || w->hidden <= 0 || w->hidden % 4 ||
       (!enc && w->embed != n_beams) || w->embed % 4 || w->actor_units <= 0 || w->actor_units % 4 || w->actor_layers < 1 || w->actor_layers > 7 ||
@@ -214,13 +247,9 @@ static inline int dreamer_init(DreamerPolicy& d, int n, int n_beams, bool lidar_
     d.err = "unsupported Dreamer architecture (need stoch 30, deter/hidden/units/embed multiples of 4, embed == n_beams (lidar agent), 1..7 actor layers)";
     return RD_ERR_INVALID;
   }
-  const float* need[] = {w->gru_kernel, w->gru_recurrent, w->gru_bias, w->img1_w, w->img1_b, w->obs1_w, w->obs1_b, w->obs2_w, w->obs2_b};
-  for (const float* p : need)
-    if (!p) { d.err = "null weight pointer"; return RD_ERR_INVALID; }
-  for (int i = 0; i <= w->actor_layers; ++i)
-    if (!w->actor_w[i] || !w->actor_b[i]) { d.err = "null actor weight pointer"; return RD_ERR_INVALID; }
   if (!gm_get_encoder()) { d.err = "cuTensorMapEncodeTiled is not available from this driver"; return RD_ERR_CUDA; }
   if (w->precision != RD_PRECISION_TF32X3 && w->precision != RD_PRECISION_TF32) { d.err = "bad precision"; return RD_ERR_INVALID; }
+  if (int rc = dr_check_sources(d, w, enc, false)) return rc;   // all checks before dreamer_free: a rejected init changes nothing
   dreamer_free(d);
   d.x3 = w->precision == RD_PRECISION_TF32X3;
   d.lidar_normalised = lidar_normalised;
@@ -230,35 +259,33 @@ static inline int dreamer_init(DreamerPolicy& d, int n, int n_beams, bool lidar_
   d.raw_init_std = (float)std::log(std::exp((double)w->init_std) - 1.0);   // [REF models.py:321]
   d.min_std = w->min_std; d.mean_scale = w->mean_scale; d.bn_eps = w->bn_eps; d.n_samples = w->n_samples;
   const int H = d.hidden, D = d.deter, E = d.embed, U = d.units;
+  int dev = 0;
+  DR_TRY(cudaGetDevice(&dev));
+  DR_TRY(cudaDeviceGetAttribute(&d.sm_count, cudaDevAttrMultiProcessorCount, dev));
+  // the weights' buffers (matrices zero-filled: the K slots k_pack_weights skips stay zero) and the stage that holds
+  // a copy of every host source, the table's arrays and then conv2..conv4's kernels
   DrPart parts[DR_MAX_PARTS];
   const int n_parts = dr_parts(d, w, enc, parts);
   size_t stage_floats = 0;
   for (int k = 0; k < n_parts; ++k) {
     const DrPart& p = parts[k];
-    if (p.op) DR_TRY(dr_upload_t(d, *p.op, p.src, p.in, p.out, p.ld, p.k_from, p.k_shift));
-    else DR_TRY(dr_upload(d, p.vec, p.src, (size_t)p.out));
+    if (p.op) {
+      DR_TRY(dr_alloc(d, *p.op, (size_t)p.out, (size_t)p.ld));
+    } else {
+      DR_TRY(cudaMalloc(p.vec, (size_t)p.out * sizeof(float)));
+      d.owned.push_back(*p.vec);
+    }
     stage_floats += (size_t)p.in * p.out;
   }
-  size_t conv_floats = 0;   // conv2..conv4 kernels: packed on the device from the stage, as dreamer_set_weights packs them
   for (int l = 1; d.depth && l < 4; ++l) {
     const int cin = dr_conv_cin(d.depth, l);
     DR_TRY(dr_alloc(d, d.w_conv[l - 1], (size_t)2 * cin, (size_t)16 * cin));
-    conv_floats += (size_t)32 * cin * cin;
+    stage_floats += (size_t)32 * cin * cin;
   }
-  DR_TRY(cudaMalloc(&d.stage, (stage_floats + conv_floats) * sizeof(float)));
+  DR_TRY(cudaMalloc(&d.stage, stage_floats * sizeof(float)));
   d.owned.push_back(d.stage);
-  if (d.depth) {
-    const float* src[3];
-    size_t off = 0;
-    for (int l = 1; l < 4; ++l) {
-      const size_t count = (size_t)32 * dr_conv_cin(d.depth, l) * dr_conv_cin(d.depth, l);
-      DR_TRY(cudaMemcpy(d.stage + off, enc->w[l], count * sizeof(float), cudaMemcpyHostToDevice));
-      src[l - 1] = d.stage + off;
-      off += count;
-    }
-    DR_TRY(dr_pack_conv(d, src, 0));
-    DR_TRY(cudaDeviceSynchronize());
-  }
+  if (int rc = dr_pack(d, w, enc, false, 0)) return rc;
+  DR_TRY(cudaDeviceSynchronize());
   const size_t N = (size_t)n;
   for (int p = 0; p < 2; ++p) {
     DR_TRY(dr_alloc(d, d.feat[p], N, d.ldf));
@@ -272,9 +299,6 @@ static inline int dreamer_init(DreamerPolicy& d, int n, int n_beams, bool lidar_
     d.owned.push_back(reinterpret_cast<float*>(d.chain_flags));
     DR_TRY(cudaMemset(d.chain_flags, 0, GM_CHAIN_MAX * row_blocks * sizeof(unsigned)));
     for (unsigned& c : d.chain_count) c = 0;
-    int dev = 0;
-    DR_TRY(cudaGetDevice(&dev));
-    DR_TRY(cudaDeviceGetAttribute(&d.sm_count, cudaDevAttrMultiProcessorCount, dev));
     d.chain = true;
     if (const char* ev = std::getenv("RD_DREAMER_CHAIN")) d.chain = std::atoi(ev) != 0;
   }
@@ -330,10 +354,10 @@ static inline float dreamer_expl_amount(const DreamerPolicy& d) {
   return (float)a;
 }
 
-// New values for every weight of an initialised policy, packed on the device on `s` into the buffers it already owns
-// (no allocation; the tensor maps stay valid) bit for bit as dreamer_init packs them.  Latent state, Philox step and
-// env_steps are kept.  w holds device pointers (on_device) or host pointers, which are first copied to d.stage.  The
-// architecture, precision and head scalars must be the init's; otherwise RD_ERR_INVALID and nothing changes.
+// New values for every weight of an initialised policy, packed on `s` by init's packer (dr_pack) into the buffers the
+// policy already owns (no allocation; the tensor maps stay valid).  Latent state, Philox step and env_steps are kept.
+// w holds device pointers (on_device) or host pointers, which are first copied to d.stage.  The architecture, precision
+// and head scalars must be the init's; otherwise RD_ERR_INVALID and nothing changes.
 static inline int dreamer_set_weights(DreamerPolicy& d, const rd_dreamer_weights* w, const rd_dreamer_conv_encoder* enc,
                                       bool on_device, cudaStream_t s) {
   if (!w) { d.err = "null weights"; return RD_ERR_INVALID; }
@@ -350,59 +374,8 @@ static inline int dreamer_set_weights(DreamerPolicy& d, const rd_dreamer_weights
     d.err = "the weights' architecture, precision or head scalars differ from the ones the policy was initialised with";
     return RD_ERR_INVALID;
   }
-  DrPart parts[DR_MAX_PARTS];
-  const int n_parts = dr_parts(d, w, enc, parts);
-  int dev = 0;
-  DR_TRY(cudaGetDevice(&dev));
-  const float* srcs[DR_MAX_PARTS + 3];   // every source array: the table's, then conv2..conv4's kernels
-  int n_src = 0;
-  for (int k = 0; k < n_parts; ++k) srcs[n_src++] = parts[k].src;
-  for (int l = 1; enc && l < 4; ++l) srcs[n_src++] = enc->w[l];
-  for (int k = 0; k < n_src; ++k) {
-    if (!srcs[k]) { d.err = "null weight pointer"; return RD_ERR_INVALID; }
-    cudaPointerAttributes at{};
-    DR_TRY(cudaPointerGetAttributes(&at, srcs[k]));
-    const bool device_ptr = at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged;
-    if (on_device && (!device_ptr || at.device != dev)) { d.err = "on_device: a weight pointer is not memory of the policy's device"; return RD_ERR_INVALID; }
-    if (!on_device && at.type == cudaMemoryTypeDevice) { d.err = "a device pointer was passed with on_device = 0"; return RD_ERR_INVALID; }
-  }
-  PackArgs a{};
-  a.n_jobs = n_parts;
-  size_t off = 0;
-  for (int k = 0; k < n_parts; ++k) {
-    const DrPart& p = parts[k];
-    const size_t count = (size_t)p.in * p.out;
-    const float* src = p.src;
-    if (!on_device) {
-      DR_TRY(cudaMemcpyAsync(d.stage + off, p.src, count * sizeof(float), cudaMemcpyHostToDevice, s));
-      src = d.stage + off;
-    }
-    PackJob& J = a.job[k];
-    J.src = src;
-    J.hi = p.op ? p.op->p[0] : *p.vec;
-    J.lo = p.op ? p.op->p[1] : nullptr;
-    J.in = p.in; J.out = p.out; J.ld = p.ld; J.k_from = p.k_from; J.k_shift = p.k_shift; J.raw = p.op ? 0 : 1;
-    J.begin = (long long)off;
-    off += count;
-  }
-  a.total = (long long)off;
-  const unsigned grid = (unsigned)std::min<size_t>((off + 255) / 256, (size_t)d.sm_count * 8);
-  k_pack_weights<<<grid, 256, 0, s>>>(a);
-  DR_TRY(cudaGetLastError());
-  if (enc) {
-    const float* src[3];
-    for (int l = 1; l < 4; ++l) {
-      const size_t count = (size_t)32 * dr_conv_cin(d.depth, l) * dr_conv_cin(d.depth, l);
-      src[l - 1] = enc->w[l];
-      if (!on_device) {
-        DR_TRY(cudaMemcpyAsync(d.stage + off, enc->w[l], count * sizeof(float), cudaMemcpyHostToDevice, s));
-        src[l - 1] = d.stage + off;
-      }
-      off += count;
-    }
-    DR_TRY(dr_pack_conv(d, src, s));
-  }
-  return RD_OK;
+  if (int rc = dr_check_sources(d, w, enc, on_device)) return rc;
+  return dr_pack(d, w, enc, on_device, s);
 }
 
 // One layer's launch description: up to two (A source, W, K range) terms.  dr_build expands them into phases:

@@ -1076,6 +1076,16 @@ RD_API void rd_gap_follower_defaults(const rd_config* cfg, rd_gap_follower* g) {
   g->speed_gain = 1.0;
 }
 
+namespace {
+// the [n][2] actions the rollouts of every on-device policy write when the caller passes none (one per handle)
+int ensure_rollout_actions(rd_env* env) {
+  if (env->pol.d_actions) return RD_OK;
+  CUDA_TRY(env, cudaMalloc(&env->pol.d_actions, sizeof(float) * 2 * (size_t)env->n));
+  CUDA_TRY(env, cudaMemset(env->pol.d_actions, 0, sizeof(float) * 2 * (size_t)env->n));
+  return RD_OK;
+}
+}  // namespace
+
 RD_API int rd_policy_gap_follower_init(rd_env* env, const rd_gap_follower* g_or_null) {
   if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
   if (env->cfg.obs_flags & RD_OBS_LIDAR_F16) return fail(env, RD_ERR_INVALID, "the on-device policies read float32 scans: RD_OBS_LIDAR_F16 is set");
@@ -1092,9 +1102,8 @@ RD_API int rd_policy_gap_follower_init(rd_env* env, const rd_gap_follower* g_or_
   if (!p.st.f64) {
     CUDA_TRY(env, cudaMalloc(&p.st.f64, sizeof(double) * RD_NP_F64 * n));
     CUDA_TRY(env, cudaMalloc(&p.st.i32, sizeof(int32_t) * RD_NP_I32 * n));
-    CUDA_TRY(env, cudaMalloc(&p.d_actions, sizeof(float) * 2 * n));
-    CUDA_TRY(env, cudaMemset(p.d_actions, 0, sizeof(float) * 2 * n));
   }
+  if (int rc = ensure_rollout_actions(env)) return rc;
   std::vector<double> f(RD_NP_F64 * n, 0.0);
   for (size_t e = 0; e < n; ++e) f[(size_t)RD_P_PREV * n + e] = std::nan("");
   CUDA_TRY(env, cudaMemcpy(p.st.f64, f.data(), sizeof(double) * f.size(), cudaMemcpyHostToDevice));
@@ -1157,18 +1166,6 @@ RD_API int rd_rollout_gap_follower(rd_env* env, int n_steps, const rd_outputs* o
   return RD_OK;
 }
 
-RD_API int rd_policy_dreamer_init(rd_env* env, const rd_dreamer_weights* w) {
-  if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
-  if (env->cfg.obs_flags & RD_OBS_LIDAR_F16) return fail(env, RD_ERR_INVALID, "the on-device policies read float32 scans: RD_OBS_LIDAR_F16 is set");
-  const int rc = dreamer_init(env->dr, env->n, env->cfg.n_beams, (env->cfg.obs_flags & RD_OBS_LIDAR_NORM) != 0, w);
-  if (rc) return fail(env, rc, "rd_policy_dreamer_init: %s", env->dr.err.c_str());
-  if (!env->pol.d_actions) {
-    CUDA_TRY(env, cudaMalloc(&env->pol.d_actions, sizeof(float) * 2 * (size_t)env->n));
-    CUDA_TRY(env, cudaMemset(env->pol.d_actions, 0, sizeof(float) * 2 * (size_t)env->n));
-  }
-  return RD_OK;
-}
-
 namespace {
 // training: Dreamer.policy(training=True) -- one sample + exploration (k_actor_train), and the env-step counter of the
 // exploration schedule advances by n_envs * action_repeat [REF dreamer/dreamer.py, Dreamer.__call__ self._step]
@@ -1197,21 +1194,80 @@ int dreamer_kind(rd_env* env, bool encoder, const char* fn) {
                 "occupancy entry points", fn);
   return RD_OK;
 }
-// what a rollout feeds the agent: the scans, or the images for an encoder agent (null if the env does not produce them)
-const void* dreamer_obs(rd_env* env, const rd_outputs* out) {
-  if (!env->dr.depth) return out->lidar_dev;
-  return (env->cfg.obs_flags & RD_OBS_OCCUPANCY) ? out->occupancy_dev : nullptr;
+// rd_policy_dreamer_init and _init_occupancy (encoder: the latter, enc its image encoder)
+int init_dreamer(rd_env* env, const rd_dreamer_weights* w, bool encoder, const rd_dreamer_conv_encoder* enc, const char* fn) {
+  if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
+  if (encoder && !enc) return fail(env, RD_ERR_INVALID, "%s: null encoder", fn);
+  if (encoder && !(env->cfg.obs_flags & RD_OBS_OCCUPANCY))
+    return fail(env, RD_ERR_INVALID, "%s: the env does not produce lidar_occupancy (RD_OBS_OCCUPANCY)", fn);
+  if (!encoder && (env->cfg.obs_flags & RD_OBS_LIDAR_F16))
+    return fail(env, RD_ERR_INVALID, "the on-device policies read float32 scans: RD_OBS_LIDAR_F16 is set");
+  const bool lidar_normalised = !encoder && (env->cfg.obs_flags & RD_OBS_LIDAR_NORM);
+  const int rc = dreamer_init(env->dr, env->n, env->cfg.n_beams, lidar_normalised, w, enc);
+  if (rc) return fail(env, rc, "%s: %s", fn, env->dr.err.c_str());
+  return ensure_rollout_actions(env);
+}
+// the four agent-step entry points: obs_dev is the scans or (encoder) the images; training reads eps_expl_dev as well
+int step_dreamer(rd_env* env, const void* obs_dev, bool encoder, bool training, float* actions_dev, int noise,
+                 const float* eps_stoch_dev, const float* eps_actor_dev, const float* eps_expl_dev, float* debug_dev,
+                 void* stream, const char* fn) {
+  if (!env || !obs_dev || !actions_dev) return fail(env, RD_ERR_INVALID, "null argument");
+  if (int rc = dreamer_kind(env, encoder, fn)) return rc;
+  if (noise < RD_NOISE_ZERO || noise > RD_NOISE_EXPLICIT) return fail(env, RD_ERR_INVALID, "bad noise mode %d", noise);
+  if (noise == RD_NOISE_EXPLICIT && (!eps_stoch_dev || !eps_actor_dev || (training && !eps_expl_dev)))
+    return fail(env, RD_ERR_INVALID, training ? "RD_NOISE_EXPLICIT needs eps_stoch_dev, eps_sample_dev and eps_expl_dev"
+                                              : "RD_NOISE_EXPLICIT needs eps_stoch_dev and eps_actor_dev");
+  return launch_dreamer(env, obs_dev, actions_dev, noise, eps_stoch_dev, eps_actor_dev, debug_dev, (cudaStream_t)stream,
+                        training, eps_expl_dev);
+}
+// the checks every Dreamer rollout makes; *obs = what it feeds the agent: the scans, or an encoder agent's images
+int dreamer_rollout_obs(rd_env* env, const rd_outputs* out, int noise, const void** obs) {
+  if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
+  if (!env->dr.depth) *obs = out->lidar_dev;
+  else *obs = (env->cfg.obs_flags & RD_OBS_OCCUPANCY) ? out->occupancy_dev : nullptr;
+  if (!*obs)
+    return fail(env, RD_ERR_INVALID, env->dr.depth ? "the rollout needs out->occupancy_dev and an env that produces it (RD_OBS_OCCUPANCY)"
+                                                   : "the rollout needs out->lidar_dev");
+  if (noise != RD_NOISE_ZERO && noise != RD_NOISE_PHILOX)
+    return fail(env, RD_ERR_INVALID, "a rollout draws its own noise (RD_NOISE_ZERO or RD_NOISE_PHILOX)");
+  return RD_OK;
+}
+// rd_rollout_dreamer and _train
+int rollout_dreamer(rd_env* env, int n_steps, const rd_outputs* out, float* actions_dev, int noise, void* stream,
+                    bool training) {
+  if (!env || !out || n_steps < 0) return fail(env, RD_ERR_INVALID, "bad argument");
+  const void* obs = nullptr;
+  if (int rc = dreamer_rollout_obs(env, out, noise, &obs)) return rc;
+  if (!env->was_reset) return fail(env, RD_ERR_STATE, "Must reset environment.");
+  float* act = actions_dev ? actions_dev : env->pol.d_actions;
+  for (int k = 0; k < n_steps; ++k) {
+    int rc = launch_dreamer(env, obs, act, noise, nullptr, nullptr, nullptr, (cudaStream_t)stream, training);
+    if (rc) return rc;
+    if ((rc = rd_step(env, act, out, stream))) return rc;
+  }
+  return RD_OK;
+}
+// rd_policy_dreamer_set_weights and _set_weights_occupancy (encoder: the latter, enc its image encoder)
+int set_dreamer_weights(rd_env* env, const rd_dreamer_weights* w, bool encoder, const rd_dreamer_conv_encoder* enc,
+                        int on_device, void* stream, const char* fn) {
+  if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
+  if (encoder && !enc) return fail(env, RD_ERR_INVALID, "%s: null encoder", fn);
+  if (int rc = dreamer_kind(env, encoder, fn)) return rc;
+  const int rc = dreamer_set_weights(env->dr, w, enc, on_device != 0, (cudaStream_t)stream);
+  if (rc) return fail(env, rc, "%s: %s", fn, env->dr.err.c_str());
+  env->launches += encoder ? 4 : 1;   // k_pack_weights, then k_pack_conv for conv2..conv4
+  return RD_OK;
 }
 }  // namespace
 
+RD_API int rd_policy_dreamer_init(rd_env* env, const rd_dreamer_weights* w) {
+  return init_dreamer(env, w, false, nullptr, "rd_policy_dreamer_init");
+}
+
 RD_API int rd_policy_dreamer(rd_env* env, const float* lidar_dev, float* actions_dev, int noise, const float* eps_stoch_dev,
                              const float* eps_actor_dev, float* debug_dev, void* stream) {
-  if (!env || !lidar_dev || !actions_dev) return fail(env, RD_ERR_INVALID, "null argument");
-  if (int rc = dreamer_kind(env, false, "rd_policy_dreamer")) return rc;
-  if (noise < RD_NOISE_ZERO || noise > RD_NOISE_EXPLICIT) return fail(env, RD_ERR_INVALID, "bad noise mode %d", noise);
-  if (noise == RD_NOISE_EXPLICIT && (!eps_stoch_dev || !eps_actor_dev))
-    return fail(env, RD_ERR_INVALID, "RD_NOISE_EXPLICIT needs eps_stoch_dev and eps_actor_dev");
-  return launch_dreamer(env, lidar_dev, actions_dev, noise, eps_stoch_dev, eps_actor_dev, debug_dev, (cudaStream_t)stream);
+  return step_dreamer(env, lidar_dev, false, false, actions_dev, noise, eps_stoch_dev, eps_actor_dev, nullptr, debug_dev,
+                      stream, "rd_policy_dreamer");
 }
 
 RD_API int rd_policy_dreamer_get_state(rd_env* env, float* stoch_dev, float* deter_dev, float* action_dev, void* stream) {
@@ -1233,50 +1289,17 @@ RD_API int rd_policy_dreamer_set_state(rd_env* env, const float* stoch_dev, cons
 }
 
 RD_API int rd_rollout_dreamer(rd_env* env, int n_steps, const rd_outputs* out, float* actions_dev, int noise, void* stream) {
-  if (!env || !out || n_steps < 0) return fail(env, RD_ERR_INVALID, "bad argument");
-  if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
-  const void* obs = dreamer_obs(env, out);
-  if (!obs)
-    return fail(env, RD_ERR_INVALID, env->dr.depth ? "the rollout needs out->occupancy_dev and an env that produces it (RD_OBS_OCCUPANCY)"
-                                                   : "bad argument (the rollout needs out->lidar_dev)");
-  if (noise != RD_NOISE_ZERO && noise != RD_NOISE_PHILOX) return fail(env, RD_ERR_INVALID, "a rollout draws its own noise (RD_NOISE_ZERO or RD_NOISE_PHILOX)");
-  if (!env->was_reset) return fail(env, RD_ERR_STATE, "Must reset environment.");
-  float* act = actions_dev ? actions_dev : env->pol.d_actions;
-  for (int k = 0; k < n_steps; ++k) {
-    int rc = launch_dreamer(env, obs, act, noise, nullptr, nullptr, nullptr, (cudaStream_t)stream);
-    if (rc) return rc;
-    if ((rc = rd_step(env, act, out, stream))) return rc;
-  }
-  return RD_OK;
+  return rollout_dreamer(env, n_steps, out, actions_dev, noise, stream, false);
 }
 
 RD_API int rd_policy_dreamer_train(rd_env* env, const float* lidar_dev, float* actions_dev, int noise, const float* eps_stoch_dev,
                                    const float* eps_sample_dev, const float* eps_expl_dev, float* debug_dev, void* stream) {
-  if (!env || !lidar_dev || !actions_dev) return fail(env, RD_ERR_INVALID, "null argument");
-  if (int rc = dreamer_kind(env, false, "rd_policy_dreamer_train")) return rc;
-  if (noise < RD_NOISE_ZERO || noise > RD_NOISE_EXPLICIT) return fail(env, RD_ERR_INVALID, "bad noise mode %d", noise);
-  if (noise == RD_NOISE_EXPLICIT && (!eps_stoch_dev || !eps_sample_dev || !eps_expl_dev))
-    return fail(env, RD_ERR_INVALID, "RD_NOISE_EXPLICIT needs eps_stoch_dev, eps_sample_dev and eps_expl_dev");
-  return launch_dreamer(env, lidar_dev, actions_dev, noise, eps_stoch_dev, eps_sample_dev, debug_dev, (cudaStream_t)stream,
-                        true, eps_expl_dev);
+  return step_dreamer(env, lidar_dev, false, true, actions_dev, noise, eps_stoch_dev, eps_sample_dev, eps_expl_dev, debug_dev,
+                      stream, "rd_policy_dreamer_train");
 }
 
 RD_API int rd_rollout_dreamer_train(rd_env* env, int n_steps, const rd_outputs* out, float* actions_dev, int noise, void* stream) {
-  if (!env || !out || n_steps < 0) return fail(env, RD_ERR_INVALID, "bad argument");
-  if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
-  const void* obs = dreamer_obs(env, out);
-  if (!obs)
-    return fail(env, RD_ERR_INVALID, env->dr.depth ? "the rollout needs out->occupancy_dev and an env that produces it (RD_OBS_OCCUPANCY)"
-                                                   : "bad argument (the rollout needs out->lidar_dev)");
-  if (noise != RD_NOISE_ZERO && noise != RD_NOISE_PHILOX) return fail(env, RD_ERR_INVALID, "a rollout draws its own noise (RD_NOISE_ZERO or RD_NOISE_PHILOX)");
-  if (!env->was_reset) return fail(env, RD_ERR_STATE, "Must reset environment.");
-  float* act = actions_dev ? actions_dev : env->pol.d_actions;
-  for (int k = 0; k < n_steps; ++k) {
-    int rc = launch_dreamer(env, obs, act, noise, nullptr, nullptr, nullptr, (cudaStream_t)stream, true);
-    if (rc) return rc;
-    if ((rc = rd_step(env, act, out, stream))) return rc;
-  }
-  return RD_OK;
+  return rollout_dreamer(env, n_steps, out, actions_dev, noise, stream, true);
 }
 
 RD_API int rd_policy_dreamer_set_exploration(rd_env* env, const rd_dreamer_exploration* x) {
@@ -1302,59 +1325,29 @@ RD_API int rd_policy_dreamer_get_exploration(rd_env* env, rd_dreamer_exploration
 }
 
 RD_API int rd_policy_dreamer_set_weights(rd_env* env, const rd_dreamer_weights* w, int on_device, void* stream) {
-  if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
-  if (int rc = dreamer_kind(env, false, "rd_policy_dreamer_set_weights")) return rc;
-  const int rc = dreamer_set_weights(env->dr, w, nullptr, on_device != 0, (cudaStream_t)stream);
-  if (rc) return fail(env, rc, "rd_policy_dreamer_set_weights: %s", env->dr.err.c_str());
-  env->launches++;
-  return RD_OK;
+  return set_dreamer_weights(env, w, false, nullptr, on_device, stream, "rd_policy_dreamer_set_weights");
 }
 
 RD_API int rd_policy_dreamer_init_occupancy(rd_env* env, const rd_dreamer_weights* w, const rd_dreamer_conv_encoder* enc) {
-  if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
-  if (!enc) return fail(env, RD_ERR_INVALID, "rd_policy_dreamer_init_occupancy: null encoder");
-  if (!(env->cfg.obs_flags & RD_OBS_OCCUPANCY))
-    return fail(env, RD_ERR_INVALID, "rd_policy_dreamer_init_occupancy: the env does not produce lidar_occupancy (RD_OBS_OCCUPANCY)");
-  const int rc = dreamer_init(env->dr, env->n, env->cfg.n_beams, false, w, enc);
-  if (rc) return fail(env, rc, "rd_policy_dreamer_init_occupancy: %s", env->dr.err.c_str());
-  if (!env->pol.d_actions) {
-    CUDA_TRY(env, cudaMalloc(&env->pol.d_actions, sizeof(float) * 2 * (size_t)env->n));
-    CUDA_TRY(env, cudaMemset(env->pol.d_actions, 0, sizeof(float) * 2 * (size_t)env->n));
-  }
-  return RD_OK;
+  return init_dreamer(env, w, true, enc, "rd_policy_dreamer_init_occupancy");
 }
 
 RD_API int rd_policy_dreamer_occupancy(rd_env* env, const uint8_t* occupancy_dev, float* actions_dev, int noise,
                                        const float* eps_stoch_dev, const float* eps_actor_dev, float* debug_dev, void* stream) {
-  if (!env || !occupancy_dev || !actions_dev) return fail(env, RD_ERR_INVALID, "null argument");
-  if (int rc = dreamer_kind(env, true, "rd_policy_dreamer_occupancy")) return rc;
-  if (noise < RD_NOISE_ZERO || noise > RD_NOISE_EXPLICIT) return fail(env, RD_ERR_INVALID, "bad noise mode %d", noise);
-  if (noise == RD_NOISE_EXPLICIT && (!eps_stoch_dev || !eps_actor_dev))
-    return fail(env, RD_ERR_INVALID, "RD_NOISE_EXPLICIT needs eps_stoch_dev and eps_actor_dev");
-  return launch_dreamer(env, occupancy_dev, actions_dev, noise, eps_stoch_dev, eps_actor_dev, debug_dev, (cudaStream_t)stream);
+  return step_dreamer(env, occupancy_dev, true, false, actions_dev, noise, eps_stoch_dev, eps_actor_dev, nullptr, debug_dev,
+                      stream, "rd_policy_dreamer_occupancy");
 }
 
 RD_API int rd_policy_dreamer_occupancy_train(rd_env* env, const uint8_t* occupancy_dev, float* actions_dev, int noise,
                                              const float* eps_stoch_dev, const float* eps_sample_dev, const float* eps_expl_dev,
                                              float* debug_dev, void* stream) {
-  if (!env || !occupancy_dev || !actions_dev) return fail(env, RD_ERR_INVALID, "null argument");
-  if (int rc = dreamer_kind(env, true, "rd_policy_dreamer_occupancy_train")) return rc;
-  if (noise < RD_NOISE_ZERO || noise > RD_NOISE_EXPLICIT) return fail(env, RD_ERR_INVALID, "bad noise mode %d", noise);
-  if (noise == RD_NOISE_EXPLICIT && (!eps_stoch_dev || !eps_sample_dev || !eps_expl_dev))
-    return fail(env, RD_ERR_INVALID, "RD_NOISE_EXPLICIT needs eps_stoch_dev, eps_sample_dev and eps_expl_dev");
-  return launch_dreamer(env, occupancy_dev, actions_dev, noise, eps_stoch_dev, eps_sample_dev, debug_dev, (cudaStream_t)stream,
-                        true, eps_expl_dev);
+  return step_dreamer(env, occupancy_dev, true, true, actions_dev, noise, eps_stoch_dev, eps_sample_dev, eps_expl_dev,
+                      debug_dev, stream, "rd_policy_dreamer_occupancy_train");
 }
 
 RD_API int rd_policy_dreamer_set_weights_occupancy(rd_env* env, const rd_dreamer_weights* w, const rd_dreamer_conv_encoder* enc,
                                                    int on_device, void* stream) {
-  if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
-  if (!enc) return fail(env, RD_ERR_INVALID, "rd_policy_dreamer_set_weights_occupancy: null encoder");
-  if (int rc = dreamer_kind(env, true, "rd_policy_dreamer_set_weights_occupancy")) return rc;
-  const int rc = dreamer_set_weights(env->dr, w, enc, on_device != 0, (cudaStream_t)stream);
-  if (rc) return fail(env, rc, "rd_policy_dreamer_set_weights_occupancy: %s", env->dr.err.c_str());
-  env->launches += 4;
-  return RD_OK;
+  return set_dreamer_weights(env, w, true, enc, on_device, stream, "rd_policy_dreamer_set_weights_occupancy");
 }
 
 RD_API int rd_dreamer_encode_occupancy(rd_env* env, const uint8_t* occupancy_dev, float* embed_dev, void* stream) {
@@ -1746,11 +1739,7 @@ RD_API int rd_rollout_store(rd_env* env, int policy, int n_steps, const rd_outpu
     if (!out->lidar_dev) return fail(env, RD_ERR_INVALID, "the rollout needs out->lidar_dev");
     if (!env->pol.ready) return fail(env, RD_ERR_STATE, "rd_policy_gap_follower_init has not been called");
   } else if (policy == RD_STORE_POLICY_DREAMER || policy == RD_STORE_POLICY_DREAMER_TRAIN) {
-    if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
-    if (!(dr_obs = dreamer_obs(env, out)))
-      return fail(env, RD_ERR_INVALID, env->dr.depth ? "the rollout needs out->occupancy_dev and an env that produces it (RD_OBS_OCCUPANCY)"
-                                                     : "the rollout needs out->lidar_dev");
-    if (noise != RD_NOISE_ZERO && noise != RD_NOISE_PHILOX) return fail(env, RD_ERR_INVALID, "a rollout draws its own noise (RD_NOISE_ZERO or RD_NOISE_PHILOX)");
+    if ((rc = dreamer_rollout_obs(env, out, noise, &dr_obs))) return rc;
   } else {
     return fail(env, RD_ERR_INVALID, "bad policy %d", policy);
   }

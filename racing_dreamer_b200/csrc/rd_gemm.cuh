@@ -808,10 +808,10 @@ __global__ void __launch_bounds__(256) k_actor_train(const GemmArgs g, const flo
   }
 }
 
-// Weight refresh (rd_policy_dreamer_set_weights): checkpoint arrays -> the policy's packed operands, on the device.
+// The Dreamer weights' packer (dr_pack: init and weight refresh): checkpoint arrays -> the policy's packed operands.
 // Job j: src [in][out] -> dst (o, kmap(i)) = tf32(x) and, if lo, tf32(x - tf32(x)), kmap(i) = i >= k_from ? i + k_shift
-// : i (dr_upload_t's layout; the K slots it skips keep their zeros); raw jobs copy [out] values as they are (biases,
-// BN).  The rounding is dr_tf32's integer one, so the packed bits equal the host packing of rd_policy_dreamer_init.
+// : i (dr_parts' layout; the K slots it skips keep init's zeros); raw jobs copy [out] values as they are (biases, BN).
+// The rounding is an integer round-to-nearest on the bits (gm_tf32_bits).
 #define GM_PACK_MAX 32
 struct PackJob {
   const float* src; float* hi; float* lo;
@@ -819,7 +819,7 @@ struct PackJob {
   long long begin;         // first element of the job in the launch's flat index
 };
 struct PackArgs { int n_jobs; long long total; PackJob job[GM_PACK_MAX]; };
-__device__ __forceinline__ float gm_tf32_bits(float x) {   // == dr_tf32 (rd_dreamer.cuh)
+__device__ __forceinline__ float gm_tf32_bits(float x) {   // round to TF32, ties away from zero (finite values)
   return __uint_as_float((__float_as_uint(x) + 0x1000u) & ~0x1fffu);
 }
 __global__ void __launch_bounds__(256) k_pack_weights(const __grid_constant__ PackArgs a) {
@@ -903,7 +903,7 @@ __global__ void __launch_bounds__(256) k_conv1(const uint8_t* __restrict__ occ, 
 }
 // Conv2D kernel [4][4][cin][cout] (Keras) -> the K-major operand [cout][16 cin] of k_dense<..., CONV> in its K-block
 // order (see gm_conv_a): (ky, kx, c) -> block 8 cb + (4 py + 2 px + dy), element cc % 32, with ky = 2 py + dy,
-// kx = 2 px + dx, cc = dx cin + c, cb = cc / 32.  Rounding as k_pack_weights'; init and weight refresh both pack with it.
+// kx = 2 px + dx, cc = dx cin + c, cb = cc / 32.  Rounding as k_pack_weights'; dr_pack launches it after k_pack_weights.
 __global__ void __launch_bounds__(256) k_pack_conv(const float* __restrict__ src, float* __restrict__ hi, float* __restrict__ lo,
                                                    int cin, int cout) {
   const int total = 16 * cin * cout;

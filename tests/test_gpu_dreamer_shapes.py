@@ -368,8 +368,9 @@ def test_chain_more_row_blocks_than_resident_clusters(torch_cuda, monkeypatch):
 
 
 def test_rejected_architectures_leave_the_policy_working(torch_cuda):
-    """widths that are not multiples of 4, 0 or 8 trunk layers, n_samples 0, embed != n_beams: each raises (in
-    DreamerPolicy or in rd_policy_dreamer_init), and the policy already on the env computes what it did before"""
+    """widths that are not multiples of 4, 0 or 8 trunk layers, n_samples 0, embed != n_beams, a device pointer among
+    the weights: each raises (in DreamerPolicy or in rd_policy_dreamer_init), and the policy already on the env computes
+    what it did before"""
     torch = torch_cuda
     import ctypes as C
     from racing_dreamer_b200 import DreamerPolicy
@@ -405,5 +406,10 @@ def test_rejected_architectures_leave_the_policy_working(torch_cuda):
         s = pol._weights_struct(w, None, lambda a: a.ctypes.data_as(C.c_void_p))
         setattr(s, field, value)
         assert env.lib.rd_policy_dreamer_init(env._handle, C.byref(s)) != 0, field
+    # init reads host memory: a CUDA tensor's pointer among the weights is rejected, not read on the host
+    s = pol._weights_struct(w, None, lambda a: a.ctypes.data_as(C.c_void_p))
+    obs2_dev = torch.from_numpy(w["obs2_w"]).cuda()
+    s.obs2_w = obs2_dev.data_ptr()
+    assert env.lib.rd_policy_dreamer_init(env._handle, C.byref(s)) != 0
     same_bits(torch, explicit_step(torch, pol, lidar, state, es, ea), want, "after the rejected inits")
     env.close()
