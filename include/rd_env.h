@@ -387,6 +387,38 @@ int rd_dreamer_encode_occupancy(rd_env* env, const uint8_t* occupancy_dev, float
  * per-env state zeroing serve both agent kinds; an encoder agent's rollout reads out->occupancy_dev.  The lidar entry
  * points fail for an encoder agent and the occupancy ones for a lidar agent (RD_ERR_INVALID). */
 
+/* ---- several Dreamer agents in one env batch: env e is driven by agent agent_of_env[e].  Replaces the reference's ways
+ *      of running more than one checkpoint: one agent per car of a multi-agent scenario
+ *      [REF baselines/scenarios/max_progress/austria.yml:3-34 (cars A..D, each with its own agent)], the evaluation of
+ *      several checkpoints [REF dreamer/evaluations/run_evaluation.py:43-94 (a loop over checkpoints and tracks)], and
+ *      Dreamer._exploration per learner [REF dreamer/dreamer.py, Dreamer._exploration].
+ *      Env e's actions, state rows, debug rows and Philox draws are bit for bit what the single-agent policy with agent
+ *      agent_of_env[e]'s weights gives env e on the same batch: the draws stay keyed by the env id.  Internally the rows
+ *      are ordered by agent, each agent's from a multiple of 128 (csrc/rd_dreamer.cuh); every entry point keeps env order.
+ *      rd_policy_dreamer[_train], _occupancy[_train], rd_rollout_dreamer[_train], rd_rollout_store (both Dreamer
+ *      policies), get/set_state, rd_dreamer_encode_occupancy and the per-env state zeroing serve a multi-agent policy
+ *      unchanged.  On a policy with more than one agent, rd_policy_dreamer_set_weights[_occupancy] and
+ *      rd_policy_dreamer_set/get_exploration return RD_ERR_INVALID: use the per-agent calls below. ---- */
+#define RD_MAX_DREAMER_AGENTS 8
+/* n_agents = G in 1..RD_MAX_DREAMER_AGENTS; w[G]; enc: NULL (lidar agents, as rd_policy_dreamer_init) or enc[G]
+ * (ConvEncoder agents, as rd_policy_dreamer_init_occupancy); agent_of_env_host int32 [N] host values in [0, G), every
+ * agent owning at least one env, in any arrangement.  Every agent has agent 0's architecture, precision, n_samples,
+ * head scalars and encoder depth; BN presence may differ per agent.  Otherwise, and for everything
+ * rd_policy_dreamer_init rejects, RD_ERR_INVALID and the current agent keeps working.  Replaces the current agent(s),
+ * zeroes the state and every agent's env_steps, and returns after the packing finished.  G = 1 is
+ * rd_policy_dreamer_init[_occupancy]. */
+int rd_policy_dreamer_init_agents(rd_env* env, int32_t n_agents, const rd_dreamer_weights* w,
+                                  const rd_dreamer_conv_encoder* enc, const int32_t* agent_of_env_host);
+/* rd_policy_dreamer_set_weights[_occupancy] for agent `agent` (enc: NULL for lidar agents): packs that agent's weights
+ * on `stream` with no allocation; the other agents' weights and every env's latent state are untouched.  The agent's
+ * BN presence must be the one it was initialised with. */
+int rd_policy_dreamer_set_agent_weights(rd_env* env, int32_t agent, const rd_dreamer_weights* w,
+                                        const rd_dreamer_conv_encoder* enc, int on_device, void* stream);
+/* rd_policy_dreamer_set/get_exploration for agent `agent`.  A training step advances the agent's env_steps by
+ * (its envs) x action_repeat, Dreamer's len(reset) x action_repeat over the envs it drives. */
+int rd_policy_dreamer_set_agent_exploration(rd_env* env, int32_t agent, const rd_dreamer_exploration* x);
+int rd_policy_dreamer_get_agent_exploration(rd_env* env, int32_t agent, rd_dreamer_exploration* x);
+
 /* ---- device-resident episode store (SURVEY.md §8-f1): records the Collect rows of every env's episodes on the device
  *      [REF dreamer/wrappers.py:198-250], exactly the episodes episodes.EpisodeRecorder hands to its callbacks, and
  *      samples fixed-length chunks the way tools.load_episodes does [REF dreamer/tools.py:235-264].  The env must have

@@ -18,7 +18,7 @@ def __getattr__(name):
                 "load_scenario"):
         from . import compat as _compat
         return getattr(_compat, name)
-    if name in ("GapFollowerPolicy", "DreamerPolicy", "load_dreamer_checkpoint", "save_dreamer_checkpoint"):
+    if name in ("GapFollowerPolicy", "DreamerPolicy", "DreamerAgents", "load_dreamer_checkpoint", "save_dreamer_checkpoint"):
         from . import policy as _policy
         return getattr(_policy, name)
     raise AttributeError(name)

@@ -173,6 +173,7 @@ STORE_POLICY_GAP_FOLLOWER, STORE_POLICY_DREAMER, STORE_POLICY_DREAMER_TRAIN = 0,
 RD_NOISE_ZERO, RD_NOISE_PHILOX, RD_NOISE_EXPLICIT = 0, 1, 2
 RD_DREAMER_DEBUG_FLOATS = 68
 RD_PRECISION_TF32X3, RD_PRECISION_TF32 = 0, 1
+RD_MAX_DREAMER_AGENTS = 8
 
 EXPORTS = (
     "rd_default_config", "rd_create", "rd_destroy", "rd_last_error", "rd_abi_version", "rd_upload_map",
@@ -185,6 +186,8 @@ EXPORTS = (
     "rd_policy_dreamer_train", "rd_rollout_dreamer_train", "rd_policy_dreamer_set_weights",
     "rd_policy_dreamer_init_occupancy", "rd_policy_dreamer_occupancy", "rd_policy_dreamer_occupancy_train",
     "rd_policy_dreamer_set_weights_occupancy", "rd_dreamer_encode_occupancy",
+    "rd_policy_dreamer_init_agents", "rd_policy_dreamer_set_agent_weights", "rd_policy_dreamer_set_agent_exploration",
+    "rd_policy_dreamer_get_agent_exploration",
     "rd_store_init", "rd_store_reset", "rd_store_step", "rd_rollout_store", "rd_store_sample", "rd_store_info",
     "rd_store_import_init", "rd_store_import", "rd_store_import_info",
 )
@@ -300,6 +303,15 @@ def load_library() -> C.CDLL:
     lib.rd_policy_dreamer_set_weights_occupancy.restype = i32
     lib.rd_dreamer_encode_occupancy.argtypes = [vp, vp, vp, vp]
     lib.rd_dreamer_encode_occupancy.restype = i32
+    lib.rd_policy_dreamer_init_agents.argtypes = [vp, i32, C.POINTER(RdDreamerWeights), C.POINTER(RdDreamerConvEncoder), vp]
+    lib.rd_policy_dreamer_init_agents.restype = i32
+    lib.rd_policy_dreamer_set_agent_weights.argtypes = [vp, i32, C.POINTER(RdDreamerWeights), C.POINTER(RdDreamerConvEncoder),
+                                                        i32, vp]
+    lib.rd_policy_dreamer_set_agent_weights.restype = i32
+    lib.rd_policy_dreamer_set_agent_exploration.argtypes = [vp, i32, C.POINTER(RdDreamerExploration)]
+    lib.rd_policy_dreamer_set_agent_exploration.restype = i32
+    lib.rd_policy_dreamer_get_agent_exploration.argtypes = [vp, i32, C.POINTER(RdDreamerExploration)]
+    lib.rd_policy_dreamer_get_agent_exploration.restype = i32
     lib.rd_store_init.argtypes = [vp, C.POINTER(RdStoreConfig)]
     lib.rd_store_init.restype = i32
     lib.rd_store_reset.argtypes = [vp, C.POINTER(RdOutputs), vp]

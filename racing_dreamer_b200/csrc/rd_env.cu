@@ -428,7 +428,7 @@ StepParams step_params(rd_env* env) {
   }
   P.pol = env->pol.st;
   P.hist = env->d_hist;
-  if (env->dr.ready) { P.pol.dr_feat = env->dr.feat[env->dr.cur].p[0]; P.pol.dr_feat_lo = env->dr.feat[env->dr.cur].p[1]; P.pol.dr_ld = env->dr.ldf; }
+  if (env->dr.ready) { P.pol.dr_feat = env->dr.feat[env->dr.cur].p[0]; P.pol.dr_feat_lo = env->dr.feat[env->dr.cur].p[1]; P.pol.dr_ld = env->dr.ldf; P.pol.dr_row = env->dr.row_of_env; }
   P.n = env->n;
   return P;
 }
@@ -1167,13 +1167,14 @@ RD_API int rd_rollout_gap_follower(rd_env* env, int n_steps, const rd_outputs* o
 }
 
 namespace {
-// training: Dreamer.policy(training=True) -- one sample + exploration (k_actor_train), and the env-step counter of the
-// exploration schedule advances by n_envs * action_repeat [REF dreamer/dreamer.py, Dreamer.__call__ self._step]
+// training: Dreamer.policy(training=True) -- one sample + exploration (k_actor_train), and each agent's env-step counter
+// of the exploration schedule advances by (its envs) x action_repeat [REF dreamer/dreamer.py, Dreamer.__call__ self._step]
 int launch_dreamer(rd_env* env, const void* obs_dev, float* actions_dev, int noise, const float* eps_stoch_dev,
                    const float* eps_actor_dev, float* debug_dev, cudaStream_t s, bool training = false,
                    const float* eps_expl_dev = nullptr) {
   int launched = 0, rc;
-  const DrTrain tr{eps_expl_dev, dreamer_expl_amount(env->dr)};
+  DrTrain tr{eps_expl_dev, {}};
+  for (int a = 0; a < env->dr.n_agents; ++a) tr.amount.a[a] = dreamer_expl_amount(env->dr, a);
   {
     ScopedTiming tm(env, s, T_POLICY);
     rc = dreamer_step(env->dr, obs_dev, actions_dev, noise, eps_stoch_dev, eps_actor_dev, debug_dev, env->cfg.seed,
@@ -1181,7 +1182,7 @@ int launch_dreamer(rd_env* env, const void* obs_dev, float* actions_dev, int noi
   }
   env->launches += launched;
   if (rc) return fail(env, rc, "rd_policy_dreamer: %s", env->dr.err.c_str());
-  if (training) env->dr.env_steps += (int64_t)env->n * env->cfg.action_repeat;
+  for (int a = 0; training && a < env->dr.n_agents; ++a) env->dr.expl[a].env_steps += (int64_t)env->dr.n_of[a] * env->cfg.action_repeat;
   return RD_OK;
 }
 // the entry point's agent kind (encoder: the occupancy entry points) must be the initialised agent's
@@ -1194,8 +1195,10 @@ int dreamer_kind(rd_env* env, bool encoder, const char* fn) {
                 "occupancy entry points", fn);
   return RD_OK;
 }
-// rd_policy_dreamer_init and _init_occupancy (encoder: the latter, enc its image encoder)
-int init_dreamer(rd_env* env, const rd_dreamer_weights* w, bool encoder, const rd_dreamer_conv_encoder* enc, const char* fn) {
+// rd_policy_dreamer_init, _init_occupancy (encoder: the latter, enc its image encoder) and _init_agents (G agents:
+// w[G], enc[G] or null, agent_of_env [n])
+int init_dreamer(rd_env* env, int G, const rd_dreamer_weights* w, bool encoder, const rd_dreamer_conv_encoder* enc,
+                 const int32_t* agent_of_env, const char* fn) {
   if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
   if (encoder && !enc) return fail(env, RD_ERR_INVALID, "%s: null encoder", fn);
   if (encoder && !(env->cfg.obs_flags & RD_OBS_OCCUPANCY))
@@ -1203,7 +1206,7 @@ int init_dreamer(rd_env* env, const rd_dreamer_weights* w, bool encoder, const r
   if (!encoder && (env->cfg.obs_flags & RD_OBS_LIDAR_F16))
     return fail(env, RD_ERR_INVALID, "the on-device policies read float32 scans: RD_OBS_LIDAR_F16 is set");
   const bool lidar_normalised = !encoder && (env->cfg.obs_flags & RD_OBS_LIDAR_NORM);
-  const int rc = dreamer_init(env->dr, env->n, env->cfg.n_beams, lidar_normalised, w, enc);
+  const int rc = dreamer_init(env->dr, env->n, env->cfg.n_beams, lidar_normalised, G, w, enc, agent_of_env);
   if (rc) return fail(env, rc, "%s: %s", fn, env->dr.err.c_str());
   return ensure_rollout_actions(env);
 }
@@ -1247,21 +1250,38 @@ int rollout_dreamer(rd_env* env, int n_steps, const rd_outputs* out, float* acti
   }
   return RD_OK;
 }
-// rd_policy_dreamer_set_weights and _set_weights_occupancy (encoder: the latter, enc its image encoder)
-int set_dreamer_weights(rd_env* env, const rd_dreamer_weights* w, bool encoder, const rd_dreamer_conv_encoder* enc,
+// rd_policy_dreamer_set_weights, _set_weights_occupancy (encoder: the latter, enc its image encoder) and
+// _set_agent_weights (agent >= 0; -1: the single agent of the other two)
+int set_dreamer_weights(rd_env* env, int agent, const rd_dreamer_weights* w, bool encoder, const rd_dreamer_conv_encoder* enc,
                         int on_device, void* stream, const char* fn) {
   if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
   if (encoder && !enc) return fail(env, RD_ERR_INVALID, "%s: null encoder", fn);
   if (int rc = dreamer_kind(env, encoder, fn)) return rc;
-  const int rc = dreamer_set_weights(env->dr, w, enc, on_device != 0, (cudaStream_t)stream);
+  if (agent < 0 && env->dr.n_agents > 1)
+    return fail(env, RD_ERR_INVALID, "%s: the policy has %d agents; use rd_policy_dreamer_set_agent_weights", fn, env->dr.n_agents);
+  const int rc = dreamer_set_weights(env->dr, std::max(agent, 0), w, enc, on_device != 0, (cudaStream_t)stream);
   if (rc) return fail(env, rc, "%s: %s", fn, env->dr.err.c_str());
   env->launches += encoder ? 4 : 1;   // k_pack_weights, then k_pack_conv for conv2..conv4
+  return RD_OK;
+}
+// the exploration state of agent `agent` (-1: the single agent of rd_policy_dreamer_get/set_exploration)
+int dreamer_exploration(rd_env* env, int agent, rd_dreamer_exploration* x, bool set, const char* fn) {
+  if (!env || !x) return fail(env, RD_ERR_INVALID, "null argument");
+  if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
+  if (agent < 0 && env->dr.n_agents > 1)
+    return fail(env, RD_ERR_INVALID, "%s: the policy has %d agents; use the per-agent exploration calls", fn, env->dr.n_agents);
+  if (agent >= env->dr.n_agents) return fail(env, RD_ERR_INVALID, "%s: agent %d is not in [0, n_agents)", fn, agent);
+  rd_dreamer_exploration& e = env->dr.expl[std::max(agent, 0)];
+  if (!set) { *x = e; return RD_OK; }
+  if (!(x->amount >= 0.0) || !(x->decay >= 0.0) || !(x->min_amount >= 0.0) || x->env_steps < 0)
+    return fail(env, RD_ERR_INVALID, "exploration: amount, decay, min_amount and env_steps must be >= 0");
+  e = *x;
   return RD_OK;
 }
 }  // namespace
 
 RD_API int rd_policy_dreamer_init(rd_env* env, const rd_dreamer_weights* w) {
-  return init_dreamer(env, w, false, nullptr, "rd_policy_dreamer_init");
+  return init_dreamer(env, 1, w, false, nullptr, nullptr, "rd_policy_dreamer_init");
 }
 
 RD_API int rd_policy_dreamer(rd_env* env, const float* lidar_dev, float* actions_dev, int noise, const float* eps_stoch_dev,
@@ -1303,33 +1323,43 @@ RD_API int rd_rollout_dreamer_train(rd_env* env, int n_steps, const rd_outputs* 
 }
 
 RD_API int rd_policy_dreamer_set_exploration(rd_env* env, const rd_dreamer_exploration* x) {
-  if (!env || !x) return fail(env, RD_ERR_INVALID, "null argument");
-  if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
-  if (!(x->amount >= 0.0) || !(x->decay >= 0.0) || !(x->min_amount >= 0.0) || x->env_steps < 0)
-    return fail(env, RD_ERR_INVALID, "exploration: amount, decay, min_amount and env_steps must be >= 0");
-  env->dr.expl_amount = x->amount;
-  env->dr.expl_decay = x->decay;
-  env->dr.expl_min = x->min_amount;
-  env->dr.env_steps = x->env_steps;
-  return RD_OK;
+  return dreamer_exploration(env, -1, const_cast<rd_dreamer_exploration*>(x), true, "rd_policy_dreamer_set_exploration");
 }
 
 RD_API int rd_policy_dreamer_get_exploration(rd_env* env, rd_dreamer_exploration* x) {
-  if (!env || !x) return fail(env, RD_ERR_INVALID, "null argument");
-  if (!env->dr.ready) return fail(env, RD_ERR_STATE, "rd_policy_dreamer_init has not been called");
-  x->amount = env->dr.expl_amount;
-  x->decay = env->dr.expl_decay;
-  x->min_amount = env->dr.expl_min;
-  x->env_steps = env->dr.env_steps;
-  return RD_OK;
+  return dreamer_exploration(env, -1, x, false, "rd_policy_dreamer_get_exploration");
 }
 
 RD_API int rd_policy_dreamer_set_weights(rd_env* env, const rd_dreamer_weights* w, int on_device, void* stream) {
-  return set_dreamer_weights(env, w, false, nullptr, on_device, stream, "rd_policy_dreamer_set_weights");
+  return set_dreamer_weights(env, -1, w, false, nullptr, on_device, stream, "rd_policy_dreamer_set_weights");
 }
 
 RD_API int rd_policy_dreamer_init_occupancy(rd_env* env, const rd_dreamer_weights* w, const rd_dreamer_conv_encoder* enc) {
-  return init_dreamer(env, w, true, enc, "rd_policy_dreamer_init_occupancy");
+  return init_dreamer(env, 1, w, true, enc, nullptr, "rd_policy_dreamer_init_occupancy");
+}
+
+RD_API int rd_policy_dreamer_init_agents(rd_env* env, int32_t n_agents, const rd_dreamer_weights* w,
+                                         const rd_dreamer_conv_encoder* enc, const int32_t* agent_of_env_host) {
+  if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
+  if (!w || !agent_of_env_host) return fail(env, RD_ERR_INVALID, "rd_policy_dreamer_init_agents: null argument");
+  return init_dreamer(env, n_agents, w, enc != nullptr, enc, agent_of_env_host, "rd_policy_dreamer_init_agents");
+}
+
+RD_API int rd_policy_dreamer_set_agent_weights(rd_env* env, int32_t agent, const rd_dreamer_weights* w,
+                                               const rd_dreamer_conv_encoder* enc, int on_device, void* stream) {
+  if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
+  if (agent < 0) return fail(env, RD_ERR_INVALID, "rd_policy_dreamer_set_agent_weights: agent %d is not in [0, n_agents)", agent);
+  return set_dreamer_weights(env, agent, w, enc != nullptr, enc, on_device, stream, "rd_policy_dreamer_set_agent_weights");
+}
+
+RD_API int rd_policy_dreamer_set_agent_exploration(rd_env* env, int32_t agent, const rd_dreamer_exploration* x) {
+  if (agent < 0) return fail(env, RD_ERR_INVALID, "rd_policy_dreamer_set_agent_exploration: agent %d is not in [0, n_agents)", agent);
+  return dreamer_exploration(env, agent, const_cast<rd_dreamer_exploration*>(x), true, "rd_policy_dreamer_set_agent_exploration");
+}
+
+RD_API int rd_policy_dreamer_get_agent_exploration(rd_env* env, int32_t agent, rd_dreamer_exploration* x) {
+  if (agent < 0) return fail(env, RD_ERR_INVALID, "rd_policy_dreamer_get_agent_exploration: agent %d is not in [0, n_agents)", agent);
+  return dreamer_exploration(env, agent, x, false, "rd_policy_dreamer_get_agent_exploration");
 }
 
 RD_API int rd_policy_dreamer_occupancy(rd_env* env, const uint8_t* occupancy_dev, float* actions_dev, int noise,
@@ -1347,7 +1377,7 @@ RD_API int rd_policy_dreamer_occupancy_train(rd_env* env, const uint8_t* occupan
 
 RD_API int rd_policy_dreamer_set_weights_occupancy(rd_env* env, const rd_dreamer_weights* w, const rd_dreamer_conv_encoder* enc,
                                                    int on_device, void* stream) {
-  return set_dreamer_weights(env, w, true, enc, on_device, stream, "rd_policy_dreamer_set_weights_occupancy");
+  return set_dreamer_weights(env, -1, w, true, enc, on_device, stream, "rd_policy_dreamer_set_weights_occupancy");
 }
 
 RD_API int rd_dreamer_encode_occupancy(rd_env* env, const uint8_t* occupancy_dev, float* embed_dev, void* stream) {
@@ -1359,7 +1389,8 @@ RD_API int rd_dreamer_encode_occupancy(rd_env* env, const uint8_t* occupancy_dev
   int rc = dreamer_encode(d, occupancy_dev, s, &launched);
   if (!rc) {   // embed = hi + lo: the latent copy kernel over [n][embed] rows
     const size_t total = (size_t)d.n * d.embed;
-    k_latent_copy<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(d.lidar.p[0], d.lidar.p[1], d.embed, 0, d.embed, embed_dev, d.n, 0);
+    k_latent_copy<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(d.lidar.p[0], d.lidar.p[1], d.embed, 0, d.embed, embed_dev, d.n, 0,
+                                                                  d.row_of_env);
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) { rc = RD_ERR_CUDA; d.err = std::string("k_latent_copy: ") + cudaGetErrorString(e); }
     ++launched;

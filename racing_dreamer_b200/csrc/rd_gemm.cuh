@@ -66,6 +66,25 @@ enum { GM_NOISE_ZERO = 0, GM_NOISE_PHILOX = 1, GM_NOISE_EXPLICIT = 2 };
 #define RD_STREAM_ACTOR 0x41435452u
 #define RD_STREAM_TRAIN 0x5452414eu   // training head: the action sample and its exploration noise (k_actor_train)
 
+// Several agents in one batch (rd_policy_dreamer_init_agents): the policy's internal rows are ordered by agent, agent a
+// owning rows [start[a], start[a + 1]), every start a multiple of GM_BM, so each 128-row tile belongs to one agent.  The
+// weights are stacked per agent: operand rows [agents x out][ld], biases [agents][...], BN [agents][16].  A tile finds its
+// agent by counting the starts at or below its first row.  start[k] = 0 for k >= 1 means there is no agent k (a real
+// start of agent k >= 1 is at least GM_BM), so a zero-initialised GmAgents -- GemmArgs g{} -- is the single agent.
+// w_row: k_dense's W row offset of each agent (agent x W rows per agent; gm_launch fills it), which its producer selects
+// by compares on constant indices -- computing agent x rows there instead made the compiler address the epilogue's
+// global loads through extra vector-to-uniform register moves (R2UR), 170 more in the GRU cell.
+#define GM_MAX_AGENTS 8
+struct GmAgents { int start[GM_MAX_AGENTS]; int w_row[GM_MAX_AGENTS]; };
+// agent k >= 1 exists and owns rows from `row` on
+__device__ __forceinline__ bool gm_from(const GmAgents& ag, int k, int row) { return ag.start[k] > 0 && row >= ag.start[k]; }
+__device__ __forceinline__ int gm_agent(const GmAgents& ag, int row) {
+  int a = 0;
+#pragma unroll
+  for (int k = 1; k < GM_MAX_AGENTS; ++k) a += gm_from(ag, k, row) ? 1 : 0;
+  return a;
+}
+
 struct GemmArgs {
   int M, N;                 // rows (envs), valid output columns
   int n_phases;
@@ -86,6 +105,12 @@ struct GemmArgs {
   const float* bn;          // ACTOR "normalized" head: [4][4] gamma, beta, moving_mean, moving_variance (or null)
   float raw_init_std, min_std, mean_scale, bn_eps;
   int n_samples;
+  // agents: W rows per agent = N (GRU: 3 N), bias floats per agent = N (GRU: 6 N); bn [agents][16], used by agent a
+  // if bit a of bn_mask is set.  STOCH / ACTOR rows map to envs through env_of_row ([M], -1 = padding; null = identity):
+  // Philox ids, explicit draws, debug rows and actions are in env order.
+  GmAgents ag;
+  const int* env_of_row;
+  int bn_mask;
 };
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -303,6 +328,7 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
   const uint32_t smem_base = (rd_smem_u32(gm_smem_raw) + 1023u) & ~1023u;   // SWIZZLE_128B tiles: 1024-byte aligned
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int m0 = blockIdx.x * GM_BM, n0 = blockIdx.y * BN;
+  const int agent = gm_agent(g.ag, CONV > 0 ? m0 / (CONV * CONV) : m0);   // a conv tile: the env row of its first position
 
   if (threadIdx.x == 0) {
     for (int p = 0; p < g.n_phases; ++p) {
@@ -345,7 +371,12 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
           const CUtensorMap* mw2 = &maps.w[X3 ? ph.w_map_lo : ph.w_map];
           const uint32_t tx = (X3 ? 2u : 1u) * (GM_A_BYTES + (uint32_t)nb * W_BYTES);
           int ak = ph.a_k0, wk = ph.w_k0;
-          const int r0 = ph.w_row0[0] + n0, r1 = ph.w_row0[1] + n0, r2 = ph.w_row0[2] + n0;
+          const int arow = CONV > 0 ? m0 / (CONV * CONV) : m0;
+          int wsel = g.ag.w_row[0];   // the agent's slice of the stacked W rows
+#pragma unroll
+          for (int k = 1; k < GM_MAX_AGENTS; ++k) wsel = gm_from(g.ag, k, arow) ? g.ag.w_row[k] : wsel;
+          const int wa = n0 + wsel;
+          const int r0 = ph.w_row0[0] + wa, r1 = ph.w_row0[1] + wa, r2 = ph.w_row0[2] + wa;
           for (int kb = 0; kb < kbs; ++kb, ++it, ak += GM_BK, wk += GM_BK) {
             if (pass == 0 && it >= (uint32_t)GM_STAGES) break;
             const uint32_t s = it % GM_STAGES, par = (it / GM_STAGES) & 1u;
@@ -444,14 +475,18 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
     const int cbeg = part * PART_COLS, cend = cbeg + PART_COLS;
     const int row = m0 + q * 32 + lane;
     const uint32_t tl = tmem + ((uint32_t)(q * 32) << 16);
+    // the agent's bias floats start at bo; loads index g.bias (the parameter) with bo folded into the per-thread offset
+    const int bo = agent * (EPI == EPI_GRU ? 6 : 1) * g.N;
+    [[maybe_unused]] int env = row;   // STOCH: the env of the row (Philox id, explicit draws, debug row)
+    if constexpr (EPI == EPI_STOCH) env = (g.env_of_row && row < g.M) ? g.env_of_row[row] : row;
     asm volatile("griddepcontrol.wait;" ::: "memory");
-    const bool live = row < g.M;
+    const bool live = row < g.M && (EPI != EPI_STOCH || env >= 0);
     // What does not depend on the accumulators is done here, while the K loop runs: the posterior's normal draws
     // (Philox + Box-Muller: most of that epilogue's arithmetic) and the GRU's previous state (row-strided loads).
     [[maybe_unused]] float zpre[2][4] = {{0.f, 0.f, 0.f, 0.f}, {0.f, 0.f, 0.f, 0.f}};
     if constexpr (EPI == EPI_STOCH && EW == 4) {
       if (live && g.noise == GM_NOISE_PHILOX) {
-        const uint32_t gid = g.gid0 + (uint32_t)row;
+        const uint32_t gid = g.gid0 + (uint32_t)env;
         gm_normal4(gid, g.step, (uint32_t)(8 * part), RD_STREAM_STOCH, g.key0, g.key1, zpre[0]);
         gm_normal4(gid, g.step, (uint32_t)(8 * part + 4), RD_STREAM_STOCH, g.key0, g.key1, zpre[1]);
       }
@@ -494,7 +529,7 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
             float* pl = &ol.x;
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
-              float x = v[j + t] + __ldg(g.bias + col + t);
+              float x = v[j + t] + __ldg(g.bias + (bo + col + t));
               if constexpr (CONV > 0) x = fmaxf(x, 0.f);   // tf.nn.relu
               else if (g.act) x = gm_elu(x);
               po[t] = gm_round_tf32(x);
@@ -514,8 +549,7 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
     } else if constexpr (EPI == EPI_GRU) {
       // tf.keras GRUCell (reset_after=True): z, r, h gates; bias[0] input side, bias[1] recurrent side
       const int H = g.N;
-      const float* bx = g.bias;
-      const float* bh = g.bias + 3 * H;
+      const int bh = bo + 3 * H;
 #pragma unroll
       for (int c0 = cbeg; c0 < cend; c0 += 8) {   // (unrolled: hpre is indexed statically)
         if (n0 + c0 >= H) break;
@@ -546,9 +580,9 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
               const int c = col + t;
-              const float z = gm_sigmoid((az[j + t] + __ldg(bx + c)) + __ldg(bh + c));
-              const float r = gm_sigmoid((ar[j + t] + __ldg(bx + H + c)) + __ldg(bh + H + c));
-              const float hh = tanhf((axh[j + t] + __ldg(bx + 2 * H + c)) + r * (arh[j + t] + __ldg(bh + 2 * H + c)));
+              const float z = gm_sigmoid((az[j + t] + __ldg(g.bias + (bo + c))) + __ldg(g.bias + (bh + c)));
+              const float r = gm_sigmoid((ar[j + t] + __ldg(g.bias + (bo + H + c))) + __ldg(g.bias + (bh + H + c)));
+              const float hh = tanhf((axh[j + t] + __ldg(g.bias + (bo + 2 * H + c))) + r * (arh[j + t] + __ldg(g.bias + (bh + 2 * H + c))));
               const float hn = z * ph_[t] + (1.f - z) * hh;
               po[t] = gm_round_tf32(hn);
               pl[t] = gm_round_tf32(hn - po[t]);
@@ -586,14 +620,14 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
             for (int t = 0; t < 4; ++t) {
               const int j = j0 + t;
               if (j < GM_STOCH) {
-                const float mean = mu[4 * h + t] + __ldg(g.bias + j);
-                const float sd = gm_softplus(sr[6 + 4 * h + t] + __ldg(g.bias + GM_STOCH + j)) + 0.1f;
+                const float mean = mu[4 * h + t] + __ldg(g.bias + (bo + j));
+                const float sd = gm_softplus(sr[6 + 4 * h + t] + __ldg(g.bias + (bo + GM_STOCH + j))) + 0.1f;
                 float e = zpre[h][t];
-                if (g.noise == GM_NOISE_EXPLICIT) e = g.eps[(size_t)row * g.ld_eps + j];
+                if (g.noise == GM_NOISE_EXPLICIT) e = g.eps[(size_t)env * g.ld_eps + j];
                 const float sv = mean + sd * e;
                 po[t] = gm_round_tf32(sv);
                 pl[t] = gm_round_tf32(sv - po[t]);
-                if (g.dbg) { g.dbg[(size_t)row * 2 * GM_STOCH + j] = mean; g.dbg[(size_t)row * 2 * GM_STOCH + GM_STOCH + j] = sd; }
+                if (g.dbg) { g.dbg[(size_t)env * 2 * GM_STOCH + j] = mean; g.dbg[(size_t)env * 2 * GM_STOCH + GM_STOCH + j] = sd; }
               }
             }
             *reinterpret_cast<float4*>(g.feat + (size_t)row * g.ldf + j0) = o;
@@ -619,7 +653,7 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
       }
       if (live) {
         float* frow = g.feat + (size_t)row * g.ldf;
-        const uint32_t gid = g.gid0 + (uint32_t)row;
+        const uint32_t gid = g.gid0 + (uint32_t)env;
 #pragma unroll
         for (int j0 = 0; j0 < 32; j0 += 4) {
           if (j0 / (32 / EW) != part) continue;   // warp-uniform: this group's share of the 30 latents
@@ -629,16 +663,16 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
           for (int t = 0; t < 4; ++t) {
             const int j = j0 + t;
             if (j < GM_STOCH) {
-              const float mean = lo[j] + __ldg(g.bias + j);
-              const float sraw = (j + GM_STOCH < 32 ? lo[(j + GM_STOCH) & 31] : hi[(j + GM_STOCH - 32) & 31]) + __ldg(g.bias + GM_STOCH + j);
+              const float mean = lo[j] + __ldg(g.bias + (bo + j));
+              const float sraw = (j + GM_STOCH < 32 ? lo[(j + GM_STOCH) & 31] : hi[(j + GM_STOCH - 32) & 31]) + __ldg(g.bias + (bo + GM_STOCH + j));
               const float sd = gm_softplus(sraw) + 0.1f;
               float e = z[t];
-              if (g.noise == GM_NOISE_EXPLICIT) e = g.eps[(size_t)row * g.ld_eps + j];
+              if (g.noise == GM_NOISE_EXPLICIT) e = g.eps[(size_t)env * g.ld_eps + j];
               const float sv = mean + sd * e;
               const float sh = gm_round_tf32(sv);
               frow[j] = sh;
               if (g.feat_lo) g.feat_lo[(size_t)row * g.ldf + j] = gm_round_tf32(sv - sh);
-              if (g.dbg) { g.dbg[(size_t)row * 2 * GM_STOCH + j] = mean; g.dbg[(size_t)row * 2 * GM_STOCH + GM_STOCH + j] = sd; }
+              if (g.dbg) { g.dbg[(size_t)env * 2 * GM_STOCH + j] = mean; g.dbg[(size_t)env * 2 * GM_STOCH + GM_STOCH + j] = sd; }
             }
           }
         }
@@ -651,7 +685,8 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
       gm_tmem_sum8(tl, g.n_acc, 1, v);
       if (live && part == 0) {
         float4 o;
-        o.x = v[0] + __ldg(g.bias + 0); o.y = v[1] + __ldg(g.bias + 1); o.z = v[2] + __ldg(g.bias + 2); o.w = v[3] + __ldg(g.bias + 3);
+        o.x = v[0] + __ldg(g.bias + bo); o.y = v[1] + __ldg(g.bias + (bo + 1)); o.z = v[2] + __ldg(g.bias + (bo + 2));
+        o.w = v[3] + __ldg(g.bias + (bo + 3));
         *reinterpret_cast<float4*>(g.out + (size_t)row * 4) = o;
       }
     }
@@ -665,14 +700,16 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
 }
 
 // ActionDecoder distribution head [REF models.py:323-346]: mean and sd of the pre-tanh Normal from hout's
-// pre-activations g.out[row][0..3]
+// pre-activations g.out[row][0..3]; the row's agent's BN, if it has one
 __device__ __forceinline__ void gm_actor_dist(const GemmArgs& g, int row, float (&mean)[2], float (&sd)[2]) {
   const float4 x4 = *reinterpret_cast<const float4*>(g.out + (size_t)row * 4);
   float x[4] = {x4.x, x4.y, x4.z, x4.w};
-  if (g.bn) {   // 'normalized_tanhtransformed_normal': BatchNormalization in inference mode, linear mean
+  const int agent = gm_agent(g.ag, row);
+  if (g.bn && ((g.bn_mask >> agent) & 1)) {   // 'normalized_tanhtransformed_normal': BatchNormalization in inference mode, linear mean
+    const float* bn = g.bn + 16 * agent;
 #pragma unroll
     for (int t = 0; t < 4; ++t)
-      x[t] = (x[t] - __ldg(g.bn + 8 + t)) * (__ldg(g.bn + t) * rsqrtf(__ldg(g.bn + 12 + t) + g.bn_eps)) + __ldg(g.bn + 4 + t);
+      x[t] = (x[t] - __ldg(bn + 8 + t)) * (__ldg(bn + t) * rsqrtf(__ldg(bn + 12 + t) + g.bn_eps)) + __ldg(bn + 4 + t);
     mean[0] = x[0]; mean[1] = x[1];
     sd[0] = gm_softplus(x[2]) + g.min_std; sd[1] = gm_softplus(x[3]) + g.min_std;
   } else {      // 'tanh_normal'
@@ -680,10 +717,10 @@ __device__ __forceinline__ void gm_actor_dist(const GemmArgs& g, int row, float 
     sd[0] = gm_softplus(x[2] + g.raw_init_std) + g.min_std; sd[1] = gm_softplus(x[3] + g.raw_init_std) + g.min_std;
   }
 }
-// the chosen action -> g.actions[row] and the latent's action slots (TF32 hi [+ lo]), which the next img1 reads
-__device__ __forceinline__ void gm_actor_store(const GemmArgs& g, int row, float a0, float a1) {
-  g.actions[2 * (size_t)row] = a0;
-  g.actions[2 * (size_t)row + 1] = a1;
+// the chosen action -> g.actions[env] and the latent's action slots of the row (TF32 hi [+ lo]), which the next img1 reads
+__device__ __forceinline__ void gm_actor_store(const GemmArgs& g, int row, int env, float a0, float a1) {
+  g.actions[2 * (size_t)env] = a0;
+  g.actions[2 * (size_t)env + 1] = a1;
   float* frow = g.feat + (size_t)row * g.ldf;
   const float h0 = gm_round_tf32(a0), h1 = gm_round_tf32(a1);
   frow[GM_STOCH] = h0;
@@ -697,9 +734,12 @@ __device__ __forceinline__ void gm_actor_store(const GemmArgs& g, int row, float
 // ActionDecoder distribution head + SampleDist.mode() [REF ros_agent/helpers/tools.py:70-73]:
 // one warp per env, lanes over pairs of draws (one Philox block = the four normals of two draws), warp arg-max.
 // `g.out` holds hout's pre-activations [M][4] (k_dense<EPI_ACTOR>); the other fields are the ACTOR ones of GemmArgs.
+// Rows are the policy's internal rows; padding rows (env_of_row -1) are skipped.
 __global__ void __launch_bounds__(256) k_actor_mode(const GemmArgs g) {
   const int row = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (row >= g.M) return;
+  const int env = g.env_of_row ? g.env_of_row[row] : row;
+  if (env < 0) return;
   // Launched while the head's k_dense still runs (programmatic dependent launch): the normal draws -- Philox and
   // Box-Muller, most of this kernel's arithmetic -- depend on nothing it produces and are made before the wait.
   constexpr int PRE = 4;   // draws 2 lane + 64 it, it < PRE, kept in registers; beyond 256 draws they are made in the loop
@@ -708,7 +748,7 @@ __global__ void __launch_bounds__(256) k_actor_mode(const GemmArgs g) {
 #pragma unroll
     for (int it = 0; it < PRE; ++it)
       if (2 * lane + 64 * it < g.n_samples)
-        gm_normal4(g.gid0 + (uint32_t)row, g.step, (uint32_t)(2 * lane + 64 * it), RD_STREAM_ACTOR, g.key0, g.key1, zp[it]);
+        gm_normal4(g.gid0 + (uint32_t)env, g.step, (uint32_t)(2 * lane + 64 * it), RD_STREAM_ACTOR, g.key0, g.key1, zp[it]);
   }
   asm volatile("griddepcontrol.wait;" ::: "memory");
   float mean[2], sd[2];
@@ -716,7 +756,7 @@ __global__ void __launch_bounds__(256) k_actor_mode(const GemmArgs g) {
   // mode(): argmax over n_samples draws of log_prob(tanh(u)), u ~ N(mean, sd): the Normal's log density minus the tanh
   // bijector's forward log-det-Jacobian 2 (log 2 - u - softplus(-2u)), summed over the two actions
   const float log2f_ = 0.69314718f, half_log_2pi = 0.91893853f;
-  const uint32_t gid = g.gid0 + (uint32_t)row;
+  const uint32_t gid = g.gid0 + (uint32_t)env;
   float best = -INFINITY, bu0 = mean[0], bu1 = mean[1];
   int bi = 0x7fffffff;
   if (g.noise == GM_NOISE_ZERO) {
@@ -748,7 +788,7 @@ __global__ void __launch_bounds__(256) k_actor_mode(const GemmArgs g) {
         float lp = 0.f, u[2];
 #pragma unroll
         for (int d = 0; d < 2; ++d) {
-          const float e = (g.noise == GM_NOISE_EXPLICIT) ? g.eps[(size_t)row * g.ld_eps + 2 * s + d] : z[2 * h + d];
+          const float e = (g.noise == GM_NOISE_EXPLICIT) ? g.eps[(size_t)env * g.ld_eps + 2 * s + d] : z[2 * h + d];
           u[d] = mean[d] + sd[d] * e;
           lp += ((-0.5f * e * e - logf(sd[d])) - half_log_2pi) - 2.f * ((log2f_ - u[d]) - gm_softplus(-2.f * u[d]));
         }
@@ -765,9 +805,9 @@ __global__ void __launch_bounds__(256) k_actor_mode(const GemmArgs g) {
   }
   if (lane == 0) {
     const float a0 = tanhf(bu0), a1 = tanhf(bu1);
-    gm_actor_store(g, row, a0, a1);
+    gm_actor_store(g, row, env, a0, a1);
     if (g.dbg) {
-      float* d = g.dbg + (size_t)row * 8;
+      float* d = g.dbg + (size_t)env * 8;
       d[0] = mean[0]; d[1] = mean[1]; d[2] = sd[0]; d[3] = sd[1]; d[4] = a0; d[5] = a1; d[6] = best; d[7] = (float)bi;
     }
   }
@@ -778,10 +818,14 @@ __global__ void __launch_bounds__(256) k_actor_mode(const GemmArgs g) {
 // a' = clip(a + amount e2, -1, 1), rounded once per operation so that a' is reproducible bit for bit from a.  a' is the
 // executed action and the one the latent keeps for the next obs_step.  One thread per env; noise: Philox block
 // (env id, step, 0, RD_STREAM_TRAIN) -> e1 = z0..1, e2 = z2..3, zero (a = tanh(mean), a' = a) or explicit
-// (g.eps [M][2] = e1, eps_expl [M][2] = e2).  Debug row: mean, sd, a (before exploration), log_prob(a), index 0.
-__global__ void __launch_bounds__(256) k_actor_train(const GemmArgs g, const float* __restrict__ eps_expl, float amount) {
-  const int row = blockIdx.x * blockDim.x + threadIdx.x;
-  if (row >= g.M) return;
+// (g.eps [envs][2] = e1, eps_expl [envs][2] = e2).  Debug row: mean, sd, a (before exploration), log_prob(a), index 0.
+// amount.a[agent]: each agent's exploration amount.  Rows as k_actor_mode's.
+struct GmAmounts { float a[GM_MAX_AGENTS]; };
+__global__ void __launch_bounds__(256) k_actor_train(const GemmArgs g, const float* __restrict__ eps_expl, const GmAmounts amounts) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;   // the policy's row
+  if (r >= g.M) return;
+  const int row = g.env_of_row ? g.env_of_row[r] : r;    // its env: the Philox id, explicit draws, action and debug row
+  if (row < 0) return;
   float z[4] = {0.f, 0.f, 0.f, 0.f};
   // made before the wait, as in k_actor_mode: the draws do not depend on the head's k_dense
   if (g.noise == GM_NOISE_PHILOX) gm_normal4(g.gid0 + (uint32_t)row, g.step, 0u, RD_STREAM_TRAIN, g.key0, g.key1, z);
@@ -790,8 +834,9 @@ __global__ void __launch_bounds__(256) k_actor_train(const GemmArgs g, const flo
     z[0] = g.eps[2 * (size_t)row]; z[1] = g.eps[2 * (size_t)row + 1];
     z[2] = eps_expl[2 * (size_t)row]; z[3] = eps_expl[2 * (size_t)row + 1];
   }
+  const float amount = amounts.a[gm_agent(g.ag, r)];
   float mean[2], sd[2];
-  gm_actor_dist(g, row, mean, sd);
+  gm_actor_dist(g, r, mean, sd);
   const float log2f_ = 0.69314718f, half_log_2pi = 0.91893853f;
   float a[2], x[2], lp = 0.f;
 #pragma unroll
@@ -801,7 +846,7 @@ __global__ void __launch_bounds__(256) k_actor_train(const GemmArgs g, const flo
     a[d] = tanhf(u);
     x[d] = fminf(fmaxf(__fadd_rn(a[d], __fmul_rn(amount, z[2 + d])), -1.f), 1.f);
   }
-  gm_actor_store(g, row, x[0], x[1]);
+  gm_actor_store(g, r, row, x[0], x[1]);
   if (g.dbg) {
     float* d = g.dbg + (size_t)row * 8;
     d[0] = mean[0]; d[1] = mean[1]; d[2] = sd[0]; d[3] = sd[1]; d[4] = a[0]; d[5] = a[1]; d[6] = lp; d[7] = 0.f;
@@ -840,11 +885,24 @@ __global__ void __launch_bounds__(256) k_pack_weights(const __grid_constant__ Pa
 
 // RacingDreamer._preprocess_lidar [REF ros_agent/models/dreamer/racing_dreamer.py:45-52] in its own float32 arithmetic
 // (clip to [0, 15], / 15, - 0.5; `normalise` = 0 when the env already emits that), then the TF32 split (hi, lo) the
-// tensor-core passes read; lo may be null (single-pass mode).  count % 4 == 0.
+// tensor-core passes read; lo may be null (single-pass mode).  count % 4 == 0.  Output rows are the policy's rows of
+// row4 float4s each: row r holds the scan of env env_of_row[r] (null: env r), zeros for a padding row (-1).
 __global__ void __launch_bounds__(256) k_embed_lidar(const float4* __restrict__ src, float4* __restrict__ hi,
-                                                     float4* __restrict__ lo, size_t count4, int normalise) {
+                                                     float4* __restrict__ lo, size_t count4, int normalise,
+                                                     const int* __restrict__ env_of_row, int row4) {
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < count4; i += (size_t)gridDim.x * blockDim.x) {
-    const float4 x4 = src[i];
+    size_t si = i;
+    if (env_of_row) {
+      const size_t r = i / (size_t)row4;
+      const int env = env_of_row[r];
+      if (env < 0) {
+        hi[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (lo) lo[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+        continue;
+      }
+      si = (size_t)env * row4 + (i - r * row4);
+    }
+    const float4 x4 = src[si];
     const float* x = &x4.x;
     float4 h4, l4;
     float* h = &h4.x;
@@ -867,20 +925,26 @@ __global__ void __launch_bounds__(256) k_embed_lidar(const float4* __restrict__ 
 // occupancy image cast to float, on CUDA cores (K = 16 is too short for a tensor-core K block).  The inputs are 0 / 1 (any
 // u8 is cast exactly), so every product is exact and the float32 sums are float32-grade in both precisions.  Output: NHWC
 // [env][32][32][32] TF32 hi (+ lo) on a 32 x 32 grid whose last row and column (outside the 31 x 31 valid outputs) are
-// zero -- the grid conv2's 5-D view reads.  One CTA per (env, output row), thread = (ox, 4 channels).
+// zero -- the grid conv2's 5-D view reads.  One CTA per (policy row, output row), thread = (ox, 4 channels).  Row r reads
+// the image of env env_of_row[r] (null: env r) with its agent's kernel and bias (w [agents][16][32], b [agents][32]);
+// a padding row (-1) is all zeros.
 #define GM_CONV1_C 32
 __global__ void __launch_bounds__(256) k_conv1(const uint8_t* __restrict__ occ, const float* __restrict__ w,
-                                               const float* __restrict__ b, float4* __restrict__ hi, float4* __restrict__ lo) {
+                                               const float* __restrict__ b, float4* __restrict__ hi, float4* __restrict__ lo,
+                                               const int* __restrict__ env_of_row, const GmAgents ag) {
   __shared__ float ws[16 * GM_CONV1_C];
   __shared__ float img[4][64];
   const int oy = blockIdx.x & 31, t = threadIdx.x;
-  const size_t env = blockIdx.x >> 5;
+  const size_t row = blockIdx.x >> 5;
+  const int env = env_of_row ? env_of_row[row] : (int)row, agent = gm_agent(ag, (int)row);
+  w += agent * 16 * GM_CONV1_C;
+  b += agent * GM_CONV1_C;
   for (int i = t; i < 16 * GM_CONV1_C; i += 256) ws[i] = w[i];
-  img[t >> 6][t & 63] = oy < 31 ? (float)occ[env * 4096 + (size_t)(2 * oy + (t >> 6)) * 64 + (t & 63)] : 0.f;
+  img[t >> 6][t & 63] = (oy < 31 && env >= 0) ? (float)occ[(size_t)env * 4096 + (size_t)(2 * oy + (t >> 6)) * 64 + (t & 63)] : 0.f;
   __syncthreads();
   const int ox = t >> 3, c0 = (t & 7) * 4;
   float v[4] = {0.f, 0.f, 0.f, 0.f};
-  if (oy < 31 && ox < 31) {
+  if (oy < 31 && ox < 31 && env >= 0) {
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       float acc = b[c0 + j];
@@ -897,7 +961,7 @@ __global__ void __launch_bounds__(256) k_conv1(const uint8_t* __restrict__ occ, 
     h[j] = gm_round_tf32(v[j]);
     l[j] = gm_round_tf32(v[j] - h[j]);
   }
-  const size_t o = ((env * 32 + oy) * 32 + ox) * (GM_CONV1_C / 4) + (c0 >> 2);
+  const size_t o = ((row * 32 + oy) * 32 + ox) * (GM_CONV1_C / 4) + (c0 >> 2);
   hi[o] = h4;
   if (lo) lo[o] = l4;
 }
@@ -917,13 +981,15 @@ __global__ void __launch_bounds__(256) k_pack_conv(const float* __restrict__ src
     if (lo) lo[k] = gm_tf32_bits(__fsub_rn(x, h));
   }
 }
-// latent rows <-> the reference's state tuple.  dir 0: out = hi + lo; dir 1: (hi, lo) = split(in)
+// latent rows <-> the reference's state tuple.  dir 0: out = hi + lo; dir 1: (hi, lo) = split(in).  ext is in env order,
+// env e's row is row_of_env[e] (null: e).
 __global__ void __launch_bounds__(256) k_latent_copy(float* __restrict__ feat, float* __restrict__ feat_lo, int ldf, int col0,
-                                                      int width, float* __restrict__ ext, int n, int dir) {
+                                                      int width, float* __restrict__ ext, int n, int dir,
+                                                      const int* __restrict__ row_of_env) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (size_t)n * width) return;
   const int e = (int)(i / width), c = (int)(i % width);
-  const size_t f = (size_t)e * ldf + col0 + c;
+  const size_t f = (size_t)(row_of_env ? row_of_env[e] : e) * ldf + col0 + c;
   if (dir == 0) {
     ext[i] = feat[f] + (feat_lo ? feat_lo[f] : 0.f);
   } else {
@@ -972,6 +1038,7 @@ struct ChainArgs {
   int M, N, ldo, n_layers, row_blocks;
   unsigned* flags;         // [GM_CHAIN_MAX][row_blocks]
   ChainLayer L[GM_CHAIN_MAX];
+  GmAgents ag;             // a row block's agent: W rows [agent N, (agent + 1) N), bias [agent N, ...)
 };
 
 __device__ __forceinline__ void gm_flag_wait(const unsigned* flag, unsigned target) {
@@ -1025,7 +1092,7 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
       uint32_t it = 0, tile = 0;
       bool first = true;
       for (int mb = blockIdx.y; mb < g.row_blocks; mb += gridDim.y) {
-        const int m0 = mb * GM_BM;
+        const int m0 = mb * GM_BM, wn0 = n0 + gm_agent(g.ag, m0) * g.N;
         for (int l = 0; l < g.n_layers; ++l) {
           const CUtensorMap* ma = &maps.a[l][0];
           const CUtensorMap* ma2 = &maps.a[l][1];
@@ -1040,8 +1107,8 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
             const uint32_t sa = smem_base + s * STAGE_BYTES, sb = sa + SUB_BYTES;
             if (i >= (uint32_t)GM_STAGES) gm_mbar_wait(&empty_bar[s], par ^ 1u);
             rd_mbar_expect_tx(&full_bar[s], STAGE_BYTES);
-            gm_tma_2d(sa + GM_A_BYTES, mw, j * GM_BK, n0, &full_bar[s]);
-            gm_tma_2d(sb + GM_A_BYTES, mw2, j * GM_BK, n0, &full_bar[s]);
+            gm_tma_2d(sa + GM_A_BYTES, mw, j * GM_BK, wn0, &full_bar[s]);
+            gm_tma_2d(sb + GM_A_BYTES, mw2, j * GM_BK, wn0, &full_bar[s]);
           }
           // the layer's input rows: the kernel in front of this one (first layer) or every N tile of the layer before
           if (first) { asm volatile("griddepcontrol.wait;" ::: "memory"); first = false; }
@@ -1058,8 +1125,8 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
             const uint32_t sa = smem_base + s * STAGE_BYTES, sb = sa + SUB_BYTES;
             gm_mbar_wait(&empty_bar[s], par ^ 1u);
             rd_mbar_expect_tx(&full_bar[s], STAGE_BYTES);
-            gm_tma_2d(sa + GM_A_BYTES, mw, j * GM_BK, n0, &full_bar[s]);
-            gm_tma_2d(sb + GM_A_BYTES, mw2, j * GM_BK, n0, &full_bar[s]);
+            gm_tma_2d(sa + GM_A_BYTES, mw, j * GM_BK, wn0, &full_bar[s]);
+            gm_tma_2d(sb + GM_A_BYTES, mw2, j * GM_BK, wn0, &full_bar[s]);
             gm_tma_2d(sa, ma, j * GM_BK, m0, &full_bar[s]);
             gm_tma_2d(sb, ma2, j * GM_BK, m0, &full_bar[s]);
           }
@@ -1131,6 +1198,7 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
     asm volatile("griddepcontrol.wait;" ::: "memory");
     uint32_t tile = 0, it_end = 0;
     for (int mb = blockIdx.y; mb < g.row_blocks; mb += gridDim.y) {
+      const int bias0 = gm_agent(g.ag, mb * GM_BM) * g.N;
       for (int l = 0; l < g.n_layers; ++l, ++tile) {
         const ChainLayer& L = g.L[l];
         it_end += (uint32_t)L.kb_total;
@@ -1154,7 +1222,7 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
               float* pl = &ol.x;
 #pragma unroll
               for (int t = 0; t < 4; ++t) {
-                const float x = gm_elu(v[j + t] + __ldg(L.bias + col + t));
+                const float x = gm_elu(v[j + t] + __ldg(L.bias + bias0 + col + t));
                 po[t] = gm_round_tf32(x);
                 pl[t] = gm_round_tf32(x - po[t]);
               }
@@ -1253,7 +1321,9 @@ static inline bool gm_make_map_conv(CUtensorMap* m, const float* base, int cin, 
 }
 
 template <int EPI, int NSLAB, int NACC, int GM_STAGES, bool X3 = false, int EW = GM_EPI_GROUPS, int BN = GM_BN, int CONV = 0>
-static inline cudaError_t gm_launch(const GemmMaps& maps, const GemmArgs& g, cudaStream_t s) {
+static inline cudaError_t gm_launch(const GemmMaps& maps, const GemmArgs& g_in, cudaStream_t s) {
+  GemmArgs g = g_in;
+  for (int a = 0; a < GM_MAX_AGENTS; ++a) g.ag.w_row[a] = a * (EPI == EPI_GRU ? 3 : 1) * g.N;
   constexpr size_t smem = (size_t)GM_STAGES * (X3 ? 2 : 1) * (GM_A_BYTES + NSLAB * BN * 128) + 1024;
   static bool attr = false;
   if (!attr) {

@@ -24,16 +24,18 @@ struct PolicyState {
   float* dr_feat; // Dreamer agent: current latent rows [n][dr_ld] = stoch | previous action | deter (null: not attached)
   float* dr_feat_lo;   // their TF32 remainder parts (null in single-pass mode)
   int dr_ld;
+  const int* dr_row;   // env -> latent row (several agents: rows ordered by agent); null: row = env
 };
 enum { RD_P_PREV = 0, RD_P_INT, RD_P_STEER, RD_P_SPEED, RD_NP_F64 };
 enum { RD_P_SCANS = 0, RD_P_HEADINGS, RD_NP_I32 };
 
 __device__ __forceinline__ void rd_policy_clear(const PolicyState& ps, int n, int e) {
   if (ps.dr_feat) {   // `state is None`: zero latent, zero previous action [REF ros_agent/models/dreamer/racing_dreamer.py:66-68]
-    float4* row = reinterpret_cast<float4*>(ps.dr_feat + (size_t)e * ps.dr_ld);
+    const size_t r = ps.dr_row ? (size_t)ps.dr_row[e] : (size_t)e;
+    float4* row = reinterpret_cast<float4*>(ps.dr_feat + r * ps.dr_ld);
     for (int k = 0; k < ps.dr_ld / 4; ++k) row[k] = make_float4(0.f, 0.f, 0.f, 0.f);
     if (ps.dr_feat_lo) {
-      float4* lo = reinterpret_cast<float4*>(ps.dr_feat_lo + (size_t)e * ps.dr_ld);
+      float4* lo = reinterpret_cast<float4*>(ps.dr_feat_lo + r * ps.dr_ld);
       for (int k = 0; k < ps.dr_ld / 4; ++k) lo[k] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
   }

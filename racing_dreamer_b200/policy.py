@@ -261,21 +261,9 @@ class DreamerPolicy:
         if (actor_version == "normalized") != has_bn:
             raise ValueError(f"actor_version {actor_version!r} does not match the checkpoint (hnorm variables "
                              f"{'present' if has_bn else 'absent'})")
-        if noise not in self.NOISE:
-            raise ValueError(f"noise {noise!r}: expected one of {sorted(self.NOISE)}")
-        self.noise = noise
         self.weights = w
         self._arch = _dreamer_arch(w)
-        deter, hidden, units, embed, layers, _ = self._arch
-        self.depth = _encoder_depth(w, deter, embed)
-        if self.depth and not env.cfg.obs_flags & _abi.OBS_OCCUPANCY:
-            raise ValueError("a ConvEncoder agent reads lidar_occupancy: the env needs obs_type='lidar_occupancy'")
-        if not self.depth and embed != env.n_beams:
-            raise ValueError(f"the checkpoint embeds {embed} beams, the env casts {env.n_beams}")
-        if precision not in self.PRECISION:
-            raise ValueError(f"precision {precision!r}: expected one of {sorted(self.PRECISION)}")
-        self.precision = precision
-        self.n_samples, self.deter = int(n_samples), deter
+        self._configure(self._arch, _encoder_depth(w, self._arch[0], self._arch[3]), noise, precision, n_samples)
         self._bn = None
         if has_bn:
             self._bn = np.ascontiguousarray(np.stack([w["bn_gamma"], w["bn_beta"], w["bn_mean"], w["bn_var"]]), np.float32)
@@ -286,11 +274,31 @@ class DreamerPolicy:
                 env._check(env.lib.rd_policy_dreamer_init_occupancy(env._handle, C.byref(s), C.byref(e)))
             else:
                 env._check(env.lib.rd_policy_dreamer_init(env._handle, C.byref(s)))
-        self.actions = torch.zeros((env.n, 2), dtype=torch.float32, device=env.device)
-        self.debug = torch.zeros(env.n * _abi.RD_DREAMER_DEBUG_FLOATS, dtype=torch.float32, device=env.device)
+        self._buffers()
         self.expl_amount, self.expl_decay, self.expl_min = float(expl_amount), float(expl_decay), float(expl_min)
         self._set_exploration(0)
         self._staged = None
+
+    def _configure(self, arch, depth, noise: str, precision: str, n_samples: int) -> None:
+        """What every Dreamer policy of an env checks and keeps, before any device work: the noise and precision names,
+        and that the env produces what the agent reads (its images, or as many beams as it embeds)."""
+        env = self.env
+        if noise not in self.NOISE:
+            raise ValueError(f"noise {noise!r}: expected one of {sorted(self.NOISE)}")
+        deter, _, _, embed, _, _ = arch
+        if depth and not env.cfg.obs_flags & _abi.OBS_OCCUPANCY:
+            raise ValueError("a ConvEncoder agent reads lidar_occupancy: the env needs obs_type='lidar_occupancy'")
+        if not depth and embed != env.n_beams:
+            raise ValueError(f"the checkpoint embeds {embed} beams, the env casts {env.n_beams}")
+        if precision not in self.PRECISION:
+            raise ValueError(f"precision {precision!r}: expected one of {sorted(self.PRECISION)}")
+        self.noise, self.precision, self.n_samples, self.deter, self.depth = noise, precision, int(n_samples), deter, depth
+
+    def _buffers(self) -> None:
+        """the actions and diagnostics buffers act() writes"""
+        env = self.env
+        self.actions = torch.zeros((env.n, 2), dtype=torch.float32, device=env.device)
+        self.debug = torch.zeros(env.n * _abi.RD_DREAMER_DEBUG_FLOATS, dtype=torch.float32, device=env.device)
 
     def _weights_struct(self, w, bn, ptr) -> "_abi.RdDreamerWeights":
         deter, hidden, units, embed, layers, _ = self._arch
@@ -344,13 +352,26 @@ class DreamerPolicy:
         use the old weights, steps enqueued after the new ones, with no host synchronisation when the sources are
         CUDA tensors.  The recurrent state, the noise counter and ``env_steps`` are kept.  The sources stay referenced
         by the policy until the next call; writing to them afterwards on another stream needs the caller's ordering."""
+        s, e, on_device = self._stage_weights(weights, self._arch)
+        env = self.env
+        with torch.cuda.device(env.device):
+            if e is not None:
+                env._check(env.lib.rd_policy_dreamer_set_weights_occupancy(env._handle, C.byref(s), C.byref(e), int(on_device),
+                                                                           env._stream()))
+            else:
+                env._check(env.lib.rd_policy_dreamer_set_weights(env._handle, C.byref(s), int(on_device), env._stream()))
+
+    def _stage_weights(self, weights, expect_arch):
+        """load_weights' validation (architecture and BN presence ``expect_arch``) and staging: the weights and encoder
+        structs of the staged arrays, and whether they are device pointers.  The staged arrays are kept in
+        ``self._staged``."""
         env = self.env
         if not isinstance(weights, dict):
             raise TypeError("weights must be a dict of arrays")
         arch = _dreamer_arch(weights)
-        if arch != self._arch:
+        if arch != expect_arch:
             names = ("deter", "hidden", "units", "embed", "actor layers", "BN head")
-            diff = [f"{n} {a} != {b}" for n, a, b in zip(names, arch, self._arch) if a != b]
+            diff = [f"{n} {a} != {b}" for n, a, b in zip(names, arch, expect_arch) if a != b]
             raise ValueError("the weights do not match the policy's architecture: " + ", ".join(diff))
         deter, _, _, embed, layers, _ = arch
         depth = _encoder_depth(weights, deter, embed)
@@ -385,15 +406,8 @@ class DreamerPolicy:
             bn = np.ascontiguousarray(np.stack([staged[k] for k in ("bn_gamma", "bn_beta", "bn_mean", "bn_var")]),
                                       np.float32) if arch[5] else None
             ptr = lambda a: a.ctypes.data_as(C.c_void_p)   # noqa: E731
-        s = self._weights_struct(staged, bn, ptr)
-        with torch.cuda.device(env.device):
-            if depth:
-                e = self._encoder_struct(staged, ptr)
-                env._check(env.lib.rd_policy_dreamer_set_weights_occupancy(env._handle, C.byref(s), C.byref(e), int(on_device),
-                                                                           env._stream()))
-            else:
-                env._check(env.lib.rd_policy_dreamer_set_weights(env._handle, C.byref(s), int(on_device), env._stream()))
         self._staged = (staged, bn)
+        return self._weights_struct(staged, bn, ptr), self._encoder_struct(staged, ptr) if depth else None, on_device
 
     def act(self, lidar: Optional[torch.Tensor] = None, eps_stoch: Optional[torch.Tensor] = None,
             eps_actor: Optional[torch.Tensor] = None, debug: bool = False, noise: Optional[str] = None,
@@ -511,3 +525,117 @@ class DreamerPolicy:
                 run = env.lib.rd_rollout_dreamer_train if training else env.lib.rd_rollout_dreamer
                 env._check(run(env._handle, int(n_steps), C.byref(env._out), self.actions.data_ptr(), mode, env._stream()))
         return env._obs(), env.buf["reward"], env.buf["done_bool"], env._info()
+
+
+class DreamerAgents(DreamerPolicy):
+    """Several Dreamer agents on one ``BatchedRaceEnv``: env ``e`` is driven by agent ``agent_of_env[e]``, whose weights
+    are ``checkpoints[agent_of_env[e]]`` (``rd_policy_dreamer_init_agents``).  What env ``e`` gets -- actions, state,
+    diagnostics, Philox draws -- is bit for bit what a ``DreamerPolicy`` with that agent's weights gives it on the same
+    batch, in one agent step for the whole batch instead of one per agent.  Uses: cars of one world driven by different
+    checkpoints (a head-to-head race with ``agents_per_world = 4``, ``agent_of_env = np.arange(n) % 4 % 2``
+    [REF baselines/scenarios/max_progress/austria.yml:3-34]), evaluating a grid of checkpoints over tracks in one batch
+    [REF dreamer/evaluations/run_evaluation.py:43-94], or several learners collecting into one episode store.
+
+    checkpoints: 1..8 weight dicts or checkpoint names / paths (``load_dreamer_checkpoint``), all of one architecture
+    (deter, hidden, units, embed, actor layers, ConvEncoder depth); BN heads may differ per agent.  agent_of_env: integer
+    array [n_envs] with values in [0, len(checkpoints)), every agent driving at least one env.  noise, n_samples and
+    precision are the policy's, shared by every agent; expl_amount / expl_decay / expl_min are one value for every agent
+    or one per agent (``Dreamer._exploration`` per learner).  ``act``, ``rollout`` (also with a store), ``get_state``,
+    ``set_state``, ``reset``, ``diagnostics`` and ``encode`` are ``DreamerPolicy``'s, in env order.  What is per agent
+    takes the agent: ``load_weights(weights, agent)``, ``env_steps(agent)`` / ``set_env_steps(agent, value)`` and
+    ``exploration_amount(agent)`` (methods here, where ``DreamerPolicy`` has one ``env_steps`` property)."""
+
+    def __init__(self, env: BatchedRaceEnv, checkpoints, agent_of_env, noise: str = "philox", n_samples: int = 100,
+                 precision: str = "tf32x3", expl_amount=0.3, expl_decay=0.0, expl_min=0.0):
+        self.env = env
+        if isinstance(checkpoints, (dict, str, pathlib.Path)):
+            raise TypeError("checkpoints must be a sequence of weight dicts or checkpoint names, one per agent")
+        ws = [c if isinstance(c, dict) else load_dreamer_checkpoint(c) for c in checkpoints]
+        ws = [{k: np.ascontiguousarray(v, np.float32) for k, v in w.items()} for w in ws]
+        G = len(ws)
+        if not 1 <= G <= _abi.RD_MAX_DREAMER_AGENTS:
+            raise ValueError(f"{G} checkpoints: expected 1..{_abi.RD_MAX_DREAMER_AGENTS} agents")
+        archs = [_dreamer_arch(w) for w in ws]
+        depths = [_encoder_depth(w, a[0], a[3]) for w, a in zip(ws, archs)]
+        names = ("deter", "hidden", "units", "embed", "actor layers")
+        for g in range(1, G):
+            diff = [f"{n} {a} != {b}" for n, a, b in zip(names, archs[g], archs[0]) if a != b]
+            if depths[g] != depths[0]:
+                diff.append(f"ConvEncoder depth {depths[g]} != {depths[0]}")
+            if diff:
+                raise ValueError(f"checkpoint {g} does not match checkpoint 0's architecture: " + ", ".join(diff))
+        if isinstance(agent_of_env, torch.Tensor):
+            agent_of_env = agent_of_env.detach().cpu().numpy()
+        aoe = np.asarray(agent_of_env)
+        if aoe.shape != (env.n,) or not np.issubdtype(aoe.dtype, np.integer):
+            raise ValueError(f"agent_of_env must be an integer array of shape ({env.n},), got {aoe.dtype} {aoe.shape}")
+        if aoe.size and (aoe.min() < 0 or aoe.max() >= G):
+            raise ValueError(f"agent_of_env values must be in [0, {G})")
+        idle = sorted(set(range(G)) - set(aoe.tolist()))
+        if idle:
+            raise ValueError(f"agents {idle} drive no env: every agent needs at least one")
+        self._configure(archs[0], depths[0], noise, precision, n_samples)
+
+        def per_agent(v, name):
+            v = [float(x) for x in v] if np.ndim(v) else [float(v)] * G
+            if len(v) != G:
+                raise ValueError(f"{name}: one value, or one per agent ({G})")
+            return v
+        self._expl = list(zip(per_agent(expl_amount, "expl_amount"), per_agent(expl_decay, "expl_decay"),
+                              per_agent(expl_min, "expl_min")))
+        self.n_agents = G
+        self.agent_of_env = aoe.astype(np.int32)
+        self.agent_of_env.setflags(write=False)
+        self.weights = ws
+        self._arch = archs[0][:5] + (False,)
+        self._agent_arch = archs
+        bns = [np.ascontiguousarray(np.stack([w["bn_gamma"], w["bn_beta"], w["bn_mean"], w["bn_var"]]), np.float32)
+               if a[5] else None for w, a in zip(ws, archs)]
+        self._bns = bns
+        host = lambda a: a.ctypes.data_as(C.c_void_p)   # noqa: E731
+        structs = (_abi.RdDreamerWeights * G)(*[self._weights_struct(w, bn, host) for w, bn in zip(ws, bns)])
+        encs = (_abi.RdDreamerConvEncoder * G)(*[self._encoder_struct(w, host) for w in ws]) if self.depth else None
+        with torch.cuda.device(env.device):
+            env._check(env.lib.rd_policy_dreamer_init_agents(env._handle, G, structs, encs,
+                                                             self.agent_of_env.ctypes.data_as(C.c_void_p)))
+        self._buffers()
+        for g in range(G):
+            self.set_env_steps(g, 0)
+        self._staged, self._staged_by_agent = None, {}
+
+    def _agent(self, agent: int) -> int:
+        if not 0 <= int(agent) < self.n_agents:
+            raise ValueError(f"agent {agent} is not in [0, {self.n_agents})")
+        return int(agent)
+
+    def _exploration(self, agent: int) -> "_abi.RdDreamerExploration":
+        x = _abi.RdDreamerExploration()
+        self.env._check(self.env.lib.rd_policy_dreamer_get_agent_exploration(self.env._handle, self._agent(agent), C.byref(x)))
+        return x
+
+    def env_steps(self, agent: int) -> int:
+        """Agent ``agent``'s env-step counter: (its envs) x action_repeat per training step."""
+        return int(self._exploration(agent).env_steps)
+
+    def set_env_steps(self, agent: int, value: int) -> None:
+        g = self._agent(agent)
+        if int(value) < 0:
+            raise ValueError("env_steps must be >= 0")
+        x = _abi.RdDreamerExploration(*self._expl[g], int(value))
+        self.env._check(self.env.lib.rd_policy_dreamer_set_agent_exploration(self.env._handle, g, C.byref(x)))
+
+    def exploration_amount(self, agent: int) -> np.float32:
+        """The exploration amount agent ``agent``'s next training step applies."""
+        g = self._agent(agent)
+        return exploration_amount(*self._expl[g], self.env_steps(g))
+
+    def load_weights(self, weights, agent: int) -> None:
+        """``DreamerPolicy.load_weights`` for agent ``agent``: its BN presence must be the one it was built with.  The
+        other agents' weights and every env's state are untouched."""
+        g = self._agent(agent)
+        s, e, on_device = self._stage_weights(weights, self._agent_arch[g])
+        self._staged_by_agent[g] = self._staged   # kept until the agent's next load, as DreamerPolicy keeps its sources
+        env = self.env
+        with torch.cuda.device(env.device):
+            env._check(env.lib.rd_policy_dreamer_set_agent_weights(env._handle, g, C.byref(s), C.byref(e) if e is not None else None,
+                                                                   int(on_device), env._stream()))
