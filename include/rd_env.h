@@ -419,6 +419,59 @@ int rd_policy_dreamer_set_agent_weights(rd_env* env, int32_t agent, const rd_dre
 int rd_policy_dreamer_set_agent_exploration(rd_env* env, int32_t agent, const rd_dreamer_exploration* x);
 int rd_policy_dreamer_get_agent_exploration(rd_env* env, int32_t agent, rd_dreamer_exploration* x);
 
+/* ---- feed-forward Gaussian actor (the model-free baselines' actors, e.g. SB3's SAC and PPO policies): a trunk of
+ *      1..RD_MLP_MAX_LAYERS Linear + activation layers over the env's scan, then a head of two action means and two
+ *      log standard deviations.  The trunk and head products run on the tcgen05 tensor cores in three TF32 passes over
+ *      hi/lo split operands (float32-grade).  The actor reads the baselines chain's observation, the flattened scan
+ *      normalised to [0, 1]: init needs RD_OBS_NORM_BASELINES, float32 lidar without occupancy, clip_actions = 1 and
+ *      rescale_actions = 0 (RD_ERR_INVALID otherwise).  One actor per handle, stateless per env. ---- */
+#define RD_MLP_MAX_LAYERS 4
+#define RD_MLP_MAX_WIDTH 1024
+#define RD_MLP_DEBUG_FLOATS 4   /* per env: mean[2] std[2] of the Gaussian before the squash */
+enum { RD_ACT_RELU = 0, RD_ACT_TANH = 1 };
+enum { RD_HEAD_SQUASHED = 0, /* per-state log_std layer clamped to [log_std_min, log_std_max]; a = tanh(mean + std e) */
+       RD_HEAD_DIAG = 1      /* state-independent log_std vector [2]; a = mean + std e, unclipped */ };
+typedef struct rd_mlp_actor {
+  int32_t n_layers;             /* trunk layers, 1..RD_MLP_MAX_LAYERS */
+  int32_t in_features;          /* = cfg.n_beams */
+  int32_t width[RD_MLP_MAX_LAYERS];   /* output width of each trunk layer, 1..RD_MLP_MAX_WIDTH */
+  int32_t activation;           /* RD_ACT_* after every trunk layer */
+  int32_t head;                 /* RD_HEAD_* */
+  float log_std_min, log_std_max;     /* RD_HEAD_SQUASHED clamp */
+  /* PyTorch layout (nn.Linear): weight [out][in], bias [out]; host pointers, or device pointers with on_device */
+  const float* w[RD_MLP_MAX_LAYERS];
+  const float* b[RD_MLP_MAX_LAYERS];
+  const float* mean_w;          /* [2][width[n_layers - 1]] */
+  const float* mean_b;          /* [2] */
+  const float* log_std_w;       /* RD_HEAD_SQUASHED: [2][width[n_layers - 1]]; else ignored */
+  const float* log_std_b;       /* RD_HEAD_SQUASHED: [2]; else ignored */
+  const float* log_std;         /* RD_HEAD_DIAG: [2]; else ignored */
+} rd_mlp_actor;
+/* Packs the actor's weights (host pointers) for the handle's envs; replaces an earlier actor.  Every check (the env
+ * config above, the architecture, the pointers) runs before any device work: a rejected init changes nothing. */
+int rd_policy_mlp_init(rd_env* env, const rd_mlp_actor* a);
+/* One actor step for every env: obs_dev f32 [N, n_beams] (the env's lidar output) -> actions_dev f32 [N, 2], the
+ * agent-facing action rd_step reads.  deterministic: e = 0 (SAC: tanh(mean); PPO: mean); else e ~ N(0, 1) per noise mode
+ * (RD_NOISE_PHILOX: block (env id, step, 0, stream tag) of Philox4x32-10 keyed (seed_lo, seed_hi ^ tag), Box-Muller
+ * normals z0, z1; RD_NOISE_ZERO: e = 0; RD_NOISE_EXPLICIT: eps_dev f32 [N, 2]).  debug_dev (may be NULL) f32
+ * [N, RD_MLP_DEBUG_FLOATS].  The step counter advances by one per call. */
+int rd_policy_mlp(rd_env* env, const float* obs_dev, float* actions_dev, int deterministic, int noise, const float* eps_dev,
+                  float* debug_dev, void* stream);
+/* New weights of the init's architecture (n_layers, widths, in_features, activation, head, clamp bounds; else
+ * RD_ERR_INVALID and nothing changes), packed on `stream` by init's packer.  on_device: the pointers are device memory
+ * of the handle's device, read on `stream` without a host synchronisation.  The step counter is kept. */
+int rd_policy_mlp_set_weights(rd_env* env, const rd_mlp_actor* w, int on_device, void* stream);
+/* n_steps x (rd_policy_mlp on out->lidar_dev -> rd_step); noise RD_NOISE_PHILOX or RD_NOISE_ZERO; the actions of the
+ * last step are left in actions_dev (may be NULL). */
+int rd_rollout_mlp(rd_env* env, int n_steps, const rd_outputs* out, float* actions_dev, int deterministic, int noise,
+                   void* stream);
+/* Uniform random actions, any env config: per env and call, Philox4x32-10 block (env id, step, 0, stream tag) keyed
+ * (seed_lo, seed_hi ^ tag), a_k = 2 (x_k >> 8) 2^-24 - 1 in [-1, 1) for k = 0, 1 (exact in float32).  The handle's
+ * random-action step counter advances by one per call. */
+int rd_policy_random(rd_env* env, float* actions_dev, void* stream);
+/* n_steps x (rd_policy_random -> rd_step); actions_dev as rd_rollout_mlp */
+int rd_rollout_random(rd_env* env, int n_steps, const rd_outputs* out, float* actions_dev, void* stream);
+
 /* ---- device-resident episode store (SURVEY.md §8-f1): records the Collect rows of every env's episodes on the device
  *      [REF dreamer/wrappers.py:198-250], exactly the episodes episodes.EpisodeRecorder hands to its callbacks, and
  *      samples fixed-length chunks the way tools.load_episodes does [REF dreamer/tools.py:235-264].  The env must have
@@ -429,7 +482,10 @@ int rd_policy_dreamer_get_agent_exploration(rd_env* env, int32_t agent, rd_dream
 enum { RD_STORE_LIDAR = 1, RD_STORE_POSE = 2, RD_STORE_VELOCITY = 4, RD_STORE_SPEED = 8,
        RD_STORE_OCCUPANCY = 16 /* 'lidar_occupancy', u8 [64,64,1]; needs RD_OBS_OCCUPANCY */ };   /* keep_obs bits */
 enum { RD_STORE_POLICY_GAP_FOLLOWER = 0, RD_STORE_POLICY_DREAMER = 1,
-       RD_STORE_POLICY_DREAMER_TRAIN = 2 /* rd_rollout_dreamer_train's agent step */ };          /* rd_rollout_store */
+       RD_STORE_POLICY_DREAMER_TRAIN = 2, /* rd_rollout_dreamer_train's agent step */
+       RD_STORE_POLICY_MLP = 3,           /* rd_rollout_mlp, deterministic actions */
+       RD_STORE_POLICY_MLP_TRAIN = 4,     /* rd_rollout_mlp, sampled actions (noise RD_NOISE_PHILOX or RD_NOISE_ZERO) */
+       RD_STORE_POLICY_RANDOM = 5         /* rd_rollout_random */ };                                  /* rd_rollout_store */
 typedef struct rd_store_config {
   int32_t capacity_rows;      /* rows per env */
   int32_t precision;          /* 32 | 16: float keys as float32 | IEEE half [REF dreamer/wrappers.py:240-250 _convert] */

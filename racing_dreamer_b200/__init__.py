@@ -15,10 +15,11 @@ def __getattr__(name):
         from . import env as _env
         return getattr(_env, name)
     if name in ("RaceCarGymCompat", "ReferenceEnv", "SingleAgentRaceCompat", "BaselinesEnv", "make_reference_env",
-                "load_scenario"):
+                "load_scenario", "baselines_config"):
         from . import compat as _compat
         return getattr(_compat, name)
-    if name in ("GapFollowerPolicy", "DreamerPolicy", "DreamerAgents", "load_dreamer_checkpoint", "save_dreamer_checkpoint"):
+    if name in ("GapFollowerPolicy", "DreamerPolicy", "DreamerAgents", "load_dreamer_checkpoint", "save_dreamer_checkpoint",
+                "Sb3Policy", "RandomPolicy", "load_sb3_checkpoint"):
         from . import policy as _policy
         return getattr(_policy, name)
     raise AttributeError(name)

@@ -11,6 +11,7 @@ from pathlib import Path
 ABI_VERSION = 3
 MAX_AGENTS = 4   # RD_MAX_AGENTS
 MAX_NSTEP = 32   # RD_MAX_NSTEP
+RD_MLP_MAX_LAYERS, RD_MLP_MAX_WIDTH, RD_MLP_DEBUG_FLOATS = 4, 1024, 4
 
 # enums (include/rd_env.h)
 RESET_GRID, RESET_RANDOM, RESET_RANDOM_BIDIRECTIONAL, RESET_RANDOM_BALL = 0, 1, 2, 3
@@ -125,6 +126,15 @@ class RdDreamerExploration(C.Structure):
     _fields_ = [("amount", C.c_double), ("decay", C.c_double), ("min_amount", C.c_double), ("env_steps", C.c_int64)]
 
 
+class RdMlpActor(C.Structure):
+    """rd_mlp_actor (include/rd_env.h): a feed-forward Gaussian actor's architecture and pointers to its PyTorch-layout
+    weights ([out][in]) and biases."""
+    _fields_ = [("n_layers", C.c_int32), ("in_features", C.c_int32), ("width", C.c_int32 * RD_MLP_MAX_LAYERS),
+                ("activation", C.c_int32), ("head", C.c_int32), ("log_std_min", C.c_float), ("log_std_max", C.c_float),
+                ("w", C.c_void_p * RD_MLP_MAX_LAYERS), ("b", C.c_void_p * RD_MLP_MAX_LAYERS)] + [
+        (n, C.c_void_p) for n in ("mean_w", "mean_b", "log_std_w", "log_std_b", "log_std")]
+
+
 class RdStoreConfig(C.Structure):
     """rd_store_config (include/rd_env.h): the device-resident episode store."""
     _fields_ = [("capacity_rows", C.c_int32), ("precision", C.c_int32), ("keep_obs", C.c_int32), ("reset_mode", C.c_int32),
@@ -169,11 +179,14 @@ STORE_LIDAR, STORE_POSE, STORE_VELOCITY, STORE_SPEED, STORE_OCCUPANCY = 1, 2, 4,
 STORE_KEYS = {"lidar": STORE_LIDAR, "pose": STORE_POSE, "velocity": STORE_VELOCITY, "speed": STORE_SPEED,
               "lidar_occupancy": STORE_OCCUPANCY}
 STORE_POLICY_GAP_FOLLOWER, STORE_POLICY_DREAMER, STORE_POLICY_DREAMER_TRAIN = 0, 1, 2
+STORE_POLICY_MLP, STORE_POLICY_MLP_TRAIN, STORE_POLICY_RANDOM = 3, 4, 5
 
 RD_NOISE_ZERO, RD_NOISE_PHILOX, RD_NOISE_EXPLICIT = 0, 1, 2
 RD_DREAMER_DEBUG_FLOATS = 68
 RD_PRECISION_TF32X3, RD_PRECISION_TF32 = 0, 1
 RD_MAX_DREAMER_AGENTS = 8
+RD_ACT_RELU, RD_ACT_TANH = 0, 1
+RD_HEAD_SQUASHED, RD_HEAD_DIAG = 0, 1
 
 EXPORTS = (
     "rd_default_config", "rd_create", "rd_destroy", "rd_last_error", "rd_abi_version", "rd_upload_map",
@@ -188,6 +201,8 @@ EXPORTS = (
     "rd_policy_dreamer_set_weights_occupancy", "rd_dreamer_encode_occupancy",
     "rd_policy_dreamer_init_agents", "rd_policy_dreamer_set_agent_weights", "rd_policy_dreamer_set_agent_exploration",
     "rd_policy_dreamer_get_agent_exploration",
+    "rd_policy_mlp_init", "rd_policy_mlp", "rd_policy_mlp_set_weights", "rd_rollout_mlp", "rd_policy_random",
+    "rd_rollout_random",
     "rd_store_init", "rd_store_reset", "rd_store_step", "rd_rollout_store", "rd_store_sample", "rd_store_info",
     "rd_store_import_init", "rd_store_import", "rd_store_import_info",
 )
@@ -312,6 +327,18 @@ def load_library() -> C.CDLL:
     lib.rd_policy_dreamer_set_agent_exploration.restype = i32
     lib.rd_policy_dreamer_get_agent_exploration.argtypes = [vp, i32, C.POINTER(RdDreamerExploration)]
     lib.rd_policy_dreamer_get_agent_exploration.restype = i32
+    lib.rd_policy_mlp_init.argtypes = [vp, C.POINTER(RdMlpActor)]
+    lib.rd_policy_mlp_init.restype = i32
+    lib.rd_policy_mlp.argtypes = [vp, vp, vp, i32, i32, vp, vp, vp]
+    lib.rd_policy_mlp.restype = i32
+    lib.rd_policy_mlp_set_weights.argtypes = [vp, C.POINTER(RdMlpActor), i32, vp]
+    lib.rd_policy_mlp_set_weights.restype = i32
+    lib.rd_rollout_mlp.argtypes = [vp, i32, C.POINTER(RdOutputs), vp, i32, i32, vp]
+    lib.rd_rollout_mlp.restype = i32
+    lib.rd_policy_random.argtypes = [vp, vp, vp]
+    lib.rd_policy_random.restype = i32
+    lib.rd_rollout_random.argtypes = [vp, i32, C.POINTER(RdOutputs), vp, vp]
+    lib.rd_rollout_random.restype = i32
     lib.rd_store_init.argtypes = [vp, C.POINTER(RdStoreConfig)]
     lib.rd_store_init.restype = i32
     lib.rd_store_reset.argtypes = [vp, C.POINTER(RdOutputs), vp]

@@ -18,6 +18,7 @@ as the batched path.  Training-scale callers should use ``BatchedRaceEnv`` direc
 """
 from __future__ import annotations
 
+import dataclasses
 import types
 from pathlib import Path
 from typing import Dict as TDict, Optional, Union
@@ -42,6 +43,25 @@ SCENARIO_DEFAULTS = {
 
 
 AGENT_IDS = ("A", "B", "C", "D")
+
+
+def baselines_config(tracks, n_envs: int, action_repeat: int = 4, mode: str = "train", **overrides) -> EnvConfig:
+    """The model-free baselines' wrap chain (``BaselinesEnv``) as the config of a batched env of ``n_envs`` cars:
+    flattened lidar normalised to [0, 1] (``normalize_obs='baselines'``), actions in [-1, 1] clipped by the env
+    (``clip_actions``, no rescale), ``repeat_semantics='baselines'`` and the tick-based TimeLimit inside ActionRepeat
+    [REF baselines/racing/experiments/acme/experiment.py:66-88; baselines/racing/experiments/sb3/sb_experiment.py:42-58].
+    mode 'train': reset mode 'random', 2000 ticks; 'test': 'grid', 4000 ticks.  The max_progress scenario's task
+    parameters unless ``overrides`` name others; ``overrides`` may set any ``EnvConfig`` field."""
+    if mode not in ("train", "test"):
+        raise ValueError("mode must be 'train' or 'test'")
+    test = mode == "test"
+    kw = dict(SCENARIO_DEFAULTS["max_progress"])
+    kw.update(obs_type="lidar", action_repeat=int(action_repeat), reset_mode="grid" if test else "random",
+              time_limit_steps=0, time_limit_ticks=4000 if test else 2000, rescale_actions=False, clip_actions=True,
+              repeat_semantics="baselines", normalize_obs="baselines")
+    kw.update(overrides)
+    tracks = tuple(tracks) if isinstance(tracks, (list, tuple)) else (tracks,)
+    return EnvConfig(tracks=tracks, n_envs=int(n_envs), **kw)
 
 
 def load_scenario(path: Union[str, Path], agent_id: str = "A") -> dict:
@@ -445,11 +465,14 @@ class BaselinesEnv(_SingleAgentBase):
                 sc.pop(k, None)
             params.update(sc)
         params.update(overrides)
-        self._limit = int(time_limit if time_limit is not None else (4000 if self._test else 2000))
-        self._reset_mode = "grid" if self._test else "random"
-        self._make(track, n_agents=1, order=order, action_repeat=int(action_repeat), reset_mode=self._reset_mode,
-                   obs_type="lidar", time_limit_steps=0, time_limit_ticks=self._limit, rescale_actions=False,
-                   clip_actions=True, repeat_semantics="baselines", normalize_obs="baselines", **params)
+        if time_limit is not None:
+            params["time_limit_ticks"] = int(time_limit)
+        ec = baselines_config(track, 1, action_repeat, mode, **params)
+        self._limit = int(ec.time_limit_ticks)
+        self._reset_mode = ec.reset_mode
+        # _make sets the tracks, the car count and the manual resets itself
+        self._make(track, n_agents=1, order=order, **{f.name: getattr(ec, f.name) for f in dataclasses.fields(ec)
+                                                      if f.name not in ("tracks", "n_envs", "map_ids", "auto_reset")})
         self._needs_reset = True
         self._action = torch.zeros((1, 2), dtype=torch.float32, device=self._env.device)
 

@@ -149,7 +149,9 @@ static inline cudaError_t dr_pack_conv(DreamerPolicy& d, const float* const* src
 
 // zero-initialised operand array(s) [rows][ld].  In single-pass mode p[1] is null -- the packer and the epilogues test it
 // -- also where the operand held a freed remainder array of an earlier tf32x3 agent (dr_view likewise).
-static inline cudaError_t dr_alloc(DreamerPolicy& d, DreamerPolicy::Operand& op, size_t rows, size_t ld) {
+// P: DreamerPolicy or MlpPolicy (rd_mlp.cuh), which read their x3 / owned / ag members the same way (dr_view, dr_build too).
+template <class P>
+static inline cudaError_t dr_alloc(P& d, DreamerPolicy::Operand& op, size_t rows, size_t ld) {
   op.p[1] = nullptr;
   for (int part = 0; part < (d.x3 ? 2 : 1); ++part) {
     cudaError_t e = cudaMalloc(&op.p[part], rows * ld * sizeof(float));
@@ -161,7 +163,8 @@ static inline cudaError_t dr_alloc(DreamerPolicy& d, DreamerPolicy::Operand& op,
   return cudaSuccess;
 }
 // TMA views of both parts: columns [col0, col0 + inner) of rows of pitch ld
-static inline bool dr_view(const DreamerPolicy& d, DreamerPolicy::Operand& view, const DreamerPolicy::Operand& base, size_t col0,
+template <class P>
+static inline bool dr_view(const P& d, DreamerPolicy::Operand& view, const DreamerPolicy::Operand& base, size_t col0,
                            uint64_t inner, uint64_t rows, uint64_t ld, uint32_t box_rows) {
   for (int part = 0; part < (d.x3 ? 2 : 1); ++part) {
     view.p[part] = base.p[part] + col0;
@@ -233,7 +236,7 @@ static inline int dr_pack(DreamerPolicy& d, const rd_dreamer_weights* w, const r
   }
   a.total = (long long)off;
   const unsigned grid = (unsigned)std::min<size_t>((off + 255) / 256, (size_t)d.sm_count * 8);
-  k_pack_weights<<<grid, 256, 0, s>>>(a);
+  k_pack_weights<false><<<grid, 256, 0, s>>>(a);
   DR_TRY(cudaGetLastError());
   if (enc) {
     const float* src[3];
@@ -481,7 +484,8 @@ static inline int dreamer_set_weights(DreamerPolicy& d, int agent, const rd_drea
 // cut into K groups of at most ~6 blocks, one accumulator group each (see "truncation" in rd_gemm.cuh).
 // Accumulator slot = group * gates + gate; `gate[t][i]` maps slab i of term t to its gate (Dense layers: one gate).
 struct DrTerm { const DreamerPolicy::Operand* a; const DreamerPolicy::Operand* w; int k_elems; int w_k0; };
-static inline void dr_build(const DreamerPolicy& d, GemmMaps& maps, GemmArgs& g, const DrTerm* terms, int n_terms, int nb,
+template <class P>
+static inline void dr_build(const P& d, GemmMaps& maps, GemmArgs& g, const DrTerm* terms, int n_terms, int nb,
                             const int* w_row0, const int (*gate)[3], int gates, int slots) {
   g.n_phases = 0;
   g.ag = d.ag;

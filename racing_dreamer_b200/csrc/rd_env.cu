@@ -23,6 +23,7 @@
 #include "rd_occupancy.cuh"
 #include "rd_policy.cuh"
 #include "rd_dreamer.cuh"
+#include "rd_mlp.cuh"
 #include "rd_store.cuh"
 
 #define RD_API extern "C" __attribute__((visibility("default")))
@@ -111,6 +112,8 @@ struct rd_env {
     bool attr_set = false;        // kernel opted in to > 48 KB of dynamic shared memory
   } pol;
   DreamerPolicy dr;   // on-device Dreamer agent (rd_policy_dreamer_init)
+  MlpPolicy mlp;      // on-device feed-forward Gaussian actor (rd_policy_mlp_init)
+  uint32_t random_step = 0;   // rd_policy_random calls so far (Philox counter)
   // device-resident episode store (rd_store_init, csrc/rd_store.cuh)
   struct Store {
     bool ready = false, started = false;   // started: rd_store_reset has run
@@ -684,6 +687,7 @@ RD_API void rd_destroy(rd_env* env) {
   cudaFree(env->d_stage_recs); cudaFree(env->d_stage_ids);
   cudaFree(env->pol.st.f64); cudaFree(env->pol.st.i32); cudaFree(env->pol.d_actions);
   dreamer_free(env->dr);
+  mlp_free(env->mlp);
   store_free(env->st);
   occ_free(env->occ);
   {
@@ -1400,6 +1404,106 @@ RD_API int rd_dreamer_encode_occupancy(rd_env* env, const uint8_t* occupancy_dev
   return RD_OK;
 }
 
+namespace {
+int launch_mlp(rd_env* env, const float* obs_dev, float* actions_dev, int deterministic, int noise, const float* eps_dev,
+               float* debug_dev, cudaStream_t s) {
+  int launched = 0, rc;
+  {
+    ScopedTiming tm(env, s, T_POLICY);
+    rc = mlp_step(env->mlp, obs_dev, actions_dev, deterministic, noise, eps_dev, debug_dev, env->cfg.seed,
+                  (uint32_t)env->cfg.env_id_offset, s, &launched);
+  }
+  env->launches += launched;
+  if (rc) return fail(env, rc, "rd_policy_mlp: %s", env->mlp.err.c_str());
+  return RD_OK;
+}
+int launch_random(rd_env* env, float* actions_dev, cudaStream_t s) {
+  const uint64_t seed = env->cfg.seed;
+  {
+    ScopedTiming tm(env, s, T_POLICY);
+    k_random_actions<<<(unsigned)((env->n + 255) / 256), 256, 0, s>>>(actions_dev, env->n, (uint32_t)seed,
+                                                                      (uint32_t)(seed >> 32) ^ RD_STREAM_RANDOM,
+                                                                      env->random_step, (uint32_t)env->cfg.env_id_offset);
+  }
+  env->launches++;
+  CUDA_TRY(env, cudaGetLastError());
+  env->random_step++;
+  return RD_OK;
+}
+// the checks every MLP rollout makes (rd_rollout_mlp, rd_rollout_store)
+int mlp_rollout_check(rd_env* env, const rd_outputs* out, int noise) {
+  if (!env->mlp.ready) return fail(env, RD_ERR_STATE, "rd_policy_mlp_init has not been called");
+  if (!out->lidar_dev) return fail(env, RD_ERR_INVALID, "the rollout needs out->lidar_dev");
+  if (noise != RD_NOISE_ZERO && noise != RD_NOISE_PHILOX)
+    return fail(env, RD_ERR_INVALID, "a rollout draws its own noise (RD_NOISE_ZERO or RD_NOISE_PHILOX)");
+  return RD_OK;
+}
+}  // namespace
+
+RD_API int rd_policy_mlp_init(rd_env* env, const rd_mlp_actor* a) {
+  if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
+  const rd_config& c = env->cfg;
+  // the actor reads what the baselines were trained on: the flattened scan normalised to [0, 1], float32, and hands
+  // the env actions in [-1, 1] that the env clips (Flatten) without rescaling
+  if (!(c.obs_flags & RD_OBS_NORM_BASELINES) || (c.obs_flags & (RD_OBS_LIDAR_F16 | RD_OBS_OCCUPANCY)) ||
+      !c.clip_actions || c.rescale_actions)
+    return fail(env, RD_ERR_INVALID, "rd_policy_mlp_init: the env must be the baselines chain (RD_OBS_NORM_BASELINES, "
+                "float32 lidar without occupancy, clip_actions = 1, rescale_actions = 0)");
+  const int rc = mlp_init(env->mlp, env->n, c.n_beams, a);
+  if (rc) return fail(env, rc, "rd_policy_mlp_init: %s", env->mlp.err.c_str());
+  return ensure_rollout_actions(env);
+}
+
+RD_API int rd_policy_mlp(rd_env* env, const float* obs_dev, float* actions_dev, int deterministic, int noise,
+                         const float* eps_dev, float* debug_dev, void* stream) {
+  if (!env || !obs_dev || !actions_dev) return fail(env, RD_ERR_INVALID, "null argument");
+  if (!env->mlp.ready) return fail(env, RD_ERR_STATE, "rd_policy_mlp_init has not been called");
+  if (noise < RD_NOISE_ZERO || noise > RD_NOISE_EXPLICIT) return fail(env, RD_ERR_INVALID, "bad noise mode %d", noise);
+  if (!deterministic && noise == RD_NOISE_EXPLICIT && !eps_dev) return fail(env, RD_ERR_INVALID, "RD_NOISE_EXPLICIT needs eps_dev");
+  return launch_mlp(env, obs_dev, actions_dev, deterministic, noise, eps_dev, debug_dev, (cudaStream_t)stream);
+}
+
+RD_API int rd_policy_mlp_set_weights(rd_env* env, const rd_mlp_actor* w, int on_device, void* stream) {
+  if (!env) return fail(nullptr, RD_ERR_INVALID, "null handle");
+  if (!env->mlp.ready) return fail(env, RD_ERR_STATE, "rd_policy_mlp_init has not been called");
+  const int rc = mlp_set_weights(env->mlp, w, env->cfg.n_beams, on_device != 0, (cudaStream_t)stream);
+  if (rc) return fail(env, rc, "rd_policy_mlp_set_weights: %s", env->mlp.err.c_str());
+  env->launches++;   // k_pack_weights
+  return RD_OK;
+}
+
+RD_API int rd_rollout_mlp(rd_env* env, int n_steps, const rd_outputs* out, float* actions_dev, int deterministic, int noise,
+                          void* stream) {
+  if (!env || !out || n_steps < 0) return fail(env, RD_ERR_INVALID, "bad argument");
+  if (int rc = mlp_rollout_check(env, out, noise)) return rc;
+  if (!env->was_reset) return fail(env, RD_ERR_STATE, "Must reset environment.");
+  float* act = actions_dev ? actions_dev : env->pol.d_actions;
+  for (int k = 0; k < n_steps; ++k) {
+    int rc = launch_mlp(env, out->lidar_dev, act, deterministic, noise, nullptr, nullptr, (cudaStream_t)stream);
+    if (rc) return rc;
+    if ((rc = rd_step(env, act, out, stream))) return rc;
+  }
+  return RD_OK;
+}
+
+RD_API int rd_policy_random(rd_env* env, float* actions_dev, void* stream) {
+  if (!env || !actions_dev) return fail(env, RD_ERR_INVALID, "null argument");
+  return launch_random(env, actions_dev, (cudaStream_t)stream);
+}
+
+RD_API int rd_rollout_random(rd_env* env, int n_steps, const rd_outputs* out, float* actions_dev, void* stream) {
+  if (!env || !out || n_steps < 0) return fail(env, RD_ERR_INVALID, "bad argument");
+  if (!env->was_reset) return fail(env, RD_ERR_STATE, "Must reset environment.");
+  if (int rc = ensure_rollout_actions(env)) return rc;
+  float* act = actions_dev ? actions_dev : env->pol.d_actions;
+  for (int k = 0; k < n_steps; ++k) {
+    int rc = launch_random(env, act, (cudaStream_t)stream);
+    if (rc) return rc;
+    if ((rc = rd_step(env, act, out, stream))) return rc;
+  }
+  return RD_OK;
+}
+
 RD_API int rd_lidar_cast(rd_env* env, const double* poses_dev, const int32_t* map_ids_host, int n, float* ranges_dev,
                          void* stream) {
   if (!env || n < 0) return fail(env, RD_ERR_INVALID, "bad argument");
@@ -1771,15 +1875,24 @@ RD_API int rd_rollout_store(rd_env* env, int policy, int n_steps, const rd_outpu
     if (!env->pol.ready) return fail(env, RD_ERR_STATE, "rd_policy_gap_follower_init has not been called");
   } else if (policy == RD_STORE_POLICY_DREAMER || policy == RD_STORE_POLICY_DREAMER_TRAIN) {
     if ((rc = dreamer_rollout_obs(env, out, noise, &dr_obs))) return rc;
+  } else if (policy == RD_STORE_POLICY_MLP || policy == RD_STORE_POLICY_MLP_TRAIN) {
+    if ((rc = mlp_rollout_check(env, out, noise))) return rc;
+  } else if (policy == RD_STORE_POLICY_RANDOM) {
+    if ((rc = ensure_rollout_actions(env))) return rc;
   } else {
     return fail(env, RD_ERR_INVALID, "bad policy %d", policy);
   }
   cudaStream_t s = (cudaStream_t)stream;
   float* act = actions_dev ? actions_dev : env->pol.d_actions;
   for (int k = 0; k < n_steps; ++k) {
-    rc = policy == RD_STORE_POLICY_GAP_FOLLOWER ? launch_gap_follower(env, out->lidar_dev, nullptr, act, nullptr, s)
-                                                : launch_dreamer(env, dr_obs, act, noise, nullptr, nullptr, nullptr, s,
-                                                                 policy == RD_STORE_POLICY_DREAMER_TRAIN);
+    if (policy == RD_STORE_POLICY_MLP || policy == RD_STORE_POLICY_MLP_TRAIN)
+      rc = launch_mlp(env, out->lidar_dev, act, policy == RD_STORE_POLICY_MLP, noise, nullptr, nullptr, s);
+    else if (policy == RD_STORE_POLICY_RANDOM)
+      rc = launch_random(env, act, s);
+    else
+      rc = policy == RD_STORE_POLICY_GAP_FOLLOWER ? launch_gap_follower(env, out->lidar_dev, nullptr, act, nullptr, s)
+                                                  : launch_dreamer(env, dr_obs, act, noise, nullptr, nullptr, nullptr, s,
+                                                                   policy == RD_STORE_POLICY_DREAMER_TRAIN);
     if (rc) return rc;
     if ((rc = store_step(env, act, out, s))) return rc;
   }

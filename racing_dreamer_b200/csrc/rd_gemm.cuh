@@ -60,11 +60,15 @@ struct GemmPhase {
   int acc_small[3];
 };
 
-enum { EPI_DENSE = 0, EPI_GRU = 1, EPI_STOCH = 2, EPI_ACTOR = 3 };
+// EPI_DENSE_RELU / EPI_DENSE_TANH: EPI_DENSE's epilogue with relu / tanh fixed at compile time (the MLP actor's trunk,
+// rd_mlp.cuh) instead of the runtime ELU switch g.act
+enum { EPI_DENSE = 0, EPI_GRU = 1, EPI_STOCH = 2, EPI_ACTOR = 3, EPI_DENSE_RELU = 4, EPI_DENSE_TANH = 5 };
 enum { GM_NOISE_ZERO = 0, GM_NOISE_PHILOX = 1, GM_NOISE_EXPLICIT = 2 };
 #define RD_STREAM_STOCH 0x53544f43u
 #define RD_STREAM_ACTOR 0x41435452u
 #define RD_STREAM_TRAIN 0x5452414eu   // training head: the action sample and its exploration noise (k_actor_train)
+#define RD_STREAM_MLP 0x4d4c5041u     // MLP actor's Gaussian sample (k_mlp_head)
+#define RD_STREAM_RANDOM 0x524e4441u  // uniform random actions (k_random_actions)
 
 // Several agents in one batch (rd_policy_dreamer_init_agents): the policy's internal rows are ordered by agent, agent a
 // owning rows [start[a], start[a + 1]), every start a multiple of GM_BM, so each 128-row tile belongs to one agent.  The
@@ -471,7 +475,8 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
     // 14 us actor layer and 21 us of the GRU cell, profiles/r3t_dreamer_kdense_analysis.txt.) =====
     const int q = warp & 3;
     const int part = (warp - 2) >> 2;                        // 0 .. EW - 1
-    constexpr int PART_COLS = (EPI == EPI_DENSE ? BN : GM_BN) / EW;
+    constexpr bool DENSE = EPI == EPI_DENSE || EPI == EPI_DENSE_RELU || EPI == EPI_DENSE_TANH;
+    constexpr int PART_COLS = (DENSE ? BN : GM_BN) / EW;
     const int cbeg = part * PART_COLS, cend = cbeg + PART_COLS;
     const int row = m0 + q * 32 + lane;
     const uint32_t tl = tmem + ((uint32_t)(q * 32) << 16);
@@ -513,7 +518,7 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
     constexpr int TILE_PARTS = PART_COLS >= 32 ? 1 : 32 / PART_COLS;       // column parts per staging tile
     static_assert(PART_COLS == 16 || PART_COLS % 32 == 0, "staging tiles are 32 columns wide");
     const uint32_t rt = (uint32_t)(q * 32 + lane);                          // tile row
-    if constexpr (EPI == EPI_DENSE) {
+    if constexpr (DENSE) {
 #pragma unroll 1
       for (int c0 = cbeg; c0 < cend; c0 += 16) {
         if (n0 + c0 >= g.N) break;   // warp-uniform
@@ -530,7 +535,8 @@ __global__ void __launch_bounds__(64 + 128 * EW, 1)
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
               float x = v[j + t] + __ldg(g.bias + (bo + col + t));
-              if constexpr (CONV > 0) x = fmaxf(x, 0.f);   // tf.nn.relu
+              if constexpr (CONV > 0 || EPI == EPI_DENSE_RELU) x = fmaxf(x, 0.f);   // tf.nn.relu / torch.nn.ReLU
+              else if constexpr (EPI == EPI_DENSE_TANH) x = tanhf(x);             // torch.nn.Tanh
               else if (g.act) x = gm_elu(x);
               po[t] = gm_round_tf32(x);
               pl[t] = gm_round_tf32(x - po[t]);
@@ -853,9 +859,11 @@ __global__ void __launch_bounds__(256) k_actor_train(const GemmArgs g, const flo
   }
 }
 
-// The Dreamer weights' packer (dr_pack: init and weight refresh): checkpoint arrays -> the policy's packed operands.
+// The weights' packer (init and weight refresh of the Dreamer agent, dr_pack, and of the MLP actor, mlp_pack):
+// checkpoint arrays -> the policy's packed operands.
 // Job j: src [in][out] -> dst (o, kmap(i)) = tf32(x) and, if lo, tf32(x - tf32(x)), kmap(i) = i >= k_from ? i + k_shift
 // : i (dr_parts' layout; the K slots it skips keep init's zeros); raw jobs copy [out] values as they are (biases, BN).
+// KMAJOR: the matrix sources are already K-major, src [out][in] (PyTorch's nn.Linear weight), kmap(i) = i.
 // The rounding is an integer round-to-nearest on the bits (gm_tf32_bits).
 #define GM_PACK_MAX 32
 struct PackJob {
@@ -867,6 +875,7 @@ struct PackArgs { int n_jobs; long long total; PackJob job[GM_PACK_MAX]; };
 __device__ __forceinline__ float gm_tf32_bits(float x) {   // round to TF32, ties away from zero (finite values)
   return __uint_as_float((__float_as_uint(x) + 0x1000u) & ~0x1fffu);
 }
+template <bool KMAJOR>
 __global__ void __launch_bounds__(256) k_pack_weights(const __grid_constant__ PackArgs a) {
   for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < a.total; t += (long long)gridDim.x * blockDim.x) {
     int j = 0;
@@ -875,8 +884,13 @@ __global__ void __launch_bounds__(256) k_pack_weights(const __grid_constant__ Pa
     const long long e = t - J.begin;
     const float x = J.src[e];
     if (J.raw) { J.hi[e] = x; continue; }
-    const int i = (int)(e / J.out), o = (int)(e % J.out);
-    const size_t f = (size_t)o * J.ld + (i >= J.k_from ? i + J.k_shift : i);
+    size_t f;
+    if constexpr (KMAJOR) {
+      f = (size_t)(e / J.in) * J.ld + (size_t)(e % J.in);
+    } else {
+      const int i = (int)(e / J.out), o = (int)(e % J.out);
+      f = (size_t)o * J.ld + (i >= J.k_from ? i + J.k_shift : i);
+    }
     const float h = gm_tf32_bits(x);
     J.hi[f] = h;
     if (J.lo) J.lo[f] = gm_tf32_bits(__fsub_rn(x, h));

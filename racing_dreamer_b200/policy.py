@@ -639,3 +639,318 @@ class DreamerAgents(DreamerPolicy):
         with torch.cuda.device(env.device):
             env._check(env.lib.rd_policy_dreamer_set_agent_weights(env._handle, g, C.byref(s), C.byref(e) if e is not None else None,
                                                                    int(on_device), env._stream()))
+
+
+# ----------------------------------------------------------------------------------------------------------------------
+# Model-free baselines: SB3's SAC and PPO / A2C actors on the tensor cores, and uniform random actions
+# ----------------------------------------------------------------------------------------------------------------------
+import io
+import json
+import re
+import zipfile
+
+from .compat import baselines_config   # noqa: F401  (the env config these actors read; exported here too)
+
+_SB3_ACTIVATIONS = {"relu": _abi.RD_ACT_RELU, "tanh": _abi.RD_ACT_TANH}
+_SB3_DEFAULT_ACTIVATION = {"sac": "relu", "ppo": "tanh"}   # SACPolicy / ActorCriticPolicy defaults [UPSTREAM-RECALL]
+SAC_LOG_STD_MIN, SAC_LOG_STD_MAX = -20.0, 2.0               # SB3 sac/policies.py LOG_STD_MIN / MAX [UPSTREAM-RECALL]
+
+
+def _sequential_linears(sd, prefix: str):
+    """the keys of the Linear layers of an nn.Sequential `prefix` (Linear at even indices, activations between)"""
+    idx = sorted({int(m.group(1)) for k in sd for m in [re.fullmatch(re.escape(prefix) + r"\.(\d+)\.weight", k)] if m})
+    if idx != list(range(0, 2 * len(idx), 2)):
+        raise ValueError(f"{prefix}: Linear layers at indices {idx}, expected 0, 2, 4, ...")
+    for i in idx:
+        if f"{prefix}.{i}.bias" not in sd:
+            raise ValueError(f"{prefix}.{i}.bias is missing")
+    return [(f"{prefix}.{i}.weight", f"{prefix}.{i}.bias") for i in idx]
+
+
+def _sb3_layout(sd, n_beams: Optional[int] = None):
+    """(algo, {canonical name: state-dict key}, widths, in_features) of an SB3 policy state dict; ValueError for anything
+    but a SAC actor or an ActorCriticPolicy (PPO / A2C) with a parameter-free feature extractor and a Gaussian head.
+    Canonical names: w0, b0, ... (trunk), mean_w, mean_b, then log_std_w, log_std_b (SAC) or log_std (PPO)."""
+    keys = set(sd)
+    if any(k.startswith(("actor_target.", "critic_target.")) for k in keys) and not any(k.startswith("actor.latent_pi.") for k in keys):
+        raise ValueError("TD3 / DDPG policies are not supported (deterministic actor without a Gaussian head)")
+    if any(k.startswith(("features_extractor.", "actor.features_extractor.", "pi_features_extractor.",
+                         "vf_features_extractor.")) for k in keys):
+        raise ValueError("a feature extractor with parameters is not supported (the actor reads the flattened scan)")
+    names = {}
+    if any(k.startswith("actor.") for k in keys):
+        algo = "sac"
+        if "actor.log_std" in keys or any(k.startswith("actor.mu.0.") for k in keys):
+            raise ValueError("gSDE (use_sde=True) is not supported")
+        trunk = _sequential_linears(sd, "actor.latent_pi")
+        heads = {"mean_w": "actor.mu.weight", "mean_b": "actor.mu.bias", "log_std_w": "actor.log_std.weight",
+                 "log_std_b": "actor.log_std.bias"}
+    elif any(k.startswith(("mlp_extractor.", "action_net.")) for k in keys):
+        algo = "ppo"
+        trunk = _sequential_linears(sd, "mlp_extractor.shared_net") + _sequential_linears(sd, "mlp_extractor.policy_net")
+        heads = {"mean_w": "action_net.weight", "mean_b": "action_net.bias", "log_std": "log_std"}
+    else:
+        raise ValueError("not an SB3 SAC or ActorCriticPolicy (PPO / A2C) state dict: no actor.* / mlp_extractor.* keys")
+    missing = [v for v in heads.values() if v not in keys]
+    if missing:
+        raise ValueError(f"the actor head is incomplete: {', '.join(missing)} missing")
+    if not trunk:
+        raise ValueError("the actor has no hidden layer (net_arch=[]): at least one is needed")
+    if len(trunk) > _abi.RD_MLP_MAX_LAYERS:
+        raise ValueError(f"{len(trunk)} hidden layers: at most {_abi.RD_MLP_MAX_LAYERS} are supported")
+    shape = lambda k: tuple(sd[k].shape)   # noqa: E731
+    widths, prev = [], None
+    for i, (kw, kb) in enumerate(trunk):
+        if len(shape(kw)) != 2 or shape(kb) != shape(kw)[:1]:
+            raise ValueError(f"{kw} / {kb}: shapes {shape(kw)} / {shape(kb)} are not a Linear layer's")
+        out, inp = shape(kw)
+        if prev is not None and inp != prev:
+            raise ValueError(f"{kw} reads {inp} features, the layer before writes {prev}")
+        if out > _abi.RD_MLP_MAX_WIDTH:
+            raise ValueError(f"{kw}: width {out} > {_abi.RD_MLP_MAX_WIDTH}")
+        names[f"w{i}"], names[f"b{i}"] = kw, kb
+        widths.append(out)
+        prev = out
+    in_features = shape(trunk[0][0])[1]
+    if n_beams is not None and in_features != n_beams:
+        raise ValueError(f"the actor reads {in_features} features, the env casts {n_beams} beams")
+    if shape(heads["mean_w"]) != (2, prev) or shape(heads["mean_b"]) != (2,):
+        raise ValueError(f"{heads['mean_w']}: shape {shape(heads['mean_w'])}, expected (2, {prev}) for 2 actions")
+    if algo == "sac" and (shape(heads["log_std_w"]) != (2, prev) or shape(heads["log_std_b"]) != (2,)):
+        raise ValueError(f"actor.log_std.weight: shape {shape(heads['log_std_w'])}, expected (2, {prev})")
+    if algo == "ppo" and shape("log_std") != (2,):
+        raise ValueError(f"log_std has shape {shape('log_std')}: a state-dependent (gSDE) log_std is not supported, "
+                         "expected (2,)")
+    names.update(heads)
+    return algo, names, widths, in_features
+
+
+def _zip_activation(data_text: Optional[str]):
+    """the activation named in an SB3 zip's ``data`` JSON: 'relu' / 'tanh', None = the algorithm's default; ValueError
+    when it names another one or cannot be read without unpickling"""
+    if data_text is None:
+        return None
+    try:
+        pk = json.loads(data_text).get("policy_kwargs", {})
+    except (ValueError, AttributeError):
+        raise ValueError("the zip's data is not readable JSON: pass activation='relu' or 'tanh'") from None
+    if not isinstance(pk, dict):
+        raise ValueError("policy_kwargs cannot be read without unpickling: pass activation='relu' or 'tanh'")
+    readable = {k: v for k, v in pk.items() if k not in (":type:", ":serialized:")}
+    if ":serialized:" in pk and not readable:
+        raise ValueError("policy_kwargs cannot be read without unpickling: pass activation='relu' or 'tanh'")
+    fn = readable.get("activation_fn")
+    if fn is None:
+        return None
+    m = re.search(r"(\w+)'?>?\s*$", str(fn))
+    name = m.group(1).lower() if m else str(fn).lower()
+    if name not in _SB3_ACTIVATIONS:
+        raise ValueError(f"activation_fn {fn}: only ReLU and Tanh are supported")
+    return name
+
+
+def _read_sb3_source(path_or_state_dict):
+    """(state dict, data JSON text or None) of an SB3 .zip, a bare policy .pth or a state dict"""
+    if isinstance(path_or_state_dict, dict):
+        return path_or_state_dict, None
+    p = pathlib.Path(path_or_state_dict)
+    if zipfile.is_zipfile(p):   # (torch.save writes a zip too: an SB3 model is the one holding policy.pth)
+        with zipfile.ZipFile(p) as z:
+            if "policy.pth" in z.namelist():
+                sd = torch.load(io.BytesIO(z.read("policy.pth")), map_location="cpu", weights_only=True)
+                data = z.read("data").decode("utf-8", "replace") if "data" in z.namelist() else None
+                return sd, data
+    return torch.load(p, map_location="cpu", weights_only=True), None
+
+
+def load_sb3_checkpoint(path_or_state_dict, activation: Optional[str] = None, n_beams: Optional[int] = None):
+    """An SB3 policy's actor: ``(algo, weights, meta)``.
+
+    ``path_or_state_dict``: an SB3 model ``.zip`` (its ``policy.pth`` is read with ``torch.load(weights_only=True)``;
+    nothing else is unpickled), a bare ``policy.pth``, or a state dict of tensors / arrays.  ``algo`` is 'sac' (SACPolicy:
+    ``actor.latent_pi`` trunk, ``actor.mu`` / ``actor.log_std`` Linear heads) or 'ppo' (ActorCriticPolicy of PPO and A2C:
+    ``mlp_extractor.shared_net`` then ``mlp_extractor.policy_net`` trunk, ``action_net`` head, ``log_std`` vector); the
+    critic keys are ignored.  ``weights``: float32 arrays named w0, b0, ... , mean_w, mean_b and log_std_w, log_std_b
+    (SAC) or log_std (PPO), PyTorch layout.  ``meta``: activation ('relu' | 'tanh': ``activation``, else the zip's
+    ``policy_kwargs``, else the algorithm's default), widths, in_features.  n_beams: the env's beam count the first layer
+    must read.  [UPSTREAM-RECALL: SB3 1.x / 2.x key layouts]"""
+    sd, data = _read_sb3_source(path_or_state_dict)
+    algo, names, widths, in_features = _sb3_layout(sd, n_beams)
+    if activation is None:
+        activation = _zip_activation(data) or _SB3_DEFAULT_ACTIVATION[algo]
+    if activation not in _SB3_ACTIVATIONS:
+        raise ValueError(f"activation {activation!r}: expected 'relu' or 'tanh'")
+    host = lambda v: v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v)   # noqa: E731
+    weights = {n: np.ascontiguousarray(host(sd[k]), np.float32) for n, k in names.items()}
+    return algo, weights, {"activation": activation, "widths": tuple(widths), "in_features": in_features}
+
+
+def _check_baselines_env(env: BatchedRaceEnv) -> None:
+    c = env.cfg
+    if (not c.obs_flags & _abi.OBS_NORM_BASELINES or c.obs_flags & (_abi.OBS_LIDAR_F16 | _abi.OBS_OCCUPANCY)
+            or not c.clip_actions or c.rescale_actions):
+        raise ValueError("the actor reads the baselines chain's observation: the env needs normalize_obs='baselines', "
+                         "obs_type='lidar', float32 lidar, clip_actions=True and rescale_actions=False "
+                         "(baselines_config builds such a config)")
+
+
+class Sb3Policy:
+    """An SB3 SAC or PPO / A2C policy's actor (``load_sb3_checkpoint``) for every env of a ``BatchedRaceEnv`` built with
+    the baselines chain (``baselines_config``): what ``model.predict(obs, deterministic)`` computes, as one
+    ``k_embed_lidar`` split, one tcgen05 ``k_dense`` launch per hidden layer and one for the head (tf32x3,
+    float32-grade), and ``k_mlp_head`` (rd_policy_mlp, include/rd_env.h).
+
+    SAC: deterministic a = tanh(mu); else a = tanh(mu + exp(clamp(log_std, -20, 2)) e).  SB3 hands the env
+    ``low + 0.5 (a + 1) (high - low)``, which on the [-1, 1] box is ``a`` up to one float32 rounding; the actor writes
+    ``a`` itself, the value SB3's replay buffer stores (the difference is below every test bar).
+    PPO / A2C: deterministic a = mean; else a = mean + exp(log_std) e, unclipped -- the value SB3's rollout buffer keeps;
+    the env's ``clip_actions`` is the clip SB3 applies before stepping.
+    noise: 'philox' (Philox4x32-10 normals per env and step), 'zero' or 'explicit' (``act(eps=[N, 2])``), as in
+    ``DreamerPolicy``.  Stateless per env: nothing to clear on reset."""
+
+    NOISE = DreamerPolicy.NOISE
+
+    def __init__(self, env: BatchedRaceEnv, checkpoint, activation: Optional[str] = None, noise: str = "philox"):
+        self.env = env
+        _check_baselines_env(env)
+        if noise not in self.NOISE:
+            raise ValueError(f"noise {noise!r}: expected one of {sorted(self.NOISE)}")
+        self.noise = noise
+        self.algo, w, self.meta = load_sb3_checkpoint(checkpoint, activation=activation, n_beams=env.n_beams)
+        self.weights = w
+        s = self._struct(w, lambda a: a.ctypes.data_as(C.c_void_p))
+        with torch.cuda.device(env.device):
+            env._check(env.lib.rd_policy_mlp_init(env._handle, C.byref(s)))
+        self.actions = torch.zeros((env.n, 2), dtype=torch.float32, device=env.device)
+        self.debug = torch.zeros((env.n, _abi.RD_MLP_DEBUG_FLOATS), dtype=torch.float32, device=env.device)
+        self._staged = None
+
+    def _struct(self, w, ptr) -> "_abi.RdMlpActor":
+        s = _abi.RdMlpActor()
+        widths = self.meta["widths"]
+        s.n_layers, s.in_features = len(widths), self.meta["in_features"]
+        for i, u in enumerate(widths):
+            s.width[i], s.w[i], s.b[i] = u, ptr(w[f"w{i}"]), ptr(w[f"b{i}"])
+        s.activation = _SB3_ACTIVATIONS[self.meta["activation"]]
+        s.mean_w, s.mean_b = ptr(w["mean_w"]), ptr(w["mean_b"])
+        if self.algo == "sac":
+            s.head, s.log_std_min, s.log_std_max = _abi.RD_HEAD_SQUASHED, SAC_LOG_STD_MIN, SAC_LOG_STD_MAX
+            s.log_std_w, s.log_std_b = ptr(w["log_std_w"]), ptr(w["log_std_b"])
+        else:
+            s.head = _abi.RD_HEAD_DIAG
+            s.log_std = ptr(w["log_std"])
+        return s
+
+    def load_weights(self, state_dict) -> None:
+        """New weights from a learner, e.g. ``model.policy.state_dict()`` (tensors, CUDA tensors on the env's device are
+        read there) or an SB3 zip.  Algorithm, layer widths and activation must be the init's (a plain state dict is
+        taken to have the init's activation); everything is checked before any device work, so a rejected refresh
+        changes nothing.  Packed on the current stream: steps enqueued before use the old weights, steps after the new
+        ones, with no host synchronisation for CUDA sources.  The Philox step counter is kept.  The sources stay
+        referenced until the next call."""
+        env = self.env
+        sd, data = _read_sb3_source(state_dict)
+        algo, names, widths, in_features = _sb3_layout(sd, env.n_beams)
+        act = _zip_activation(data) or self.meta["activation"]
+        if (algo, tuple(widths), act) != (self.algo, self.meta["widths"], self.meta["activation"]):
+            raise ValueError(f"the weights ({algo}, widths {tuple(widths)}, {act}) do not match the policy's "
+                             f"({self.algo}, widths {self.meta['widths']}, {self.meta['activation']})")
+        on_device = False
+        for n, k in names.items():
+            v = sd[k]
+            if isinstance(v, torch.Tensor):
+                if v.device.type != "cpu" and v.device != env.device:
+                    raise ValueError(f"{k} is on {v.device}, the policy on {env.device}")
+                if not v.dtype.is_floating_point:
+                    raise ValueError(f"{k} has dtype {v.dtype}, expected a float dtype")
+                on_device |= v.is_cuda
+            elif not np.issubdtype(np.asarray(v).dtype, np.floating):
+                raise ValueError(f"{k} has dtype {np.asarray(v).dtype}, expected a float dtype")
+        if on_device:
+            def dev(v):
+                t = v.detach() if isinstance(v, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(v, np.float32))
+                return t.to(device=env.device, dtype=torch.float32).contiguous()
+            staged = {n: dev(sd[k]) for n, k in names.items()}
+            ptr = lambda t: C.c_void_p(t.data_ptr())   # noqa: E731
+        else:
+            host = lambda v: v.detach().numpy() if isinstance(v, torch.Tensor) else v   # noqa: E731
+            staged = {n: np.ascontiguousarray(host(sd[k]), np.float32) for n, k in names.items()}
+            ptr = lambda a: a.ctypes.data_as(C.c_void_p)   # noqa: E731
+        self._staged = staged
+        s = self._struct(staged, ptr)
+        with torch.cuda.device(env.device):
+            env._check(env.lib.rd_policy_mlp_set_weights(env._handle, C.byref(s), int(on_device), env._stream()))
+
+    def act(self, obs: Optional[torch.Tensor] = None, deterministic: bool = True, eps: Optional[torch.Tensor] = None,
+            debug: bool = False) -> torch.Tensor:
+        """obs f32 [N, n_beams] (default: the env's current scan) -> actions f32 [N, 2] (a persistent buffer), SB3's
+        ``predict``.  noise='explicit' takes ``eps`` [N, 2] for a stochastic step."""
+        env = self.env
+        li = env.buf["lidar"] if obs is None else obs
+        if li.shape != (env.n, env.n_beams) or li.dtype != torch.float32 or li.device != env.device or not li.is_contiguous():
+            raise ValueError(f"obs must be a contiguous float32 CUDA tensor of shape ({env.n}, {env.n_beams})")
+        mode = self.NOISE[self.noise]
+        e = None
+        if mode == _abi.RD_NOISE_EXPLICIT and not deterministic:
+            if eps is None:
+                raise ValueError("noise='explicit' needs eps [N, 2] for a stochastic step")
+            e = eps.to(device=env.device, dtype=torch.float32).contiguous()
+            if e.shape != (env.n, 2):
+                raise ValueError("eps must be [N, 2]")
+        with torch.cuda.device(env.device):
+            env._check(env.lib.rd_policy_mlp(env._handle, li.data_ptr(), self.actions.data_ptr(), int(deterministic), mode,
+                                              e.data_ptr() if e is not None else None,
+                                              self.debug.data_ptr() if debug else None, env._stream()))
+        return self.actions
+
+    def diagnostics(self) -> Dict[str, torch.Tensor]:
+        """Valid after ``act(debug=True)``: the Gaussian's mean and std per env, before the squash."""
+        return {"mean": self.debug[:, 0:2], "std": self.debug[:, 2:4]}
+
+    def rollout(self, n_steps: int, deterministic: bool = False, store=None):
+        """n_steps x (actor step -> env.step) enqueued on the current stream, no host round trip; ``store``: a
+        ``DeviceEpisodeStore`` of this env that records every step (the actor's actions, unclipped for PPO) and resets
+        the finished envs.  Returns the env's (obs, reward, done, info) views of the last step."""
+        env = self.env
+        mode = self.NOISE[self.noise]
+        with torch.cuda.device(env.device):
+            if store is not None:
+                _check_store(env, store)
+                policy = _abi.STORE_POLICY_MLP if deterministic else _abi.STORE_POLICY_MLP_TRAIN
+                env._check(env.lib.rd_rollout_store(env._handle, policy, int(n_steps), C.byref(env._out),
+                                                    self.actions.data_ptr(), mode, env._stream()))
+            else:
+                env._check(env.lib.rd_rollout_mlp(env._handle, int(n_steps), C.byref(env._out), self.actions.data_ptr(),
+                                                  int(deterministic), mode, env._stream()))
+        return env._obs(), env.buf["reward"], env.buf["done_bool"], env._info()
+
+
+class RandomPolicy:
+    """Uniform random actions in [-1, 1)^2 for every env of any ``BatchedRaceEnv`` (``rd_policy_random``): SB3's
+    ``action_space.sample()`` before ``learning_starts`` and Dreamer's random prefill [UPSTREAM-RECALL], drawn on the
+    device.  Law [NEW-SPEC; the reference draws from numpy's RNG]: Philox4x32-10 block (env id, step, 0,
+    RD_STREAM_RANDOM) keyed (seed_lo, seed_hi ^ tag), a_k = 2 (x_k >> 8) 2^-24 - 1; the step counter is the env
+    handle's and advances by one per call."""
+
+    def __init__(self, env: BatchedRaceEnv):
+        self.env = env
+        self.actions = torch.zeros((env.n, 2), dtype=torch.float32, device=env.device)
+
+    def act(self) -> torch.Tensor:
+        env = self.env
+        with torch.cuda.device(env.device):
+            env._check(env.lib.rd_policy_random(env._handle, self.actions.data_ptr(), env._stream()))
+        return self.actions
+
+    def rollout(self, n_steps: int, store=None):
+        """n_steps x (random actions -> env.step), as ``Sb3Policy.rollout``."""
+        env = self.env
+        with torch.cuda.device(env.device):
+            if store is not None:
+                _check_store(env, store)
+                env._check(env.lib.rd_rollout_store(env._handle, _abi.STORE_POLICY_RANDOM, int(n_steps), C.byref(env._out),
+                                                    self.actions.data_ptr(), 0, env._stream()))
+            else:
+                env._check(env.lib.rd_rollout_random(env._handle, int(n_steps), C.byref(env._out), self.actions.data_ptr(),
+                                                     env._stream()))
+        return env._obs(), env.buf["reward"], env.buf["done_bool"], env._info()

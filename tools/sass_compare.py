@@ -1,6 +1,7 @@
 """Compare the SASS of two builds of librd_env.so kernel by kernel: which kernels of the first build compile to different
 instructions (or are missing) in the second, and which kernels are new.  k_dense's trailing CONV template argument
-(0 = a dense layer) is added to the first build's names, so a build from before that argument compares too.
+(0 = a dense layer) is added to the first build's names, so a build from before that argument compares too; likewise
+k_pack_weights' KMAJOR argument (false = the Keras-layout packer it was before the argument existed).
 
     cuobjdump -sass old/librd_env.so > old.sass; cuobjdump -sass racing_dreamer_b200/librd_env.so > new.sass
     python tools/sass_compare.py old.sass new.sass
@@ -21,6 +22,7 @@ def functions(path):
 
 
 def with_conv0(name):
+    name = re.sub(r"^_Z14k_pack_weights8PackArgs$", "_Z14k_pack_weightsILb0EEv8PackArgs", name)
     return re.sub(r"^(_Z7k_denseI(?:Li\d+E|Lb\dE){7})(Ev8GemmMaps)", r"\1Li0E\2", name)
 
 
