@@ -30,13 +30,14 @@ def _linear(rng, out: int, inp: int, scale: float = 1.0):
 
 
 def sac_state_dict(seed: int, n_beams: int = 1080, widths: Sequence[int] = (256, 256), log_std_bias: float = -1.0,
-                   critic: bool = True) -> Dict[str, np.ndarray]:
+                   critic: bool = True, scale: float = 1.0) -> Dict[str, np.ndarray]:
     """A SACPolicy state dict (key names and shapes of SB3's), with nn.Linear-style random weights and the critic's
-    keys, which the actor ignores.  log_std_bias shifts the log_std head (SB3's initial std is ~1)."""
+    keys, which the actor ignores.  log_std_bias shifts the log_std head (SB3's initial std is ~1); scale multiplies
+    the trunk's weights and biases (saturated tanh, dead relu units, activations beyond the init's range)."""
     rng = np.random.default_rng(seed)
     sd, prev = {}, n_beams
     for i, u in enumerate(widths):
-        sd[f"actor.latent_pi.{2 * i}.weight"], sd[f"actor.latent_pi.{2 * i}.bias"] = _linear(rng, u, prev)
+        sd[f"actor.latent_pi.{2 * i}.weight"], sd[f"actor.latent_pi.{2 * i}.bias"] = _linear(rng, u, prev, scale)
         prev = u
     sd["actor.mu.weight"], sd["actor.mu.bias"] = _linear(rng, 2, prev)
     sd["actor.log_std.weight"], sd["actor.log_std.bias"] = _linear(rng, 2, prev)
@@ -50,17 +51,20 @@ def sac_state_dict(seed: int, n_beams: int = 1080, widths: Sequence[int] = (256,
 
 
 def ppo_state_dict(seed: int, n_beams: int = 1080, widths: Sequence[int] = (64, 64), shared: Sequence[int] = (),
-                   log_std: Sequence[float] = (-0.5, 0.25), critic: bool = True) -> Dict[str, np.ndarray]:
+                   log_std: Sequence[float] = (-0.5, 0.25), critic: bool = True, scale: float = 1.0) -> Dict[str, np.ndarray]:
     """An ActorCriticPolicy state dict: ``shared`` widths under mlp_extractor.shared_net (older SB3), ``widths`` under
-    mlp_extractor.policy_net, action_net, log_std, and the value side, which the actor ignores."""
+    mlp_extractor.policy_net, action_net, log_std, and the value side, which the actor ignores.  scale multiplies the
+    actor trunk's weights and biases, as in sac_state_dict."""
     rng = np.random.default_rng(seed)
     sd, prev = {}, n_beams
     for i, u in enumerate(shared):
-        sd[f"mlp_extractor.shared_net.{2 * i}.weight"], sd[f"mlp_extractor.shared_net.{2 * i}.bias"] = _linear(rng, u, prev)
+        sd[f"mlp_extractor.shared_net.{2 * i}.weight"], sd[f"mlp_extractor.shared_net.{2 * i}.bias"] = _linear(
+            rng, u, prev, scale)
         prev = u
     trunk_in = prev
     for i, u in enumerate(widths):
-        sd[f"mlp_extractor.policy_net.{2 * i}.weight"], sd[f"mlp_extractor.policy_net.{2 * i}.bias"] = _linear(rng, u, prev)
+        sd[f"mlp_extractor.policy_net.{2 * i}.weight"], sd[f"mlp_extractor.policy_net.{2 * i}.bias"] = _linear(
+            rng, u, prev, scale)
         prev = u
     sd["action_net.weight"], sd["action_net.bias"] = _linear(rng, 2, prev)
     sd["log_std"] = np.asarray(log_std, np.float32)
@@ -75,20 +79,24 @@ def n_layers(w) -> int:
 
 
 def actor(w, algo: str, activation: str, obs: np.ndarray, eps: Optional[np.ndarray] = None,
-          deterministic: bool = True):
-    """obs [N, n_beams] -> (mean [N, 2], std [N, 2], action [N, 2]) in float64; eps [N, 2] standard normals (stochastic)."""
-    act = {"relu": lambda x: np.maximum(x, 0.0), "tanh": np.tanh}[activation]
-    f = lambda k: np.asarray(w[k], np.float64)   # noqa: E731
-    x = np.asarray(obs, np.float64)
+          deterministic: bool = True, dtype=np.float64, log_std_bounds=(LOG_STD_MIN, LOG_STD_MAX), matmul=None):
+    """obs [N, n_beams] -> (mean [N, 2], std [N, 2], action [N, 2]) in `dtype`; eps [N, 2] standard normals
+    (stochastic).  dtype=np.float32 is a float32 evaluation (float32 weights, products, sums and activations), the
+    yardstick of a float32-grade kernel.  log_std_bounds: the SAC head's clamp.  matmul(x, w) -> x w^T, the products
+    of every Linear layer (default: in `dtype`; the tests pass emulations of tensor-core arithmetic)."""
+    act = {"relu": lambda x: np.maximum(x, dtype(0)), "tanh": np.tanh}[activation]
+    f = lambda k: np.asarray(w[k], dtype)   # noqa: E731
+    mm = matmul or (lambda a, b: a @ b.T)
+    x = np.asarray(obs, dtype)
     for i in range(n_layers(w)):
-        x = act(x @ f(f"w{i}").T + f(f"b{i}"))
-    mean = x @ f("mean_w").T + f("mean_b")
+        x = act(mm(x, f(f"w{i}")) + f(f"b{i}"))
+    mean = mm(x, f("mean_w")) + f("mean_b")
     if algo == "sac":
-        log_std = np.clip(x @ f("log_std_w").T + f("log_std_b"), LOG_STD_MIN, LOG_STD_MAX)
+        log_std = np.clip(mm(x, f("log_std_w")) + f("log_std_b"), dtype(log_std_bounds[0]), dtype(log_std_bounds[1]))
     else:
         log_std = np.broadcast_to(f("log_std"), mean.shape)
     std = np.exp(log_std)
-    u = mean if deterministic or eps is None else mean + std * np.asarray(eps, np.float64)
+    u = mean if deterministic or eps is None else mean + std * np.asarray(eps, dtype)
     return mean, std, (np.tanh(u) if algo == "sac" else u)
 
 

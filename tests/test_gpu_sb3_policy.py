@@ -2,13 +2,15 @@
 k_mlp_head) against the float64 restatement oracle/sb3_policy.py, their rollouts and weight refresh, and the uniform
 random actions (RandomPolicy: k_random_actions) against their NumPy law, bit for bit.
 
-Bars: test_gpu_dreamer's tf32x3 bars for the Gaussian's mean and std and for the actions; the Philox path is compared
-with the explicit path fed the float64 Box-Muller restatement of the same blocks (a few float32 ulp per normal)."""
+Bars: the evaluation against float64 is held to test_cpu_sb3_shapes' bar (float32-grade, 8x better than one TF32 pass),
+the explicit-noise actions to test_gpu_dreamer's tf32x3 bars; the Philox path is compared with the explicit path fed the
+float64 Box-Muller restatement of the same blocks (a few float32 ulp per normal)."""
 import numpy as np
 import pytest
 
 from oracle import sb3_policy as sp
 from test_cpu_sb3_policy import make_sd, mlp_normals, random_actions
+from test_cpu_sb3_shapes import check, reference
 from test_gpu_dreamer import BARS, close
 
 pytestmark = pytest.mark.gpu
@@ -59,38 +61,39 @@ def test_evaluation_matches_restatement(torch_cuda, arch, n):
     a = pol.act(scans, deterministic=True, debug=True).cpu().numpy()
     d = {k: v.cpu().numpy() for k, v in pol.diagnostics().items()}
     _, w, meta = load_sb3_checkpoint(sd)
-    mean, std, act = sp.actor(w, algo, meta["activation"], scans.cpu().numpy())
-    close("mean", d["mean"], mean)
-    close("std", d["std"], std, rtol=HEAD * RTOL, atol=HEAD * ATOL)
-    close("action", a, act)
+    ref, bars = reference(w, dict(algo=algo, activation=meta["activation"]), scans.cpu().numpy())
+    check(arch, (d["mean"], d["std"], a), ref, bars)
     env.close()
 
 
 @pytest.mark.parametrize("arch", ["sac256", "ppo64"])
 def test_training_mode(torch_cuda, arch):
+    """Philox normals of block (env_id_offset + env, step, 0, RD_STREAM_MLP), at offsets 0 and 12345"""
     torch = torch_cuda
     from racing_dreamer_b200.policy import Sb3Policy, load_sb3_checkpoint
     algo, kw = ARCHS[arch]
     sd = make_sd(algo, 12, **kw)
     n = 4096
-    env_p, env_e = make_env(n, seed=21), make_env(n, seed=21)
-    scans = scans_of(env_p, torch)
-    pol_p, pol_e = Sb3Policy(env_p, sd, noise="philox"), Sb3Policy(env_e, sd, noise="explicit")
     _, w, meta = load_sb3_checkpoint(sd)
-    seed = int(env_p.cfg.seed)
-    for step in range(3):
-        e = mlp_normals(seed, n, step)
-        a_e = pol_e.act(scans, deterministic=False, eps=torch.from_numpy(e.astype(np.float32))).cpu().numpy()
-        mean, std, act = sp.actor(w, algo, meta["activation"], scans.cpu().numpy(), e.astype(np.float32),
-                                  deterministic=False)
-        close("explicit action", a_e, act, rtol=HEAD * RTOL, atol=HEAD * ATOL)
-        a_p = pol_p.act(scans, deterministic=False).cpu().numpy()
-        assert np.abs(a_p - a_e).max() < 1e-4, np.abs(a_p - a_e).max()
+    for gid0 in (0, 12345):
+        env_p, env_e = make_env(n, seed=21, env_id_offset=gid0), make_env(n, seed=21, env_id_offset=gid0)
+        scans = scans_of(env_p, torch)
+        pol_p, pol_e = Sb3Policy(env_p, sd, noise="philox"), Sb3Policy(env_e, sd, noise="explicit")
+        seed = int(env_p.cfg.seed)
+        for step in range(3):
+            e = mlp_normals(seed, n, step, gid0)
+            a_e = pol_e.act(scans, deterministic=False, eps=torch.from_numpy(e.astype(np.float32))).cpu().numpy()
+            mean, std, act = sp.actor(w, algo, meta["activation"], scans.cpu().numpy(), e.astype(np.float32),
+                                      deterministic=False)
+            close("explicit action", a_e, act, rtol=HEAD * RTOL, atol=HEAD * ATOL)
+            a_p = pol_p.act(scans, deterministic=False).cpu().numpy()
+            assert np.abs(a_p - a_e).max() < 1e-4, np.abs(a_p - a_e).max()
+        env_p.close()
+        env_e.close()
     if algo == "ppo":   # unclipped in the actions buffer; the env's clip = stepping with clip(a, -1, 1)
         big = make_sd("ppo", 12, widths=(64, 64), log_std=(1.5, 1.5))
         env_c = make_env(n, seed=21)
         scans_of(env_c, torch)
-        env_p.close()
         env_p = make_env(n, seed=21)
         scans_of(env_p, torch)
         pol = Sb3Policy(env_p, big)
@@ -100,8 +103,7 @@ def test_training_mode(torch_cuda, arch):
         o2 = env_c.step(a.clamp(-1, 1))[0]["lidar"]
         assert torch.equal(o1, o2)
         env_c.close()
-    env_p.close()
-    env_e.close()
+        env_p.close()
 
 
 @pytest.mark.parametrize("arch", ["sac256", "ppo64"])
@@ -127,7 +129,7 @@ def test_rollout_equals_act_step_loop(torch_cuda, arch):
         assert torch.equal(a, b)
 
 
-@pytest.mark.parametrize("policy", ["ppo", "random"])
+@pytest.mark.parametrize("policy", ["ppo", "ppo_deterministic", "random"])
 def test_rollout_store_equals_store_step(torch_cuda, policy):
     torch = torch_cuda
     from racing_dreamer_b200.episodes import DeviceEpisodeStore
@@ -137,16 +139,17 @@ def test_rollout_store_equals_store_step(torch_cuda, policy):
     for mode in ("rollout", "loop"):
         env = make_env(16, seed=11, auto_reset=False, time_limit_ticks=120)
         store = DeviceEpisodeStore(env, capacity_rows=400)
-        pol = Sb3Policy(env, sd) if policy == "ppo" else RandomPolicy(env)
+        det = policy == "ppo_deterministic"   # RD_STORE_POLICY_MLP (else _MLP_TRAIN)
+        pol = RandomPolicy(env) if policy == "random" else Sb3Policy(env, sd)
         store.reset()
         if mode == "rollout":
             if policy == "random":
                 pol.rollout(70, store=store)
             else:
-                pol.rollout(70, deterministic=False, store=store)
+                pol.rollout(70, deterministic=det, store=store)
         else:
             for _ in range(70):
-                store.step(pol.act() if policy == "random" else pol.act(deterministic=False))
+                store.step(pol.act() if policy == "random" else pol.act(deterministic=det))
         torch.cuda.synchronize()
         runs.append(store.episodes())
         env.close()
@@ -158,7 +161,7 @@ def test_rollout_store_equals_store_step(torch_cuda, policy):
     acts = np.concatenate([x["action"][1:] for x in e1])
     if policy == "ppo":
         assert np.abs(acts).max() > 1.0   # the recorded actions are the actor's, unclipped
-    else:
+    elif policy == "random":
         assert acts.min() >= -1.0 and acts.max() < 1.0
 
 
@@ -265,9 +268,10 @@ def test_multi_car_rows(torch_cuda):
     env = make_env(64, agents_per_world=4, reset_mode="random_ball")
     scans = scans_of(env, torch)
     pol = Sb3Policy(env, sd)
-    a = pol.act(deterministic=True).cpu().numpy()
+    a = pol.act(deterministic=True, debug=True).cpu().numpy()
+    d = {k: v.cpu().numpy() for k, v in pol.diagnostics().items()}
     _, w, meta = load_sb3_checkpoint(sd)
-    _, _, act = sp.actor(w, "ppo", meta["activation"], scans.cpu().numpy())
-    close("action", a, act)
+    ref, bars = reference(w, dict(algo="ppo", activation=meta["activation"]), scans.cpu().numpy())
+    check("multi-car rows", (d["mean"], d["std"], a), ref, bars)
     assert len({bytes(r) for r in a}) > 32
     env.close()
